@@ -2,6 +2,7 @@
 """bench.py — whole-encode throughput of the B200 JPEG encode path (BASELINE.json: "encode Mpx/s").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload image16k|frame4k]
+                    [--dump-outputs DIR]
 
 A "step" is one complete encode (K1 colour/DCT/quant -> K2 symbol statistics -> host Huffman table build ->
 K3 Huffman pack -> K4 byte stuffing) of one synthetic image per GPU.  Default workload: the 16384x16384 (268 Mpx)
@@ -22,6 +23,10 @@ cpu_baseline = the reference encoder itself (oracle/_ref, built from /root/refer
 --impl reference = the same binary on the headline workload itself: the 16384x16384 file, OMP_NUM_THREADS=1 (north_star:
           "single-threaded"; its three std::async channel tasks still run), ONE timed encode whatever --steps says (an
           encode takes ~45 s + ~9 s of PPM loading); the best multi-threaded figure is reported beside it.
+--dump-outputs DIR = after the timed steps, rank 0 writes what its last timed step produced as float32/float64 .npy files
+          in DIR, so that two builds can be compared output for output on the same seeded input: the JPEG file (jpeg.npy,
+          one value per byte), and for batch1080p the files of its frames back to back (jpeg.npy) and their sizes
+          (sizes.npy).  Past DUMP_BYTES the bytes are a fixed, seeded sample (jpeg_sample.npy, jpeg_sample_offsets.npy).
 """
 from __future__ import annotations
 
@@ -48,6 +53,7 @@ CPU_SAMPLE = (2048, 2048)          # bounded sample of the same generator for th
 if os.environ.get("JPGENC_BENCH_CPU_SAMPLE"):                      # tests use a smaller one
     CPU_SAMPLE = tuple(int(x) for x in os.environ["JPGENC_BENCH_CPU_SAMPLE"].split("x"))
 METRIC, UNIT = "encode_throughput", "Mpx/s"
+DUMP_BYTES = 60 << 20              # --dump-outputs writes at most this much
 
 
 def measured_peak():
@@ -295,6 +301,7 @@ def run_ours(args):
         jpeg_bytes = enc.encode_bound(None)
     ms_total = enc.timer_end()
     s1 = enc.stats()
+    dump = output_arrays(last_file(enc, jpeg_bytes)) if args.dump_outputs and rank == 0 else None
     n_timed = max(1, s1.timed_encodes - s0.timed_encodes)
     k1_ms = [(s1.sum_ms_k1 - s0.sum_ms_k1) / n_timed]
     launches = enc.launch_count() - launches0
@@ -451,11 +458,39 @@ def run_ours(args):
                                              what="bounded sample of the workload (the full 16384x16384 image is what --impl reference times)")
     line["extra"] = extra
     enc.close()
+    if dump is not None:
+        write_outputs(args.dump_outputs, dump)
     if dist is not None:
         dist.barrier()
         dist.destroy_process_group()
     if rank == 0:
         emit(line)
+
+
+def last_file(enc, jpeg_bytes: int):
+    """the JPEG file of the context's last encode_bound (jpgenc_assemble_last: headers + scan + EOI, no new encode)"""
+    import ctypes
+    import numpy as np
+    out = np.empty(jpeg_bytes, np.uint8)
+    n = ctypes.c_uint64()
+    enc._check(enc.lib.jpgenc_assemble_last(enc.h, out.ctypes.data, out.size, ctypes.byref(n)))
+    return out[: n.value]
+
+
+def output_arrays(jpeg, budget=DUMP_BYTES):
+    """the bytes as float32 values, one per byte; past `budget` a fixed, seeded sample of the bytes and their offsets"""
+    import numpy as np
+    if jpeg.size * 4 <= budget:
+        return {"jpeg": jpeg.astype(np.float32)}
+    idx = np.sort(np.random.default_rng(0).choice(jpeg.size, budget // 12, replace=False))
+    return {"jpeg_sample": jpeg[idx].astype(np.float32), "jpeg_sample_offsets": idx.astype(np.float64)}
+
+
+def write_outputs(dirname, arrays):
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 def batch_golden():
@@ -466,13 +501,14 @@ def batch_golden():
         return None
 
 
-def batch_section(enc, rank, world, barrier, max_over_ranks, reps=3, frames_total=BATCH_FRAMES):
+def batch_section(enc, rank, world, barrier, max_over_ranks, reps=3, frames_total=BATCH_FRAMES, keep_files=False):
     """BASELINE configs[4]: `frames_total` synthetic 1920x1080 frames (frame k = seed k), frame k encoded by the rank that
     owns it (contiguous shards, no data-path collective) -> strong scaling over the ranks.  Every figure is the host wall
     clock around ONE synchronous library call on this rank's shard, between barriers, max over ranks, mean of `reps`.
       resident        frames in HBM, files left in HBM (sizes and offsets reported)
       files_returned  frames in HBM, complete files back in ONE pinned host buffer (one device-to-host copy per pass)
-      e2e             frames in pinned host memory, files back in pinned host memory (H2D + D2H inside)"""
+      e2e             frames in pinned host memory, files back in pinned host memory (H2D + D2H inside)
+    keep_files: res["files"] = the files of the last timed call, back to back (the three passes return the same files)"""
     import hashlib
     import numpy as np
     from jpgenc_b200.capi import pinned_empty, pinned_free
@@ -525,6 +561,7 @@ def batch_section(enc, rank, world, barrier, max_over_ranks, reps=3, frames_tota
         ok = ok and out[offs[k]] == 0xFF and out[offs[k] + 1] == 0xD8 and out[offs[k] + sizes[k] - 1] == 0xD9
     parity["ok"] = bool(ok)
     assert ok, f"batch output differs from the golden/reference data: {parity}"
+    files = out[:total].copy() if keep_files else None
     pinned_free(host_ptr); pinned_free(out_ptr); enc.dev_free(d_all)
     mpx = frames_total * w * h / 1e6
     sec = {"resident": dt_res, "files_returned": dt_files, "e2e": dt_e2e}
@@ -538,6 +575,8 @@ def batch_section(enc, rank, world, barrier, max_over_ranks, reps=3, frames_tota
         res[k] = {"frames_per_s": round(frames_total / dt, 1), "mpx_per_s": round(mpx / dt, 1), "ms": round(dt * 1e3, 3)}
     res["e2e"]["h2d_bytes_per_gpu"] = nf * fbytes
     res["e2e"]["h2d_gbps_per_gpu"] = round(nf * fbytes / dt_e2e / 1e9, 2)
+    if keep_files:
+        res["files"], res["sizes"] = files, sizes
     return res
 
 
@@ -569,8 +608,13 @@ def run_batch(args):
     enc = Encoder(local)
     sampler = ClockSampler(local)
     sampler.start()
-    reps = max(3, args.steps // 20)
-    b = batch_section(enc, rank, world, barrier, max_over_ranks, reps=reps)
+    reps = args.steps
+    dump = bool(args.dump_outputs) and rank == 0
+    b = batch_section(enc, rank, world, barrier, max_over_ranks, reps=reps, keep_files=dump)
+    if dump:
+        import numpy as np
+        sizes = np.array(b.pop("sizes"), np.float64)
+        write_outputs(args.dump_outputs, {"sizes": sizes, **output_arrays(b.pop("files"), DUMP_BYTES - sizes.nbytes)})
     clocks = sampler.summary()
     w, h, desc = WORKLOADS["batch1080p"]
     line = {"metric": METRIC, "value": b["resident"]["mpx_per_s"], "unit": UNIT, "n_gpus": world, "steps": reps, "warmup": 1,
@@ -700,7 +744,12 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="image16k", choices=list(WORKLOADS))
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path computed in its last step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs: --impl ours only")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
     if args.impl == "reference":
         run_reference(args)

@@ -22,16 +22,14 @@ def oracle():
 
 @pytest.fixture(scope="session")
 def reference():
-    """The compiled reference (oracle/_ref); tests that need it are skipped where it was never built."""
+    """The compiled reference (oracle/_ref), or None where it was never built (no reference tree to build it from)."""
     from oracle.pyoracle import REF_SO, Reference, build
     if not REF_SO.exists():
         try:
             build()
         except Exception:
             pass
-    if not REF_SO.exists():
-        pytest.skip("oracle/_ref not built (no /root/reference here)")
-    return Reference()
+    return Reference() if REF_SO.exists() else None
 
 
 @pytest.fixture(scope="session")
