@@ -107,11 +107,6 @@ int ensure_coef(jpgenc_ctx* c) {
     return rc;
 }
 
-// JPGENC_TRACE=1: host wall-clock of the phases of every batched pass on stderr (development aid)
-bool trace_on() {
-    static const bool on = [] { const char* v = std::getenv("JPGENC_TRACE"); return v && *v && *v != '0'; }();
-    return on;
-}
 double now_us() {
     return std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now().time_since_epoch()).count();
 }
@@ -168,8 +163,8 @@ void ensure_host_pool(jpgenc_ctx* c) {
 // chroma AC while the caller builds luma AC, which is about the same work (a photograph: 3 + 3 + 3 us against 10; noise: both AC
 // tables are large and the same holds).  Measured against a thread per table (3840x2160 / 16384^2 / 2048^2 noise, all 16 cores
 // and pinned to 4): 0.0887 / 0.6787 / 0.1529 ms against 0.0913 / 0.6806 / 0.1540 -- fewer threads to wake and to wait for, and
-// a process that shares its host with seven other ranks keeps two of its four cores.  JPGENC_TABLE_THREADS (1..3) overrides.
-static int table_workers() { return static_cast<int>(std::min(3u, std::max(1u, env_u32("JPGENC_TABLE_THREADS", 1u)))); }
+// a process that shares its host with seven other ranks keeps two of its four cores.
+constexpr int kTableWorkers = 1;
 
 // pinned staging: [statistics F * kStatsBytes + 16][device tables F * 8 KB][PassMeta block (common.cuh)]
 size_t stage_tables_off(uint32_t F) { return ((F * kStatsBytes + 16 + 255) / 256) * 256; }
@@ -268,7 +263,6 @@ int jpgenc_create(int device, jpgenc_ctx** out) {
         return JPGENC_ERR_NO_DEVICE;
     }
     c->sm_count = prop.multiProcessorCount;
-    c->stage_timing = static_cast<int>(std::min(2u, env_u32("JPGENC_STAGE_TIMING", 0)));    // jpgenc_set_stage_timing
     if ((e = cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking)) != cudaSuccess) return bail("cudaStreamCreate", e);
     if ((e = cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking)) != cudaSuccess) return bail("cudaStreamCreate", e);
     for (cudaEvent_t& ev : c->ev_band)
@@ -317,7 +311,6 @@ void jpgenc_destroy(jpgenc_ctx* c) {
     for (cudaEvent_t ev : {c->ev_a, c->ev_b, c->ev_t0, c->ev_t1, c->ev_u0, c->ev_u1, c->ev_k0, c->ev_k1}) if (ev) cudaEventDestroy(ev);
     for (cudaEvent_t ev : c->ev_band) if (ev) cudaEventDestroy(ev);
     if (c->ev_done) cudaEventDestroy(c->ev_done);
-    if (c->ev_wide) cudaEventDestroy(c->ev_wide);
     if (c->ev_fwd) cudaEventDestroy(c->ev_fwd);
     if (c->ev_k4) cudaEventDestroy(c->ev_k4);
     if (c->ev_copied) cudaEventDestroy(c->ev_copied);
@@ -588,7 +581,7 @@ static int prepare_entropy(jpgenc_ctx* c, const jpgenc_huff_table* tables, uint3
     if (bits == 0) return fail(c, JPGENC_ERR_ARG, "symbol statistics missing: run jpgenc_symbol_stats first");
     const uint64_t nbytes = (bits + 7) / 8, tiles = (nbytes + kK4TileBytes - 1) / kK4TileBytes;
     if (tiles > 0x7FFFFFFFull) return fail(c, JPGENC_ERR_ARG, "scan too large");
-    c->frame_bits.assign(1, bits); c->frame_out_off.assign(1, 0); c->frame_ff.assign(1, 0);
+    c->frame_bits.assign(1, bits);
     m.raw_off[0] = 0;
     m.raw_bytes[0] = nbytes;
     m.frame_bits[0] = bits;
@@ -633,7 +626,6 @@ static int wait_entropy(jpgenc_ctx* c) {
         c->error = "entropy coder wrote " + std::to_string(bits) + " bits, statistics predicted " + std::to_string(c->frame_bits[0]);
         return JPGENC_ERR_ARG;
     }
-    c->frame_ff[0] = ff;
     c->stats.scan_bits = bits;
     c->stats.stuffed_ff = ff;
     c->stats.scan_bytes = (bits + 7) / 8 + ff;
@@ -644,12 +636,10 @@ static int wait_entropy(jpgenc_ctx* c) {
 // tables[4], built on the host.  Afterwards the stuffed scan is in d_scan, its size in c->stats.
 static int entropy_frames(jpgenc_ctx* c, const jpgenc_huff_table* tables) {
     JPGENC_CUDA(c, cudaSetDevice(c->device));
-    const double t_conv = trace_on() ? now_us() : 0;
     uint32_t k4_tiles = 0;
     int rc = prepare_entropy(c, tables, &k4_tiles);
     if (rc) return rc;
     if ((rc = enqueue_entropy_phase(c, k4_tiles))) return rc;
-    if (trace_on()) c->trace_convert_us = now_us() - t_conv;
     return wait_entropy(c);
 }
 
@@ -740,7 +730,6 @@ static int run_entropy_stages(jpgenc_ctx* c, jpgenc_huff_table tables[4], uint64
     int rc;
     uint32_t count[4][256];
     uint64_t first_pos[4][256];
-    const double t0 = trace_on() ? now_us() : 0;
     // the pool's workers spin from arm() until the statistics arrive: fine for the ~0.2 ms of K2 on resident pixels, not for
     // the milliseconds an upload takes (VERDICT round 1: 3 spinning workers x 8 ranks on a 32-core host)
     if (!c->parallel_tables || c->upload_pending) {
@@ -748,19 +737,15 @@ static int run_entropy_stages(jpgenc_ctx* c, jpgenc_huff_table tables[4], uint64
         for (int t = 0; t < 4; ++t)
             if ((rc = jpgenc_build_huffman(count[t], first_pos[t], &tables[t]))) return fail(c, rc, "Huffman table build failed");
     } else {
-        if (!c->pool) c->pool = new TablePool(table_workers());
+        if (!c->pool) c->pool = new TablePool(kTableWorkers);
         c->pool->arm();                                             // the workers wake up while K2 runs
         if ((rc = jpgenc_symbol_stats(c, count, first_pos))) {
             c->pool->build(nullptr, nullptr, nullptr);              // release them again
             return rc;
         }
-        const double t1 = trace_on() ? now_us() : 0;
         if ((rc = c->pool->build(count, first_pos, tables))) return fail(c, rc, "Huffman table build failed");
-        if (trace_on()) std::fprintf(stderr, "[jpgenc image] K2 launch+sync %.1f us, tables %.1f us, ", t1 - t0, now_us() - t1);
     }
-    const double t2 = trace_on() ? now_us() : 0;
     if ((rc = jpgenc_entropy_encode(c, tables, scan))) return rc;
-    if (trace_on()) std::fprintf(stderr, "convert+K3+K4+sync %.1f us (convert+enqueue %.1f)\n", now_us() - t2, c->trace_convert_us);
     std::memcpy(c->last_tables, tables, sizeof c->last_tables);
     c->have_tables = true;
     return JPGENC_OK;
@@ -823,14 +808,13 @@ static int run_pipeline(jpgenc_ctx* c, jpgenc_huff_table tables[4], uint64_t* sc
     int rc;
     if ((rc = ensure_coef(c))) return rc;
     if ((rc = ensure_stats_buffers(c))) return rc;
-    const double t0 = trace_on() ? now_us() : 0;
     // ---- phase A: K1, refinement, K2, statistics into the mailbox ----
     c->k2_tiles_done = 0;
     const uint64_t key_a[5] = {c->alloc_gen, reinterpret_cast<uint64_t>(c->d_rgb), (static_cast<uint64_t>(c->real_w) << 32) | c->real_h, c->maxval,
                                1u | static_cast<uint64_t>(c->stage_timing) << 8};
     const bool pool = c->parallel_tables;
     if (pool) {
-        if (!c->pool) c->pool = new TablePool(table_workers());
+        if (!c->pool) c->pool = new TablePool(kTableWorkers);
         c->pool->arm();                                             // the table builders wake up while K1 / K2 run
     }
     rc = run_phase(c, c->graph_a, key_a, [&]() -> int {
@@ -846,7 +830,6 @@ static int run_pipeline(jpgenc_ctx* c, jpgenc_huff_table tables[4], uint64_t* sc
         if (pool) c->pool->build(nullptr, nullptr, nullptr);        // release the workers again
         return rc;
     }
-    const double t1 = trace_on() ? now_us() : 0;
     // ---- host: the four tables ----
     const uint32_t(*count)[256] = c->stat_count;
     const uint64_t(*first_pos)[256] = c->stat_first;
@@ -856,7 +839,6 @@ static int run_pipeline(jpgenc_ctx* c, jpgenc_huff_table tables[4], uint64_t* sc
         for (int t = 0; t < 4; ++t)
             if ((rc = jpgenc_build_huffman(count[t], first_pos[t], &tables[t]))) return fail(c, rc, "Huffman table build failed");
     }
-    const double t2 = trace_on() ? now_us() : 0;
     // ---- phase B: tables to the device, K3a, K3b, K4, totals into the mailbox ----
     uint32_t k4_tiles = 0;
     if ((rc = prepare_entropy(c, tables, &k4_tiles))) return rc;
@@ -868,11 +850,7 @@ static int run_pipeline(jpgenc_ctx* c, jpgenc_huff_table tables[4], uint64_t* sc
     const uint32_t k4_grid = std::min(c->k4_grid_hint, static_cast<uint32_t>(c->raw_cap / kK4TileBytes + 1));   // raw_cap holds the scan: >= k4_tiles
     const uint64_t key_b[5] = {c->alloc_gen, k4_grid, (static_cast<uint64_t>(c->real_w) << 32) | c->real_h, 0, 1u | static_cast<uint64_t>(c->stage_timing) << 8};
     if ((rc = run_phase(c, c->graph_b, key_b, [&]() -> int { return enqueue_entropy_phase(c, k4_grid); }))) return rc;
-    const double t3 = trace_on() ? now_us() : 0;
     if ((rc = wait_entropy(c))) return rc;
-    if (trace_on())
-        std::fprintf(stderr, "[jpgenc image] phase A + wait %.1f us, tables %.1f us, convert + phase B enqueue %.1f us, wait %.1f us\n", t1 - t0, t2 - t1,
-                     t3 - t2, now_us() - t3);
     if (scan) *scan = c->stats.scan_bytes;
     std::memcpy(c->last_tables, tables, sizeof c->last_tables);
     c->have_tables = true;

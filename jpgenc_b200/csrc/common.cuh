@@ -200,14 +200,12 @@ struct jpgenc_ctx {
     uint64_t batch_raw_per_frame = 0;     // batched calls: raw-scan bytes reserved per frame (1.5 x the largest seen so far; 0 = nothing seen yet)
     uint32_t batch_geom_w = 0, batch_geom_h = 0;   // ... the frame size that figure was learnt on (kept across calls of one size)
     cudaEvent_t ev_done = nullptr;        // batched calls: end of the slot's current pass
-    cudaEvent_t ev_wide = nullptr;        // ... its K1/refinement/K2 are through (JPGENC_STAGGER=1: the next pass's wide kernels wait for it)
     cudaEvent_t ev_k4 = nullptr;          // ... its K4 is through (the next pass's K3 waits for it: passes finish one after the other)
-    cudaEvent_t ev_fwd = nullptr;         // ... its K1/refinement are through (JPGENC_STAGGER=2: the next pass's K1 waits for it)
+    cudaEvent_t ev_fwd = nullptr;         // ... its K1/refinement are through (a call of two passes: the next pass's K1 waits for it)
     cudaEvent_t ev_copied = nullptr;      // ... its files have left d_scan (recorded on out_stream)
     cudaStream_t out_stream = nullptr;    // device-to-host copies of finished passes, beside the slot's kernels
     bool copy_pending = false;
     uint8_t hdr_prefix_host[256] = {};    // what d_hdr_prefix holds
-    uint32_t debug_tables_valid = 0;      // JPGENC_DEBUG_SKIP_TABLES (development): tables in d_built_tables from an earlier call
     uint32_t* d_items = nullptr;          // K2's symbol stream (blockwalk.cuh), consumed by K3
     size_t items_cap = 0;
     uint32_t* d_tile_cnt = nullptr;             // per K2 tile: number of items in its slab
@@ -219,7 +217,7 @@ struct jpgenc_ctx {
     bool have_items = false;
     uint32_t k2_tiles_done = 0;           // K2 tiles already processed behind the bands of an upload (jpgenc_encode_rgb)
     std::vector<uint32_t> host_hist;      // K2's histograms as last read back, [nframes][4][256]
-    std::vector<uint64_t> frame_bits, frame_out_off, frame_ff;   // per frame after K3/K4: scan bits, byte offset of its stuffed scan in d_scan, stuffed FFs
+    std::vector<uint64_t> frame_bits;     // per frame: scan bits the statistics predict (checked against K3's count)
     bool k2_configured = false;
     // launch_forward_rows(first) clears K1's counters AND what K2 / K3a accumulate into in one kernel; launch_symbol_stats(first)
     // then skips its own clears -- valid while no buffer was reallocated and the frame count is the same
@@ -251,11 +249,6 @@ struct jpgenc_ctx {
     uint32_t mailbox_seq = 0;             // announced by K2 / K4 of the current encode
     void* h_pinned = nullptr;             // small pinned staging (stats, totals)
     size_t pinned_bytes = 0;
-
-    std::vector<jpgenc_huff_table> pass_tables;   // batched-frame calls: tables of the lane's current pass
-    std::vector<const void*> pass_ptrs;           // ... device pointers of its frames
-    double trace_convert_us = 0;
-    std::vector<uint32_t> hdr_len;                // ... header length of every frame's file
 
     jpgenc_stats stats{};
     jpgenc_huff_table last_tables[4];     // tables of the last whole-image run (for jpgenc_assemble_last)
@@ -331,10 +324,8 @@ int launch_entropy(jpgenc_ctx* c, uint32_t k4_grid);
 int launch_publish_stats(jpgenc_ctx* c);
 // batches: built tables + K2's histograms -> DeviceTables and the PassMeta block, all on the device
 int launch_finalize_tables(jpgenc_ctx* c);
-#ifndef JPGENC_K4_THREADS
-#define JPGENC_K4_THREADS 256
-#endif
-constexpr uint32_t kK4TileBytes = JPGENC_K4_THREADS * 16;   // input bytes per K4 tile: 16 per thread (entropy.cu)
+constexpr uint32_t kK4Threads = 256;
+constexpr uint32_t kK4TileBytes = kK4Threads * 16;   // input bytes per K4 tile: 16 per thread (entropy.cu)
 size_t table_scratch_bytes();
 int build_table_arrays_host(const uint32_t count[256], const uint64_t first_pos[256], jpgenc_huff_table* out);
 int launch_build_tables(jpgenc_ctx* c, const uint8_t* d_stats, uint32_t stats_stride, uint32_t ntables, void* d_scratch,

@@ -368,7 +368,7 @@ __global__ void __launch_bounds__(kPackThreads) huffman_pack_kernel(const __grid
 // 16 input bytes (SIMD byte compare), a CTA scan + look-back give the output position, the tile's output is assembled
 // in shared memory (word stores; byte stores only at a thread's unaligned ends or where an FF actually occurs) and
 // leaves as coalesced 32-bit stores, funnel-shifted to the alignment of the global position.
-constexpr int kStuffThreads = JPGENC_K4_THREADS;
+constexpr int kStuffThreads = kK4Threads;
 constexpr int kStuffBytesPerThread = 16;
 constexpr int kStuffTile = kStuffThreads * kStuffBytesPerThread;
 static_assert(kStuffTile == kK4TileBytes, "capi.cu numbers K4 tiles with kK4TileBytes");

@@ -17,7 +17,6 @@
 //    already in the MCU-interleaved order the entropy coder consumes.
 #include <algorithm>
 #include <cmath>
-#include <cstdlib>
 
 #include "common.cuh"
 #include "exact.cuh"
@@ -745,12 +744,6 @@ static bool make_block_map(void* base, uint64_t nblocks, uint32_t box_blocks, CU
     return encode(map, CU_TENSOR_MAP_DATA_TYPE_UINT16, 2, base, gdim, gstride, box, estride, CU_TENSOR_MAP_INTERLEAVE_NONE,
                   CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
-// JPGENC_TENSOR_STORE=0 falls back to the per-thread copy-out (A/B measurements)
-static bool tensor_store_enabled() {
-    static const bool on = [] { const char* v = std::getenv("JPGENC_TENSOR_STORE"); return !(v && *v == '0'); }();
-    return on;
-}
-
 // Everything K1 needs to know about the image(s) bound to the context
 static void fill_forward_params(const jpgenc_ctx* c, ForwardParams* p) {
     p->rgb = c->d_rgb;
@@ -782,10 +775,8 @@ static int launch_refine(jpgenc_ctx* c, bool all) {
     const uint64_t total = static_cast<uint64_t>(bpf) * c->nframes;
     const unsigned grid = static_cast<unsigned>(std::max<uint64_t>(c->sm_count, std::min<uint64_t>(c->sm_count * 16, total / 256 + 1)));
     // 64 threads per block where the flagged blocks are few (latency: 3840x2160 15 -> 6 us), 8 per block where they are many
-    // (throughput: at 16384^2 the 64-thread form's barriers cost 42 us against 28).  JPGENC_REFINE64=0/1 forces one form.
-    static const int forced = [] { const char* v = std::getenv("JPGENC_REFINE64"); return v && *v ? (*v == '0' ? 0 : 1) : -1; }();
-    const bool wide = forced >= 0 ? forced == 1 : total < (3u << 19);
-    if (wide)
+    // (throughput: at 16384^2 the 64-thread form's barriers cost 42 us against 28)
+    if (total < (3u << 19))
         refine_kernel<true><<<grid, kRefineThreads, 0, c->stream>>>(
             c->d_rgb, c->nframes > 1 ? c->d_frame_ptrs : nullptr, bpf, c->d_coef, c->d_refine_list, c->d_counters,
             all ? 0u : static_cast<uint32_t>(c->refine_cap), all ? 1 : 0, bpf * c->nframes, c->real_w, c->real_h, c->mcu_w, e);
@@ -805,11 +796,8 @@ int launch_forward_rows(jpgenc_ctx* c, uint32_t y0, uint32_t rows, bool first, b
     ForwardParams p{};
     fill_forward_params(c, &p);
     p.mcu_y0 = y0;
-    {
-        // measured on 16384^2 (740 resident CTAs): 150..550 strips ahead all take K1 from 0.328 to 0.317 ms; further ahead loses
-        static const int ahead = [] { const char* v = std::getenv("JPGENC_K1_PREFETCH"); return v && *v ? std::atoi(v) : 256; }();
-        p.prefetch_ahead = static_cast<uint32_t>(ahead);
-    }
+    // measured on 16384^2 (740 resident CTAs): 150..550 strips ahead all take K1 from 0.328 to 0.317 ms; further ahead loses
+    p.prefetch_ahead = 256;
     if (first && !launch_encode_clear(c))                                                          // counters + K2's / K3a's accumulators in one kernel
         JPGENC_CUDA(c, cudaMemsetAsync(c->d_counters, 0, 4 * sizeof(uint32_t), c->stream));          // (no statistics buffers yet) list length .. refined so far
     bool aligned = (c->real_w % 16 == 0) && (reinterpret_cast<uintptr_t>(c->d_rgb) % 16 == 0);
@@ -817,7 +805,7 @@ int launch_forward_rows(jpgenc_ctx* c, uint32_t y0, uint32_t rows, bool first, b
     // (strips of 24 and of 40 MCUs, which divide 1920- and 3840-pixel rows evenly, were measured: no gain on those frames
     // -- the partial fourth strip is not what costs -- and 24 is 7 % slower where 32 divides the row)
     const dim3 grid((c->mcu_w + 31) / 32, rows, c->nframes);
-    const bool bulk_out = tensor_store_enabled() && aligned &&
+    const bool bulk_out = aligned &&
                           make_block_map(c->d_coef, static_cast<uint64_t>(c->mcu_w) * c->mcu_h * kBlocksPerMcu * c->nframes, 32 * kBlocksPerMcu, &p.coef_map);
     if (bulk_out) forward_kernel<32, true, true><<<grid, 128, 0, c->stream>>>(p);
     else if (aligned) forward_kernel<32, true><<<grid, 128, 0, c->stream>>>(p);

@@ -100,7 +100,7 @@ public:
     // `workers` 1..3 threads beside the caller.  The caller always builds the luma AC table (normally the largest alphabet:
     // 10 us against 3 us for each of the others on a photograph); with three workers each of the other tables has a thread
     // of its own, with one worker that thread builds all three one after the other -- about as long as the luma AC table
-    // takes, with one spinning thread instead of three (the default, capi.cu: table_workers).
+    // takes, with one spinning thread instead of three (what capi.cu uses: kTableWorkers).
     explicit TablePool(int workers = 1) : nworkers_(workers < 1 ? 1 : workers > 3 ? 3 : workers) {
         for (int i = 0; i < nworkers_; ++i) workers_[i] = std::thread([this, i] { run(i); });
     }

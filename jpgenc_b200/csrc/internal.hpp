@@ -38,7 +38,6 @@ size_t stage_meta_off(uint32_t F);
 size_t stage_bytes(uint32_t F);
 
 uint32_t env_u32(const char* name, uint32_t dflt);
-bool trace_on();                                                 // JPGENC_TRACE=1: host wall-clock of the phases on stderr
 double now_us();
 
 }}  // namespace jpgenc::detail

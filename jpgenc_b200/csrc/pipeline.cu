@@ -32,34 +32,6 @@ namespace {
 constexpr uint32_t kDefaultSlots = 4, kMaxSlots = 6;
 constexpr uint32_t kMaxHeaderBytes = 2 + 18 + 2 * 69 + 19 + 4 * (21 + 256) + 14;   // SOI APP0 DQTx2 SOF0 DHTx4 SOS
 
-// JPGENC_TRACE=2: a device-side timeline of the call -- timing events between the stages of every pass, printed relative to
-// the first one when the call ends (development aid; the extra event records cost a few microseconds per pass)
-struct Timeline {
-    struct Mark { cudaEvent_t ev; uint32_t pass; const char* what; };
-    std::vector<Mark> marks;
-    bool on = false;
-    void mark(jpgenc_ctx* l, uint32_t pass, const char* what) {
-        if (!on) return;
-        cudaEvent_t ev = nullptr;
-        if (cudaEventCreate(&ev) != cudaSuccess) return;
-        cudaEventRecord(ev, l->stream);
-        marks.push_back({ev, pass, what});
-    }
-    void print() {
-        if (marks.empty()) return;
-        cudaEventSynchronize(marks.back().ev);
-        for (const Mark& m : marks) {
-            float ms = 0;
-            cudaEventSynchronize(m.ev);
-            cudaEventElapsedTime(&ms, marks.front().ev, m.ev);
-            std::fprintf(stderr, "[jpgenc timeline] pass %u %-10s %8.1f us\n", m.pass, m.what, ms * 1e3);
-        }
-        for (const Mark& m : marks) cudaEventDestroy(m.ev);
-        marks.clear();
-    }
-};
-Timeline g_timeline;
-
 struct Job {
     uint32_t n = 0;
     uint32_t w = 0, h = 0, maxval = 255;
@@ -116,7 +88,6 @@ int prepare_slot(jpgenc_ctx* root, jpgenc_ctx* l, const Job& job, const uint8_t*
         l->hdr_prefix_len = prefix_len;
     }
     if (!l->ev_done) JPGENC_CUDA(l, cudaEventCreateWithFlags(&l->ev_done, cudaEventDisableTiming));
-    if (!l->ev_wide) JPGENC_CUDA(l, cudaEventCreateWithFlags(&l->ev_wide, cudaEventDisableTiming));
     if (!l->ev_fwd) JPGENC_CUDA(l, cudaEventCreateWithFlags(&l->ev_fwd, cudaEventDisableTiming));
     if (!l->ev_k4) JPGENC_CUDA(l, cudaEventCreateWithFlags(&l->ev_k4, cudaEventDisableTiming));
     if (!l->ev_copied) JPGENC_CUDA(l, cudaEventCreateWithFlags(&l->ev_copied, cudaEventDisableTiming));
@@ -141,9 +112,7 @@ int enqueue_entropy(jpgenc_ctx* l, Pass& ps, cudaEvent_t prev_k4 = nullptr) {
     // after the other and the files of pass p travel while pass p + 1 is packed, instead of all slots' files queueing up
     // behind the last kernel (trace of 4 slots in step: 4 x 11 MB = 0.8 ms of copies after the last K4)
     if (prev_k4) JPGENC_CUDA(l, cudaStreamWaitEvent(l->stream, prev_k4, 0));
-    g_timeline.mark(l, ps.f0, "finalize");
     if ((rc = launch_entropy(l, ps.k4_grid))) return rc;
-    g_timeline.mark(l, ps.f0, "K3+K4");
     JPGENC_CUDA(l, cudaEventRecord(l->ev_k4, l->stream));
     uint8_t* h = static_cast<uint8_t*>(l->h_pinned) + stage_meta_off(F);
     JPGENC_CUDA(l, cudaMemcpyAsync(h, l->d_meta, pass_meta_bytes(F), cudaMemcpyDeviceToHost, l->stream));
@@ -153,7 +122,7 @@ int enqueue_entropy(jpgenc_ctx* l, Pass& ps, cudaEvent_t prev_k4 = nullptr) {
 }
 
 // the whole chain of one pass on slot `l`; `ready` (optional): event after which the pixels are valid
-// `after` (optional): the previous pass's "wide kernels done" event (see run_passes)
+// `after` (optional): the event after the previous pass's K1 (see run_passes)
 int enqueue_pass(jpgenc_ctx* root, jpgenc_ctx* l, Pass& ps, const void* const* dev_frames, cudaEvent_t ready, cudaEvent_t after, cudaEvent_t prev_k4) {
     const uint32_t F = ps.F;
     int rc;
@@ -180,27 +149,17 @@ int enqueue_pass(jpgenc_ctx* root, jpgenc_ctx* l, Pass& ps, const void* const* d
     JPGENC_CUDA(l, cudaMemcpyAsync(l->d_frame_ptrs, l->h_pinned, F * sizeof(void*), cudaMemcpyHostToDevice, l->stream));
     if (ready) JPGENC_CUDA(l, cudaStreamWaitEvent(l->stream, ready, 0));
     if (after) JPGENC_CUDA(l, cudaStreamWaitEvent(l->stream, after, 0));
-    g_timeline.mark(l, ps.f0, "start");
     if ((rc = launch_forward_rows(l, 0, l->mcu_h, true, true))) return rc;                       // K1 + exact refinement
-    g_timeline.mark(l, ps.f0, "K1+refine");
     l->have_coef = true;
     JPGENC_CUDA(l, cudaEventRecord(l->ev_fwd, l->stream));
     const size_t nblocks = static_cast<size_t>(l->mcu_w) * l->mcu_h * kBlocksPerMcu, tiles = (nblocks + 383) / 384;
     if ((rc = launch_symbol_stats(l, 0, static_cast<uint32_t>(tiles * F), true))) return rc;     // K2
     l->have_items = true;
-    g_timeline.mark(l, ps.f0, "K2");
-    JPGENC_CUDA(l, cudaEventRecord(l->ev_wide, l->stream));
     const uint32_t nt = 4 * F;
     if ((rc = ensure(l, reinterpret_cast<uint8_t**>(&l->d_tab_scratch), &l->tab_scratch_cap, nt * table_scratch_bytes()))) return rc;
     if ((rc = ensure(l, &l->d_built_tables, &l->built_tables_cap, nt * (sizeof(jpgenc_huff_table) + sizeof(uint32_t))))) return rc;
-    // (JPGENC_DEBUG_SKIP_TABLES=1, development only: keep the tables of the previous call -- valid output only when the same
-    // frames are encoded again; shows what the pipeline would do with a free table build)
-    static const bool skip_tables = env_u32("JPGENC_DEBUG_SKIP_TABLES", 0) != 0;
-    if (!(skip_tables && l->debug_tables_valid >= nt))
-        if ((rc = launch_build_tables(l, l->d_stats, static_cast<uint32_t>(kStatsBytes), nt, l->d_tab_scratch, l->d_built_tables,
-                                      reinterpret_cast<uint32_t*>(l->d_built_tables + nt)))) return rc;
-    l->debug_tables_valid = nt;
-    g_timeline.mark(l, ps.f0, "tables");
+    if ((rc = launch_build_tables(l, l->d_stats, static_cast<uint32_t>(kStatsBytes), nt, l->d_tab_scratch, l->d_built_tables,
+                                  reinterpret_cast<uint32_t*>(l->d_built_tables + nt)))) return rc;
     // how much raw scan / output the pass may use: 1.5 x the largest frame the batch has produced so far
     // (root->batch_raw_per_frame), before the first pass has finished a guess of 12 bytes per block; a pass that needs more
     // is refused by finalize_tables_kernel and its entropy stage re-run with what it asked for (finish_pass)
@@ -301,16 +260,14 @@ int run_passes(jpgenc_ctx* c, Job& job, uint32_t per_pass, uint32_t nslots, Fram
         if ((rc = prepare_slot(c, slot[k], job, hdr, prefix_len))) return k ? fail(c, rc, jpgenc_last_error(slot[k])) : rc;
     }
     std::vector<Pass> pass(npasses);
-    // (measured: 128 frames 1.26 -> 1.33 ms, 1024 frames 6.9 -> 7.2 ms: the cross-stream waits cost more than the earlier
-    // table builds gain; kept as a switch)
-    // default: the streams run side by side, except for a call of exactly two passes -- there nothing else will ever run beside
-    // the table builds, and letting pass 1's K1 start when pass 0's K1 is through (mode 2) puts pass 0's table build beside pass 1's
-    // wide kernels (timeline, 128 frames: 1.057 -> 1.014 ms; 256 and 1024 frames are 2-4 % slower staggered)
-    const uint32_t stagger = env_u32("JPGENC_STAGGER", npasses == 2 ? 2u : 0u);
+    // The streams run side by side, except in a call of exactly two passes: there nothing else will ever run beside the table
+    // builds, and letting pass 1's K1 start when pass 0's K1 is through puts pass 0's table build beside pass 1's wide kernels
+    // (timeline, 128 frames: 1.057 -> 1.014 ms).  Staggering more passes does not pay: 256 and 1024 frames are 2-4 % slower
+    // that way, and making every pass wait for the previous pass's K2 took 128 frames 1.26 -> 1.33 ms, 1024 frames 6.9 -> 7.2 ms
+    // -- the cross-stream waits cost more than the earlier table builds gain.
+    const bool stagger = npasses == 2 && nslots > 1;
     rc = JPGENC_OK;
     jpgenc_ctx* failed = nullptr;
-    const double t0 = trace_on() ? now_us() : 0;
-    g_timeline.on = env_u32("JPGENC_TRACE", 0) >= 2;
     for (uint32_t p = 0; p < npasses + nslots && rc == JPGENC_OK; ++p) {
         if (p >= nslots) {                                          // the slot's previous pass: results, files, slot free again
             const uint32_t q = p - nslots;
@@ -318,7 +275,6 @@ int run_passes(jpgenc_ctx* c, Job& job, uint32_t per_pass, uint32_t nslots, Fram
             rc = finish_pass(c, l, pass[q], job);
             if (rc) { failed = l; break; }
             done_with(q);
-            if (trace_on()) std::fprintf(stderr, "[jpgenc batch] pass %u (%u frames, slot %u) finished at %.0f us\n", q, pass[q].F, q % nslots, now_us() - t0);
         }
         if (p < npasses) {
             jpgenc_ctx* l = slot[p % nslots];
@@ -327,15 +283,13 @@ int run_passes(jpgenc_ctx* c, Job& job, uint32_t per_pass, uint32_t nslots, Fram
             const void* const* ptrs = nullptr;
             cudaEvent_t ready = nullptr;
             rc = frames_of(p, l, &ptrs, &ready);
-            // Staggering: the wide kernels of pass p (K1, refinement, K2) start when those of pass p - 1 are through.  Left
-            // alone, the streams run the same stage of all passes side by side, every table build then starts at the same
-            // (late) moment and nothing wide is left to run beside it.
-            cudaEvent_t after = nullptr;
-            if (stagger && p > 0 && nslots > 1) after = stagger == 2 ? slot[(p - 1) % nslots]->ev_fwd : slot[(p - 1) % nslots]->ev_wide;
+            // Staggering: the wide kernels of pass p start when pass p - 1's K1 is through.  Left alone, the streams run the
+            // same stage of all passes side by side, every table build then starts at the same (late) moment and nothing wide
+            // is left to run beside it.
+            cudaEvent_t after = (stagger && p > 0) ? slot[(p - 1) % nslots]->ev_fwd : nullptr;
             // (only when files travel back: sizes-only calls are 2-5 % faster with the slots' K3/K4 side by side.  Measured,
-            // 1024 frames, in order / not: files returned 6.61 / 7.00 ms, sizes only 6.30 / 6.20 ms; JPGENC_ENTROPY_ORDER=0/1 forces)
-            static const uint32_t order_env = env_u32("JPGENC_ENTROPY_ORDER", 2);
-            const bool in_order = order_env == 2 ? (job.packed != nullptr || job.out_ptrs != nullptr) : order_env != 0;
+            // 1024 frames, in order / not: files returned 6.61 / 7.00 ms, sizes only 6.30 / 6.20 ms)
+            const bool in_order = job.packed != nullptr || job.out_ptrs != nullptr;
             cudaEvent_t prev_k4 = (in_order && p > 0 && nslots > 1) ? slot[(p - 1) % nslots]->ev_k4 : nullptr;
             if (rc == JPGENC_OK) rc = enqueue_pass(c, l, pass[p], ptrs, ready, after, prev_k4);
             if (rc) { failed = l; break; }
@@ -348,7 +302,6 @@ int run_passes(jpgenc_ctx* c, Job& job, uint32_t per_pass, uint32_t nslots, Fram
         slot[k]->copy_pending = false;
         if (e != cudaSuccess && rc == JPGENC_OK) { rc = JPGENC_ERR_CUDA; c->error = std::string("batched pass: ") + cudaGetErrorString(e); }
     }
-    g_timeline.print();
     if (failed && failed != c) c->error = failed->error;
     for (uint32_t k = 1; k < nslots; ++k) {
         c->launches += slot[k]->launches;
@@ -361,7 +314,7 @@ int run_passes(jpgenc_ctx* c, Job& job, uint32_t per_pass, uint32_t nslots, Fram
 
 uint32_t slots_for(uint32_t n, uint32_t per_pass) {
     const uint32_t npasses = (n + per_pass - 1) / per_pass;
-    uint32_t s = env_u32("JPGENC_SLOTS", env_u32("JPGENC_LANES", kDefaultSlots));
+    uint32_t s = env_u32("JPGENC_SLOTS", kDefaultSlots);
     return std::max(1u, std::min({s, kMaxSlots, npasses}));
 }
 
@@ -381,7 +334,7 @@ int encode_device_frames(jpgenc_ctx* c, Job& job, const void* const* dev_frames)
     // what earlier calls learnt about the size of such frames' scans stays valid (a later frame that needs more is refused on the
     // device and re-run, finish_pass); a new frame size starts from the guess again
     if (c->batch_geom_w != job.w || c->batch_geom_h != job.h) { c->batch_raw_per_frame = 0; c->batch_geom_w = job.w; c->batch_geom_h = job.h; }
-    const uint32_t nslots0 = std::min(kMaxSlots, env_u32("JPGENC_SLOTS", env_u32("JPGENC_LANES", kDefaultSlots)));
+    const uint32_t nslots0 = std::min(kMaxSlots, env_u32("JPGENC_SLOTS", kDefaultSlots));
     const uint32_t per_pass = pass_frames(c, job.n, std::max(1u, nslots0));
     const uint32_t nslots = slots_for(job.n, per_pass);
     return run_passes(c, job, per_pass, nslots,
@@ -405,7 +358,7 @@ int encode_host_frames(jpgenc_ctx* c, Job& job, const uint8_t* const* frames) {
     // what earlier calls learnt about the size of such frames' scans stays valid (a later frame that needs more is refused on the
     // device and re-run, finish_pass); a new frame size starts from the guess again
     if (c->batch_geom_w != job.w || c->batch_geom_h != job.h) { c->batch_raw_per_frame = 0; c->batch_geom_w = job.w; c->batch_geom_h = job.h; }
-    const uint32_t nslots0 = std::min(kMaxSlots, env_u32("JPGENC_SLOTS", env_u32("JPGENC_LANES", kDefaultSlots)));
+    const uint32_t nslots0 = std::min(kMaxSlots, env_u32("JPGENC_SLOTS", kDefaultSlots));
     const uint32_t per_pass = pass_frames(c, job.n, std::max(1u, nslots0));
     const uint32_t nslots = slots_for(job.n, per_pass);
     const uint32_t npasses = (job.n + per_pass - 1) / per_pass;

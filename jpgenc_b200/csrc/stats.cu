@@ -17,7 +17,6 @@
 // like, the loop body is branch-free and the item stores are coalesced.  The DC and EOB symbols
 // exist exactly once (at most once) per block and stay with the block's own thread.
 #include <algorithm>
-#include <cstdlib>
 
 #include "blockwalk.cuh"
 
@@ -40,32 +39,13 @@ struct StatsParams {
     uint32_t* refine_copy;            // ... copied next to the statistics so that one read-back fetches everything
 };
 
-// The round-1 histogram update, kept behind JPGENC_K2_AGG=1 for A/B measurements: lanes with the same bin are counted by
-// their lowest lane, so the hot symbols (EOB, +-1 coefficients, the common DC category) cost one shared-memory atomic
-// instead of up to 32.  The default is now a plain atomic per lane: the grouping costs ~25 instructions per step in a
-// kernel bound by instruction issue, while same-address shared-memory atomics are serialised by the LSU at no issue cost
-// (typical image 0.2145 -> 0.2042 ms, uniform texture 0.0712 -> 0.0670, 4096^2 noise 0.102 -> 0.0855).
+// Histogram updates are a plain shared-memory atomic per lane: grouping lanes of the same bin (MATCH.ANY, round 1) costs
+// ~25 instructions per step in a kernel bound by instruction issue, while same-address shared-memory atomics are serialised
+// by the LSU at no issue cost (DESIGN.md, K2).
 //
 // Keys inside a tile are 32-bit and TILE-LOCAL (TileKeys): shared memory has a native 32-bit atomic minimum, a 64-bit one is
 // a compare-and-swap loop.
-__device__ __forceinline__ void warp_count(uint32_t* s_hist, uint32_t* s_first, bool has, int idx, uint32_t key) {
-    const int lane = threadIdx.x & 31;
-    const unsigned grp = __match_any_sync(0xffffffffu, has ? idx : (0x10000 | lane));
-    const bool leader = has && lane == __ffs(grp) - 1;
-    if (leader) atomicAdd(&s_hist[idx], static_cast<uint32_t>(__popc(grp)));
-    // first-occurrence key: nothing to do once the minimum is established (the steady state of a large image).  Where
-    // lanes do improve on it, 32 lanes hammering one address with atomics is what made small frames slow, and a minimum
-    // over the matching lanes (__reduce_min_sync with a partial mask) is a software loop of ~40 instructions.  Lanes hold
-    // consecutive symbols of the scan, so the lowest matching lane nearly always holds the smallest key: it updates first,
-    // and only lanes that still beat the stored value afterwards (block rows out of text order) follow.
-    const bool better = has && key < s_first[idx];
-    if (__any_sync(0xffffffffu, better)) {
-        if (leader && better) atomicMin(&s_first[idx], key);
-        __syncwarp();
-        if (better && !leader && key < s_first[idx]) atomicMin(&s_first[idx], key);
-    }
-}
-
+//
 // Tile-local first-occurrence keys.  The global key of a symbol is (block index in the reference's text order) * 256 +
 // position key.  Inside one tile (64 consecutive MCUs) the luma text indices lie within a few block rows of the tile's
 // first block, and the chroma ones are the tile's MCU numbers, once for Cb and once -- n_mcu later -- for Cr:
@@ -90,7 +70,6 @@ constexpr int kStatsSmem = kTileSmemBytes                // masks + dc
                            + 4096 + 4096                 // histogram, local first-occurrence keys
                            + 36 * 4;                     // scan scratch
 
-template <bool kAggregateAc>
 __global__ void __launch_bounds__(kTileBlocks, 5) symbol_stats_kernel(const __grid_constant__ StatsParams p) {
     extern __shared__ __align__(128) uint8_t smem[];
     const TileView tv = tile_view(smem);
@@ -168,9 +147,7 @@ __global__ void __launch_bounds__(kTileBlocks, 5) symbol_stats_kernel(const __gr
         out[base] = make_item(tdc, dcat, 0, diff);
         if (eob) out[base + count - 1] = make_item(tdc + 1, 0, 0, 0);
     }
-    if constexpr (kAggregateAc) {
-        warp_count(s_hist, s_first, live, tdc * 256 + dcat, key);
-    } else if (live) {
+    if (live) {
         atomicAdd(&s_hist[tdc * 256 + dcat], 1u);
         if (key < s_first[tdc * 256 + dcat]) atomicMin(&s_first[tdc * 256 + dcat], key);
     }
@@ -218,7 +195,7 @@ __global__ void __launch_bounds__(kTileBlocks, 5) symbol_stats_kernel(const __gr
         __syncthreads();
         // consecutive lanes take consecutive coefficients
         const uint32_t n = min(static_cast<uint32_t>(kDescCap), total_ac - win);
-        for (uint32_t j0 = 0; j0 < n; j0 += kTileBlocks) {              // uniform trip count: warp_count is a warp-wide operation
+        for (uint32_t j0 = 0; j0 < n; j0 += kTileBlocks) {              // uniform trip count: the __any_sync below is warp-wide
             const uint32_t j = j0 + tid;
             const bool has = j < n;
             int idx = 0, nzrl = 0, table = 0;
@@ -234,9 +211,7 @@ __global__ void __launch_bounds__(kTileBlocks, 5) symbol_stats_kernel(const __gr
                 const uint32_t sb = s_base[b];
                 out[(sb & 0xFFFFu) + 1u + (win + j - (sb >> 16))] = make_item(table, symbol, nzrl, value);
             }
-            if constexpr (kAggregateAc) {
-                warp_count(s_hist, s_first, has, idx, ikey);
-            } else if (has) {                                            // plain shared-memory atomics: same-address lanes are serialised by the LSU
+            if (has) {                                                   // plain shared-memory atomics: same-address lanes are serialised by the LSU
                 atomicAdd(&s_hist[idx], 1u);
                 if (ikey < s_first[idx]) atomicMin(&s_first[idx], ikey);
             }
@@ -305,9 +280,8 @@ __global__ void encode_clear_kernel(uint32_t* counters, uint32_t* stats, uint32_
 
 bool launch_encode_clear(jpgenc_ctx* c) {
     // one image only: in batches (four streams side by side) the same kernel in front of every pass's K1 costs 6 % (1024 frames
-    // 5.89 -> 6.23 ms, measured twice; the memsets stay there).  JPGENC_MERGED_CLEAR=0 switches it off everywhere.
-    static const bool off = [] { const char* v = std::getenv("JPGENC_MERGED_CLEAR"); return v && *v == '0'; }();
-    if (off || c->nframes > 1) return false;
+    // 5.89 -> 6.23 ms, measured twice; the memsets stay there)
+    if (c->nframes > 1) return false;
     const size_t stat_bytes = static_cast<size_t>(c->nframes) * kStatsBytes;
     if (!c->d_stats || !c->d_range_base || c->stats_cap < stat_bytes || stat_bytes / 4 > 0xFFFFFFFFull || c->range_base_cap / 8 > 0xFFFFFFFFull) return false;
     const uint32_t stat_words = static_cast<uint32_t>(stat_bytes / 4), range_words = static_cast<uint32_t>(c->range_base_cap / 8);
@@ -352,14 +326,10 @@ int launch_symbol_stats(jpgenc_ctx* c, uint32_t tile0, uint32_t ntiles, bool fir
     p.refine_count = c->d_counters;
     p.refine_copy = reinterpret_cast<uint32_t*>(c->d_stats + c->nframes * kStatsBytes);
     if (!c->k2_configured) {                                   // (the first encode of a context is never graph-captured)
-        JPGENC_CUDA(c, cudaFuncSetAttribute(symbol_stats_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kStatsSmem));
-        JPGENC_CUDA(c, cudaFuncSetAttribute(symbol_stats_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kStatsSmem));
+        JPGENC_CUDA(c, cudaFuncSetAttribute(symbol_stats_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kStatsSmem));
         c->k2_configured = true;
     }
-    // JPGENC_K2_AGG=1: MATCH.ANY-grouped histogram updates (round 1) instead of plain shared-memory atomics
-    static const bool aggregate = [] { const char* v = std::getenv("JPGENC_K2_AGG"); return v && *v == '1'; }();
-    if (aggregate) symbol_stats_kernel<true><<<ntiles, kTileBlocks, kStatsSmem, c->stream>>>(p);
-    else symbol_stats_kernel<false><<<ntiles, kTileBlocks, kStatsSmem, c->stream>>>(p);
+    symbol_stats_kernel<<<ntiles, kTileBlocks, kStatsSmem, c->stream>>>(p);
     JPGENC_CUDA(c, cudaGetLastError());
     c->launches += 1;
     return JPGENC_OK;

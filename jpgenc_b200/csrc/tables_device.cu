@@ -18,7 +18,6 @@
 // steps -- one thread, ~40 ns per step -- but all 4 * F tables of a pass run side by side (one warp each, lane 0
 // working) and the other lanes' kernels fill the SMs meanwhile.  A single image keeps the host build: 16 us there
 // against >= 250 us here.
-#include <cstdlib>
 #include <cstring>
 
 #include "common.cuh"
@@ -32,7 +31,6 @@ constexpr int kMaxBuckets = 600;
 constexpr int kLimit = 15;                                     // package_merge(symbol_frequency, 15)
 constexpr int kMaxNodes = kMaxSyms * (kLimit + 2) + 16;        // leaves + at most one package per pair of items per level
 constexpr int kBeforeBegin = -2;
-constexpr int kSharedSyms = 64;                               // heaps of up to this many symbols fit the CTA's shared memory
 
 struct HeapItem {
     long long w;
@@ -140,7 +138,7 @@ __host__ __device__ int um_touch(OrderedMap& m, int key) {
     return node;
 }
 
-__host__ __device__ void heap_push_hole(HeapItem* v, int hole, int top, long long val_w, int val_node) {      // std::__push_heap
+void heap_push_hole(HeapItem* v, int hole, int top, long long val_w, int val_node) {      // std::__push_heap
     int parent = (hole - 1) / 2;
     while (hole > top && v[parent].w > val_w) {
         v[hole].w = v[parent].w;
@@ -151,9 +149,9 @@ __host__ __device__ void heap_push_hole(HeapItem* v, int hole, int top, long lon
     v[hole].w = val_w;
     v[hole].node = val_node;
 }
-__host__ __device__ void heap_push(HeapItem* v, int& n, long long w, int node) { ++n; heap_push_hole(v, n - 1, 0, w, node); }
+void heap_push(HeapItem* v, int& n, long long w, int node) { ++n; heap_push_hole(v, n - 1, 0, w, node); }
 // top(), then std::pop_heap + pop_back
-__host__ __device__ void heap_pop(HeapItem* v, int& n, long long& top_w, int& top_node) {
+void heap_pop(HeapItem* v, int& n, long long& top_w, int& top_node) {
     top_w = v[0].w;
     top_node = v[0].node;
     if (n > 1) {
@@ -181,7 +179,7 @@ __host__ __device__ void heap_pop(HeapItem* v, int& n, long long& top_w, int& to
 
 // occurrences of every symbol among the leaves of package `root`: cnt[] is incremented, the symbols seen are flagged in
 // the 256-bit mask
-__host__ __device__ void count_leaves(const Node* nodes, int root, unsigned short* cnt, unsigned (&mask)[8]) {
+void count_leaves(const Node* nodes, int root, unsigned short* cnt, unsigned (&mask)[8]) {
     int stack[40], sp = 0;                                     // a package is at most kLimit levels deep: <= 17 pending nodes
     stack[sp++] = root;
     while (sp) {
@@ -210,24 +208,13 @@ __host__ __device__ void write_table(const TableScratch& s, int nsymbols, jpgenc
     t->nsymbols = nsymbols;
 }
 
-// where the serial part keeps its hot state: in the CTA's shared memory for small alphabets, in the scratch slab otherwise
-struct Work {
-    OrderedMap* map;
-    Node* nodes;
-    HeapItem *blueprint, *heap_a, *heap_b;
-    unsigned short *len_of, *cnt;
-};
-
-// The serial part: s.order[0..n) = the distinct symbols in order of first appearance, count[256] their frequencies;
-// *tab has been zeroed.  Runs on one device thread -- and, for tests without a GPU, on the host.
-// The container state (map, three heaps, package nodes, counters) lives where `wk` says: in shared memory for alphabets of
-// up to kSharedSyms symbols -- every container operation is a chain of dependent loads; from global memory a 27-symbol
-// table took 700 us -- otherwise in the table's scratch slab.
-__host__ __device__ void build_table_serial(TableScratch& s, const uint32_t* count, int n, jpgenc_huff_table* tab, const Work& wk) {
-    OrderedMap& map = *wk.map;
-    Node* nodes = wk.nodes;
-    HeapItem *blueprint = wk.blueprint, *heap_a = wk.heap_a, *heap_b = wk.heap_b;
-    unsigned short *len_of = wk.len_of, *cnt = wk.cnt;
+// The one-thread construction: s.order[0..n) = the distinct symbols in order of first appearance, count[256] their
+// frequencies; *tab has been zeroed.  Runs on the host, as the reference the CPU tests check the array restatement with.
+void build_table_serial(TableScratch& s, const uint32_t* count, int n, jpgenc_huff_table* tab) {
+    OrderedMap& map = s.map;
+    Node* nodes = s.nodes;
+    HeapItem *blueprint = s.blueprint, *heap_a = s.heap_a, *heap_b = s.heap_b;
+    unsigned short *len_of = s.len_of, *cnt = s.cnt;
     um_init(map);
     for (int i = 0; i < n; ++i) um_touch(map, s.order[i]);
     int m = 0;
@@ -282,7 +269,7 @@ __host__ __device__ void build_table_serial(TableScratch& s, const uint32_t* cou
             unsigned bits = mask[w];
             while (bits) {
                 int b = 0;
-                while (!((bits >> b) & 1u)) ++b;               // lowest set bit (portable: this function also runs on the host)
+                while (!((bits >> b) & 1u)) ++b;               // lowest set bit
                 const int sym = w * 32 + b;
                 bits &= bits - 1;
                 um_touch(map, sym);
@@ -549,7 +536,7 @@ __device__ int package_merge_warp(WarpShared& ws, uint32_t* nodes, int n, int la
 
 // The table `tab` (zeroed) from count[] / first[]; ws = the warp's shared memory, s = its scratch slab in global memory.
 __device__ void build_table_warp(WarpShared& ws, TableScratch& s, const uint32_t* count, const unsigned long long* first,
-                                 jpgenc_huff_table* tab, int lane, uint32_t* status, bool lean_ok) {
+                                 jpgenc_huff_table* tab, int lane, uint32_t* status) {
     // ---- distinct symbols in order of first appearance (= the order the reference's counting loop creates map entries) ----
     int n = 0;
     for (int base = 0; base < 256; base += 32) {
@@ -593,8 +580,8 @@ __device__ void build_table_warp(WarpShared& ws, TableScratch& s, const uint32_t
     for (int d = 16; d > 0; d >>= 1) total += __shfl_xor_sync(0xffffffffu, total, d);
     const bool small_weights = total < (1ull << 28);           // 15 x total (the heaviest a package can get) fits 32 bits
     int npk;
-    if (small_weights && n <= 32 && lean_ok) npk = package_merge_warp<LeanHeap<1>>(ws, nodes, n, lane);
-    else if (small_weights && n <= 64 && lean_ok) npk = package_merge_warp<LeanHeap<2>>(ws, nodes, n, lane);
+    if (small_weights && n <= 32) npk = package_merge_warp<LeanHeap<1>>(ws, nodes, n, lane);
+    else if (small_weights && n <= 64) npk = package_merge_warp<LeanHeap<2>>(ws, nodes, n, lane);
     else npk = package_merge_warp<WideHeap>(ws, nodes, n, lane);
     for (int i = lane; i < n; i += 32) { ws.cnt[i] = 0; ws.first[i] = 0xFFFFu; }
     __syncwarp();
@@ -656,14 +643,12 @@ __device__ void build_table_warp(WarpShared& ws, TableScratch& s, const uint32_t
 }  // namespace
 #endif
 
-// One warp per table.  status[table] = 0 ok, 1 = no symbol at all.  kCooperative = false runs the one-thread version
-// (build_table_serial, the code the CPU tests execute) for A/B checks: JPGENC_TABLES_SERIAL=1.
+// One warp per table.  status[table] = 0 ok, 1 = no symbol at all.
 // (No __restrict__ on these parameters: with it nvcc 12.9 -O3 treated the two level heaps -- members of one scratch
 // object whose pointers swap roles every level -- as never aliasing, and a popped weight read back as 0.  Found by the
 // parity test; -G, -Xcicc -O1 and non-inlined heap functions all gave the right tables.)
-template <bool kCooperative>
 __global__ void __launch_bounds__(32) build_tables_kernel(const uint8_t* stats, uint32_t stats_stride, uint32_t ntables,
-                                                          TableScratch* scratch, jpgenc_huff_table* out, uint32_t* status, int lean_ok) {
+                                                          TableScratch* scratch, jpgenc_huff_table* out, uint32_t* status) {
     const uint32_t table = blockIdx.x, lane = threadIdx.x;
     if (table >= ntables) return;
     const uint32_t frame = table >> 2, t = table & 3;
@@ -676,37 +661,9 @@ __global__ void __launch_bounds__(32) build_tables_kernel(const uint8_t* stats, 
         uint32_t* w = reinterpret_cast<uint32_t*>(tab);
         for (uint32_t i = lane; i < sizeof(jpgenc_huff_table) / 4; i += 32) w[i] = 0;
     }
-    if constexpr (kCooperative) {
-        __shared__ WarpShared ws;
-        __syncwarp();
-        build_table_warp(ws, s, count, first, tab, static_cast<int>(lane), status + table, lean_ok != 0);
-    } else {
-        __shared__ HeapItem sh_heap[3][2 * kSharedSyms + 16];
-        __shared__ Node sh_nodes[kSharedSyms * (kLimit + 2) + 16];
-        __shared__ OrderedMap sh_map;
-        __shared__ unsigned short sh_len[2][kMaxSyms];
-        // distinct symbols in order of first appearance == the order the reference's counting loop creates map entries
-        // (keys are unique: one text position holds one symbol); rank = number of present symbols that appear earlier
-        int n = 0;
-        for (int base = 0; base < 256; base += 32) {
-            const int sym = base + lane;
-            const bool here = count[sym] != 0;
-            if (here) {
-                const unsigned long long k = first[sym];
-                int rank = 0;
-                for (int o = 0; o < 256; ++o) rank += (count[o] != 0 && first[o] < k) ? 1 : 0;
-                s.order[rank] = static_cast<unsigned char>(sym);
-            }
-            n += __popc(__ballot_sync(0xffffffffu, here));
-        }
-        __syncwarp();
-        if (lane != 0) return;
-        if (n == 0) { status[table] = 1; return; }                 // the reference asserts text.size() > 0
-        status[table] = 0;
-        const Work in_shared{&sh_map, sh_nodes, sh_heap[0], sh_heap[1], sh_heap[2], sh_len[0], sh_len[1]};
-        const Work in_scratch{&s.map, s.nodes, s.blueprint, s.heap_a, s.heap_b, s.len_of, s.cnt};
-        build_table_serial(s, count, n, tab, n <= kSharedSyms ? in_shared : in_scratch);
-    }
+    __shared__ WarpShared ws;
+    __syncwarp();
+    build_table_warp(ws, s, count, first, tab, static_cast<int>(lane), status + table);
 }
 
 size_t table_scratch_bytes() { return sizeof(TableScratch); }
@@ -725,7 +682,7 @@ int build_table_arrays_host(const uint32_t count[256], const uint64_t first_pos[
         s->order[rank] = static_cast<unsigned char>(sym);
         ++n;
     }
-    if (n) build_table_serial(*s, count, n, out, Work{&s->map, s->nodes, s->blueprint, s->heap_a, s->heap_b, s->len_of, s->cnt});
+    if (n) build_table_serial(*s, count, n, out);
     delete s;
     return n ? JPGENC_OK : JPGENC_ERR_ARG;
 }
@@ -734,11 +691,7 @@ int build_table_arrays_host(const uint32_t count[256], const uint64_t first_pos[
 // frame: histogram u32[4][256], first-occurrence keys u64[4][256]); scratch: ntables * table_scratch_bytes()
 int launch_build_tables(jpgenc_ctx* c, const uint8_t* d_stats, uint32_t stats_stride, uint32_t ntables, void* d_scratch,
                         jpgenc_huff_table* d_out, uint32_t* d_status) {
-    static const bool serial = [] { const char* v = std::getenv("JPGENC_TABLES_SERIAL"); return v && *v && *v != '0'; }();
-    // JPGENC_TABLES_LEAN=0: the general heap operations for every table (A/B checks of the lean ones)
-    static const int lean = [] { const char* v = std::getenv("JPGENC_TABLES_LEAN"); return (v && *v == '0') ? 0 : 1; }();
-    if (serial) build_tables_kernel<false><<<ntables, 32, 0, c->stream>>>(d_stats, stats_stride, ntables, static_cast<TableScratch*>(d_scratch), d_out, d_status, lean);
-    else build_tables_kernel<true><<<ntables, 32, 0, c->stream>>>(d_stats, stats_stride, ntables, static_cast<TableScratch*>(d_scratch), d_out, d_status, lean);
+    build_tables_kernel<<<ntables, 32, 0, c->stream>>>(d_stats, stats_stride, ntables, static_cast<TableScratch*>(d_scratch), d_out, d_status);
     JPGENC_CUDA(c, cudaGetLastError());
     c->launches += 1;
     return JPGENC_OK;

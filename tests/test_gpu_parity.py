@@ -368,13 +368,14 @@ def test_frames_through_the_kernels_together(encoder, oracle, w, h, n):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("per_pass,lanes", [(3, 2), (1, 4), (4, 1), (7, 3), (2, 3)])
+@pytest.mark.parametrize("per_pass,lanes", [(3, 2), (1, 4), (4, 1), (7, 3), (2, 3), (12, 2)])
 def test_frames_in_many_passes_on_several_lanes(encoder, oracle, monkeypatch, per_pass, lanes):
     """The batched-frame calls cut a batch into passes and run them on several pipeline lanes (own streams and buffers, one
     host thread each; uploads of host frames travel through a ring of slices ahead of the kernels).  Forcing tiny passes
-    makes every hand-over happen many times: the files must not depend on pass size, lane count or which lane ran a pass."""
+    makes every hand-over happen many times: the files must not depend on pass size, lane count or which lane ran a pass.
+    (12, 2) gives exactly two passes, the one shape whose second pass waits for the first pass's K1 (staggered)."""
     monkeypatch.setenv("JPGENC_FRAMES_PER_PASS", str(per_pass))
-    monkeypatch.setenv("JPGENC_LANES", str(lanes))
+    monkeypatch.setenv("JPGENC_SLOTS", str(lanes))
     w, h, n = 176, 104, 23
     frames = [synth_rgb(w, h, s) if s % 4 else noise_rgb(w, h, s) for s in range(n)]
     want = [oracle.encode_rgb(f) for f in frames]

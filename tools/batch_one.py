@@ -1,6 +1,6 @@
 """one batched call over 256 frames of 1920x1080 in passes of 128, single lane (for ncu launch lists) -- development aid"""
 import os, sys
-os.environ["JPGENC_LANES"] = "1"; os.environ["JPGENC_FRAMES_PER_PASS"] = "128"
+os.environ["JPGENC_SLOTS"] = "1"; os.environ["JPGENC_FRAMES_PER_PASS"] = "128"
 sys.path.insert(0, ".")
 from jpgenc_b200.capi import Encoder
 w, h, nf = 1920, 1080, 256

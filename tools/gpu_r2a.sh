@@ -20,7 +20,6 @@ python tools/one_image.py 16384 16384 50
 python tools/one_image.py 3840 2160 200
 python tools/one_image.py 1920 1080 200
 python tools/one_image.py 512 512 200
-JPGENC_TRACE=1 python tools/one_image.py 16384 16384 3 2>&1 | tail -8
 python tools/one_image.py 16384 16384 2 > /dev/null 2>&1 &&
 ncu --metrics gpu__time_duration.sum --clock-control none --csv --log-file gpurun_out/r2a_launches16k.csv python tools/one_image.py 16384 16384 1 > gpurun_out/r2a_ncu16k.log 2>&1
 python tools/one_batch.py 128 2 &&

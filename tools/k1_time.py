@@ -1,4 +1,4 @@
-"""K1 time on the 16384^2 synthetic (CUDA events inside the library), for A/B runs with environment switches -- development aid"""
+"""K1 and K2 time and whole-encode time on the 16384^2 synthetic (CUDA events inside the library) -- development aid"""
 import sys
 sys.path.insert(0, ".")
 from jpgenc_b200.capi import Encoder
