@@ -204,6 +204,18 @@ int jpgenc_encode_frames_packed(jpgenc_ctx* ctx, uint32_t n, const void* const* 
                                 uint32_t h, uint32_t maxval, uint8_t* out, uint64_t cap, uint64_t* offsets, uint64_t* sizes,
                                 uint64_t* total_bytes);
 
+/* n images of individual sizes widths[i] x heights[i] (interleaved RGB, tightly packed rows), in host memory
+ * (images_on_device = 0; pinned for full PCIe speed) or device memory (1), through the same pass pipeline: output as
+ * jpgenc_encode_frames_packed -- the complete JFIF files back to back in input order in `out` (cap bytes; NULL = sizes and
+ * offsets only), file i at out[offsets[i] .. offsets[i] + sizes[i]), *total_bytes (optional) the end of the last one.  Every
+ * file is byte-identical to encoding that image alone.  One maxval and the context's quantisation tables apply to all images.
+ * Sides are 1..65535 (JPGENC_ERR_ARG otherwise).  Host images are checked against maxval when it is below 255
+ * (JPGENC_ERR_FORMAT); device images are the caller's promise.  n = 0 is legal and touches nothing.  When every image has the
+ * same size this is jpgenc_encode_frames_packed. */
+int jpgenc_encode_images_packed(jpgenc_ctx* ctx, uint32_t n, const void* const* images, int images_on_device, const uint32_t* widths,
+                                const uint32_t* heights, uint32_t maxval, uint8_t* out, uint64_t cap, uint64_t* offsets,
+                                uint64_t* sizes, uint64_t* total_bytes);
+
 /* ---- stage methods for the modes writeJPEG does not use (SURVEY.md 8(f)4) ------------------------------------------ */
 /* Image::applySubsampling(mode) on one chroma plane (src/Image.cpp:198-319): `plane` = height x width doubles (host), mode =
  * the order of Image::SubsamplingMode (0 S444, 1 S422, 2 S411, 3 S420, 4 S420_m, 5 S420_lm); `out` receives the

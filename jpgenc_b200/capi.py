@@ -104,6 +104,8 @@ _SIGNATURES = {
                                        C.POINTER(C.c_void_p), u64p, u64p]),
     "jpgenc_encode_frames_packed": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(C.c_void_p), C.c_int, C.c_uint32, C.c_uint32, C.c_uint32,
                                               C.c_void_p, C.c_uint64, u64p, u64p, u64p]),
+    "jpgenc_encode_images_packed": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(C.c_void_p), C.c_int, u32p, u32p, C.c_uint32,
+                                              C.c_void_p, C.c_uint64, u64p, u64p, u64p]),
     "jpgenc_batch_create": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "jpgenc_batch_destroy": (None, [C.c_void_p]),
     "jpgenc_batch_last_error": (C.c_char_p, [C.c_void_p]),
@@ -340,6 +342,40 @@ class Encoder:
         self._check(self.lib.jpgenc_encode_frames_packed(self.h, n, frames, 0 if host_frames else 1, w, h, maxval, out_ptr, cap,
                                                          offs, sizes, C.byref(total)))
         return [int(x) for x in offs], [int(x) for x in sizes], int(total.value)
+
+    def encode_images_packed(self, ptrs, widths, heights, out_ptr: int | None, cap: int, maxval: int = 255, host_images=False):
+        """images of individual sizes (device memory, or host memory with host_images=True) -> complete files back to back in
+        ONE buffer, in input order; returns (offsets, sizes, total bytes)"""
+        n = len(ptrs)
+        imgs = (C.c_void_p * n)(*ptrs)
+        w = np.ascontiguousarray(widths, np.uint32)
+        h = np.ascontiguousarray(heights, np.uint32)
+        sizes = (C.c_uint64 * n)()
+        offs = (C.c_uint64 * n)()
+        total = C.c_uint64()
+        self._check(self.lib.jpgenc_encode_images_packed(self.h, n, imgs, 0 if host_images else 1, _np_ptr(w, u32p), _np_ptr(h, u32p), maxval,
+                                                         out_ptr, cap, offs, sizes, C.byref(total)))
+        return [int(x) for x in offs], [int(x) for x in sizes], int(total.value)
+
+    def encode_images(self, images, maxval: int = 255):
+        """list of HxWx3 uint8 arrays of any sizes -> list of JPEG byte strings, through one call (a second one, sizes first,
+        only when the files outgrow the pixels)"""
+        images = [np.ascontiguousarray(a, np.uint8) for a in images]
+        if not images:
+            return []
+        ptrs = [a.ctypes.data for a in images]
+        ws = [a.shape[1] for a in images]
+        hs = [a.shape[0] for a in images]
+        out = np.empty(sum(a.size for a in images) + 4096 * len(images), np.uint8)
+        try:
+            offs, sizes, _ = self.encode_images_packed(ptrs, ws, hs, out.ctypes.data, out.size, maxval, host_images=True)
+        except JpgencError as e:
+            if e.code != ERR_CAPACITY:
+                raise
+            _, _, total = self.encode_images_packed(ptrs, ws, hs, None, 0, maxval, host_images=True)
+            out = np.empty(total, np.uint8)
+            offs, sizes, _ = self.encode_images_packed(ptrs, ws, hs, out.ctypes.data, out.size, maxval, host_images=True)
+        return [out[o: o + n].tobytes() for o, n in zip(offs, sizes)]
 
     def encode_ppm_file(self, src: str, dst: str):
         self._check(self.lib.jpgenc_encode_ppm_file(self.h, src.encode(), dst.encode()))

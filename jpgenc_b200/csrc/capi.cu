@@ -70,6 +70,7 @@ int set_geometry(jpgenc_ctx* c, uint32_t w, uint32_t h, uint32_t maxval) {
     c->real_w = w; c->real_h = h; c->maxval = maxval;
     c->mcu_w = (w + 15) / 16; c->mcu_h = (h + 15) / 16;        // src/Image.cpp:479-489
     c->nframes = 1;
+    c->mixed.on = false;
     c->have_pixels = false;                                      // whoever changes the geometry binds its pixels afterwards
     c->have_coef = c->have_scan = c->have_items = false; c->k2_tiles_done = 0;
     return JPGENC_OK;
@@ -97,7 +98,7 @@ int refresh_forward_stats(jpgenc_ctx* c) {
 }
 
 int ensure_coef(jpgenc_ctx* c) {
-    const size_t nblocks = static_cast<size_t>(c->mcu_w) * c->mcu_h * kBlocksPerMcu * c->nframes;
+    const size_t nblocks = c->mixed.on ? c->mixed.blocks : static_cast<size_t>(c->mcu_w) * c->mcu_h * kBlocksPerMcu * c->nframes;
     if (nblocks * 64 > 0xFFFFFFFFull * 16) return fail(c, JPGENC_ERR_ARG, "image (or batch) too large");
     int rc = ensure(c, &c->d_coef, &c->coef_cap, nblocks * kBlockBytes);
     if (rc) return rc;
@@ -115,14 +116,17 @@ double now_us() {
 int ensure_stats_buffers(jpgenc_ctx* c) {
     const uint32_t F = c->nframes;
     const size_t nblocks = static_cast<size_t>(c->mcu_w) * c->mcu_h * kBlocksPerMcu, tiles = (nblocks + 383) / 384;
+    // images of individual sizes: the pass's own tiles, groups and super-groups (c->mixed)
+    const size_t all_tiles = c->mixed.on ? c->mixed.tiles : F * tiles;
+    const size_t range_words = c->mixed.on ? c->mixed.groups + c->mixed.supers : F * (tiles * 4 / 8 + tiles * 4 / 2048 + 4);
     int rc;
     // one fixed slab of item slots per tile, sized for the worst case (every coefficient non-zero); typical images
     // touch a few percent of it
-    if ((rc = ensure(c, &c->d_items, &c->items_cap, F * tiles * 384 * 64 * sizeof(uint32_t)))) return rc;
-    if ((rc = ensure(c, &c->d_tile_cnt, &c->tile_cnt_cap, F * tiles * sizeof(uint32_t)))) return rc;
+    if ((rc = ensure(c, &c->d_items, &c->items_cap, all_tiles * 384 * 64 * sizeof(uint32_t)))) return rc;
+    if ((rc = ensure(c, &c->d_tile_cnt, &c->tile_cnt_cap, all_tiles * sizeof(uint32_t)))) return rc;
     // K3 may cut a tile into four ranges (small images, launch_entropy): sized for that
-    if ((rc = ensure(c, &c->d_range_bits, &c->range_bits_cap, F * tiles * 4 * sizeof(uint32_t)))) return rc;
-    if ((rc = ensure(c, &c->d_range_base, &c->range_base_cap, F * (tiles * 4 / 8 + tiles * 4 / 2048 + 4) * sizeof(unsigned long long)))) return rc;
+    if ((rc = ensure(c, &c->d_range_bits, &c->range_bits_cap, all_tiles * 4 * sizeof(uint32_t)))) return rc;
+    if ((rc = ensure(c, &c->d_range_base, &c->range_base_cap, range_words * sizeof(unsigned long long)))) return rc;
     if ((rc = ensure(c, &c->d_stats, &c->stats_cap, F * kStatsBytes + 16))) return rc;
     return ensure_pinned(c, stage_bytes(F));
 }
@@ -225,6 +229,7 @@ int poll_mailbox(jpgenc_ctx* c, int word, unsigned long long* value) {
 
 void leave_batch_state(jpgenc_ctx* c) {
     c->nframes = 1;                                                  // the context goes back to single-image state
+    c->mixed.on = false;
     c->have_pixels = c->have_coef = c->have_scan = c->have_items = false; c->k2_tiles_done = 0;
     c->file_mode = false;
     c->host_hist.clear();
@@ -297,7 +302,7 @@ void jpgenc_destroy(jpgenc_ctx* c) {
     delete c->pool;
     if (c->owns_host_pool) delete c->host_pool;
     cudaFree(c->d_rgb_owned); cudaFree(c->d_coef); cudaFree(c->d_refine_list); cudaFree(c->d_counters);
-    cudaFree(c->d_stats); cudaFree(c->d_tables);   /* d_meta lives in the same allocation */ cudaFree(c->d_frame_ptrs); cudaFree(c->d_lookback); cudaFree(c->d_raw);
+    cudaFree(c->d_stats); cudaFree(c->d_tables);   /* d_meta lives in the same allocation */ cudaFree(c->d_frame_ptrs); cudaFree(c->d_geom); cudaFree(c->d_lookback); cudaFree(c->d_raw);
     cudaFree(c->d_scan); cudaFree(c->d_hdr_prefix); cudaFree(c->d_flush);
     cudaFree(c->d_tab_scratch); cudaFree(c->d_built_tables);
     cudaFree(c->d_items); cudaFree(c->d_tile_cnt); cudaFree(c->d_range_bits); cudaFree(c->d_range_base);

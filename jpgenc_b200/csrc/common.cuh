@@ -52,6 +52,37 @@ struct ColorConsts {                      // FP32 fast path; sample scale folded
     float y[3], cb[3], cr[3];
 };
 
+// ---- a pass of images of individual sizes (jpgenc_encode_images_packed), device resident -------------------------
+// One entry per image of the pass and one behind the last, whose prefix fields hold the pass totals: the images' work
+// units are numbered through the whole pass, and a CTA finds its image by a search over the prefix of its own unit.
+// All prefixes fit 32 bits: a pass has fewer than 2^31 coefficient blocks.
+struct FrameGeom {
+    const uint8_t* rgb;
+    uint32_t real_w, real_h, mcu_w, mcu_h;
+    uint32_t block0;                      // first coefficient block (blocks are numbered through the pass)
+    uint32_t strip0;                      // first K1 strip (a CTA: kMcus MCUs of one MCU row)
+    uint32_t tile0;                       // first K2 tile = item slab; its K3 ranges start at tile0 * split
+    uint32_t group0;                      // first K3 group (a CTA of K3a / K3b)
+    uint32_t super0;                      // first K3 super-group (256 groups)
+    uint32_t pad;
+};
+static_assert(sizeof(FrameGeom) == 48, "FrameGeom is copied as an array");
+
+// the image f (0 <= f < F) whose units [geom[f].*key, geom[f + 1].*key) contain unit x, found by a whole warp in two rounds of
+// 32 parallel probes for F <= 1024 (every lane must take part; every lane returns f)
+__device__ __forceinline__ uint32_t geom_find_warp(const FrameGeom* geom, uint32_t F, uint32_t x, uint32_t FrameGeom::*key) {
+    const uint32_t lane = threadIdx.x & 31;
+    uint32_t lo = 0, n = F;                                   // the answer lies in [lo, lo + n)
+    while (n > 1) {
+        const uint32_t step = (n + 31) / 32, i = lo + lane * step;
+        const unsigned le = __ballot_sync(0xffffffffu, i < lo + n && geom[i].*key <= x);   // lane 0 always holds
+        const uint32_t k = 31 - __clz(le);
+        lo += k * step;
+        n = min(step, n - k * step);
+    }
+    return lo;
+}
+
 struct ForwardParams {
     const uint8_t* rgb;                   // one image ...
     const uint8_t* const* frames;         // ... or (non-null) one device pointer per frame of a batch of equally sized frames
@@ -68,6 +99,20 @@ struct ForwardParams {
     QuantConsts2 luma;
     QuantConsts2 chroma;
     alignas(64) CUtensorMap coef_map;     // coefficient array as rows of 128 bytes, for the tensor store of full strips
+    // images of individual sizes (forward_mixed_kernel): geom[nframes + 1], `strips` CTAs in all; the fields above that
+    // describe one size (rgb, frames, blocks_per_frame, real_w .. mcu_y0) are unused there
+    const FrameGeom* geom;
+    uint32_t nframes;
+    uint32_t strips;
+};
+
+// host side: the totals of the pass of images of individual sizes bound to a context (the device reads them from the
+// entry behind the last image of FrameGeom)
+struct MixedPass {
+    bool on = false;
+    bool aligned = false;                 // every image has real_w % 16 == 0 and a 16-byte aligned pointer (K1's bulk copies)
+    uint32_t blocks = 0, strips = 0, tiles = 0, groups = 0, supers = 0;
+    uint32_t split = 1;                   // K3 ranges per K2 tile, one choice for the whole pass (launch_entropy)
 };
 
 __host__ __device__ inline uint64_t umin64(uint64_t a, uint64_t b) { return a < b ? a : b; }
@@ -178,6 +223,9 @@ struct jpgenc_ctx {
     const uint8_t** d_frame_ptrs = nullptr;   // [nframes] device pointers of the frames (batches only)
     size_t frame_ptrs_cap = 0;
     bool frames_aligned = false;          // every frame pointer is 16-byte aligned (bulk-copy path of K1)
+    jpgenc::MixedPass mixed;              // on: the frames bound are images of individual sizes, described by d_geom
+    jpgenc::FrameGeom* d_geom = nullptr;  // [nframes + 1]
+    size_t geom_cap = 0;
     const uint8_t* d_rgb = nullptr;       // bound or owned
     uint8_t* d_rgb_owned = nullptr;
     size_t rgb_cap = 0;
@@ -311,6 +359,8 @@ __host__ __device__ inline unsigned long long mail_tag(uint32_t seq) { return st
 __host__ __device__ inline unsigned long long mail_word(unsigned long long value, uint32_t seq) { return value | (mail_tag(seq) << kMailTagShift); }
 int launch_forward(jpgenc_ctx* c);
 int launch_forward_rows(jpgenc_ctx* c, uint32_t y0, uint32_t rows, bool first, bool last);
+// K1 + exact refinement over a pass of images of individual sizes (c->mixed, c->d_geom)
+int launch_forward_mixed(jpgenc_ctx* c);
 int launch_dct_quant_blocks(jpgenc_ctx* c, const float* in, int16_t* out, uint64_t nblocks, const uint8_t q[64],
                             uint64_t* refined);
 int launch_planes_to_mcu(jpgenc_ctx* c, const int32_t* d_qy, const int32_t* d_qcb, const int32_t* d_qcr);

@@ -193,6 +193,95 @@ __global__ void __launch_bounds__(kPackThreads) range_bits_kernel(const __grid_c
     }
 }
 
+// Images of individual sizes (geom[nframes + 1], numbered through the pass): a CTA of K3a / K3b finds its image by the
+// first-group prefix and works as a group of a batch of that one image -- the parameters are rebased onto the image's
+// tables, tiles, ranges, groups, super-groups and PassMeta entries, and carry its own counts (the split is the pass's).
+__device__ __forceinline__ EntropyParams entropy_image(const EntropyParams& p, const FrameGeom* __restrict__ geom, uint32_t* group_base) {
+    const uint32_t f = geom_find_warp(geom, p.nframes, blockIdx.x, &FrameGeom::group0);
+    const FrameGeom& g = geom[f];
+    EntropyParams q = p;
+    q.ranges_per_frame = (geom[f + 1].tile0 - g.tile0) * p.split;
+    q.groups_per_frame = geom[f + 1].group0 - g.group0;
+    q.supers_per_frame = geom[f + 1].super0 - g.super0;
+    q.tables = p.tables + f;
+    q.range_cnt = p.range_cnt + g.tile0;
+    q.items = p.items + static_cast<size_t>(g.tile0) * kSlabItems;
+    q.range_bits = p.range_bits + static_cast<size_t>(g.tile0) * p.split;
+    q.group_bits = p.group_bits + g.group0;
+    q.super_bits = p.super_bits + g.super0;
+    q.raw_off = p.raw_off + f;
+    q.total_bits = p.total_bits + f;
+    *group_base = g.group0;
+    return q;
+}
+
+// K3a over images of individual sizes.  The same code as range_bits_kernel on the parameters entropy_image rebased onto the
+// CTA's image; it is a copy rather than a shared function because moving range_bits_kernel's body into a device function
+// changes that kernel's machine code (register allocation and schedule), and the single-size path is to stay as it is.
+__global__ void __launch_bounds__(kPackThreads) range_bits_mixed_kernel(const __grid_constant__ EntropyParams pass, const FrameGeom* __restrict__ geom) {
+    uint32_t group0;
+    const EntropyParams p = entropy_image(pass, geom, &group0);
+    __shared__ uint32_t s_len[1024];                           // bits of a symbol with its magnitude: code length + category; 0 = absent
+    __shared__ uint32_t s_wbits[kPackWarps];
+    if (p.hdr->error) return;                                  // the pass was refused (finalize_tables_kernel): the host re-runs it
+    const uint32_t group = blockIdx.x - group0;             // within the image; p is rebased onto it
+    const DeviceTables* tables = p.tables;
+    for (int i = threadIdx.x; i < 1024; i += kPackThreads) {
+        const uint32_t e = (&tables->entry[0][0])[i];
+        s_len[i] = e ? (e >> 16) + (i & 15u) : 0u;
+    }
+    {   // housekeeping, spread over the grid
+        const unsigned long long gtid = static_cast<unsigned long long>(blockIdx.x) * kPackThreads + threadIdx.x;
+        const unsigned long long gsize = static_cast<unsigned long long>(gridDim.x) * kPackThreads;
+        const unsigned long long raw_words16 = p.hdr->raw_total / 16;
+        uint4* raw16 = reinterpret_cast<uint4*>(p.raw);
+        for (unsigned long long i = gtid; i < raw_words16; i += gsize) raw16[i] = make_uint4(0, 0, 0, 0);
+        if (gtid == 0) *p.redo_count = 0u;
+    }
+    __syncthreads();
+    const uint32_t range = group * kPackWarps + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    uint32_t bits = 0;
+    if (range < p.ranges_per_frame) {
+        uint32_t n;
+        const uint32_t* __restrict__ items = range_items(p, 0, range, &n);
+        auto size_of = [&](uint32_t item) {
+            uint32_t b = s_len[item & 0x3FFu];
+            const uint32_t nz = (item >> 10) & 3u;
+            if (nz) b += nz * (s_len[(item & 0x300u) | 0xF0u]);
+            return b;
+        };
+        uint32_t head = min(n, static_cast<uint32_t>((16u - (reinterpret_cast<uintptr_t>(items) & 15u)) & 15u) >> 2);
+        if (lane < head) bits += size_of(__ldg(items + lane));
+        const uint4* __restrict__ q4 = reinterpret_cast<const uint4*>(items + head);
+        const uint32_t nq = (n - head) >> 2;
+        uint32_t i = lane;
+        for (; i + 96 < nq; i += 128) {
+            const uint4 a = __ldg(q4 + i), b = __ldg(q4 + i + 32), c = __ldg(q4 + i + 64), d = __ldg(q4 + i + 96);
+            bits += size_of(a.x) + size_of(a.y) + size_of(a.z) + size_of(a.w);
+            bits += size_of(b.x) + size_of(b.y) + size_of(b.z) + size_of(b.w);
+            bits += size_of(c.x) + size_of(c.y) + size_of(c.z) + size_of(c.w);
+            bits += size_of(d.x) + size_of(d.y) + size_of(d.z) + size_of(d.w);
+        }
+        for (; i < nq; i += 32) {
+            const uint4 a = __ldg(q4 + i);
+            bits += size_of(a.x) + size_of(a.y) + size_of(a.z) + size_of(a.w);
+        }
+        const uint32_t tail0 = head + 4u * nq;
+        if (tail0 + lane < n) bits += size_of(__ldg(items + tail0 + lane));
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) bits += __shfl_xor_sync(0xffffffffu, bits, d);
+        if (lane == 0) p.range_bits[range] = bits;
+    }
+    if (lane == 0) s_wbits[threadIdx.x >> 5] = bits;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        unsigned long long sum = 0;
+        for (int w = 0; w < kPackWarps; ++w) sum += s_wbits[w];
+        p.group_bits[group] = sum;
+        atomicAdd(&p.super_bits[group >> 8], sum);
+    }
+}
+
 // ---- K3b: pack ---------------------------------------------------------------------------------------------------
 // One warp per range, no block-wide synchronisation.  The range is taken in chunks of 512 items: 16 coalesced row
 // loads put the chunk into a padded shared-memory array, from which every lane reads ITS 16 consecutive items
@@ -204,14 +293,18 @@ constexpr int kChunkRows = 16;
 constexpr int kChunkItems = kChunkRows * 32;
 constexpr int kWarpBitWords = 512;                      // 16 Kbit per chunk (32 bits per item on average) before falling back
 
-__global__ void __launch_bounds__(kPackThreads) huffman_pack_kernel(const __grid_constant__ EntropyParams p) {
+// The CTA works on group blockIdx.x - group_base in the numbering of p: 0 for frames of one size, the first group of its image
+// for images of individual sizes (entropy_image).  (The thread index comes from the kernel: there the compiler knows its range
+// from the launch bounds.)
+__device__ __forceinline__ void huffman_pack_body(const EntropyParams& p, uint32_t group_base, unsigned thread) {
+    const uint32_t block = blockIdx.x - group_base;
     __shared__ uint32_t s_tab[1024], s_fast[1024];                      // DeviceTables::entry / ::fast
     __shared__ uint32_t s_items[kPackWarps][kChunkItems + kChunkRows];  // item j of the chunk at j + (j >> 5)
     __shared__ uint32_t s_bits[kPackWarps][kWarpBitWords + 2];
     __shared__ unsigned long long s_part[kPackWarps];
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int tid = thread, lane = tid & 31, warp = tid >> 5;
     if (p.hdr->error) return;
-    const uint32_t frame = blockIdx.x / p.groups_per_frame, group = blockIdx.x - frame * p.groups_per_frame;
+    const uint32_t frame = block / p.groups_per_frame, group = block - frame * p.groups_per_frame;
     const DeviceTables* tables = p.tables + frame;
     for (int i = tid; i < 1024; i += kPackThreads) {
         s_tab[i] = (&tables->entry[0][0])[i];
@@ -363,6 +456,15 @@ __global__ void __launch_bounds__(kPackThreads) huffman_pack_kernel(const __grid
     }
 }
 
+__global__ void __launch_bounds__(kPackThreads) huffman_pack_kernel(const __grid_constant__ EntropyParams p) {
+    huffman_pack_body(p, 0, threadIdx.x);
+}
+__global__ void __launch_bounds__(kPackThreads) huffman_pack_mixed_kernel(const __grid_constant__ EntropyParams p, const FrameGeom* __restrict__ geom) {
+    uint32_t group0;
+    const EntropyParams q = entropy_image(p, geom, &group0);
+    huffman_pack_body(q, group0, threadIdx.x);
+}
+
 // ---- K4 ---------------------------------------------------------------------------------------------------
 // FF -> FF 00 (BitstreamGeneric.hpp:213-224).  A tile is 16 KB of the raw scan.  Every thread counts the FF bytes of its
 // 16 input bytes (SIMD byte compare), a CTA scan + look-back give the output position, the tile's output is assembled
@@ -374,9 +476,18 @@ constexpr int kStuffTile = kStuffThreads * kStuffBytesPerThread;
 static_assert(kStuffTile == kK4TileBytes, "capi.cu numbers K4 tiles with kK4TileBytes");
 
 // header of frame `frame`'s file at `dst`: the common prefix (SOI .. SOF0), the four DHT segments from the tables as the
-// device build left them, SOS (src/Image.cpp:933-954, JpegSegments.hpp:188-218; host twin: host/jfif_writer.cpp)
-__device__ __forceinline__ void write_file_header(uint8_t* dst, const EntropyParams& p, uint32_t frame, int tid, int nthreads) {
-    for (uint32_t i = tid; i < p.hdr_prefix_len; i += nthreads) dst[i] = p.hdr_prefix[i];
+// device build left them, SOS (src/Image.cpp:933-954, JpegSegments.hpp:188-218; host twin: host/jfif_writer.cpp).
+// geom (images of individual sizes): the prefix carries some image's size, the frame's own height and width replace it
+// (SOF0 is the prefix's last segment, 19 bytes: FF C0, length, precision, height at +5, width at +7)
+__device__ __forceinline__ void write_file_header(uint8_t* dst, const EntropyParams& p, uint32_t frame, int tid, int nthreads,
+                                                  const FrameGeom* geom = nullptr) {
+    if (geom) {
+        const uint32_t hw = (geom[frame].real_h << 16) | geom[frame].real_w, at = p.hdr_prefix_len - 14;
+        for (uint32_t i = tid; i < p.hdr_prefix_len; i += nthreads)
+            dst[i] = i - at < 4 ? static_cast<uint8_t>(hw >> (8 * (3 - (i - at)))) : p.hdr_prefix[i];
+    } else {
+        for (uint32_t i = tid; i < p.hdr_prefix_len; i += nthreads) dst[i] = p.hdr_prefix[i];
+    }
     uint32_t at = p.hdr_prefix_len;
     const jpgenc_huff_table* tabs = p.built + static_cast<size_t>(frame) * 4;
     for (int t = 0; t < 4; ++t) {
@@ -464,11 +575,12 @@ __global__ void __launch_bounds__(kCountThreads) ff_count_kernel(const __grid_co
     }
 }
 
-__global__ void __launch_bounds__(kStuffThreads, 6) stuff_kernel(const __grid_constant__ EntropyParams p, uint8_t* __restrict__ scan) {
+// geom: null for frames of one size (their SOF0 is the prefix's), else the geometry of images of individual sizes
+__device__ __forceinline__ void stuff_body(const EntropyParams& p, uint8_t* __restrict__ scan, const FrameGeom* geom, unsigned thread) {
     __shared__ alignas(16) uint8_t s_out[2 * kStuffTile + 16];
     __shared__ uint32_t s_scan[33];
     __shared__ unsigned long long s_before[kStuffThreads / 32];
-    const int tid = threadIdx.x;
+    const int tid = thread;
     if (p.hdr->error) return;
     // tiles are numbered frame by frame through the whole pass; the grid is an upper bound: surplus CTAs leave at once
     const uint32_t gtile = blockIdx.x;
@@ -551,7 +663,15 @@ __global__ void __launch_bounds__(kStuffThreads, 6) stuff_kernel(const __grid_co
         }
         if (tid < p.tail) g[len + tid] = tid ? 0xD9 : 0xFF;   // EOI (JpegSegments.hpp:361-377)
     }
-    if (tile == 0 && p.hdr_len[frame]) write_file_header(file + base, p, frame, tid, kStuffThreads);
+    if (tile == 0 && p.hdr_len[frame]) write_file_header(file + base, p, frame, tid, kStuffThreads, geom);
+}
+
+__global__ void __launch_bounds__(kStuffThreads, 6) stuff_kernel(const __grid_constant__ EntropyParams p, uint8_t* __restrict__ scan) {
+    stuff_body(p, scan, nullptr, threadIdx.x);
+}
+__global__ void __launch_bounds__(kStuffThreads, 6) stuff_mixed_kernel(const __grid_constant__ EntropyParams p, uint8_t* __restrict__ scan,
+                                                                       const FrameGeom* __restrict__ geom) {
+    stuff_body(p, scan, geom, threadIdx.x);
 }
 
 // Frame geometry (raw offsets, sizes, K4 tile numbering, output positions) is read from the PassMeta block in device
@@ -575,10 +695,19 @@ int launch_entropy(jpgenc_ctx* c, uint32_t k4_grid) {
     p.range_bits = c->d_range_bits;
     p.group_bits = c->d_range_base;                                  // [F * groups] then [F * supers]
     p.super_bits = c->d_range_base + static_cast<size_t>(F) * p.groups_per_frame;
+    size_t groups = static_cast<size_t>(F) * p.groups_per_frame, supers = static_cast<size_t>(F) * p.supers_per_frame;
+    if (c->mixed.on) {
+        // images of individual sizes: the pass's own counts (FrameGeom, host-built with the same split rule over the pass's
+        // tiles); the per-frame counts above are replaced per CTA (entropy_image)
+        p.split = c->mixed.split;
+        groups = c->mixed.groups;
+        supers = c->mixed.supers;
+        p.super_bits = c->d_range_base + groups;
+    }
     if (c->entropy_runs) {
         // K3a ADDS into the super-group sums, which launch_symbol_stats cleared: a second entropy pass over the same
         // symbol items (other tables) must start from zero again
-        JPGENC_CUDA(c, cudaMemsetAsync(p.super_bits, 0, static_cast<size_t>(F) * p.supers_per_frame * sizeof(unsigned long long), c->stream));
+        JPGENC_CUDA(c, cudaMemsetAsync(p.super_bits, 0, supers * sizeof(unsigned long long), c->stream));
     }
     ++c->entropy_runs;
     p.raw = c->d_raw;
@@ -604,15 +733,22 @@ int launch_entropy(jpgenc_ctx* c, uint32_t k4_grid) {
         p.hdr_prefix_len = c->hdr_prefix_len;
         p.tail = 2;
     }
-    const unsigned grid = p.groups_per_frame * F;
-    range_bits_kernel<<<grid, kPackThreads, 0, c->stream>>>(p);
-    JPGENC_CUDA(c, cudaGetLastError());
-    huffman_pack_kernel<<<grid, kPackThreads, 0, c->stream>>>(p);
+    const unsigned grid = static_cast<unsigned>(groups);
+    if (c->mixed.on) {
+        range_bits_mixed_kernel<<<grid, kPackThreads, 0, c->stream>>>(p, c->d_geom);
+        JPGENC_CUDA(c, cudaGetLastError());
+        huffman_pack_mixed_kernel<<<grid, kPackThreads, 0, c->stream>>>(p, c->d_geom);
+    } else {
+        range_bits_kernel<<<grid, kPackThreads, 0, c->stream>>>(p);
+        JPGENC_CUDA(c, cudaGetLastError());
+        huffman_pack_kernel<<<grid, kPackThreads, 0, c->stream>>>(p);
+    }
     JPGENC_CUDA(c, cudaGetLastError());
     if (k4_grid) {
         ff_count_kernel<<<k4_grid, kCountThreads, 0, c->stream>>>(p);
         JPGENC_CUDA(c, cudaGetLastError());
-        stuff_kernel<<<k4_grid, kStuffThreads, 0, c->stream>>>(p, c->d_scan);
+        if (c->mixed.on) stuff_mixed_kernel<<<k4_grid, kStuffThreads, 0, c->stream>>>(p, c->d_scan, c->d_geom);
+        else stuff_kernel<<<k4_grid, kStuffThreads, 0, c->stream>>>(p, c->d_scan);
         JPGENC_CUDA(c, cudaGetLastError());
         c->launches += 2;
     }

@@ -207,17 +207,37 @@ struct ForwardSmem {
 
 // kAligned: real_w % 16 == 0 and 16-byte aligned base -> rows are staged with bulk copies; otherwise a clamped
 // byte loader fills the tile (odd sizes; right-edge replication, src/Image.cpp:491-530)
-template <int kMcus, bool kAligned, bool kBulkOut = false>
-__global__ void __launch_bounds__(kMcus * 4, 640 / (kMcus * 4)) forward_kernel(const __grid_constant__ ForwardParams p) {
+// kMixed: images of individual sizes (p.geom): a 1-D grid over the strips of all images; a CTA finds its image by a search
+// over the first-strip prefix.  Otherwise one size: grid (strips of a row, rows, frames).
+template <int kMcus, bool kAligned, bool kBulkOut, bool kMixed>
+// (shared memory and the thread index come from the kernel: there the compiler knows the alignment and, from the launch
+// bounds, the range of threadIdx.x)
+__device__ __forceinline__ void forward_body(const ForwardParams& p, ForwardSmem<kMcus>& sm, unsigned thread) {
     using Smem = ForwardSmem<kMcus>;
-    __shared__ Smem sm;
     constexpr int kThreads = kMcus * 4;
-    const int tid = threadIdx.x;
-    const uint32_t my = p.mcu_y0 + blockIdx.y;
-    const uint32_t mcu0 = blockIdx.x * kMcus;
-    const int nm = min(kMcus, static_cast<int>(p.mcu_w - mcu0));
-    const uint8_t* __restrict__ rgb = p.frames ? p.frames[blockIdx.z] : p.rgb;      // batch: grid.z walks over the frames
-    const uint32_t frame_block0 = blockIdx.z * p.blocks_per_frame;
+    const int tid = thread;
+    uint32_t my, mcu0, frame_block0, real_w, real_h, mcu_w;
+    const uint8_t* __restrict__ rgb;
+    if constexpr (kMixed) {
+        const FrameGeom& g = p.geom[geom_find_warp(p.geom, p.nframes, blockIdx.x, &FrameGeom::strip0)];
+        mcu_w = g.mcu_w;
+        const uint32_t per_row = (mcu_w + kMcus - 1) / kMcus, s = blockIdx.x - g.strip0;
+        my = s / per_row;
+        mcu0 = (s - my * per_row) * kMcus;
+        rgb = g.rgb;
+        frame_block0 = g.block0;
+        real_w = g.real_w;
+        real_h = g.real_h;
+    } else {
+        my = p.mcu_y0 + blockIdx.y;
+        mcu0 = blockIdx.x * kMcus;
+        rgb = p.frames ? p.frames[blockIdx.z] : p.rgb;      // batch: grid.z walks over the frames
+        frame_block0 = blockIdx.z * p.blocks_per_frame;
+        real_w = p.real_w;
+        real_h = p.real_h;
+        mcu_w = p.mcu_w;
+    }
+    const int nm = min(kMcus, static_cast<int>(mcu_w - mcu0));
 
     // ---- stage the 16-row RGB strip ----
     if constexpr (kAligned) {
@@ -230,10 +250,20 @@ __global__ void __launch_bounds__(kMcus * 4, 640 / (kMcus * 4)) forward_kernel(c
             // 16 lanes issue one row each (a single thread issuing all 16 serialises ~0.3 us of TMA issue latency)
             const uint32_t row_bytes = nm * 48;
             if (tid == 0) ptx::mbar_expect_tx(&sm.bar, 16 * row_bytes);
-            const uint32_t sy = min(my * 16 + tid, p.real_h - 1);              // bottom edge replication
-            ptx::bulk_g2s(sm.tile + tid * Smem::kPitch, rgb + (static_cast<size_t>(sy) * p.real_w + mcu0 * 16) * 3, row_bytes, &sm.bar);
+            const uint32_t sy = min(my * 16 + tid, real_h - 1);                // bottom edge replication
+            ptx::bulk_g2s(sm.tile + tid * Smem::kPitch, rgb + (static_cast<size_t>(sy) * real_w + mcu0 * 16) * 3, row_bytes, &sm.bar);
         }
-        if (p.prefetch_ahead && tid >= 32 && tid < 48) {
+        if constexpr (kMixed) {
+            // the flat strip order runs across the images: warp 1 finds the image of the strip `prefetch_ahead` CTAs later
+            const uint32_t t = blockIdx.x + p.prefetch_ahead;
+            if (p.prefetch_ahead && t < p.strips && tid >= 32 && tid < 64) {
+                const FrameGeom& g = p.geom[geom_find_warp(p.geom, p.nframes, t, &FrameGeom::strip0)];
+                const uint32_t per_row = (g.mcu_w + kMcus - 1) / kMcus, s = t - g.strip0, pby = s / per_row;
+                const uint32_t pm0 = (s - pby * per_row) * kMcus, pnm = min(static_cast<uint32_t>(kMcus), g.mcu_w - pm0);
+                const uint32_t sy = min(pby * 16 + (tid - 32), g.real_h - 1);
+                if (tid < 48) ptx::bulk_prefetch_l2(g.rgb + (static_cast<size_t>(sy) * g.real_w + pm0 * 16) * 3, pnm * 48);
+            }
+        } else if (p.prefetch_ahead && tid >= 32 && tid < 48) {
             // the CTAs are dispatched in linear order (x, then y, then frame): by the time the CTA `prefetch_ahead`
             // positions later starts, its strip is in L2 and its bulk copies wait for L2 instead of DRAM
             const uint32_t per_frame = gridDim.x * gridDim.y;
@@ -252,9 +282,9 @@ __global__ void __launch_bounds__(kMcus * 4, 640 / (kMcus * 4)) forward_kernel(c
         const int row_bytes = nm * 48;
         for (int idx = tid; idx < 16 * row_bytes; idx += kThreads) {
             const int r = idx / row_bytes, b = idx - r * row_bytes;
-            const uint32_t sx = min(mcu0 * 16 + b / 3, p.real_w - 1);
-            const uint32_t sy = min(my * 16 + r, p.real_h - 1);
-            sm.tile[r * Smem::kPitch + b] = rgb[(static_cast<size_t>(sy) * p.real_w + sx) * 3 + (b % 3)];
+            const uint32_t sx = min(mcu0 * 16 + b / 3, real_w - 1);
+            const uint32_t sy = min(my * 16 + r, real_h - 1);
+            sm.tile[r * Smem::kPitch + b] = rgb[(static_cast<size_t>(sy) * real_w + sx) * 3 + (b % 3)];
         }
         __syncthreads();
     }
@@ -305,7 +335,7 @@ __global__ void __launch_bounds__(kMcus * 4, 640 / (kMcus * 4)) forward_kernel(c
     }
     __syncthreads();   // every RGB byte has been consumed (tile may now be reused as staging); chroma planes complete
 
-    const uint32_t mcu_base = my * p.mcu_w + mcu0;
+    const uint32_t mcu_base = my * mcu_w + mcu0;
     const uint32_t block_base = frame_block0 + mcu_base * kBlocksPerMcu;     // first coefficient block of this strip
     uint32_t packed[32];
     if (active) {
@@ -348,6 +378,18 @@ __global__ void __launch_bounds__(kMcus * 4, 640 / (kMcus * 4)) forward_kernel(c
     }
     __syncthreads();
     copy_out(sm.tile, p.coef + static_cast<size_t>(block_base) * kCoefPerBlock, nm * kBlocksPerMcu, tid, kThreads);
+}
+
+template <int kMcus, bool kAligned, bool kBulkOut = false>
+__global__ void __launch_bounds__(kMcus * 4, 640 / (kMcus * 4)) forward_kernel(const __grid_constant__ ForwardParams p) {
+    __shared__ ForwardSmem<kMcus> sm;
+    forward_body<kMcus, kAligned, kBulkOut, false>(p, sm, threadIdx.x);
+}
+
+template <int kMcus, bool kAligned, bool kBulkOut>
+__global__ void __launch_bounds__(kMcus * 4, 640 / (kMcus * 4)) forward_mixed_kernel(const __grid_constant__ ForwardParams p) {
+    __shared__ ForwardSmem<kMcus> sm;
+    forward_body<kMcus, kAligned, kBulkOut, true>(p, sm, threadIdx.x);
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -506,6 +548,29 @@ __global__ void __launch_bounds__(kRefineThreads) refine_kernel(const uint8_t* _
     auto sample = [&](const ExactColumn& col, int r) { return exact_sample(col, real_w, real_h, r, e.scale); };
     if constexpr (k64) refine_loop64(n0, n, list, all != 0, coef, blocks_per_frame, e.qy, e.qc, e, locate, sample);
     else refine_loop(n0, n, list, all != 0, coef, blocks_per_frame, e.qy, e.qc, e, locate, sample);
+}
+
+// images of individual sizes: block id -> image by a search over the first-block prefix (every image starts on an MCU, so
+// id % 6 still tells luma from chroma: blocks_per_frame = 2^32 - 1 leaves ids < 2^31 as they are)
+template <bool k64>
+__global__ void __launch_bounds__(kRefineThreads) refine_mixed_kernel(const FrameGeom* __restrict__ geom, uint32_t nframes,
+                                                                          int16_t* __restrict__ coef, const uint32_t* __restrict__ list,
+                                                                          const uint32_t* __restrict__ count, uint32_t cap,
+                                                                          const __grid_constant__ ExactConsts e) {
+    const uint32_t n = min(count[0], cap), n0 = count[3];
+    struct Column { ExactColumn col; uint32_t real_w, real_h; };
+    auto locate = [&](uint32_t id, int c) {
+        uint32_t lo = 0, hi = nframes;
+        while (hi - lo > 1) {
+            const uint32_t mid = (lo + hi) >> 1;
+            if (geom[mid].block0 <= id) lo = mid; else hi = mid;
+        }
+        const FrameGeom& g = geom[lo];
+        return Column{exact_locate(g.rgb, g.mcu_w, id - g.block0, c), g.real_w, g.real_h};
+    };
+    auto sample = [&](const Column& col, int r) { return exact_sample(col.col, col.real_w, col.real_h, r, e.scale); };
+    if constexpr (k64) refine_loop64(n0, n, list, false, coef, 0xFFFFFFFFu, e.qy, e.qc, e, locate, sample);
+    else refine_loop(n0, n, list, false, coef, 0xFFFFFFFFu, e.qy, e.qc, e, locate, sample);
 }
 
 // Images that are not 8-bit samples: three planes of doubles as the reference holds them (Image::R/G/B after loadPPM, or
@@ -813,6 +878,37 @@ int launch_forward_rows(jpgenc_ctx* c, uint32_t y0, uint32_t rows, bool first, b
     JPGENC_CUDA(c, cudaGetLastError());
     c->launches += 1;
     return last ? launch_refine(c, false) : JPGENC_OK;
+}
+
+// K1 + exact refinement over a pass of images of individual sizes.  The bulk copies need every image of the pass to qualify
+// (c->mixed.aligned); the tensor store serves the full strips of every image, the copy-out the partial ones.
+int launch_forward_mixed(jpgenc_ctx* c) {
+    ForwardParams p{};
+    fill_forward_params(c, &p);                                   // (its per-size fields are not read by forward_mixed_kernel)
+    p.geom = c->d_geom;
+    p.nframes = c->nframes;
+    p.strips = c->mixed.strips;
+    p.prefetch_ahead = 256;
+    JPGENC_CUDA(c, cudaMemsetAsync(c->d_counters, 0, 4 * sizeof(uint32_t), c->stream));
+    c->stats_clear_valid = false;                                 // K2 clears the statistics and K3a's sums itself
+    const bool aligned = c->mixed.aligned;
+    const bool bulk_out = aligned && make_block_map(c->d_coef, c->mixed.blocks, 32 * kBlocksPerMcu, &p.coef_map);
+    if (bulk_out) forward_mixed_kernel<32, true, true><<<c->mixed.strips, 128, 0, c->stream>>>(p);
+    else if (aligned) forward_mixed_kernel<32, true, false><<<c->mixed.strips, 128, 0, c->stream>>>(p);
+    else forward_mixed_kernel<32, false, false><<<c->mixed.strips, 128, 0, c->stream>>>(p);
+    JPGENC_CUDA(c, cudaGetLastError());
+    ExactConsts e;
+    fill_exact(c, c->qy, c->qc, 255. / c->maxval, &e);
+    const uint64_t total = c->mixed.blocks;                       // the same grid and thread layout rules as launch_refine
+    const unsigned grid = static_cast<unsigned>(std::max<uint64_t>(c->sm_count, std::min<uint64_t>(c->sm_count * 16, total / 256 + 1)));
+    const uint32_t cap = static_cast<uint32_t>(c->refine_cap);
+    if (total < (3u << 19))
+        refine_mixed_kernel<true><<<grid, kRefineThreads, 0, c->stream>>>(c->d_geom, c->nframes, c->d_coef, c->d_refine_list, c->d_counters, cap, e);
+    else
+        refine_mixed_kernel<false><<<grid, kRefineThreads, 0, c->stream>>>(c->d_geom, c->nframes, c->d_coef, c->d_refine_list, c->d_counters, cap, e);
+    JPGENC_CUDA(c, cudaGetLastError());
+    c->launches += 2;
+    return JPGENC_OK;
 }
 
 // exact pass over the list entries that have not been refined yet (after a band of K1), and remember how far it got

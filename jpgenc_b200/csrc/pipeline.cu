@@ -23,6 +23,7 @@
 #include <vector>
 
 #include "internal.hpp"
+#include "../host/ppm_reader.hpp"
 
 using namespace jpgenc;
 using namespace jpgenc::detail;
@@ -35,6 +36,11 @@ constexpr uint32_t kMaxHeaderBytes = 2 + 18 + 2 * 69 + 19 + 4 * (21 + 256) + 14;
 struct Job {
     uint32_t n = 0;
     uint32_t w = 0, h = 0, maxval = 255;
+    // images of individual sizes (jpgenc_encode_images_packed): image i is widths[i] x heights[i] (w x h: the first one's);
+    // null: every frame is w x h
+    const uint32_t* widths = nullptr;
+    const uint32_t* heights = nullptr;
+    double raw_per_block = 0;              // ... raw-scan bytes reserved per block: 1.5 x the most this call has seen (0: nothing yet)
     // output: per-frame buffers (legacy), one packed buffer, or none (sizes only)
     uint8_t* const* out_ptrs = nullptr;
     const uint64_t* caps = nullptr;
@@ -50,6 +56,22 @@ struct Pass {
     uint32_t k4_grid = 0;
     int attempts = 0;
 };
+
+uint32_t job_w(const Job& job, uint32_t i) { return job.widths ? job.widths[i] : job.w; }
+uint32_t job_h(const Job& job, uint32_t i) { return job.heights ? job.heights[i] : job.h; }
+uint64_t job_blocks(const Job& job, uint32_t i) {
+    return static_cast<uint64_t>((job_w(job, i) + 15) / 16) * ((job_h(job, i) + 15) / 16) * kBlocksPerMcu;
+}
+
+// passes of `per_pass` frames (the last one may be shorter)
+std::vector<Pass> uniform_passes(uint32_t n, uint32_t per_pass) {
+    std::vector<Pass> pass((n + per_pass - 1) / per_pass);
+    for (size_t p = 0; p < pass.size(); ++p) {
+        pass[p].f0 = static_cast<uint32_t>(p) * per_pass;
+        pass[p].F = std::min(per_pass, n - pass[p].f0);
+    }
+    return pass;
+}
 
 // the largest pass one slot can hold: item slabs (worst-case reservation, 96 KB per tile) within ~2 GB, block ids in 31 bits
 uint32_t frames_per_pass_cap(const jpgenc_ctx* c) {
@@ -71,6 +93,58 @@ uint32_t pass_frames(const jpgenc_ctx* c, uint32_t n, uint32_t slots) {
     uint32_t per = std::min(hi, std::max(lo, (n + 2 * slots - 1) / (2 * slots)));
     per = env_u32("JPGENC_FRAMES_PER_PASS", per);
     return std::max(1u, std::min({per, frames_per_pass_cap(c), n}));
+}
+
+// Images of individual sizes: the list is cut, in input order, into passes of the same pixel budget as pass_frames (MCU-padded
+// pixels; ~128..256 Mpx, about two passes per slot) under the limits of frames_per_pass_cap (item slabs within ~2 GB, block
+// ids in 31 bits, 1024 frames); JPGENC_FRAMES_PER_PASS bounds the images per pass.  An image that exceeds a limit alone
+// gets a pass of its own.
+std::vector<Pass> image_passes(const Job& job, uint32_t slots) {
+    constexpr uint64_t kMaxSlabTiles = (2ull << 30) / (384 * 64 * 4), kMaxBlocks = 0x7FFFFFFFull;
+    uint64_t total_px = 0;
+    for (uint32_t i = 0; i < job.n; ++i) total_px += job_blocks(job, i) / kBlocksPerMcu * 256;
+    const uint64_t target = std::min<uint64_t>(256ull << 20, std::max<uint64_t>(128ull << 20, (total_px + 2 * slots - 1) / (2 * slots)));
+    const uint32_t max_frames = std::max(1u, std::min(1024u, env_u32("JPGENC_FRAMES_PER_PASS", 1024)));
+    std::vector<Pass> pass;
+    uint64_t px = 0, tiles = 0, blocks = 0;
+    for (uint32_t i = 0; i < job.n; ++i) {
+        const uint64_t b = job_blocks(job, i), t = (b + 383) / 384, x = b / kBlocksPerMcu * 256;
+        if (pass.empty() || pass.back().F == max_frames || px + x > target || tiles + t > kMaxSlabTiles || blocks + b > kMaxBlocks) {
+            pass.emplace_back();
+            pass.back().f0 = i;
+            px = tiles = blocks = 0;
+        }
+        ++pass.back().F;
+        px += x; tiles += t; blocks += b;
+    }
+    return pass;
+}
+
+// The geometry of a pass of images of individual sizes (FrameGeom, F + 1 entries) and its totals.  K3's split follows
+// launch_entropy's rule, applied to the pass's tiles.
+MixedPass image_geometry(const Job& job, const Pass& ps, const void* const* ptrs, FrameGeom* g) {
+    MixedPass m;
+    m.on = true;
+    m.aligned = true;
+    uint64_t all_tiles = 0;
+    for (uint32_t f = 0; f < ps.F; ++f) all_tiles += (job_blocks(job, ps.f0 + f) + 383) / 384;
+    m.split = all_tiles < 4096 ? 4u : 1u;
+    for (uint32_t f = 0; f <= ps.F; ++f) {
+        g[f] = FrameGeom{};
+        g[f].block0 = m.blocks; g[f].strip0 = m.strips; g[f].tile0 = m.tiles; g[f].group0 = m.groups; g[f].super0 = m.supers;
+        if (f == ps.F) break;
+        const uint32_t w = job_w(job, ps.f0 + f), h = job_h(job, ps.f0 + f);
+        g[f].rgb = static_cast<const uint8_t*>(ptrs[f]);
+        g[f].real_w = w; g[f].real_h = h; g[f].mcu_w = (w + 15) / 16; g[f].mcu_h = (h + 15) / 16;
+        const uint32_t blocks = g[f].mcu_w * g[f].mcu_h * kBlocksPerMcu, tiles = (blocks + 383) / 384, groups = (tiles * m.split + 7) / 8;
+        m.blocks += blocks;
+        m.strips += (g[f].mcu_w + 31) / 32 * g[f].mcu_h;
+        m.tiles += tiles;
+        m.groups += groups;
+        m.supers += (groups + 255) / 256;
+        m.aligned = m.aligned && w % 16 == 0 && reinterpret_cast<uintptr_t>(ptrs[f]) % 16 == 0;
+    }
+    return m;
 }
 
 int prepare_slot(jpgenc_ctx* root, jpgenc_ctx* l, const Job& job, const uint8_t* prefix, uint32_t prefix_len) {
@@ -123,7 +197,8 @@ int enqueue_entropy(jpgenc_ctx* l, Pass& ps, cudaEvent_t prev_k4 = nullptr) {
 
 // the whole chain of one pass on slot `l`; `ready` (optional): event after which the pixels are valid
 // `after` (optional): the event after the previous pass's K1 (see run_passes)
-int enqueue_pass(jpgenc_ctx* root, jpgenc_ctx* l, Pass& ps, const void* const* dev_frames, cudaEvent_t ready, cudaEvent_t after, cudaEvent_t prev_k4) {
+int enqueue_pass(jpgenc_ctx* root, jpgenc_ctx* l, const Job& job, Pass& ps, const void* const* dev_frames, cudaEvent_t ready, cudaEvent_t after,
+                 cudaEvent_t prev_k4) {
     const uint32_t F = ps.F;
     int rc;
     l->nframes = F;
@@ -134,26 +209,37 @@ int enqueue_pass(jpgenc_ctx* root, jpgenc_ctx* l, Pass& ps, const void* const* d
     l->frames_aligned = aligned;
     l->d_rgb = static_cast<const uint8_t*>(dev_frames[0]);
     l->have_pixels = true;
+    std::vector<FrameGeom> geom;
+    if (job.widths) {
+        geom.resize(F + 1);
+        l->mixed = image_geometry(job, ps, dev_frames, geom.data());
+    }
     if ((rc = ensure_coef(l))) return rc;
     if ((rc = ensure_stats_buffers(l))) return rc;               // also sizes the pinned staging (stage_bytes(F))
-    {
+    if (job.widths) {
+        // the geometry (with the frame pointers) travels through pinned memory like the pointer array below
+        const size_t bytes = geom.size() * sizeof(FrameGeom);
+        if ((rc = ensure(l, &l->d_geom, &l->geom_cap, bytes))) return rc;
+        std::memcpy(l->h_pinned, geom.data(), bytes);
+        JPGENC_CUDA(l, cudaMemcpyAsync(l->d_geom, l->h_pinned, bytes, cudaMemcpyHostToDevice, l->stream));
+    } else {
         size_t cap = l->frame_ptrs_cap;
         void* p = l->d_frame_ptrs;
         if ((rc = ensure(l, reinterpret_cast<uint8_t**>(&p), &cap, F * sizeof(void*)))) return rc;
         l->d_frame_ptrs = static_cast<const uint8_t**>(p);
         l->frame_ptrs_cap = cap;
+        // the pointer array travels through pinned memory (the statistics' staging area is unused in this path), so that the
+        // copy is asynchronous and the caller's array need not outlive the call
+        std::memcpy(l->h_pinned, dev_frames, F * sizeof(void*));
+        JPGENC_CUDA(l, cudaMemcpyAsync(l->d_frame_ptrs, l->h_pinned, F * sizeof(void*), cudaMemcpyHostToDevice, l->stream));
     }
-    // the pointer array travels through pinned memory (the statistics' staging area is unused in this path), so that the
-    // copy is asynchronous and the caller's array need not outlive the call
-    std::memcpy(l->h_pinned, dev_frames, F * sizeof(void*));
-    JPGENC_CUDA(l, cudaMemcpyAsync(l->d_frame_ptrs, l->h_pinned, F * sizeof(void*), cudaMemcpyHostToDevice, l->stream));
     if (ready) JPGENC_CUDA(l, cudaStreamWaitEvent(l->stream, ready, 0));
     if (after) JPGENC_CUDA(l, cudaStreamWaitEvent(l->stream, after, 0));
-    if ((rc = launch_forward_rows(l, 0, l->mcu_h, true, true))) return rc;                       // K1 + exact refinement
+    if ((rc = job.widths ? launch_forward_mixed(l) : launch_forward_rows(l, 0, l->mcu_h, true, true))) return rc;   // K1 + exact refinement
     l->have_coef = true;
     JPGENC_CUDA(l, cudaEventRecord(l->ev_fwd, l->stream));
     const size_t nblocks = static_cast<size_t>(l->mcu_w) * l->mcu_h * kBlocksPerMcu, tiles = (nblocks + 383) / 384;
-    if ((rc = launch_symbol_stats(l, 0, static_cast<uint32_t>(tiles * F), true))) return rc;     // K2
+    if ((rc = launch_symbol_stats(l, 0, job.widths ? l->mixed.tiles : static_cast<uint32_t>(tiles * F), true))) return rc;     // K2
     l->have_items = true;
     const uint32_t nt = 4 * F;
     if ((rc = ensure(l, reinterpret_cast<uint8_t**>(&l->d_tab_scratch), &l->tab_scratch_cap, nt * table_scratch_bytes()))) return rc;
@@ -164,8 +250,15 @@ int enqueue_pass(jpgenc_ctx* root, jpgenc_ctx* l, Pass& ps, const void* const* d
     // (root->batch_raw_per_frame), before the first pass has finished a guess of 12 bytes per block; a pass that needs more
     // is refused by finalize_tables_kernel and its entropy stage re-run with what it asked for (finish_pass)
     // (JPGENC_RAW_GUESS_PER_BLOCK: tests set it to 0 so that every first pass is refused and re-run)
-    const uint64_t per_frame = root->batch_raw_per_frame ? root->batch_raw_per_frame : nblocks * env_u32("JPGENC_RAW_GUESS_PER_BLOCK", 12) + 4096;
-    l->raw_limit = F * raw_slot_bytes(per_frame);
+    // (images of individual sizes: the same per block -- 12 bytes, then 1.5 x the most bytes per block this call has seen)
+    if (job.widths) {
+        const double per_block = job.raw_per_block ? job.raw_per_block : env_u32("JPGENC_RAW_GUESS_PER_BLOCK", 12);
+        l->raw_limit = 0;
+        for (uint32_t f = 0; f < F; ++f) l->raw_limit += raw_slot_bytes(static_cast<uint64_t>((geom[f + 1].block0 - geom[f].block0) * per_block) + 4096);
+    } else {
+        const uint64_t per_frame = root->batch_raw_per_frame ? root->batch_raw_per_frame : nblocks * env_u32("JPGENC_RAW_GUESS_PER_BLOCK", 12) + 4096;
+        l->raw_limit = F * raw_slot_bytes(per_frame);
+    }
     l->out_limit = F * (kMaxHeaderBytes + 2ull) + 2 * l->raw_limit;
     ps.attempts = 0;
     return enqueue_entropy(l, ps, prev_k4);
@@ -194,15 +287,18 @@ int finish_pass(jpgenc_ctx* root, jpgenc_ctx* l, Pass& ps, Job& job) {
             continue;
         }
         uint64_t max_raw = 0;
+        double max_per_block = 0;
         for (uint32_t f = 0; f < F; ++f) {
             if (m.total_bits[f] != m.frame_bits[f]) {
                 l->error = "entropy coder wrote " + std::to_string(m.total_bits[f]) + " bits, statistics predicted " + std::to_string(m.frame_bits[f]);
                 return JPGENC_ERR_ARG;
             }
             max_raw = std::max<uint64_t>(max_raw, m.raw_bytes[f]);
+            if (job.widths) max_per_block = std::max(max_per_block, static_cast<double>(m.raw_bytes[f]) / job_blocks(job, ps.f0 + f));
         }
-        // later passes reserve 1.5 x the largest frame seen so far
-        root->batch_raw_per_frame = std::max<uint64_t>(root->batch_raw_per_frame, max_raw + max_raw / 2 + 4096);
+        // later passes reserve 1.5 x the largest frame (images of individual sizes: bytes per block) seen so far
+        if (job.widths) job.raw_per_block = std::max(job.raw_per_block, 1.5 * max_per_block);
+        else root->batch_raw_per_frame = std::max<uint64_t>(root->batch_raw_per_frame, max_raw + max_raw / 2 + 4096);
         const uint64_t total = hd.out_total + m.ff_incl[F - 1];
         // The files go home on the slot's OUTPUT stream (behind ev_done, i.e. behind K4), so that the slot's next pass can
         // start its K1/K2/table build meanwhile; only its K3/K4, which overwrite d_scan, wait for the copy (enqueue_entropy).
@@ -239,10 +335,11 @@ int finish_pass(jpgenc_ctx* root, jpgenc_ctx* l, Pass& ps, Job& job) {
 // Runs the passes over the slots.  frames_of(p, slot context) -> device pointers of pass p's frames and the event after
 // which they are valid; done_with(p) is called when pass p's pixels are no longer needed.
 template <class FramesOf, class DoneWith>
-int run_passes(jpgenc_ctx* c, Job& job, uint32_t per_pass, uint32_t nslots, FramesOf&& frames_of, DoneWith&& done_with) {
-    const uint32_t npasses = (job.n + per_pass - 1) / per_pass;
+int run_passes(jpgenc_ctx* c, Job& job, std::vector<Pass>& pass, uint32_t nslots, FramesOf&& frames_of, DoneWith&& done_with) {
+    const uint32_t npasses = static_cast<uint32_t>(pass.size());
     // SOI .. SOF0 are the same bytes for every frame of the batch: jpgenc_write_headers with empty tables gives
-    // prefix + 4 x (DHT with no symbol: 21 bytes) + SOS (14 bytes)
+    // prefix + 4 x (DHT with no symbol: 21 bytes) + SOS (14 bytes).  (Images of individual sizes: the first image's size
+    // stands in SOF0; K4 writes every image's own.)
     uint8_t hdr[512];
     jpgenc_huff_table empty[4];
     std::memset(empty, 0, sizeof empty);
@@ -259,7 +356,6 @@ int run_passes(jpgenc_ctx* c, Job& job, uint32_t per_pass, uint32_t nslots, Fram
         slot[k] = k ? c->lanes[k - 1] : c;
         if ((rc = prepare_slot(c, slot[k], job, hdr, prefix_len))) return k ? fail(c, rc, jpgenc_last_error(slot[k])) : rc;
     }
-    std::vector<Pass> pass(npasses);
     // The streams run side by side, except in a call of exactly two passes: there nothing else will ever run beside the table
     // builds, and letting pass 1's K1 start when pass 0's K1 is through puts pass 0's table build beside pass 1's wide kernels
     // (timeline, 128 frames: 1.057 -> 1.014 ms).  Staggering more passes does not pay: 256 and 1024 frames are 2-4 % slower
@@ -278,8 +374,6 @@ int run_passes(jpgenc_ctx* c, Job& job, uint32_t per_pass, uint32_t nslots, Fram
         }
         if (p < npasses) {
             jpgenc_ctx* l = slot[p % nslots];
-            pass[p].f0 = p * per_pass;
-            pass[p].F = std::min(per_pass, job.n - pass[p].f0);
             const void* const* ptrs = nullptr;
             cudaEvent_t ready = nullptr;
             rc = frames_of(p, l, &ptrs, &ready);
@@ -291,7 +385,7 @@ int run_passes(jpgenc_ctx* c, Job& job, uint32_t per_pass, uint32_t nslots, Fram
             // 1024 frames, in order / not: files returned 6.61 / 7.00 ms, sizes only 6.30 / 6.20 ms)
             const bool in_order = job.packed != nullptr || job.out_ptrs != nullptr;
             cudaEvent_t prev_k4 = (in_order && p > 0 && nslots > 1) ? slot[(p - 1) % nslots]->ev_k4 : nullptr;
-            if (rc == JPGENC_OK) rc = enqueue_pass(c, l, pass[p], ptrs, ready, after, prev_k4);
+            if (rc == JPGENC_OK) rc = enqueue_pass(c, l, job, pass[p], ptrs, ready, after, prev_k4);
             if (rc) { failed = l; break; }
         }
     }
@@ -312,10 +406,15 @@ int run_passes(jpgenc_ctx* c, Job& job, uint32_t per_pass, uint32_t nslots, Fram
     return rc;
 }
 
-uint32_t slots_for(uint32_t n, uint32_t per_pass) {
-    const uint32_t npasses = (n + per_pass - 1) / per_pass;
+uint32_t slots_for(size_t npasses) {
     uint32_t s = env_u32("JPGENC_SLOTS", kDefaultSlots);
-    return std::max(1u, std::min({s, kMaxSlots, npasses}));
+    return std::max(1u, static_cast<uint32_t>(std::min<size_t>({s, kMaxSlots, npasses})));
+}
+
+// the passes of a call: equal frames in passes of pass_frames() frames, images of individual sizes by image_passes()
+std::vector<Pass> plan_passes(const jpgenc_ctx* c, const Job& job) {
+    const uint32_t nslots0 = std::max(1u, std::min(kMaxSlots, env_u32("JPGENC_SLOTS", kDefaultSlots)));
+    return job.widths ? image_passes(job, nslots0) : uniform_passes(job.n, pass_frames(c, job.n, nslots0));
 }
 
 int check_job(jpgenc_ctx* c, const Job& job, const void* frames) {
@@ -333,13 +432,12 @@ int encode_device_frames(jpgenc_ctx* c, Job& job, const void* const* dev_frames)
     if (rc) return rc;
     // what earlier calls learnt about the size of such frames' scans stays valid (a later frame that needs more is refused on the
     // device and re-run, finish_pass); a new frame size starts from the guess again
-    if (c->batch_geom_w != job.w || c->batch_geom_h != job.h) { c->batch_raw_per_frame = 0; c->batch_geom_w = job.w; c->batch_geom_h = job.h; }
-    const uint32_t nslots0 = std::min(kMaxSlots, env_u32("JPGENC_SLOTS", kDefaultSlots));
-    const uint32_t per_pass = pass_frames(c, job.n, std::max(1u, nslots0));
-    const uint32_t nslots = slots_for(job.n, per_pass);
-    return run_passes(c, job, per_pass, nslots,
+    if (!job.widths && (c->batch_geom_w != job.w || c->batch_geom_h != job.h)) { c->batch_raw_per_frame = 0; c->batch_geom_w = job.w; c->batch_geom_h = job.h; }
+    std::vector<Pass> pass = plan_passes(c, job);
+    const uint32_t nslots = slots_for(pass.size());
+    return run_passes(c, job, pass, nslots,
                       [&](uint32_t p, jpgenc_ctx*, const void* const** ptrs, cudaEvent_t* ready) {
-                          *ptrs = dev_frames + static_cast<size_t>(p) * per_pass;
+                          *ptrs = dev_frames + pass[p].f0;
                           *ready = nullptr;
                           return JPGENC_OK;
                       },
@@ -348,7 +446,8 @@ int encode_device_frames(jpgenc_ctx* c, Job& job, const void* const* dev_frames)
 
 // Frames in host memory (pinned for full PCIe speed): they travel on the copy stream into a ring of pass-sized slices
 // of device memory, always a few passes ahead of the kernels; when pass p is finished its slice is re-filled with the
-// frames of pass p + ring.
+// frames of pass p + ring.  A slice holds the bytes of the largest pass (passes of images of individual sizes differ);
+// every frame starts on 256 bytes.
 int encode_host_frames(jpgenc_ctx* c, Job& job, const uint8_t* const* frames) {
     // an empty batch is legal and touches nothing: an image bound to the context keeps its geometry
     if (job.n == 0) return (job.w && job.h && job.maxval && job.maxval <= 255) ? JPGENC_OK : fail(c, JPGENC_ERR_ARG, "width/height/maxval out of range");
@@ -357,24 +456,32 @@ int encode_host_frames(jpgenc_ctx* c, Job& job, const uint8_t* const* frames) {
     if (rc) return rc;
     // what earlier calls learnt about the size of such frames' scans stays valid (a later frame that needs more is refused on the
     // device and re-run, finish_pass); a new frame size starts from the guess again
-    if (c->batch_geom_w != job.w || c->batch_geom_h != job.h) { c->batch_raw_per_frame = 0; c->batch_geom_w = job.w; c->batch_geom_h = job.h; }
-    const uint32_t nslots0 = std::min(kMaxSlots, env_u32("JPGENC_SLOTS", kDefaultSlots));
-    const uint32_t per_pass = pass_frames(c, job.n, std::max(1u, nslots0));
-    const uint32_t nslots = slots_for(job.n, per_pass);
-    const uint32_t npasses = (job.n + per_pass - 1) / per_pass;
+    if (!job.widths && (c->batch_geom_w != job.w || c->batch_geom_h != job.h)) { c->batch_raw_per_frame = 0; c->batch_geom_w = job.w; c->batch_geom_h = job.h; }
+    std::vector<Pass> pass = plan_passes(c, job);
+    const uint32_t nslots = slots_for(pass.size());
+    const uint32_t npasses = static_cast<uint32_t>(pass.size());
     constexpr uint32_t kRingMax = sizeof(c->ev_band) / sizeof(c->ev_band[0]);
     const uint32_t ring = std::min({nslots + 2, npasses, kRingMax});
-    const size_t fbytes = static_cast<size_t>(job.w) * job.h * 3, fstride = (fbytes + 255) & ~static_cast<size_t>(255);
-    if ((rc = ensure(c, &c->d_rgb_owned, &c->rgb_cap, static_cast<size_t>(ring) * per_pass * fstride + 16))) return rc;
+    auto fbytes = [&](uint32_t i) { return static_cast<size_t>(job_w(job, i)) * job_h(job, i) * 3; };
+    auto fstride = [&](uint32_t i) { return (fbytes(i) + 255) & ~static_cast<size_t>(255); };
+    // frame f of pass p sits at slice (p % ring) + at[f0 + f]
+    std::vector<size_t> at(job.n);
+    size_t slice = 0;
+    for (const Pass& ps : pass) {
+        size_t o = 0;
+        for (uint32_t f = 0; f < ps.F; ++f) { at[ps.f0 + f] = o; o += fstride(ps.f0 + f); }
+        slice = std::max(slice, o);
+    }
+    if ((rc = ensure(c, &c->d_rgb_owned, &c->rgb_cap, static_cast<size_t>(ring) * slice + 16))) return rc;
     auto upload = [&](uint32_t p) -> int {
-        const uint32_t f0 = p * per_pass, F = std::min(per_pass, job.n - f0), s = p % ring;
-        // frames that follow each other in host memory (a video buffer) travel as one strided copy
+        const uint32_t f0 = pass[p].f0, F = pass[p].F, s = p % ring;
+        // equal frames that follow each other in host memory (a video buffer) travel as one strided copy
         for (uint32_t f = 0; f < F;) {
             uint32_t run = 1;
-            while (f + run < F && frames[f0 + f + run] == frames[f0 + f + run - 1] + fbytes) ++run;
-            uint8_t* dst = c->d_rgb_owned + (static_cast<size_t>(s) * per_pass + f) * fstride;
-            if (run == 1) JPGENC_CUDA(c, cudaMemcpyAsync(dst, frames[f0 + f], fbytes, cudaMemcpyHostToDevice, c->copy_stream));
-            else JPGENC_CUDA(c, cudaMemcpy2DAsync(dst, fstride, frames[f0 + f], fbytes, fbytes, run, cudaMemcpyHostToDevice, c->copy_stream));
+            while (!job.widths && f + run < F && frames[f0 + f + run] == frames[f0 + f + run - 1] + fbytes(0)) ++run;
+            uint8_t* dst = c->d_rgb_owned + static_cast<size_t>(s) * slice + at[f0 + f];
+            if (run == 1) JPGENC_CUDA(c, cudaMemcpyAsync(dst, frames[f0 + f], fbytes(f0 + f), cudaMemcpyHostToDevice, c->copy_stream));
+            else JPGENC_CUDA(c, cudaMemcpy2DAsync(dst, fstride(0), frames[f0 + f], fbytes(0), fbytes(0), run, cudaMemcpyHostToDevice, c->copy_stream));
             f += run;
         }
         JPGENC_CUDA(c, cudaEventRecord(c->ev_band[s], c->copy_stream));
@@ -384,12 +491,12 @@ int encode_host_frames(jpgenc_ctx* c, Job& job, const uint8_t* const* frames) {
         if ((rc = upload(p))) return rc;
     std::vector<std::vector<const void*>> ptrs(nslots);
     int upload_rc = JPGENC_OK;
-    rc = run_passes(c, job, per_pass, nslots,
+    rc = run_passes(c, job, pass, nslots,
                     [&](uint32_t p, jpgenc_ctx*, const void* const** out, cudaEvent_t* ready) {
-                        const uint32_t f0 = p * per_pass, F = std::min(per_pass, job.n - f0), s = p % ring;
+                        const uint32_t f0 = pass[p].f0, F = pass[p].F, s = p % ring;
                         std::vector<const void*>& v = ptrs[p % nslots];
                         v.resize(F);
-                        for (uint32_t f = 0; f < F; ++f) v[f] = c->d_rgb_owned + (static_cast<size_t>(s) * per_pass + f) * fstride;
+                        for (uint32_t f = 0; f < F; ++f) v[f] = c->d_rgb_owned + static_cast<size_t>(s) * slice + at[f0 + f];
                         *out = v.data();
                         *ready = c->ev_band[s];
                         return JPGENC_OK;
@@ -436,6 +543,33 @@ int jpgenc_encode_frames_packed(jpgenc_ctx* c, uint32_t n, const void* const* fr
     int rc = check_job(c, job, frames);
     if (rc) return rc;
     rc = frames_on_device ? encode_device_frames(c, job, frames) : encode_host_frames(c, job, reinterpret_cast<const uint8_t* const*>(frames));
+    if (total_bytes) *total_bytes = job.packed_at;
+    return rc;
+} JPGENC_CATCH(c)
+
+int jpgenc_encode_images_packed(jpgenc_ctx* c, uint32_t n, const void* const* images, int images_on_device, const uint32_t* widths,
+                                const uint32_t* heights, uint32_t maxval, uint8_t* out, uint64_t cap, uint64_t* offsets, uint64_t* sizes,
+                                uint64_t* total_bytes) try {
+    if (!c) return JPGENC_ERR_ARG;
+    if (total_bytes) *total_bytes = 0;
+    if (maxval == 0 || maxval > 255) return fail(c, JPGENC_ERR_ARG, "maxval out of range");
+    if (n == 0) return JPGENC_OK;                                // an empty batch is legal and touches nothing
+    if (!images || !widths || !heights || !offsets || !sizes) return fail(c, JPGENC_ERR_ARG, "null argument");
+    bool same = true;
+    for (uint32_t i = 0; i < n; ++i) {
+        if (!images[i]) return fail(c, JPGENC_ERR_ARG, "null image pointer");
+        if (widths[i] == 0 || heights[i] == 0 || widths[i] > 65535 || heights[i] > 65535) return fail(c, JPGENC_ERR_ARG, "image side out of range (1..65535)");
+        same = same && widths[i] == widths[0] && heights[i] == heights[0];
+    }
+    if (!images_on_device && maxval < 255)
+        for (uint32_t i = 0; i < n; ++i)
+            if (!samples_within_maxval(static_cast<const uint8_t*>(images[i]), static_cast<size_t>(widths[i]) * heights[i] * 3, maxval))
+                return fail(c, JPGENC_ERR_FORMAT, "a sample exceeds maxval");
+    Job job;
+    job.n = n; job.w = widths[0]; job.h = heights[0]; job.maxval = maxval;
+    if (!same) { job.widths = widths; job.heights = heights; }   // one size: the batched-frame path as it is
+    job.packed_mode = true; job.packed = out; job.packed_cap = cap; job.offsets = offsets; job.sizes = sizes;
+    const int rc = images_on_device ? encode_device_frames(c, job, images) : encode_host_frames(c, job, reinterpret_cast<const uint8_t* const*>(images));
     if (total_bytes) *total_bytes = job.packed_at;
     return rc;
 } JPGENC_CATCH(c)

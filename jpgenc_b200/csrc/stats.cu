@@ -70,7 +70,8 @@ constexpr int kStatsSmem = kTileSmemBytes                // masks + dc
                            + 4096 + 4096                 // histogram, local first-occurrence keys
                            + 36 * 4;                     // scan scratch
 
-__global__ void __launch_bounds__(kTileBlocks, 5) symbol_stats_kernel(const __grid_constant__ StatsParams p) {
+// (the thread index comes from the kernel: there the compiler knows its range from the launch bounds)
+__device__ __forceinline__ void symbol_stats_body(const StatsParams& p, unsigned thread) {
     extern __shared__ __align__(128) uint8_t smem[];
     const TileView tv = tile_view(smem);
     uint8_t* at = smem + kTileSmemBytes;
@@ -82,7 +83,7 @@ __global__ void __launch_bounds__(kTileBlocks, 5) symbol_stats_kernel(const __gr
     uint32_t* s_scan = reinterpret_cast<uint32_t*>(at);
     __shared__ uint32_t s_origin[2];                                      // MCU column / row of the tile's first MCU
 
-    const int tid = threadIdx.x, lane = tid & 31;
+    const int tid = thread, lane = tid & 31;
     const uint32_t gtile = p.tile0 + blockIdx.x;
     const uint32_t frame = p.tiles_total == p.tiles_per_frame ? 0u : gtile / p.tiles_per_frame;   // one image: no division
     const uint32_t first = (gtile - frame * p.tiles_per_frame) * kTileBlocks;           // first block of the tile, within its frame
@@ -238,6 +239,32 @@ __global__ void __launch_bounds__(kTileBlocks, 5) symbol_stats_kernel(const __gr
     }
 }
 
+__global__ void __launch_bounds__(kTileBlocks, 5) symbol_stats_kernel(const __grid_constant__ StatsParams p) {
+    symbol_stats_body(p, threadIdx.x);
+}
+
+// Images of individual sizes (geom[nframes + 1]): a tile finds its image by the first-tile prefix and runs as a tile of a
+// batch of that one image -- the parameters are rebased onto the image's coefficients, statistics, item slabs and tile
+// counts, and carry its own block count and MCU geometry.  (K1's refinement counter is then copied by the last tile of
+// every image: the same value each time.)
+__global__ void __launch_bounds__(kTileBlocks, 5) symbol_stats_mixed_kernel(const __grid_constant__ StatsParams p, const FrameGeom* __restrict__ geom,
+                                                                            uint32_t nframes) {
+    const uint32_t gtile = p.tile0 + blockIdx.x;
+    const uint32_t f = geom_find_warp(geom, nframes, gtile, &FrameGeom::tile0);
+    const FrameGeom& g = geom[f];
+    StatsParams q = p;
+    q.coef = p.coef + static_cast<size_t>(g.block0) * kCoefPerBlock;
+    q.nblocks = g.mcu_w * g.mcu_h * kBlocksPerMcu;
+    q.tiles_per_frame = q.tiles_total = geom[f + 1].tile0 - g.tile0;
+    q.tile0 = p.tile0 - g.tile0;                                        // tile0 + blockIdx.x = the tile within the image
+    q.mcu_w = g.mcu_w;
+    q.n_mcu = g.mcu_w * g.mcu_h;
+    q.g_stats = p.g_stats + static_cast<size_t>(f) * kStatsBytes;
+    q.items = p.items + static_cast<size_t>(g.tile0) * kSlabItems;
+    q.tile_cnt = p.tile_cnt + g.tile0;
+    symbol_stats_body(q, threadIdx.x);
+}
+
 // One image: hand the statistics to the host through its mailbox (mapped pinned memory).  A kernel of its own, in stream
 // order behind K2: making the last CTA of K2 do this needs a __threadfence per CTA behind its histogram atomics, which cost
 // K2 24 us at 16384 tiles.  Only the symbols that occur travel (a few dozen of 1024), each as two self-validating 64-bit
@@ -327,9 +354,14 @@ int launch_symbol_stats(jpgenc_ctx* c, uint32_t tile0, uint32_t ntiles, bool fir
     p.refine_copy = reinterpret_cast<uint32_t*>(c->d_stats + c->nframes * kStatsBytes);
     if (!c->k2_configured) {                                   // (the first encode of a context is never graph-captured)
         JPGENC_CUDA(c, cudaFuncSetAttribute(symbol_stats_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kStatsSmem));
+        JPGENC_CUDA(c, cudaFuncSetAttribute(symbol_stats_mixed_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kStatsSmem));
         c->k2_configured = true;
     }
-    symbol_stats_kernel<<<ntiles, kTileBlocks, kStatsSmem, c->stream>>>(p);
+    if (c->mixed.on) {                                         // images of individual sizes: the per-size fields above are replaced per tile
+        symbol_stats_mixed_kernel<<<ntiles, kTileBlocks, kStatsSmem, c->stream>>>(p, c->d_geom, c->nframes);
+    } else {
+        symbol_stats_kernel<<<ntiles, kTileBlocks, kStatsSmem, c->stream>>>(p);
+    }
     JPGENC_CUDA(c, cudaGetLastError());
     c->launches += 1;
     return JPGENC_OK;
