@@ -38,6 +38,14 @@ extern "C" {
 #define JPGENC_ERR_CAPACITY  -6   /* caller's output buffer too small */
 #define JPGENC_ERR_NOMEM     -7   /* host memory exhausted (a C++ exception was caught at the boundary; text in jpgenc_last_error) */
 
+/* Pixel formats of the *_image calls.  A 4th byte is never read into the image and takes no part in the maxval check.
+ * Together with a row pitch (bytes from one row to the next; 0 = width * bytes per pixel, never less than that) they describe
+ * the pixels only: the file is the one the reference writes for the same R,G,B samples. */
+#define JPGENC_PIXEL_RGB      0   /* 3 bytes per pixel: R,G,B */
+#define JPGENC_PIXEL_BGR      1   /* 3 bytes per pixel: B,G,R */
+#define JPGENC_PIXEL_RGBA     2   /* 4 bytes per pixel: R,G,B, then a byte that is ignored */
+#define JPGENC_PIXEL_BGRA     3   /* 4 bytes per pixel: B,G,R, then a byte that is ignored */
+
 typedef struct jpgenc_ctx jpgenc_ctx;
 
 /* Table ids everywhere: 0 = Y_DC, 1 = Y_AC, 2 = C_DC, 3 = C_AC (src/Image.cpp:908-912, 946-949). */
@@ -100,6 +108,11 @@ int jpgenc_set_dct_constants(jpgenc_ctx* ctx, const double a[5], const double s[
 int jpgenc_upload_rgb(jpgenc_ctx* ctx, const uint8_t* host_rgb, uint32_t real_w, uint32_t real_h, uint32_t maxval);
 /* same, for pixels that already live in device memory (no copy is made; the pointer must stay valid) */
 int jpgenc_bind_device_rgb(jpgenc_ctx* ctx, const void* dev_rgb, uint32_t real_w, uint32_t real_h, uint32_t maxval);
+/* same, for device pixels in any JPGENC_PIXEL_* format with a row pitch (0 = tight); crops of a larger image and pitched
+ * allocations are read where they are.  Then jpgenc_color_dct_quant / jpgenc_encode_bound as after jpgenc_bind_device_rgb.
+ * Unknown format, pitch below the row size, sides outside 1..65535: JPGENC_ERR_ARG. */
+int jpgenc_bind_device_image(jpgenc_ctx* ctx, const void* dev, uint32_t real_w, uint32_t real_h, uint32_t row_pitch, int format,
+                             uint32_t maxval);
 
 /* ---- K1: convertToColorSpace(YCbCr) + applySubsampling(S420_m) + applyDCT(Arai) + applyQuantization
  *      + zigzag (src/Image.cpp:112-148, 198-235, 540-595, 597-636; Dct.hpp:47-215; Coding.hpp:57-97) -- */
@@ -156,6 +169,11 @@ int jpgenc_assemble_last(jpgenc_ctx* ctx, uint8_t* dst, uint64_t cap, uint64_t* 
 /* upload + encode (host pixels in, JPEG bytes out) */
 int jpgenc_encode_rgb(jpgenc_ctx* ctx, const uint8_t* host_rgb, uint32_t real_w, uint32_t real_h, uint32_t maxval,
                       uint8_t* dst, uint64_t cap, uint64_t* jpeg_bytes);
+/* the same for host pixels in any JPGENC_PIXEL_* format with a row pitch (0 = tight).  The rows travel as they are, in their
+ * own format, the pitch gap dropped by the copy engine, and the device reads that format: no host core repacks them, and
+ * 4-byte pixels cost 4/3 of the PCIe bytes of RGB.  Checked against maxval when it is below 255 (colour bytes only). */
+int jpgenc_encode_image(jpgenc_ctx* ctx, const void* host, uint32_t real_w, uint32_t real_h, uint32_t row_pitch, int format,
+                        uint32_t maxval, uint8_t* dst, uint64_t cap, uint64_t* jpeg_bytes);
 /* Image::writeJPEG (src/Image.cpp:831-976) for an image given as the reference holds it: three row-major planes of doubles
  * (Image::R/G/B, include/Image.hpp:104-114), `width` x `height` = the image padded to whole 16x16 MCUs (src/Image.cpp:479-530),
  * real_w x real_h = what SOF0 reports.  ycbcr != 0: the planes already are level-shifted Y, Cb, Cr and are not converted
@@ -215,6 +233,14 @@ int jpgenc_encode_frames_packed(jpgenc_ctx* ctx, uint32_t n, const void* const* 
 int jpgenc_encode_images_packed(jpgenc_ctx* ctx, uint32_t n, const void* const* images, int images_on_device, const uint32_t* widths,
                                 const uint32_t* heights, uint32_t maxval, uint8_t* out, uint64_t cap, uint64_t* offsets,
                                 uint64_t* sizes, uint64_t* total_bytes);
+/* jpgenc_encode_images_packed for pixels in one JPGENC_PIXEL_* format per call and a row pitch per image (row_pitches may be
+ * NULL: all tight; an entry of 0 is tight too).  Tiles of one large image are pointers into it with its pitch.  Host images
+ * are uploaded in their own format as in jpgenc_encode_image.  Tight RGB is jpgenc_encode_images_packed itself; every other
+ * call runs the pass pipeline of images of individual sizes, equal sizes included. */
+int jpgenc_encode_images_packed_layout(jpgenc_ctx* ctx, uint32_t n, const void* const* images, int images_on_device,
+                                       const uint32_t* widths, const uint32_t* heights, const uint32_t* row_pitches, int format,
+                                       uint32_t maxval, uint8_t* out, uint64_t cap, uint64_t* offsets, uint64_t* sizes,
+                                       uint64_t* total_bytes);
 
 /* ---- stage methods for the modes writeJPEG does not use (SURVEY.md 8(f)4) ------------------------------------------ */
 /* Image::applySubsampling(mode) on one chroma plane (src/Image.cpp:198-319): `plane` = height x width doubles (host), mode =

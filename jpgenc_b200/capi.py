@@ -16,6 +16,9 @@ LIB_PATH = Path(__file__).resolve().parent / "lib" / "libjpgenc_b200.so"
 OK = 0
 ERR_CUDA, ERR_ARG, ERR_NO_DEVICE, ERR_FORMAT, ERR_IO, ERR_CAPACITY, ERR_NOMEM = -1, -2, -3, -4, -5, -6, -7
 
+# JPGENC_PIXEL_*: name -> (code, bytes per pixel)
+PIXEL_FORMATS = {"RGB": (0, 3), "BGR": (1, 3), "RGBA": (2, 4), "BGRA": (3, 4)}
+
 u8p = C.POINTER(C.c_uint8)
 i16p = C.POINTER(C.c_int16)
 i32p = C.POINTER(C.c_int32)
@@ -59,6 +62,9 @@ _SIGNATURES = {
     "jpgenc_set_dct_constants": (C.c_int, [C.c_void_p, f64p, f64p]),
     "jpgenc_upload_rgb": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32]),
     "jpgenc_bind_device_rgb": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32]),
+    "jpgenc_bind_device_image": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int, C.c_uint32]),
+    "jpgenc_encode_image": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int, C.c_uint32, C.c_void_p, C.c_uint64,
+                                      u64p]),
     "jpgenc_color_dct_quant": (C.c_int, [C.c_void_p]),
     "jpgenc_get_coefficients": (C.c_int, [C.c_void_p, i16p]),
     "jpgenc_set_coefficients": (C.c_int, [C.c_void_p, i32p, i32p, i32p, C.c_uint32, C.c_uint32]),
@@ -106,6 +112,8 @@ _SIGNATURES = {
                                               C.c_void_p, C.c_uint64, u64p, u64p, u64p]),
     "jpgenc_encode_images_packed": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(C.c_void_p), C.c_int, u32p, u32p, C.c_uint32,
                                               C.c_void_p, C.c_uint64, u64p, u64p, u64p]),
+    "jpgenc_encode_images_packed_layout": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(C.c_void_p), C.c_int, u32p, u32p, u32p, C.c_int,
+                                                     C.c_uint32, C.c_void_p, C.c_uint64, u64p, u64p, u64p]),
     "jpgenc_batch_create": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "jpgenc_batch_destroy": (None, [C.c_void_p]),
     "jpgenc_batch_last_error": (C.c_char_p, [C.c_void_p]),
@@ -141,6 +149,31 @@ class JpgencError(RuntimeError):
 
 def _np_ptr(a: np.ndarray, t):
     return a.ctypes.data_as(t)
+
+
+def _format_code(fmt) -> int:
+    """'RGB' / 'BGR' / 'RGBA' / 'BGRA' (or a JPGENC_PIXEL_* code) -> the code"""
+    if isinstance(fmt, str):
+        if fmt not in PIXEL_FORMATS:
+            raise ValueError(f"unknown pixel format {fmt!r}")
+        return PIXEL_FORMATS[fmt][0]
+    return int(fmt)
+
+
+def image_layout(a: np.ndarray, fmt: str = "RGB"):
+    """(pointer, width, height, row pitch) of a uint8 (H, W, C) array whose strides are (pitch, C, 1) with C the format's
+    bytes per pixel -- a tight array or a view such as big[y0:y1, x0:x1].  Anything else raises ValueError: the pixels are
+    read where they are, never copied."""
+    if fmt not in PIXEL_FORMATS:
+        raise ValueError(f"unknown pixel format {fmt!r}")
+    bpp = PIXEL_FORMATS[fmt][1]
+    if not isinstance(a, np.ndarray) or a.dtype != np.uint8 or a.ndim != 3 or a.shape[2] != bpp:
+        raise ValueError(f"{fmt} pixels must be a uint8 array of shape (H, W, {bpp})")
+    h, w, _ = a.shape
+    pitch = a.strides[0] if h > 1 else w * bpp
+    if a.strides[2] != 1 or (w > 1 and a.strides[1] != bpp) or pitch < w * bpp:
+        raise ValueError(f"{fmt} pixels must have strides (pitch, {bpp}, 1) with pitch >= {w * bpp}; got {a.strides}")
+    return a.ctypes.data, w, h, pitch
 
 
 class Encoder:
@@ -192,6 +225,10 @@ class Encoder:
 
     def bind_device_rgb(self, dev_ptr: int, w: int, h: int, maxval: int = 255):
         self._check(self.lib.jpgenc_bind_device_rgb(self.h, dev_ptr, w, h, maxval))
+
+    def bind_device_image(self, dev_ptr: int, w: int, h: int, pitch: int = 0, fmt="RGB", maxval: int = 255):
+        """device pixels in format fmt ('RGB', 'BGR', 'RGBA', 'BGRA'), rows `pitch` bytes apart (0: tight)"""
+        self._check(self.lib.jpgenc_bind_device_image(self.h, dev_ptr, w, h, pitch, _format_code(fmt), maxval))
 
     # ---- stages ---------------------------------------------------------------------------------
     def color_dct_quant(self):
@@ -280,6 +317,22 @@ class Encoder:
             self._check(rc)
             return out[: n.value].tobytes()
 
+    def encode_image(self, arr: np.ndarray, fmt: str = "RGB", maxval: int = 255) -> bytes:
+        """host pixels in format fmt: a uint8 (H, W, 3 or 4) array with strides (pitch, C, 1), e.g. a crop view of a larger
+        image (see image_layout) -> JPEG bytes"""
+        ptr, w, h, pitch = image_layout(arr, fmt)
+        code = _format_code(fmt)
+        cap = max(4096, w * h * 3 // 2 + 4096)
+        while True:
+            out = np.empty(cap, np.uint8)
+            n = C.c_uint64()
+            rc = self.lib.jpgenc_encode_image(self.h, ptr, w, h, pitch, code, maxval, out.ctypes.data, cap, C.byref(n))
+            if rc == ERR_CAPACITY:
+                cap = int(n.value) + 16
+                continue
+            self._check(rc)
+            return out[: n.value].tobytes()
+
     def encode_planes(self, p0: np.ndarray, p1: np.ndarray, p2: np.ndarray, real_w: int, real_h: int, ycbcr: bool = False) -> bytes:
         """three (H16, W16) float64 planes as the reference's Image holds them -> JPEG bytes (exact FP64 path for every block)"""
         planes = [np.ascontiguousarray(p, np.float64) for p in (p0, p1, p2)]
@@ -343,9 +396,11 @@ class Encoder:
                                                          offs, sizes, C.byref(total)))
         return [int(x) for x in offs], [int(x) for x in sizes], int(total.value)
 
-    def encode_images_packed(self, ptrs, widths, heights, out_ptr: int | None, cap: int, maxval: int = 255, host_images=False):
+    def encode_images_packed(self, ptrs, widths, heights, out_ptr: int | None, cap: int, maxval: int = 255, host_images=False,
+                             pitches=None, fmt=None):
         """images of individual sizes (device memory, or host memory with host_images=True) -> complete files back to back in
-        ONE buffer, in input order; returns (offsets, sizes, total bytes)"""
+        ONE buffer, in input order; returns (offsets, sizes, total bytes).  pitches (bytes from row to row, per image; None or 0:
+        tight) and fmt ('RGB', 'BGR', 'RGBA', 'BGRA') describe pixels in another layout than tight RGB."""
         n = len(ptrs)
         imgs = (C.c_void_p * n)(*ptrs)
         w = np.ascontiguousarray(widths, np.uint32)
@@ -353,28 +408,42 @@ class Encoder:
         sizes = (C.c_uint64 * n)()
         offs = (C.c_uint64 * n)()
         total = C.c_uint64()
-        self._check(self.lib.jpgenc_encode_images_packed(self.h, n, imgs, 0 if host_images else 1, _np_ptr(w, u32p), _np_ptr(h, u32p), maxval,
-                                                         out_ptr, cap, offs, sizes, C.byref(total)))
+        if pitches is None and fmt is None:
+            self._check(self.lib.jpgenc_encode_images_packed(self.h, n, imgs, 0 if host_images else 1, _np_ptr(w, u32p), _np_ptr(h, u32p), maxval,
+                                                             out_ptr, cap, offs, sizes, C.byref(total)))
+        else:
+            p = np.ascontiguousarray(pitches, np.uint32) if pitches is not None else None
+            self._check(self.lib.jpgenc_encode_images_packed_layout(self.h, n, imgs, 0 if host_images else 1, _np_ptr(w, u32p), _np_ptr(h, u32p),
+                                                                    _np_ptr(p, u32p) if p is not None else None, _format_code(fmt or "RGB"),
+                                                                    maxval, out_ptr, cap, offs, sizes, C.byref(total)))
         return [int(x) for x in offs], [int(x) for x in sizes], int(total.value)
 
-    def encode_images(self, images, maxval: int = 255):
+    def encode_images(self, images, maxval: int = 255, fmt: str | None = None):
         """list of HxWx3 uint8 arrays of any sizes -> list of JPEG byte strings, through one call (a second one, sizes first,
-        only when the files outgrow the pixels)"""
-        images = [np.ascontiguousarray(a, np.uint8) for a in images]
+        only when the files outgrow the pixels).  With fmt ('RGB', 'BGR', 'RGBA', 'BGRA') the arrays are read where they are,
+        with their row pitch: (H, W, C) arrays with strides (pitch, C, 1), such as crop views of a larger image (image_layout;
+        anything else raises ValueError)."""
+        if fmt is None:
+            images = [np.ascontiguousarray(a, np.uint8) for a in images]
+            layouts = [(a.ctypes.data, a.shape[1], a.shape[0], 0) for a in images]
+        else:
+            layouts = [image_layout(a, fmt) for a in images]
         if not images:
             return []
-        ptrs = [a.ctypes.data for a in images]
-        ws = [a.shape[1] for a in images]
-        hs = [a.shape[0] for a in images]
-        out = np.empty(sum(a.size for a in images) + 4096 * len(images), np.uint8)
+        ptrs = [x[0] for x in layouts]
+        ws = [x[1] for x in layouts]
+        hs = [x[2] for x in layouts]
+        pitches = [x[3] for x in layouts] if fmt is not None else None
+        out = np.empty(sum(w * h * 3 for w, h in zip(ws, hs)) + 4096 * len(images), np.uint8)
+        kw = dict(host_images=True, pitches=pitches, fmt=fmt)
         try:
-            offs, sizes, _ = self.encode_images_packed(ptrs, ws, hs, out.ctypes.data, out.size, maxval, host_images=True)
+            offs, sizes, _ = self.encode_images_packed(ptrs, ws, hs, out.ctypes.data, out.size, maxval, **kw)
         except JpgencError as e:
             if e.code != ERR_CAPACITY:
                 raise
-            _, _, total = self.encode_images_packed(ptrs, ws, hs, None, 0, maxval, host_images=True)
+            _, _, total = self.encode_images_packed(ptrs, ws, hs, None, 0, maxval, **kw)
             out = np.empty(total, np.uint8)
-            offs, sizes, _ = self.encode_images_packed(ptrs, ws, hs, out.ctypes.data, out.size, maxval, host_images=True)
+            offs, sizes, _ = self.encode_images_packed(ptrs, ws, hs, out.ctypes.data, out.size, maxval, **kw)
         return [out[o: o + n].tobytes() for o, n in zip(offs, sizes)]
 
     def encode_ppm_file(self, src: str, dst: str):

@@ -69,10 +69,21 @@ int set_geometry(jpgenc_ctx* c, uint32_t w, uint32_t h, uint32_t maxval) {
     if (w == 0 || h == 0 || maxval == 0 || maxval > 255) return fail(c, JPGENC_ERR_ARG, "width/height/maxval out of range");
     c->real_w = w; c->real_h = h; c->maxval = maxval;
     c->mcu_w = (w + 15) / 16; c->mcu_h = (h + 15) / 16;        // src/Image.cpp:479-489
+    c->pixel_format = JPGENC_PIXEL_RGB;
+    c->row_pitch = w * 3;
     c->nframes = 1;
     c->mixed.on = false;
     c->have_pixels = false;                                      // whoever changes the geometry binds its pixels afterwards
     c->have_coef = c->have_scan = c->have_items = false; c->k2_tiles_done = 0;
+    return JPGENC_OK;
+}
+
+int check_layout(jpgenc_ctx* c, uint32_t w, uint32_t h, uint32_t* row_pitch, int format) {
+    if (format < JPGENC_PIXEL_RGB || format > JPGENC_PIXEL_BGRA) return fail(c, JPGENC_ERR_ARG, "unknown pixel format");
+    if (w == 0 || h == 0 || w > 65535 || h > 65535) return fail(c, JPGENC_ERR_ARG, "image side out of range (1..65535)");
+    const uint32_t row = w * pixel_bytes(format);
+    if (*row_pitch == 0) *row_pitch = row;
+    if (*row_pitch < row) return fail(c, JPGENC_ERR_ARG, "row pitch below the row size");
     return JPGENC_OK;
 }
 
@@ -393,6 +404,18 @@ int jpgenc_bind_device_rgb(jpgenc_ctx* c, const void* dev_rgb, uint32_t w, uint3
     const int rc = set_geometry(c, w, h, maxval);
     if (rc) return rc;
     c->d_rgb = static_cast<const uint8_t*>(dev_rgb);
+    c->have_pixels = true;
+    return JPGENC_OK;
+} JPGENC_CATCH(c)
+
+int jpgenc_bind_device_image(jpgenc_ctx* c, const void* dev, uint32_t w, uint32_t h, uint32_t row_pitch, int format, uint32_t maxval) try {
+    if (!c) return JPGENC_ERR_ARG;
+    if (!dev) return fail(c, JPGENC_ERR_ARG, "null image pointer");
+    int rc = check_layout(c, w, h, &row_pitch, format);
+    if (rc || (rc = set_geometry(c, w, h, maxval))) return rc;
+    c->pixel_format = format;
+    c->row_pitch = row_pitch;
+    c->d_rgb = static_cast<const uint8_t*>(dev);
     c->have_pixels = true;
     return JPGENC_OK;
 } JPGENC_CATCH(c)
@@ -815,7 +838,9 @@ static int run_pipeline(jpgenc_ctx* c, jpgenc_huff_table tables[4], uint64_t* sc
     if ((rc = ensure_stats_buffers(c))) return rc;
     // ---- phase A: K1, refinement, K2, statistics into the mailbox ----
     c->k2_tiles_done = 0;
-    const uint64_t key_a[5] = {c->alloc_gen, reinterpret_cast<uint64_t>(c->d_rgb), (static_cast<uint64_t>(c->real_w) << 32) | c->real_h, c->maxval,
+    // (the pixel layout picks K1 and the refinement: it is part of the key)
+    const uint64_t key_a[5] = {c->alloc_gen, reinterpret_cast<uint64_t>(c->d_rgb), (static_cast<uint64_t>(c->real_w) << 32) | c->real_h,
+                               c->maxval | static_cast<uint64_t>(c->pixel_format) << 8 | static_cast<uint64_t>(c->row_pitch) << 32,
                                1u | static_cast<uint64_t>(c->stage_timing) << 8};
     const bool pool = c->parallel_tables;
     if (pool) {
@@ -878,12 +903,18 @@ static int ensure_file_staging(jpgenc_ctx* c, size_t bytes) {
 // `fill` (optional): instead of reading the pixels from `host_rgb`, every band is first produced by fill(dst, byte offset in
 // the image, bytes) into one of two pinned staging buffers (a file read, for instance) and uploaded from there: bounded
 // pinned memory, full PCIe rate, and the production of band b+1 overlaps the upload of band b.
+// Pixels in another layout (`format`, rows `pitch` bytes apart in host memory) travel as they are, in their own format, the
+// pitch gap dropped by the copy: on the device they are tight rows of that format, read by the pixel-layout kernels.
 static int upload_and_forward(jpgenc_ctx* c, const uint8_t* host_rgb, uint32_t w, uint32_t h, uint32_t maxval,
-                              const std::function<int(uint8_t*, size_t, size_t)>* fill = nullptr) {
+                              const std::function<int(uint8_t*, size_t, size_t)>* fill = nullptr, int format = JPGENC_PIXEL_RGB,
+                              size_t pitch = 0) {
     JPGENC_CUDA(c, cudaSetDevice(c->device));
     int rc = set_geometry(c, w, h, maxval);
     if (rc) return rc;
-    const size_t row_bytes = static_cast<size_t>(w) * 3, bytes = row_bytes * h;
+    const size_t row_bytes = static_cast<size_t>(w) * pixel_bytes(format), bytes = row_bytes * h;
+    if (pitch == 0) pitch = row_bytes;
+    c->pixel_format = format;
+    c->row_pitch = static_cast<uint32_t>(row_bytes);
     if ((rc = ensure(c, &c->d_rgb_owned, &c->rgb_cap, bytes + 16))) return rc;
     c->d_rgb = c->d_rgb_owned;
     c->have_pixels = true;
@@ -900,7 +931,7 @@ static int upload_and_forward(jpgenc_ctx* c, const uint8_t* host_rgb, uint32_t w
         const uint32_t rows = std::min(rows_per_band, c->mcu_h - y0);
         const size_t px0 = static_cast<size_t>(y0) * 16, px1 = std::min<size_t>(h, static_cast<size_t>(y0 + rows) * 16);
         if (px1 > px0) {
-            const uint8_t* src = host_rgb ? host_rgb + px0 * row_bytes : nullptr;
+            const uint8_t* src = host_rgb ? host_rgb + px0 * pitch : nullptr;
             if (fill) {
                 const size_t band_bytes = static_cast<size_t>(rows_per_band) * 16 * row_bytes;
                 if (band == 0) {
@@ -912,7 +943,11 @@ static int upload_and_forward(jpgenc_ctx* c, const uint8_t* host_rgb, uint32_t w
                 if ((rc = (*fill)(slot, px0 * row_bytes, (px1 - px0) * row_bytes))) return fail(c, rc, "truncated PPM payload, or a sample above maxval");
                 src = slot;
             }
-            JPGENC_CUDA(c, cudaMemcpyAsync(c->d_rgb_owned + px0 * row_bytes, src, (px1 - px0) * row_bytes, cudaMemcpyHostToDevice, c->copy_stream));
+            if (pitch == row_bytes)
+                JPGENC_CUDA(c, cudaMemcpyAsync(c->d_rgb_owned + px0 * row_bytes, src, (px1 - px0) * row_bytes, cudaMemcpyHostToDevice, c->copy_stream));
+            else
+                JPGENC_CUDA(c, cudaMemcpy2DAsync(c->d_rgb_owned + px0 * row_bytes, row_bytes, src, pitch, row_bytes, px1 - px0, cudaMemcpyHostToDevice,
+                                                 c->copy_stream));
         }
         JPGENC_CUDA(c, cudaEventRecord(c->ev_band[band], c->copy_stream));
         JPGENC_CUDA(c, cudaStreamWaitEvent(c->stream, c->ev_band[band], 0));
@@ -974,6 +1009,25 @@ int jpgenc_encode_rgb(jpgenc_ctx* c, const uint8_t* host_rgb, uint32_t w, uint32
         return fail(c, JPGENC_ERR_FORMAT, "a sample exceeds maxval");
     int rc = upload_and_forward(c, host_rgb, w, h, maxval);
     if (rc) return rc;
+    jpgenc_huff_table tables[4];
+    uint64_t scan = 0;
+    if ((rc = run_entropy_stages(c, tables, &scan))) return rc;       // its first synchronisation also covers the copies
+    const size_t hdr = jpgenc_write_headers(c->real_w, c->real_h, c->qy, c->qc, tables, nullptr);
+    if (jpeg_bytes) *jpeg_bytes = hdr + scan + 2;
+    if (!dst) return JPGENC_OK;
+    return assemble(c, tables, scan, dst, cap);
+} JPGENC_CATCH(c)
+
+int jpgenc_encode_image(jpgenc_ctx* c, const void* host, uint32_t w, uint32_t h, uint32_t row_pitch, int format, uint32_t maxval,
+                        uint8_t* dst, uint64_t cap, uint64_t* jpeg_bytes) try {
+    if (!c) return JPGENC_ERR_ARG;
+    if (!host) return fail(c, JPGENC_ERR_ARG, "null image pointer");
+    int rc = check_layout(c, w, h, &row_pitch, format);
+    if (rc) return rc;
+    const uint8_t* px = static_cast<const uint8_t*>(host);
+    if (maxval && maxval < 255 && !samples_within_maxval(px, w, h, row_pitch, pixel_bytes(format), maxval))
+        return fail(c, JPGENC_ERR_FORMAT, "a sample exceeds maxval");
+    if ((rc = upload_and_forward(c, px, w, h, maxval, nullptr, format, row_pitch))) return rc;
     jpgenc_huff_table tables[4];
     uint64_t scan = 0;
     if ((rc = run_entropy_stages(c, tables, &scan))) return rc;       // its first synchronisation also covers the copies

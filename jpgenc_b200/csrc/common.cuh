@@ -64,7 +64,7 @@ struct FrameGeom {
     uint32_t tile0;                       // first K2 tile = item slab; its K3 ranges start at tile0 * split
     uint32_t group0;                      // first K3 group (a CTA of K3a / K3b)
     uint32_t super0;                      // first K3 super-group (256 groups)
-    uint32_t pad;
+    uint32_t pitch;                       // bytes from one pixel row to the next (read only by the kernels of other pixel layouts)
 };
 static_assert(sizeof(FrameGeom) == 48, "FrameGeom is copied as an array");
 
@@ -104,13 +104,20 @@ struct ForwardParams {
     const FrameGeom* geom;
     uint32_t nframes;
     uint32_t strips;
+    // pixels in another layout than tight RGB (forward_layout_kernel, forward_mixed_layout_kernel; the format is their template
+    // parameter): bytes from one row to the next of the single image (images of individual sizes: FrameGeom::pitch)
+    uint32_t pitch;
 };
+
+// bytes per pixel of a JPGENC_PIXEL_* format
+__host__ __device__ constexpr uint32_t pixel_bytes(int format) { return format >= JPGENC_PIXEL_RGBA ? 4u : 3u; }
 
 // host side: the totals of the pass of images of individual sizes bound to a context (the device reads them from the
 // entry behind the last image of FrameGeom)
 struct MixedPass {
     bool on = false;
     bool aligned = false;                 // every image has real_w % 16 == 0 and a 16-byte aligned pointer (K1's bulk copies)
+    int format = -1;                      // JPGENC_PIXEL_*: the pixel-layout kernels (with FrameGeom::pitch); -1 tight RGB
     uint32_t blocks = 0, strips = 0, tiles = 0, groups = 0, supers = 0;
     uint32_t split = 1;                   // K3 ranges per K2 tile, one choice for the whole pass (launch_entropy)
 };
@@ -230,6 +237,8 @@ struct jpgenc_ctx {
     uint8_t* d_rgb_owned = nullptr;
     size_t rgb_cap = 0;
     uint32_t real_w = 0, real_h = 0, maxval = 255, mcu_w = 0, mcu_h = 0;
+    int pixel_format = JPGENC_PIXEL_RGB;  // layout of the single image bound (set_geometry: tight RGB)
+    uint32_t row_pitch = 0;               // ... bytes from one row to the next
     bool have_pixels = false, have_coef = false, have_scan = false, forward_pending = false, upload_pending = false;
 
     int16_t* d_coef = nullptr;

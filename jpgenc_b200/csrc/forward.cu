@@ -17,6 +17,7 @@
 //    already in the MCU-interleaved order the entropy coder consumes.
 #include <algorithm>
 #include <cmath>
+#include <type_traits>
 
 #include "common.cuh"
 #include "exact.cuh"
@@ -205,18 +206,116 @@ struct ForwardSmem {
     alignas(8) uint64_t bar;
 };
 
+// Staging of the pixel-layout kernels: the same 16-row tile of 3 bytes per pixel, in the byte order of the source (the colour
+// read below swaps R and B of BGR / BGRA at compile time).  Each CTA picks its path from its own image:
+//  * 3 bytes per pixel, base and pitch 16-byte aligned, real_w % 16 == 0: one bulk copy per row, as forward_kernel;
+//  * 4 bytes per pixel: 16-byte vector loads (4 pixels) from a 16-byte aligned base and pitch, each turned into 12 bytes of the
+//    tile by three byte permutes (the 4th byte never reaches the tile); a 4-byte strip staged whole would be 32 KB and cost
+//    K1 its 5 CTAs per SM.  Chunks past the right edge, and every chunk of an unaligned image, take clamped byte loads;
+//  * otherwise a clamped byte loader with the pitch.
+template <int kMcus, int kFmt, bool kMixed>
+__device__ __forceinline__ void stage_layout(const ForwardParams& p, ForwardSmem<kMcus>& sm, int tid, const uint8_t* __restrict__ rgb,
+                                             uint32_t pitch, uint32_t real_w, uint32_t real_h, uint32_t my, uint32_t mcu0, int nm) {
+    using Smem = ForwardSmem<kMcus>;
+    constexpr int kThreads = kMcus * 4;
+    constexpr uint32_t kBpp = pixel_bytes(kFmt);
+    const bool aligned = ((reinterpret_cast<uintptr_t>(rgb) | pitch) & 15) == 0;
+    const bool bulk = kBpp == 3 && aligned && real_w % 16 == 0;           // the same for every thread of the CTA
+    if (bulk) {
+        if (tid == 0) {
+            ptx::mbar_init(&sm.bar, 1);
+            ptx::mbar_init_fence();
+        }
+        __syncthreads();
+        if (tid < 16) {
+            const uint32_t row_bytes = nm * 48;
+            if (tid == 0) ptx::mbar_expect_tx(&sm.bar, 16 * row_bytes);
+            const uint32_t sy = min(my * 16 + tid, real_h - 1);
+            ptx::bulk_g2s(sm.tile + tid * Smem::kPitch, rgb + static_cast<size_t>(sy) * pitch + mcu0 * 48, row_bytes, &sm.bar);
+        }
+    }
+    // the strip `prefetch_ahead` CTAs later into L2, when its rows are whole 16-byte multiples inside the image (the range must
+    // not pass the end of a row)
+    if (p.prefetch_ahead && tid >= 32 && tid < 64) {
+        const uint8_t* prgb = nullptr;
+        uint32_t ppitch = 0, pw = 0, ph = 0, pm0 = 0, pnm = 0, pby = 0;
+        if constexpr (kMixed) {
+            const uint32_t t = blockIdx.x + p.prefetch_ahead;
+            if (t < p.strips) {                                             // uniform over the warp (geom_find_warp needs all lanes)
+                const FrameGeom& g = p.geom[geom_find_warp(p.geom, p.nframes, t, &FrameGeom::strip0)];
+                const uint32_t per_row = (g.mcu_w + kMcus - 1) / kMcus, s = t - g.strip0;
+                pby = s / per_row;
+                pm0 = (s - pby * per_row) * kMcus;
+                pnm = min(static_cast<uint32_t>(kMcus), g.mcu_w - pm0);
+                prgb = g.rgb; ppitch = g.pitch; pw = g.real_w; ph = g.real_h;
+            }
+        } else {
+            const uint32_t lin = blockIdx.y * gridDim.x + blockIdx.x + p.prefetch_ahead, y = lin / gridDim.x;
+            if (y < gridDim.y) {
+                pby = p.mcu_y0 + y;
+                pm0 = (lin - y * gridDim.x) * kMcus;
+                pnm = min(static_cast<uint32_t>(kMcus), p.mcu_w - pm0);
+                prgb = p.rgb; ppitch = pitch; pw = real_w; ph = real_h;
+            }
+        }
+        if (prgb && tid < 48 && ((reinterpret_cast<uintptr_t>(prgb) | ppitch | pw) & 15) == 0) {
+            const uint32_t sy = min(pby * 16 + (tid - 32), ph - 1);
+            ptx::bulk_prefetch_l2(prgb + static_cast<size_t>(sy) * ppitch + pm0 * 16 * kBpp, pnm * 16 * kBpp);
+        }
+    }
+    if (bulk) {
+        ptx::mbar_wait(&sm.bar, 0);
+        return;
+    }
+    if constexpr (kBpp == 4) {
+        if (tid < nm * 4) {                                                 // thread = 4 pixels of every row of the strip
+            const uint32_t x0 = mcu0 * 16 + tid * 4;
+            const bool vec = aligned && x0 + 4 <= real_w;
+#pragma unroll 4
+            for (int r = 0; r < 16; ++r) {
+                const uint8_t* row = rgb + static_cast<size_t>(min(my * 16 + r, real_h - 1)) * pitch;
+                uint32_t q[4];
+                if (vec) {
+                    const uint4 v = __ldg(reinterpret_cast<const uint4*>(row + x0 * 4));
+                    q[0] = v.x; q[1] = v.y; q[2] = v.z; q[3] = v.w;
+                } else {
+#pragma unroll
+                    for (int k = 0; k < 4; ++k) {
+                        const uint8_t* px = row + min(x0 + k, real_w - 1) * 4;
+                        q[k] = px[0] | (px[1] << 8) | (px[2] << 16);
+                    }
+                }
+                uint32_t* dst = reinterpret_cast<uint32_t*>(sm.tile + r * Smem::kPitch + tid * 12);
+                dst[0] = __byte_perm(q[0], q[1], 0x4210);                  // c0 c1 c2 | c0 of the next pixel ...
+                dst[1] = __byte_perm(q[1], q[2], 0x5421);
+                dst[2] = __byte_perm(q[2], q[3], 0x6542);
+            }
+        }
+    } else {
+        const int row_bytes = nm * 48;
+        for (int idx = tid; idx < 16 * row_bytes; idx += kThreads) {
+            const int r = idx / row_bytes, b = idx - r * row_bytes;
+            const uint32_t sx = min(mcu0 * 16 + b / 3, real_w - 1);
+            const uint32_t sy = min(my * 16 + r, real_h - 1);
+            sm.tile[r * Smem::kPitch + b] = rgb[static_cast<size_t>(sy) * pitch + sx * 3 + (b % 3)];
+        }
+    }
+    __syncthreads();
+}
+
 // kAligned: real_w % 16 == 0 and 16-byte aligned base -> rows are staged with bulk copies; otherwise a clamped
 // byte loader fills the tile (odd sizes; right-edge replication, src/Image.cpp:491-530)
 // kMixed: images of individual sizes (p.geom): a 1-D grid over the strips of all images; a CTA finds its image by a search
 // over the first-strip prefix.  Otherwise one size: grid (strips of a row, rows, frames).
-template <int kMcus, bool kAligned, bool kBulkOut, bool kMixed>
+// kFmt >= 0: pixels in that JPGENC_PIXEL_* format with a row pitch (stage_layout; kAligned is not used); -1: tight RGB
+template <int kMcus, bool kAligned, bool kBulkOut, bool kMixed, int kFmt = -1>
 // (shared memory and the thread index come from the kernel: there the compiler knows the alignment and, from the launch
 // bounds, the range of threadIdx.x)
 __device__ __forceinline__ void forward_body(const ForwardParams& p, ForwardSmem<kMcus>& sm, unsigned thread) {
     using Smem = ForwardSmem<kMcus>;
     constexpr int kThreads = kMcus * 4;
     const int tid = thread;
-    uint32_t my, mcu0, frame_block0, real_w, real_h, mcu_w;
+    uint32_t my, mcu0, frame_block0, real_w, real_h, mcu_w, pitch;
     const uint8_t* __restrict__ rgb;
     if constexpr (kMixed) {
         const FrameGeom& g = p.geom[geom_find_warp(p.geom, p.nframes, blockIdx.x, &FrameGeom::strip0)];
@@ -228,6 +327,7 @@ __device__ __forceinline__ void forward_body(const ForwardParams& p, ForwardSmem
         frame_block0 = g.block0;
         real_w = g.real_w;
         real_h = g.real_h;
+        pitch = g.pitch;
     } else {
         my = p.mcu_y0 + blockIdx.y;
         mcu0 = blockIdx.x * kMcus;
@@ -236,11 +336,14 @@ __device__ __forceinline__ void forward_body(const ForwardParams& p, ForwardSmem
         real_w = p.real_w;
         real_h = p.real_h;
         mcu_w = p.mcu_w;
+        pitch = p.pitch;
     }
     const int nm = min(kMcus, static_cast<int>(mcu_w - mcu0));
 
     // ---- stage the 16-row RGB strip ----
-    if constexpr (kAligned) {
+    if constexpr (kFmt >= 0) {
+        stage_layout<kMcus, kFmt, kMixed>(p, sm, tid, rgb, pitch, real_w, real_h, my, mcu0, nm);
+    } else if constexpr (kAligned) {
         if (tid == 0) {
             ptx::mbar_init(&sm.bar, 1);
             ptx::mbar_init_fence();
@@ -293,6 +396,7 @@ __device__ __forceinline__ void forward_body(const ForwardParams& p, ForwardSmem
     const int bx = tid % (kMcus * 2), by = tid / (kMcus * 2);
     const bool active = (bx >> 1) < nm;
     f2 v[32];                                     // v[r*4+p] = samples (r, 2p) and (r, 2p+1)
+    constexpr int kR = (kFmt == JPGENC_PIXEL_BGR || kFmt == JPGENC_PIXEL_BGRA) ? 2 : 0, kB = 2 - kR;   // tile bytes of R and B
     if (active) {
         const ColorConsts& cc = p.color;
 #pragma unroll
@@ -306,9 +410,9 @@ __device__ __forceinline__ void forward_body(const ForwardParams& p, ForwardSmem
                 const uint32_t w[6] = {q0.x, q0.y, q1.x, q1.y, q2.x, q2.y};
 #pragma unroll
                 for (int pp = 0; pp < 4; ++pp) {                  // pixels 2pp, 2pp+1 = bytes 6pp .. 6pp+5
-                    rr[h][pp] = bytes_to_f2(w, 6 * pp, 6 * pp + 3);
+                    rr[h][pp] = bytes_to_f2(w, 6 * pp + kR, 6 * pp + 3 + kR);
                     gg[h][pp] = bytes_to_f2(w, 6 * pp + 1, 6 * pp + 4);
-                    bb[h][pp] = bytes_to_f2(w, 6 * pp + 2, 6 * pp + 5);
+                    bb[h][pp] = bytes_to_f2(w, 6 * pp + kB, 6 * pp + 3 + kB);
                     v[r * 4 + pp] = fma2s(rr[h][pp], cc.y[0], fma2s(gg[h][pp], cc.y[1], fma2s(bb[h][pp], cc.y[2], make_float2(-128.f, -128.f))));
                 }
             }
@@ -392,6 +496,19 @@ __global__ void __launch_bounds__(kMcus * 4, 640 / (kMcus * 4)) forward_mixed_ke
     forward_body<kMcus, kAligned, kBulkOut, true>(p, sm, threadIdx.x);
 }
 
+// pixels in another layout (JPGENC_PIXEL_* kFmt, row pitch): one image (p.rgb, p.pitch) / images of individual sizes
+template <int kMcus, int kFmt, bool kBulkOut>
+__global__ void __launch_bounds__(kMcus * 4, 640 / (kMcus * 4)) forward_layout_kernel(const __grid_constant__ ForwardParams p) {
+    __shared__ ForwardSmem<kMcus> sm;
+    forward_body<kMcus, false, kBulkOut, false, kFmt>(p, sm, threadIdx.x);
+}
+
+template <int kMcus, int kFmt, bool kBulkOut>
+__global__ void __launch_bounds__(kMcus * 4, 640 / (kMcus * 4)) forward_mixed_layout_kernel(const __grid_constant__ ForwardParams p) {
+    __shared__ ForwardSmem<kMcus> sm;
+    forward_body<kMcus, false, kBulkOut, true, kFmt>(p, sm, threadIdx.x);
+}
+
 // ---------------------------------------------------------------------------------------------------
 // exact FP64 path (the reference's arithmetic, operation for operation, no contraction)
 // ---------------------------------------------------------------------------------------------------
@@ -407,12 +524,17 @@ __device__ __forceinline__ double exact_channel(int comp, double r, double g, do
     return dsub(dadd(128.0, dadd(dadd(dmul((double).5f, r), dmul((double)-.4186f, g)), dmul((double)-.0813f, b))), 128.0);
 }
 
-__device__ __forceinline__ double exact_pixel(const uint8_t* rgb, uint32_t real_w, uint32_t real_h, uint32_t x, uint32_t y,
+// kFmt: -1 tight RGB, otherwise the JPGENC_PIXEL_* format of pixels whose rows are `pitch` bytes apart
+template <int kFmt>
+__device__ __forceinline__ double exact_pixel(const uint8_t* rgb, uint32_t pitch, uint32_t real_w, uint32_t real_h, uint32_t x, uint32_t y,
                                               int comp, double scale) {
     const uint32_t sx = min(x, real_w - 1), sy = min(y, real_h - 1);            // src/Image.cpp:491-530
-    const uint8_t* px = rgb + (static_cast<size_t>(sy) * real_w + sx) * 3;
-    return exact_channel(comp, dmul(static_cast<double>(px[0]), scale), dmul(static_cast<double>(px[1]), scale),
-                         dmul(static_cast<double>(px[2]), scale));
+    const uint8_t* px;
+    if constexpr (kFmt < 0) px = rgb + (static_cast<size_t>(sy) * real_w + sx) * 3;
+    else px = rgb + static_cast<size_t>(sy) * pitch + sx * pixel_bytes(kFmt);
+    constexpr int kR = (kFmt == JPGENC_PIXEL_BGR || kFmt == JPGENC_PIXEL_BGRA) ? 2 : 0, kB = 2 - kR;
+    return exact_channel(comp, dmul(static_cast<double>(px[kR]), scale), dmul(static_cast<double>(px[1]), scale),
+                         dmul(static_cast<double>(px[kB]), scale));
 }
 
 // Column c of block `id` (mcu*6+k) of an image: located once per thread (the divisions), then sampled row by row
@@ -428,13 +550,14 @@ __device__ __forceinline__ ExactColumn exact_locate(const uint8_t* rgb, uint32_t
     return ExactColumn{rgb, mx * 16 + 2 * c, my * 16, static_cast<int>(k) - 3};
 }
 // spatial sample of row r in the reference's arithmetic
-__device__ __forceinline__ double exact_sample(const ExactColumn& b, uint32_t real_w, uint32_t real_h, int r, double scale) {
-    if (b.comp == 0) return exact_pixel(b.rgb, real_w, real_h, b.x, b.y + r, 0, scale);
+template <int kFmt = -1>
+__device__ __forceinline__ double exact_sample(const ExactColumn& b, uint32_t real_w, uint32_t real_h, int r, double scale, uint32_t pitch = 0) {
+    if (b.comp == 0) return exact_pixel<kFmt>(b.rgb, pitch, real_w, real_h, b.x, b.y + r, 0, scale);
     const uint32_t x = b.x, y = b.y + 2 * r;                                    // S420_m, src/Image.cpp:207-226
-    const double top = dadd(dadd(0.0, exact_pixel(b.rgb, real_w, real_h, x, y, b.comp, scale)),
-                            exact_pixel(b.rgb, real_w, real_h, x + 1, y, b.comp, scale));
-    const double bot = dadd(dadd(0.0, exact_pixel(b.rgb, real_w, real_h, x, y + 1, b.comp, scale)),
-                            exact_pixel(b.rgb, real_w, real_h, x + 1, y + 1, b.comp, scale));
+    const double top = dadd(dadd(0.0, exact_pixel<kFmt>(b.rgb, pitch, real_w, real_h, x, y, b.comp, scale)),
+                            exact_pixel<kFmt>(b.rgb, pitch, real_w, real_h, x + 1, y, b.comp, scale));
+    const double bot = dadd(dadd(0.0, exact_pixel<kFmt>(b.rgb, pitch, real_w, real_h, x, y + 1, b.comp, scale)),
+                            exact_pixel<kFmt>(b.rgb, pitch, real_w, real_h, x + 1, y + 1, b.comp, scale));
     return dmul(dadd(top, bot), 0.25);          // the reference divides by 4: the same double, bit for bit, without a division
 }
 
@@ -532,33 +655,34 @@ __device__ __forceinline__ void refine_loop64(uint32_t n0, uint32_t n, const uin
 }
 
 // ids are global block indices; with `frames` (a batch) block id belongs to frame id / blocks_per_frame
-template <bool k64>
+// kFmt >= 0: pixels in that JPGENC_PIXEL_* format, rows `pitch` bytes apart (-1: tight RGB, pitch unused)
+template <bool k64, int kFmt = -1>
 __global__ void __launch_bounds__(kRefineThreads) refine_kernel(const uint8_t* __restrict__ rgb, const uint8_t* const* __restrict__ frames,
                                                                     uint32_t blocks_per_frame, int16_t* __restrict__ coef,
                                                                     const uint32_t* __restrict__ list,
                                                                     const uint32_t* __restrict__ count, uint32_t cap, int all,
                                                                     uint32_t nblocks, uint32_t real_w, uint32_t real_h,
-                                                                    uint32_t mcu_w, const __grid_constant__ ExactConsts e) {
+                                                                    uint32_t mcu_w, const __grid_constant__ ExactConsts e, uint32_t pitch) {
     // count[0] = entries in the list, count[3] = entries already refined (band-wise encodes refine after every band)
     const uint32_t n = all ? nblocks : min(count[0], cap), n0 = all ? 0u : count[3];
     auto locate = [&](uint32_t id, int c) {
         const uint32_t f = frames ? id / blocks_per_frame : 0u;
         return exact_locate(frames ? frames[f] : rgb, mcu_w, id - f * blocks_per_frame, c);
     };
-    auto sample = [&](const ExactColumn& col, int r) { return exact_sample(col, real_w, real_h, r, e.scale); };
+    auto sample = [&](const ExactColumn& col, int r) { return exact_sample<kFmt>(col, real_w, real_h, r, e.scale, pitch); };
     if constexpr (k64) refine_loop64(n0, n, list, all != 0, coef, blocks_per_frame, e.qy, e.qc, e, locate, sample);
     else refine_loop(n0, n, list, all != 0, coef, blocks_per_frame, e.qy, e.qc, e, locate, sample);
 }
 
 // images of individual sizes: block id -> image by a search over the first-block prefix (every image starts on an MCU, so
 // id % 6 still tells luma from chroma: blocks_per_frame = 2^32 - 1 leaves ids < 2^31 as they are)
-template <bool k64>
+template <bool k64, int kFmt = -1>
 __global__ void __launch_bounds__(kRefineThreads) refine_mixed_kernel(const FrameGeom* __restrict__ geom, uint32_t nframes,
                                                                           int16_t* __restrict__ coef, const uint32_t* __restrict__ list,
                                                                           const uint32_t* __restrict__ count, uint32_t cap,
                                                                           const __grid_constant__ ExactConsts e) {
     const uint32_t n = min(count[0], cap), n0 = count[3];
-    struct Column { ExactColumn col; uint32_t real_w, real_h; };
+    struct Column { ExactColumn col; uint32_t real_w, real_h, pitch; };
     auto locate = [&](uint32_t id, int c) {
         uint32_t lo = 0, hi = nframes;
         while (hi - lo > 1) {
@@ -566,9 +690,9 @@ __global__ void __launch_bounds__(kRefineThreads) refine_mixed_kernel(const Fram
             if (geom[mid].block0 <= id) lo = mid; else hi = mid;
         }
         const FrameGeom& g = geom[lo];
-        return Column{exact_locate(g.rgb, g.mcu_w, id - g.block0, c), g.real_w, g.real_h};
+        return Column{exact_locate(g.rgb, g.mcu_w, id - g.block0, c), g.real_w, g.real_h, kFmt >= 0 ? g.pitch : 0u};
     };
-    auto sample = [&](const Column& col, int r) { return exact_sample(col.col, col.real_w, col.real_h, r, e.scale); };
+    auto sample = [&](const Column& col, int r) { return exact_sample<kFmt>(col.col, col.real_w, col.real_h, r, e.scale, col.pitch); };
     if constexpr (k64) refine_loop64(n0, n, list, false, coef, 0xFFFFFFFFu, e.qy, e.qc, e, locate, sample);
     else refine_loop(n0, n, list, false, coef, 0xFFFFFFFFu, e.qy, e.qc, e, locate, sample);
 }
@@ -831,6 +955,23 @@ static void fill_forward_params(const jpgenc_ctx* c, ForwardParams* p) {
     fill_quant_consts2(c->qc, c->dct_s, &p->chroma, colour_err);
 }
 
+// calls f(std::integral_constant<int, format>) for a JPGENC_PIXEL_* format: the kernels of the other pixel layouts take the
+// format as a template parameter
+template <class F>
+static void with_format(int format, F&& f) {
+    switch (format) {
+        case JPGENC_PIXEL_RGB: f(std::integral_constant<int, JPGENC_PIXEL_RGB>{}); break;
+        case JPGENC_PIXEL_BGR: f(std::integral_constant<int, JPGENC_PIXEL_BGR>{}); break;
+        case JPGENC_PIXEL_RGBA: f(std::integral_constant<int, JPGENC_PIXEL_RGBA>{}); break;
+        default: f(std::integral_constant<int, JPGENC_PIXEL_BGRA>{}); break;
+    }
+}
+
+// the single image bound is not tight RGB: K1 and the refinement take the pixel-layout kernels
+static bool layout_image(const jpgenc_ctx* c) {
+    return c->pixel_format != JPGENC_PIXEL_RGB || c->row_pitch != c->real_w * 3;
+}
+
 // exact FP64 pass over the blocks K1 flagged (all == false) or over every block (all == true)
 static int launch_refine(jpgenc_ctx* c, bool all) {
     ExactConsts e;
@@ -841,14 +982,26 @@ static int launch_refine(jpgenc_ctx* c, bool all) {
     const unsigned grid = static_cast<unsigned>(std::max<uint64_t>(c->sm_count, std::min<uint64_t>(c->sm_count * 16, total / 256 + 1)));
     // 64 threads per block where the flagged blocks are few (latency: 3840x2160 15 -> 6 us), 8 per block where they are many
     // (throughput: at 16384^2 the 64-thread form's barriers cost 42 us against 28)
-    if (total < (3u << 19))
+    const uint32_t cap = all ? 0u : static_cast<uint32_t>(c->refine_cap);
+    const uint8_t* const* frames = c->nframes > 1 ? c->d_frame_ptrs : nullptr;
+    if (layout_image(c)) {
+        with_format(c->pixel_format, [&](auto fmt) {
+            constexpr int kFmt = decltype(fmt)::value;
+            if (total < (3u << 19))
+                refine_kernel<true, kFmt><<<grid, kRefineThreads, 0, c->stream>>>(c->d_rgb, frames, bpf, c->d_coef, c->d_refine_list, c->d_counters, cap,
+                                                                                  all ? 1 : 0, bpf * c->nframes, c->real_w, c->real_h, c->mcu_w, e, c->row_pitch);
+            else
+                refine_kernel<false, kFmt><<<grid, kRefineThreads, 0, c->stream>>>(c->d_rgb, frames, bpf, c->d_coef, c->d_refine_list, c->d_counters, cap,
+                                                                                   all ? 1 : 0, bpf * c->nframes, c->real_w, c->real_h, c->mcu_w, e, c->row_pitch);
+        });
+    } else if (total < (3u << 19))
         refine_kernel<true><<<grid, kRefineThreads, 0, c->stream>>>(
-            c->d_rgb, c->nframes > 1 ? c->d_frame_ptrs : nullptr, bpf, c->d_coef, c->d_refine_list, c->d_counters,
-            all ? 0u : static_cast<uint32_t>(c->refine_cap), all ? 1 : 0, bpf * c->nframes, c->real_w, c->real_h, c->mcu_w, e);
+            c->d_rgb, frames, bpf, c->d_coef, c->d_refine_list, c->d_counters,
+            cap, all ? 1 : 0, bpf * c->nframes, c->real_w, c->real_h, c->mcu_w, e, 0u);
     else
         refine_kernel<false><<<grid, kRefineThreads, 0, c->stream>>>(
-            c->d_rgb, c->nframes > 1 ? c->d_frame_ptrs : nullptr, bpf, c->d_coef, c->d_refine_list, c->d_counters,
-            all ? 0u : static_cast<uint32_t>(c->refine_cap), all ? 1 : 0, bpf * c->nframes, c->real_w, c->real_h, c->mcu_w, e);
+            c->d_rgb, frames, bpf, c->d_coef, c->d_refine_list, c->d_counters,
+            cap, all ? 1 : 0, bpf * c->nframes, c->real_w, c->real_h, c->mcu_w, e, 0u);
     JPGENC_CUDA(c, cudaGetLastError());
     c->launches += 1;
     return JPGENC_OK;
@@ -870,6 +1023,19 @@ int launch_forward_rows(jpgenc_ctx* c, uint32_t y0, uint32_t rows, bool first, b
     // (strips of 24 and of 40 MCUs, which divide 1920- and 3840-pixel rows evenly, were measured: no gain on those frames
     // -- the partial fourth strip is not what costs -- and 24 is 7 % slower where 32 divides the row)
     const dim3 grid((c->mcu_w + 31) / 32, rows, c->nframes);
+    if (layout_image(c)) {
+        // each CTA picks its staging path from the image (stage_layout); the tensor store serves every full strip
+        p.pitch = c->row_pitch;
+        const bool bulk = make_block_map(c->d_coef, static_cast<uint64_t>(c->mcu_w) * c->mcu_h * kBlocksPerMcu, 32 * kBlocksPerMcu, &p.coef_map);
+        with_format(c->pixel_format, [&](auto fmt) {
+            constexpr int kFmt = decltype(fmt)::value;
+            if (bulk) forward_layout_kernel<32, kFmt, true><<<grid, 128, 0, c->stream>>>(p);
+            else forward_layout_kernel<32, kFmt, false><<<grid, 128, 0, c->stream>>>(p);
+        });
+        JPGENC_CUDA(c, cudaGetLastError());
+        c->launches += 1;
+        return last ? launch_refine(c, false) : JPGENC_OK;
+    }
     const bool bulk_out = aligned &&
                           make_block_map(c->d_coef, static_cast<uint64_t>(c->mcu_w) * c->mcu_h * kBlocksPerMcu * c->nframes, 32 * kBlocksPerMcu, &p.coef_map);
     if (bulk_out) forward_kernel<32, true, true><<<grid, 128, 0, c->stream>>>(p);
@@ -881,7 +1047,8 @@ int launch_forward_rows(jpgenc_ctx* c, uint32_t y0, uint32_t rows, bool first, b
 }
 
 // K1 + exact refinement over a pass of images of individual sizes.  The bulk copies need every image of the pass to qualify
-// (c->mixed.aligned); the tensor store serves the full strips of every image, the copy-out the partial ones.
+// (c->mixed.aligned); the tensor store serves the full strips of every image, the copy-out the partial ones.  Pixels in another
+// layout (c->mixed.format >= 0) take the pixel-layout kernels, where each CTA picks its staging path from its own image.
 int launch_forward_mixed(jpgenc_ctx* c) {
     ForwardParams p{};
     fill_forward_params(c, &p);                                   // (its per-size fields are not read by forward_mixed_kernel)
@@ -891,9 +1058,16 @@ int launch_forward_mixed(jpgenc_ctx* c) {
     p.prefetch_ahead = 256;
     JPGENC_CUDA(c, cudaMemsetAsync(c->d_counters, 0, 4 * sizeof(uint32_t), c->stream));
     c->stats_clear_valid = false;                                 // K2 clears the statistics and K3a's sums itself
+    const bool layout = c->mixed.format >= 0;
     const bool aligned = c->mixed.aligned;
-    const bool bulk_out = aligned && make_block_map(c->d_coef, c->mixed.blocks, 32 * kBlocksPerMcu, &p.coef_map);
-    if (bulk_out) forward_mixed_kernel<32, true, true><<<c->mixed.strips, 128, 0, c->stream>>>(p);
+    const bool bulk_out = (aligned || layout) && make_block_map(c->d_coef, c->mixed.blocks, 32 * kBlocksPerMcu, &p.coef_map);
+    if (layout) {
+        with_format(c->mixed.format, [&](auto fmt) {
+            constexpr int kFmt = decltype(fmt)::value;
+            if (bulk_out) forward_mixed_layout_kernel<32, kFmt, true><<<c->mixed.strips, 128, 0, c->stream>>>(p);
+            else forward_mixed_layout_kernel<32, kFmt, false><<<c->mixed.strips, 128, 0, c->stream>>>(p);
+        });
+    } else if (bulk_out) forward_mixed_kernel<32, true, true><<<c->mixed.strips, 128, 0, c->stream>>>(p);
     else if (aligned) forward_mixed_kernel<32, true, false><<<c->mixed.strips, 128, 0, c->stream>>>(p);
     else forward_mixed_kernel<32, false, false><<<c->mixed.strips, 128, 0, c->stream>>>(p);
     JPGENC_CUDA(c, cudaGetLastError());
@@ -902,7 +1076,15 @@ int launch_forward_mixed(jpgenc_ctx* c) {
     const uint64_t total = c->mixed.blocks;                       // the same grid and thread layout rules as launch_refine
     const unsigned grid = static_cast<unsigned>(std::max<uint64_t>(c->sm_count, std::min<uint64_t>(c->sm_count * 16, total / 256 + 1)));
     const uint32_t cap = static_cast<uint32_t>(c->refine_cap);
-    if (total < (3u << 19))
+    if (layout) {
+        with_format(c->mixed.format, [&](auto fmt) {
+            constexpr int kFmt = decltype(fmt)::value;
+            if (total < (3u << 19))
+                refine_mixed_kernel<true, kFmt><<<grid, kRefineThreads, 0, c->stream>>>(c->d_geom, c->nframes, c->d_coef, c->d_refine_list, c->d_counters, cap, e);
+            else
+                refine_mixed_kernel<false, kFmt><<<grid, kRefineThreads, 0, c->stream>>>(c->d_geom, c->nframes, c->d_coef, c->d_refine_list, c->d_counters, cap, e);
+        });
+    } else if (total < (3u << 19))
         refine_mixed_kernel<true><<<grid, kRefineThreads, 0, c->stream>>>(c->d_geom, c->nframes, c->d_coef, c->d_refine_list, c->d_counters, cap, e);
     else
         refine_mixed_kernel<false><<<grid, kRefineThreads, 0, c->stream>>>(c->d_geom, c->nframes, c->d_coef, c->d_refine_list, c->d_counters, cap, e);

@@ -40,6 +40,11 @@ struct Job {
     // null: every frame is w x h
     const uint32_t* widths = nullptr;
     const uint32_t* heights = nullptr;
+    // pixels in another layout (jpgenc_encode_images_packed_layout; needs widths): JPGENC_PIXEL_* format, -1 tight RGB, and the
+    // row pitch of every image as the caller holds it.  `staged`: host images, uploaded into tight rows of their format.
+    int format = -1;
+    const uint32_t* pitches = nullptr;
+    bool staged = false;
     double raw_per_block = 0;              // ... raw-scan bytes reserved per block: 1.5 x the most this call has seen (0: nothing yet)
     // output: per-frame buffers (legacy), one packed buffer, or none (sizes only)
     uint8_t* const* out_ptrs = nullptr;
@@ -59,6 +64,9 @@ struct Pass {
 
 uint32_t job_w(const Job& job, uint32_t i) { return job.widths ? job.widths[i] : job.w; }
 uint32_t job_h(const Job& job, uint32_t i) { return job.heights ? job.heights[i] : job.h; }
+uint32_t job_bpp(const Job& job) { return job.format < 0 ? 3u : pixel_bytes(job.format); }
+// bytes from one row of image i to the next where the kernels read it
+uint32_t job_pitch(const Job& job, uint32_t i) { return job.pitches && !job.staged ? job.pitches[i] : job_w(job, i) * job_bpp(job); }
 uint64_t job_blocks(const Job& job, uint32_t i) {
     return static_cast<uint64_t>((job_w(job, i) + 15) / 16) * ((job_h(job, i) + 15) / 16) * kBlocksPerMcu;
 }
@@ -126,6 +134,7 @@ MixedPass image_geometry(const Job& job, const Pass& ps, const void* const* ptrs
     MixedPass m;
     m.on = true;
     m.aligned = true;
+    m.format = job.format;
     uint64_t all_tiles = 0;
     for (uint32_t f = 0; f < ps.F; ++f) all_tiles += (job_blocks(job, ps.f0 + f) + 383) / 384;
     m.split = all_tiles < 4096 ? 4u : 1u;
@@ -136,6 +145,7 @@ MixedPass image_geometry(const Job& job, const Pass& ps, const void* const* ptrs
         const uint32_t w = job_w(job, ps.f0 + f), h = job_h(job, ps.f0 + f);
         g[f].rgb = static_cast<const uint8_t*>(ptrs[f]);
         g[f].real_w = w; g[f].real_h = h; g[f].mcu_w = (w + 15) / 16; g[f].mcu_h = (h + 15) / 16;
+        if (job.format >= 0) g[f].pitch = job_pitch(job, ps.f0 + f);
         const uint32_t blocks = g[f].mcu_w * g[f].mcu_h * kBlocksPerMcu, tiles = (blocks + 383) / 384, groups = (tiles * m.split + 7) / 8;
         m.blocks += blocks;
         m.strips += (g[f].mcu_w + 31) / 32 * g[f].mcu_h;
@@ -447,7 +457,7 @@ int encode_device_frames(jpgenc_ctx* c, Job& job, const void* const* dev_frames)
 // Frames in host memory (pinned for full PCIe speed): they travel on the copy stream into a ring of pass-sized slices
 // of device memory, always a few passes ahead of the kernels; when pass p is finished its slice is re-filled with the
 // frames of pass p + ring.  A slice holds the bytes of the largest pass (passes of images of individual sizes differ);
-// every frame starts on 256 bytes.
+// every frame starts on 256 bytes.  Pixels in another layout travel in their own format, the pitch gap dropped by the copy.
 int encode_host_frames(jpgenc_ctx* c, Job& job, const uint8_t* const* frames) {
     // an empty batch is legal and touches nothing: an image bound to the context keeps its geometry
     if (job.n == 0) return (job.w && job.h && job.maxval && job.maxval <= 255) ? JPGENC_OK : fail(c, JPGENC_ERR_ARG, "width/height/maxval out of range");
@@ -462,7 +472,7 @@ int encode_host_frames(jpgenc_ctx* c, Job& job, const uint8_t* const* frames) {
     const uint32_t npasses = static_cast<uint32_t>(pass.size());
     constexpr uint32_t kRingMax = sizeof(c->ev_band) / sizeof(c->ev_band[0]);
     const uint32_t ring = std::min({nslots + 2, npasses, kRingMax});
-    auto fbytes = [&](uint32_t i) { return static_cast<size_t>(job_w(job, i)) * job_h(job, i) * 3; };
+    auto fbytes = [&](uint32_t i) { return static_cast<size_t>(job_w(job, i)) * job_h(job, i) * job_bpp(job); };
     auto fstride = [&](uint32_t i) { return (fbytes(i) + 255) & ~static_cast<size_t>(255); };
     // frame f of pass p sits at slice (p % ring) + at[f0 + f]
     std::vector<size_t> at(job.n);
@@ -480,13 +490,17 @@ int encode_host_frames(jpgenc_ctx* c, Job& job, const uint8_t* const* frames) {
             uint32_t run = 1;
             while (!job.widths && f + run < F && frames[f0 + f + run] == frames[f0 + f + run - 1] + fbytes(0)) ++run;
             uint8_t* dst = c->d_rgb_owned + static_cast<size_t>(s) * slice + at[f0 + f];
-            if (run == 1) JPGENC_CUDA(c, cudaMemcpyAsync(dst, frames[f0 + f], fbytes(f0 + f), cudaMemcpyHostToDevice, c->copy_stream));
+            const size_t row = static_cast<size_t>(job_w(job, f0 + f)) * job_bpp(job);
+            if (job.pitches && job.pitches[f0 + f] != row)
+                JPGENC_CUDA(c, cudaMemcpy2DAsync(dst, row, frames[f0 + f], job.pitches[f0 + f], row, job_h(job, f0 + f), cudaMemcpyHostToDevice, c->copy_stream));
+            else if (run == 1) JPGENC_CUDA(c, cudaMemcpyAsync(dst, frames[f0 + f], fbytes(f0 + f), cudaMemcpyHostToDevice, c->copy_stream));
             else JPGENC_CUDA(c, cudaMemcpy2DAsync(dst, fstride(0), frames[f0 + f], fbytes(0), fbytes(0), run, cudaMemcpyHostToDevice, c->copy_stream));
             f += run;
         }
         JPGENC_CUDA(c, cudaEventRecord(c->ev_band[s], c->copy_stream));
         return JPGENC_OK;
     };
+    job.staged = true;
     for (uint32_t p = 0; p < ring; ++p)
         if ((rc = upload(p))) return rc;
     std::vector<std::vector<const void*>> ptrs(nslots);
@@ -568,6 +582,39 @@ int jpgenc_encode_images_packed(jpgenc_ctx* c, uint32_t n, const void* const* im
     Job job;
     job.n = n; job.w = widths[0]; job.h = heights[0]; job.maxval = maxval;
     if (!same) { job.widths = widths; job.heights = heights; }   // one size: the batched-frame path as it is
+    job.packed_mode = true; job.packed = out; job.packed_cap = cap; job.offsets = offsets; job.sizes = sizes;
+    const int rc = images_on_device ? encode_device_frames(c, job, images) : encode_host_frames(c, job, reinterpret_cast<const uint8_t* const*>(images));
+    if (total_bytes) *total_bytes = job.packed_at;
+    return rc;
+} JPGENC_CATCH(c)
+
+int jpgenc_encode_images_packed_layout(jpgenc_ctx* c, uint32_t n, const void* const* images, int images_on_device, const uint32_t* widths,
+                                       const uint32_t* heights, const uint32_t* row_pitches, int format, uint32_t maxval, uint8_t* out,
+                                       uint64_t cap, uint64_t* offsets, uint64_t* sizes, uint64_t* total_bytes) try {
+    if (!c) return JPGENC_ERR_ARG;
+    if (total_bytes) *total_bytes = 0;
+    if (format < JPGENC_PIXEL_RGB || format > JPGENC_PIXEL_BGRA) return fail(c, JPGENC_ERR_ARG, "unknown pixel format");
+    if (maxval == 0 || maxval > 255) return fail(c, JPGENC_ERR_ARG, "maxval out of range");
+    if (n == 0) return JPGENC_OK;                                // an empty batch is legal and touches nothing
+    if (!images || !widths || !heights || !offsets || !sizes) return fail(c, JPGENC_ERR_ARG, "null argument");
+    std::vector<uint32_t> pitch(n);
+    bool tight_rgb = format == JPGENC_PIXEL_RGB;
+    for (uint32_t i = 0; i < n; ++i) {
+        if (!images[i]) return fail(c, JPGENC_ERR_ARG, "null image pointer");
+        pitch[i] = row_pitches ? row_pitches[i] : 0;
+        const int rc = check_layout(c, widths[i], heights[i], &pitch[i], format);
+        if (rc) return rc;
+        tight_rgb = tight_rgb && pitch[i] == widths[i] * 3;
+    }
+    if (tight_rgb) return jpgenc_encode_images_packed(c, n, images, images_on_device, widths, heights, maxval, out, cap, offsets, sizes, total_bytes);
+    if (!images_on_device && maxval < 255)
+        for (uint32_t i = 0; i < n; ++i)
+            if (!samples_within_maxval(static_cast<const uint8_t*>(images[i]), widths[i], heights[i], pitch[i], pixel_bytes(format), maxval))
+                return fail(c, JPGENC_ERR_FORMAT, "a sample exceeds maxval");
+    Job job;
+    job.n = n; job.w = widths[0]; job.h = heights[0]; job.maxval = maxval;
+    job.widths = widths; job.heights = heights;                  // the pass pipeline of images of individual sizes, equal sizes too
+    job.format = format; job.pitches = pitch.data();
     job.packed_mode = true; job.packed = out; job.packed_cap = cap; job.offsets = offsets; job.sizes = sizes;
     const int rc = images_on_device ? encode_device_frames(c, job, images) : encode_host_frames(c, job, reinterpret_cast<const uint8_t* const*>(images));
     if (total_bytes) *total_bytes = job.packed_at;

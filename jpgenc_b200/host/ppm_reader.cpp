@@ -94,6 +94,23 @@ bool samples_within_maxval(const uint8_t* px, size_t count, uint32_t maxval) {
     return over == 0;
 }
 
+bool samples_within_maxval(const uint8_t* px, uint32_t w, uint32_t h, size_t pitch, uint32_t bpp, uint32_t maxval) {
+    if (maxval >= 255) return true;
+    if (bpp == 3) {
+        for (uint32_t y = 0; y < h; ++y)
+            if (!samples_within_maxval(px + y * pitch, static_cast<size_t>(w) * 3, maxval)) return false;
+        return true;
+    }
+    uint8_t over = 0;
+    for (uint32_t y = 0; y < h; ++y) {
+        const uint8_t* row = px + y * pitch;
+        for (uint32_t x = 0; x < w; ++x)
+            over |= static_cast<uint8_t>(row[x * bpp] > maxval) | static_cast<uint8_t>(row[x * bpp + 1] > maxval) |
+                    static_cast<uint8_t>(row[x * bpp + 2] > maxval);
+    }
+    return over == 0;
+}
+
 int ppm_samples(const uint8_t* file, size_t n, const PpmHeader& h, std::vector<uint8_t>* storage, const uint8_t** view) {
     const size_t count = static_cast<size_t>(h.width) * h.height * 3;
     if (h.magic == 6) {                                         // loadP6PPM, src/Image.cpp:411-418
