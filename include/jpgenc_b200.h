@@ -45,6 +45,7 @@ extern "C" {
 #define JPGENC_PIXEL_BGR      1   /* 3 bytes per pixel: B,G,R */
 #define JPGENC_PIXEL_RGBA     2   /* 4 bytes per pixel: R,G,B, then a byte that is ignored */
 #define JPGENC_PIXEL_BGRA     3   /* 4 bytes per pixel: B,G,R, then a byte that is ignored */
+#define JPGENC_PIXEL_GRAY    16   /* 1 byte per pixel v, encoded as the pixel (v, v, v): the reference's file for that RGB image */
 
 typedef struct jpgenc_ctx jpgenc_ctx;
 
@@ -113,6 +114,11 @@ int jpgenc_bind_device_rgb(jpgenc_ctx* ctx, const void* dev_rgb, uint32_t real_w
  * Unknown format, pitch below the row size, sides outside 1..65535: JPGENC_ERR_ARG. */
 int jpgenc_bind_device_image(jpgenc_ctx* ctx, const void* dev, uint32_t real_w, uint32_t real_h, uint32_t row_pitch, int format,
                              uint32_t maxval);
+/* same, for planar RGB: one plane of 1 byte per pixel per channel, the three with one row pitch (0 = real_w).  BGR or GBR plane
+ * order is a different assignment of the pointers; planes may alias (r == g == b gives the JPGENC_PIXEL_GRAY file).
+ * A null plane, pitch below real_w, sides outside 1..65535: JPGENC_ERR_ARG. */
+int jpgenc_bind_device_planar(jpgenc_ctx* ctx, const void* r, const void* g, const void* b, uint32_t real_w, uint32_t real_h,
+                              uint32_t row_pitch, uint32_t maxval);
 
 /* ---- K1: convertToColorSpace(YCbCr) + applySubsampling(S420_m) + applyDCT(Arai) + applyQuantization
  *      + zigzag (src/Image.cpp:112-148, 198-235, 540-595, 597-636; Dct.hpp:47-215; Coding.hpp:57-97) -- */
@@ -174,6 +180,11 @@ int jpgenc_encode_rgb(jpgenc_ctx* ctx, const uint8_t* host_rgb, uint32_t real_w,
  * 4-byte pixels cost 4/3 of the PCIe bytes of RGB.  Checked against maxval when it is below 255 (colour bytes only). */
 int jpgenc_encode_image(jpgenc_ctx* ctx, const void* host, uint32_t real_w, uint32_t real_h, uint32_t row_pitch, int format,
                         uint32_t maxval, uint8_t* dst, uint64_t cap, uint64_t* jpeg_bytes);
+/* the same for planar RGB in host memory (see jpgenc_bind_device_planar): every plane travels as it is, one copy per plane and
+ * band (one for all three when they lie back to back, as in a tight (3, H, W) buffer).  Checked against maxval when it is below
+ * 255, in all three planes. */
+int jpgenc_encode_planar(jpgenc_ctx* ctx, const void* r, const void* g, const void* b, uint32_t real_w, uint32_t real_h,
+                         uint32_t row_pitch, uint32_t maxval, uint8_t* dst, uint64_t cap, uint64_t* jpeg_bytes);
 /* Image::writeJPEG (src/Image.cpp:831-976) for an image given as the reference holds it: three row-major planes of doubles
  * (Image::R/G/B, include/Image.hpp:104-114), `width` x `height` = the image padded to whole 16x16 MCUs (src/Image.cpp:479-530),
  * real_w x real_h = what SOF0 reports.  ycbcr != 0: the planes already are level-shifted Y, Cb, Cr and are not converted
@@ -241,6 +252,11 @@ int jpgenc_encode_images_packed_layout(jpgenc_ctx* ctx, uint32_t n, const void* 
                                        const uint32_t* widths, const uint32_t* heights, const uint32_t* row_pitches, int format,
                                        uint32_t maxval, uint8_t* out, uint64_t cap, uint64_t* offsets, uint64_t* sizes,
                                        uint64_t* total_bytes);
+/* jpgenc_encode_images_packed_layout for planar RGB: planes[3i], planes[3i + 1], planes[3i + 2] are the R, G and B planes of
+ * image i, row_pitches[i] their common row pitch (row_pitches may be NULL: all tight; an entry of 0 is tight too). */
+int jpgenc_encode_images_packed_planar(jpgenc_ctx* ctx, uint32_t n, const void* const* planes, int images_on_device,
+                                       const uint32_t* widths, const uint32_t* heights, const uint32_t* row_pitches, uint32_t maxval,
+                                       uint8_t* out, uint64_t cap, uint64_t* offsets, uint64_t* sizes, uint64_t* total_bytes);
 
 /* ---- stage methods for the modes writeJPEG does not use (SURVEY.md 8(f)4) ------------------------------------------ */
 /* Image::applySubsampling(mode) on one chroma plane (src/Image.cpp:198-319): `plane` = height x width doubles (host), mode =

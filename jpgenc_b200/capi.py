@@ -16,8 +16,8 @@ LIB_PATH = Path(__file__).resolve().parent / "lib" / "libjpgenc_b200.so"
 OK = 0
 ERR_CUDA, ERR_ARG, ERR_NO_DEVICE, ERR_FORMAT, ERR_IO, ERR_CAPACITY, ERR_NOMEM = -1, -2, -3, -4, -5, -6, -7
 
-# JPGENC_PIXEL_*: name -> (code, bytes per pixel)
-PIXEL_FORMATS = {"RGB": (0, 3), "BGR": (1, 3), "RGBA": (2, 4), "BGRA": (3, 4)}
+# JPGENC_PIXEL_*: name -> (code, bytes per pixel); a GRAY pixel v is encoded as the pixel (v, v, v)
+PIXEL_FORMATS = {"RGB": (0, 3), "BGR": (1, 3), "RGBA": (2, 4), "BGRA": (3, 4), "GRAY": (16, 1)}
 
 u8p = C.POINTER(C.c_uint8)
 i16p = C.POINTER(C.c_int16)
@@ -63,6 +63,9 @@ _SIGNATURES = {
     "jpgenc_upload_rgb": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32]),
     "jpgenc_bind_device_rgb": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32]),
     "jpgenc_bind_device_image": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int, C.c_uint32]),
+    "jpgenc_bind_device_planar": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32]),
+    "jpgenc_encode_planar": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32,
+                                       C.c_void_p, C.c_uint64, u64p]),
     "jpgenc_encode_image": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int, C.c_uint32, C.c_void_p, C.c_uint64,
                                       u64p]),
     "jpgenc_color_dct_quant": (C.c_int, [C.c_void_p]),
@@ -114,6 +117,8 @@ _SIGNATURES = {
                                               C.c_void_p, C.c_uint64, u64p, u64p, u64p]),
     "jpgenc_encode_images_packed_layout": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(C.c_void_p), C.c_int, u32p, u32p, u32p, C.c_int,
                                                      C.c_uint32, C.c_void_p, C.c_uint64, u64p, u64p, u64p]),
+    "jpgenc_encode_images_packed_planar": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(C.c_void_p), C.c_int, u32p, u32p, u32p, C.c_uint32,
+                                                     C.c_void_p, C.c_uint64, u64p, u64p, u64p]),
     "jpgenc_batch_create": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "jpgenc_batch_destroy": (None, [C.c_void_p]),
     "jpgenc_batch_last_error": (C.c_char_p, [C.c_void_p]),
@@ -162,11 +167,19 @@ def _format_code(fmt) -> int:
 
 def image_layout(a: np.ndarray, fmt: str = "RGB"):
     """(pointer, width, height, row pitch) of a uint8 (H, W, C) array whose strides are (pitch, C, 1) with C the format's
-    bytes per pixel -- a tight array or a view such as big[y0:y1, x0:x1].  Anything else raises ValueError: the pixels are
-    read where they are, never copied."""
+    bytes per pixel -- a tight array or a view such as big[y0:y1, x0:x1]; GRAY: a uint8 (H, W) array with strides (pitch, 1).
+    Anything else raises ValueError: the pixels are read where they are, never copied."""
     if fmt not in PIXEL_FORMATS:
         raise ValueError(f"unknown pixel format {fmt!r}")
     bpp = PIXEL_FORMATS[fmt][1]
+    if fmt == "GRAY":
+        if not isinstance(a, np.ndarray) or a.dtype != np.uint8 or a.ndim != 2 or a.size == 0:
+            raise ValueError("GRAY pixels must be a uint8 array of shape (H, W)")
+        h, w = a.shape
+        pitch = a.strides[0] if h > 1 else w
+        if (w > 1 and a.strides[1] != 1) or pitch < w:
+            raise ValueError(f"GRAY pixels must have strides (pitch, 1) with pitch >= {w}; got {a.strides}")
+        return a.ctypes.data, w, h, pitch
     if not isinstance(a, np.ndarray) or a.dtype != np.uint8 or a.ndim != 3 or a.shape[2] != bpp:
         raise ValueError(f"{fmt} pixels must be a uint8 array of shape (H, W, {bpp})")
     h, w, _ = a.shape
@@ -174,6 +187,58 @@ def image_layout(a: np.ndarray, fmt: str = "RGB"):
     if a.strides[2] != 1 or (w > 1 and a.strides[1] != bpp) or pitch < w * bpp:
         raise ValueError(f"{fmt} pixels must have strides (pitch, {bpp}, 1) with pitch >= {w * bpp}; got {a.strides}")
     return a.ctypes.data, w, h, pitch
+
+
+def tensor_layout(t, order: str = "RGB"):
+    """How a torch uint8 image tensor is read in place: (fmt, pointers, width, height, row pitch in bytes).
+
+    fmt is "planar" (pointers = the R, G, B planes) or a PIXEL_FORMATS name (one pointer).  Accepted:
+      (3, H, W) with stride(2) == 1     planar, one plane per channel (crop views t[:, y0:y1, x0:x1] too);
+                                        a channel stride of 0 (g.expand(3, H, W)) is GRAY
+      (3, H, W) in channels_last        interleaved RGB (strides (1, pitch, 3))
+      (H, W, 3) / (H, W, 4)             interleaved RGB / RGBA with strides (pitch, C, 1)
+      (H, W), (1, H, W)                 GRAY with strides (pitch, 1)
+    order="BGR" reads the channels as B, G, R (BGR / BGRA, or the planes in that order).  Anything else raises ValueError;
+    nothing is ever copied.  Pure: only the tensor's metadata is read."""
+    if order not in ("RGB", "BGR"):
+        raise ValueError(f"order must be 'RGB' or 'BGR', not {order!r}")
+    if type(t).__module__.split(".")[0] != "torch" or not hasattr(t, "stride"):
+        raise ValueError("expected a torch.Tensor")
+    if str(t.dtype) != "torch.uint8":
+        raise ValueError(f"image tensors must be uint8, not {t.dtype}")
+    if t.numel() == 0:
+        raise ValueError("empty image tensor")
+    shape, stride, base = tuple(t.shape), tuple(t.stride()), t.data_ptr()
+
+    def plane(h, w, sh, sw):                  # (H, W) with strides (sh, sw): the row pitch of one byte per pixel, or None
+        if w > 1 and sw != 1:
+            return None
+        pitch = sh if h > 1 else w
+        return pitch if pitch >= w else None
+
+    if len(shape) == 2 or (len(shape) == 3 and shape[0] == 1):
+        h, w = shape[-2:]
+        pitch = plane(h, w, stride[-2], stride[-1])
+        if pitch is not None:
+            return "GRAY", (base,), w, h, pitch
+    elif len(shape) == 3 and shape[0] == 3:
+        _, h, w = shape
+        pitch = plane(h, w, stride[1], stride[2])
+        if pitch is not None:
+            if stride[0] == 0:
+                return "GRAY", (base,), w, h, pitch
+            ptrs = tuple(base + k * stride[0] for k in range(3))
+            return "planar", ptrs[::-1] if order == "BGR" else ptrs, w, h, pitch
+        pitch = stride[1] if h > 1 else 3 * w
+        if stride[0] == 1 and (w == 1 or stride[2] == 3) and pitch >= 3 * w:
+            return order, (base,), w, h, pitch
+    elif len(shape) == 3 and shape[2] in (3, 4):
+        h, w, c = shape
+        pitch = stride[0] if h > 1 else c * w
+        if stride[2] == 1 and (w == 1 or stride[1] == c) and pitch >= c * w:
+            return order + ("A" if c == 4 else ""), (base,), w, h, pitch
+    raise ValueError(f"cannot read a tensor of shape {shape} and strides {stride} in place: expected (3, H, W) planes, (3, H, W) "
+                     "channels_last, (H, W, 3|4) with strides (pitch, C, 1), or (H, W) / (1, H, W) grey")
 
 
 class Encoder:
@@ -227,8 +292,12 @@ class Encoder:
         self._check(self.lib.jpgenc_bind_device_rgb(self.h, dev_ptr, w, h, maxval))
 
     def bind_device_image(self, dev_ptr: int, w: int, h: int, pitch: int = 0, fmt="RGB", maxval: int = 255):
-        """device pixels in format fmt ('RGB', 'BGR', 'RGBA', 'BGRA'), rows `pitch` bytes apart (0: tight)"""
+        """device pixels in format fmt ('RGB', 'BGR', 'RGBA', 'BGRA', 'GRAY'), rows `pitch` bytes apart (0: tight)"""
         self._check(self.lib.jpgenc_bind_device_image(self.h, dev_ptr, w, h, pitch, _format_code(fmt), maxval))
+
+    def bind_device_planar(self, r: int, g: int, b: int, w: int, h: int, pitch: int = 0, maxval: int = 255):
+        """planar RGB in device memory: three planes of one byte per pixel, rows `pitch` bytes apart (0: tight)"""
+        self._check(self.lib.jpgenc_bind_device_planar(self.h, r, g, b, w, h, pitch, maxval))
 
     # ---- stages ---------------------------------------------------------------------------------
     def color_dct_quant(self):
@@ -333,6 +402,19 @@ class Encoder:
             self._check(rc)
             return out[: n.value].tobytes()
 
+    def encode_planar(self, r: int, g: int, b: int, w: int, h: int, pitch: int = 0, maxval: int = 255) -> bytes:
+        """planar RGB in host memory (three plane pointers, one row pitch; 0: tight) -> JPEG bytes"""
+        cap = max(4096, w * h * 3 // 2 + 4096)
+        while True:
+            out = np.empty(cap, np.uint8)
+            n = C.c_uint64()
+            rc = self.lib.jpgenc_encode_planar(self.h, r, g, b, w, h, pitch, maxval, out.ctypes.data, cap, C.byref(n))
+            if rc == ERR_CAPACITY:
+                cap = int(n.value) + 16
+                continue
+            self._check(rc)
+            return out[: n.value].tobytes()
+
     def encode_planes(self, p0: np.ndarray, p1: np.ndarray, p2: np.ndarray, real_w: int, real_h: int, ycbcr: bool = False) -> bytes:
         """three (H16, W16) float64 planes as the reference's Image holds them -> JPEG bytes (exact FP64 path for every block)"""
         planes = [np.ascontiguousarray(p, np.float64) for p in (p0, p1, p2)]
@@ -418,11 +500,84 @@ class Encoder:
                                                                     maxval, out_ptr, cap, offs, sizes, C.byref(total)))
         return [int(x) for x in offs], [int(x) for x in sizes], int(total.value)
 
+    def encode_images_packed_planar(self, planes, widths, heights, out_ptr: int | None, cap: int, maxval: int = 255, host_images=False,
+                                    pitches=None):
+        """planar RGB images of individual sizes: planes[3i:3i + 3] = the R, G, B plane pointers of image i (device memory, or host
+        memory with host_images=True), pitches per image (None or 0: tight) -> files back to back as encode_images_packed"""
+        n = len(widths)
+        pl = (C.c_void_p * (3 * n))(*planes)
+        w = np.ascontiguousarray(widths, np.uint32)
+        h = np.ascontiguousarray(heights, np.uint32)
+        p = np.ascontiguousarray(pitches, np.uint32) if pitches is not None else None
+        sizes = (C.c_uint64 * n)()
+        offs = (C.c_uint64 * n)()
+        total = C.c_uint64()
+        self._check(self.lib.jpgenc_encode_images_packed_planar(self.h, n, pl, 0 if host_images else 1, _np_ptr(w, u32p), _np_ptr(h, u32p),
+                                                                _np_ptr(p, u32p) if p is not None else None, maxval, out_ptr, cap, offs,
+                                                                sizes, C.byref(total)))
+        return [int(x) for x in offs], [int(x) for x in sizes], int(total.value)
+
+    def _files(self, encode, pixels: int, n: int):
+        """encode(out_ptr, cap) -> (offsets, sizes, total) into a host buffer, again with the reported size when the files
+        outgrow the first guess -> list of the files"""
+        out = np.empty(pixels * 3 + 4096 * n, np.uint8)
+        try:
+            offs, sizes, _ = encode(out.ctypes.data, out.size)
+        except JpgencError as e:
+            if e.code != ERR_CAPACITY:
+                raise
+            _, _, total = encode(None, 0)
+            out = np.empty(total, np.uint8)
+            offs, sizes, _ = encode(out.ctypes.data, out.size)
+        return [out[o: o + k].tobytes() for o, k in zip(offs, sizes)]
+
+    def encode_tensor(self, t, order: str = "RGB") -> bytes:
+        """one torch uint8 image tensor, on the CPU or on this encoder's GPU, read in place (see tensor_layout) -> JPEG bytes"""
+        return self.encode_tensors([t], order)[0]
+
+    def encode_tensors(self, ts, order: str = "RGB", maxval: int = 255):
+        """torch uint8 image tensors of any sizes, all on the CPU or all on this encoder's GPU and all of one layout kind
+        (tensor_layout), through one batched call -> list of JPEG byte strings.  Nothing is copied or converted: any other
+        tensor raises ValueError.  CUDA tensors are read once the work queued on torch's current stream has finished."""
+        import torch
+
+        ts = list(ts)
+        if not ts:
+            return []
+        layouts = [tensor_layout(t, order) for t in ts]
+        kinds = {x[0] for x in layouts}
+        if len(kinds) != 1:
+            raise ValueError(f"one layout kind per call; got {sorted(kinds)}")
+        devices = {t.device for t in ts}
+        if len(devices) != 1:
+            raise ValueError(f"tensors on several devices in one call: {sorted(str(d) for d in devices)}")
+        dev = devices.pop()
+        if dev.type == "cuda":
+            if dev.index != self.device:
+                raise ValueError(f"tensor on {dev}, encoder on cuda:{self.device}")
+            ev = torch.cuda.Event()
+            ev.record(torch.cuda.current_stream(dev))
+            ev.synchronize()
+        elif dev.type != "cpu":
+            raise ValueError(f"tensors on {dev} cannot be read")
+        kind = layouts[0][0]
+        ws = [x[2] for x in layouts]
+        hs = [x[3] for x in layouts]
+        pitches = [x[4] for x in layouts]
+        host = dev.type == "cpu"
+        if kind == "planar":
+            planes = [p for x in layouts for p in x[1]]
+            enc = lambda o, c: self.encode_images_packed_planar(planes, ws, hs, o, c, maxval, host_images=host, pitches=pitches)
+        else:
+            ptrs = [x[1][0] for x in layouts]
+            enc = lambda o, c: self.encode_images_packed(ptrs, ws, hs, o, c, maxval, host_images=host, pitches=pitches, fmt=kind)
+        return self._files(enc, sum(w * h for w, h in zip(ws, hs)), len(ts))
+
     def encode_images(self, images, maxval: int = 255, fmt: str | None = None):
         """list of HxWx3 uint8 arrays of any sizes -> list of JPEG byte strings, through one call (a second one, sizes first,
-        only when the files outgrow the pixels).  With fmt ('RGB', 'BGR', 'RGBA', 'BGRA') the arrays are read where they are,
-        with their row pitch: (H, W, C) arrays with strides (pitch, C, 1), such as crop views of a larger image (image_layout;
-        anything else raises ValueError)."""
+        only when the files outgrow the pixels).  With fmt ('RGB', 'BGR', 'RGBA', 'BGRA', 'GRAY') the arrays are read where they
+        are, with their row pitch: (H, W, C) arrays with strides (pitch, C, 1), such as crop views of a larger image, or (H, W)
+        grey arrays with strides (pitch, 1) (image_layout; anything else raises ValueError)."""
         if fmt is None:
             images = [np.ascontiguousarray(a, np.uint8) for a in images]
             layouts = [(a.ctypes.data, a.shape[1], a.shape[0], 0) for a in images]
@@ -434,17 +589,8 @@ class Encoder:
         ws = [x[1] for x in layouts]
         hs = [x[2] for x in layouts]
         pitches = [x[3] for x in layouts] if fmt is not None else None
-        out = np.empty(sum(w * h * 3 for w, h in zip(ws, hs)) + 4096 * len(images), np.uint8)
-        kw = dict(host_images=True, pitches=pitches, fmt=fmt)
-        try:
-            offs, sizes, _ = self.encode_images_packed(ptrs, ws, hs, out.ctypes.data, out.size, maxval, **kw)
-        except JpgencError as e:
-            if e.code != ERR_CAPACITY:
-                raise
-            _, _, total = self.encode_images_packed(ptrs, ws, hs, None, 0, maxval, **kw)
-            out = np.empty(total, np.uint8)
-            offs, sizes, _ = self.encode_images_packed(ptrs, ws, hs, out.ctypes.data, out.size, maxval, **kw)
-        return [out[o: o + n].tobytes() for o, n in zip(offs, sizes)]
+        return self._files(lambda o, c: self.encode_images_packed(ptrs, ws, hs, o, c, maxval, host_images=True, pitches=pitches, fmt=fmt),
+                           sum(w * h for w, h in zip(ws, hs)), len(images))
 
     def encode_ppm_file(self, src: str, dst: str):
         self._check(self.lib.jpgenc_encode_ppm_file(self.h, src.encode(), dst.encode()))

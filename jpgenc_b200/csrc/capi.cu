@@ -79,7 +79,7 @@ int set_geometry(jpgenc_ctx* c, uint32_t w, uint32_t h, uint32_t maxval) {
 }
 
 int check_layout(jpgenc_ctx* c, uint32_t w, uint32_t h, uint32_t* row_pitch, int format) {
-    if (format < JPGENC_PIXEL_RGB || format > JPGENC_PIXEL_BGRA) return fail(c, JPGENC_ERR_ARG, "unknown pixel format");
+    if ((format < JPGENC_PIXEL_RGB || format > JPGENC_PIXEL_BGRA) && format != JPGENC_PIXEL_GRAY) return fail(c, JPGENC_ERR_ARG, "unknown pixel format");
     if (w == 0 || h == 0 || w > 65535 || h > 65535) return fail(c, JPGENC_ERR_ARG, "image side out of range (1..65535)");
     const uint32_t row = w * pixel_bytes(format);
     if (*row_pitch == 0) *row_pitch = row;
@@ -416,6 +416,21 @@ int jpgenc_bind_device_image(jpgenc_ctx* c, const void* dev, uint32_t w, uint32_
     c->pixel_format = format;
     c->row_pitch = row_pitch;
     c->d_rgb = static_cast<const uint8_t*>(dev);
+    c->have_pixels = true;
+    return JPGENC_OK;
+} JPGENC_CATCH(c)
+
+int jpgenc_bind_device_planar(jpgenc_ctx* c, const void* r, const void* g, const void* b, uint32_t w, uint32_t h, uint32_t row_pitch,
+                              uint32_t maxval) try {
+    if (!c) return JPGENC_ERR_ARG;
+    if (!r || !g || !b) return fail(c, JPGENC_ERR_ARG, "null plane pointer");
+    int rc = check_layout(c, w, h, &row_pitch, JPGENC_PIXEL_GRAY);        // every plane: one byte per pixel
+    if (rc || (rc = set_geometry(c, w, h, maxval))) return rc;
+    c->pixel_format = kPixelPlanar;
+    c->row_pitch = row_pitch;
+    c->d_rgb = static_cast<const uint8_t*>(r);
+    c->d_plane_g = static_cast<const uint8_t*>(g);
+    c->d_plane_b = static_cast<const uint8_t*>(b);
     c->have_pixels = true;
     return JPGENC_OK;
 } JPGENC_CATCH(c)
@@ -793,7 +808,7 @@ static bool graphs_enabled() {
 }
 
 // replays (capturing first, if the key is new for the second time) the phase that `enqueue` puts on the stream
-static int run_phase(jpgenc_ctx* c, jpgenc_ctx::PhaseGraph& g, const uint64_t (&key)[5], const std::function<int()>& enqueue) {
+static int run_phase(jpgenc_ctx* c, jpgenc_ctx::PhaseGraph& g, const uint64_t (&key)[kGraphKeyWords], const std::function<int()>& enqueue) {
     const bool same_as_graph = g.exec && std::memcmp(g.key, key, sizeof key) == 0;
     if (!same_as_graph) {
         const bool repeat = std::memcmp(g.seen, key, sizeof key) == 0;
@@ -839,9 +854,11 @@ static int run_pipeline(jpgenc_ctx* c, jpgenc_huff_table tables[4], uint64_t* sc
     // ---- phase A: K1, refinement, K2, statistics into the mailbox ----
     c->k2_tiles_done = 0;
     // (the pixel layout picks K1 and the refinement: it is part of the key)
-    const uint64_t key_a[5] = {c->alloc_gen, reinterpret_cast<uint64_t>(c->d_rgb), (static_cast<uint64_t>(c->real_w) << 32) | c->real_h,
-                               c->maxval | static_cast<uint64_t>(c->pixel_format) << 8 | static_cast<uint64_t>(c->row_pitch) << 32,
-                               1u | static_cast<uint64_t>(c->stage_timing) << 8};
+    const bool planar = c->pixel_format == kPixelPlanar;
+    const uint64_t key_a[kGraphKeyWords] = {c->alloc_gen, reinterpret_cast<uint64_t>(c->d_rgb), (static_cast<uint64_t>(c->real_w) << 32) | c->real_h,
+                                            c->maxval | static_cast<uint64_t>(c->pixel_format) << 8 | static_cast<uint64_t>(c->row_pitch) << 32,
+                                            1u | static_cast<uint64_t>(c->stage_timing) << 8,
+                                            planar ? reinterpret_cast<uint64_t>(c->d_plane_g) : 0, planar ? reinterpret_cast<uint64_t>(c->d_plane_b) : 0};
     const bool pool = c->parallel_tables;
     if (pool) {
         if (!c->pool) c->pool = new TablePool(kTableWorkers);
@@ -878,7 +895,8 @@ static int run_pipeline(jpgenc_ctx* c, jpgenc_huff_table tables[4], uint64_t* sc
     // CTAs for the 83 tiles of every 3840x2160 frame: 10 us), never more than the raw buffer holds
     if (k4_tiles > c->k4_grid_hint || k4_tiles < c->k4_grid_hint / 4) c->k4_grid_hint = k4_tiles + k4_tiles / 2 + 8;
     const uint32_t k4_grid = std::min(c->k4_grid_hint, static_cast<uint32_t>(c->raw_cap / kK4TileBytes + 1));   // raw_cap holds the scan: >= k4_tiles
-    const uint64_t key_b[5] = {c->alloc_gen, k4_grid, (static_cast<uint64_t>(c->real_w) << 32) | c->real_h, 0, 1u | static_cast<uint64_t>(c->stage_timing) << 8};
+    const uint64_t key_b[kGraphKeyWords] = {c->alloc_gen, k4_grid, (static_cast<uint64_t>(c->real_w) << 32) | c->real_h, 0,
+                                            1u | static_cast<uint64_t>(c->stage_timing) << 8, 0, 0};
     if ((rc = run_phase(c, c->graph_b, key_b, [&]() -> int { return enqueue_entropy_phase(c, k4_grid); }))) return rc;
     if ((rc = wait_entropy(c))) return rc;
     if (scan) *scan = c->stats.scan_bytes;
@@ -905,23 +923,32 @@ static int ensure_file_staging(jpgenc_ctx* c, size_t bytes) {
 // pinned memory, full PCIe rate, and the production of band b+1 overlaps the upload of band b.
 // Pixels in another layout (`format`, rows `pitch` bytes apart in host memory) travel as they are, in their own format, the
 // pitch gap dropped by the copy: on the device they are tight rows of that format, read by the pixel-layout kernels.
+// Planar RGB (kPixelPlanar; host_rgb, host_g, host_b are the planes) lands as three tight planes back to back.
 static int upload_and_forward(jpgenc_ctx* c, const uint8_t* host_rgb, uint32_t w, uint32_t h, uint32_t maxval,
                               const std::function<int(uint8_t*, size_t, size_t)>* fill = nullptr, int format = JPGENC_PIXEL_RGB,
-                              size_t pitch = 0) {
+                              size_t pitch = 0, const uint8_t* host_g = nullptr, const uint8_t* host_b = nullptr) {
     JPGENC_CUDA(c, cudaSetDevice(c->device));
     int rc = set_geometry(c, w, h, maxval);
     if (rc) return rc;
     const size_t row_bytes = static_cast<size_t>(w) * pixel_bytes(format), bytes = row_bytes * h;
+    const uint32_t nplanes = format == kPixelPlanar ? 3 : 1;
     if (pitch == 0) pitch = row_bytes;
     c->pixel_format = format;
     c->row_pitch = static_cast<uint32_t>(row_bytes);
-    if ((rc = ensure(c, &c->d_rgb_owned, &c->rgb_cap, bytes + 16))) return rc;
+    if ((rc = ensure(c, &c->d_rgb_owned, &c->rgb_cap, nplanes * bytes + 16))) return rc;
     c->d_rgb = c->d_rgb_owned;
+    c->d_plane_g = c->d_rgb_owned + bytes;
+    c->d_plane_b = c->d_rgb_owned + 2 * bytes;
     c->have_pixels = true;
     if ((rc = ensure_coef(c))) return rc;
+    const uint8_t* host_plane[3] = {host_rgb, host_g, host_b};
+    // planes that lie `gap` bytes apart with tight rows (a (3, H, W) buffer) travel as ONE strided copy per band
+    const uintptr_t gap = reinterpret_cast<uintptr_t>(host_g) - reinterpret_cast<uintptr_t>(host_rgb);
+    const bool one_copy = nplanes == 3 && pitch == row_bytes && gap >= bytes && gap <= (uintptr_t{1} << 48) &&
+                          reinterpret_cast<uintptr_t>(host_b) - reinterpret_cast<uintptr_t>(host_g) == gap;
     constexpr uint32_t kMaxBands = sizeof(c->ev_band) / sizeof(c->ev_band[0]);
     // bands of at least ~8 MB (a copy that size already runs at full PCIe rate), at most kMaxBands of them
-    uint32_t rows_per_band = static_cast<uint32_t>(std::max<size_t>(1, (8u << 20) / (row_bytes * 16)));
+    uint32_t rows_per_band = static_cast<uint32_t>(std::max<size_t>(1, (8u << 20) / (row_bytes * nplanes * 16)));
     rows_per_band = std::max(rows_per_band, (c->mcu_h + kMaxBands - 1) / kMaxBands);
     if ((rc = ensure_stats_buffers(c))) return rc;
     const uint32_t tiles = (c->mcu_w * c->mcu_h * kBlocksPerMcu + 383) / 384;
@@ -943,11 +970,18 @@ static int upload_and_forward(jpgenc_ctx* c, const uint8_t* host_rgb, uint32_t w
                 if ((rc = (*fill)(slot, px0 * row_bytes, (px1 - px0) * row_bytes))) return fail(c, rc, "truncated PPM payload, or a sample above maxval");
                 src = slot;
             }
-            if (pitch == row_bytes)
-                JPGENC_CUDA(c, cudaMemcpyAsync(c->d_rgb_owned + px0 * row_bytes, src, (px1 - px0) * row_bytes, cudaMemcpyHostToDevice, c->copy_stream));
-            else
-                JPGENC_CUDA(c, cudaMemcpy2DAsync(c->d_rgb_owned + px0 * row_bytes, row_bytes, src, pitch, row_bytes, px1 - px0, cudaMemcpyHostToDevice,
+            if (one_copy)
+                JPGENC_CUDA(c, cudaMemcpy2DAsync(c->d_rgb_owned + px0 * row_bytes, bytes, src, gap, (px1 - px0) * row_bytes, 3, cudaMemcpyHostToDevice,
                                                  c->copy_stream));
+            else
+                for (uint32_t k = 0; k < nplanes; ++k) {
+                    if (k) src = host_plane[k] + px0 * pitch;
+                    uint8_t* dst = c->d_rgb_owned + k * bytes + px0 * row_bytes;
+                    if (pitch == row_bytes)
+                        JPGENC_CUDA(c, cudaMemcpyAsync(dst, src, (px1 - px0) * row_bytes, cudaMemcpyHostToDevice, c->copy_stream));
+                    else
+                        JPGENC_CUDA(c, cudaMemcpy2DAsync(dst, row_bytes, src, pitch, row_bytes, px1 - px0, cudaMemcpyHostToDevice, c->copy_stream));
+                }
         }
         JPGENC_CUDA(c, cudaEventRecord(c->ev_band[band], c->copy_stream));
         JPGENC_CUDA(c, cudaStreamWaitEvent(c->stream, c->ev_band[band], 0));
@@ -1018,6 +1052,18 @@ int jpgenc_encode_rgb(jpgenc_ctx* c, const uint8_t* host_rgb, uint32_t w, uint32
     return assemble(c, tables, scan, dst, cap);
 } JPGENC_CATCH(c)
 
+// the rest of an encode after upload_and_forward: K2 .. K4, then the file into dst (NULL: the size only)
+static int finish_upload_encode(jpgenc_ctx* c, uint8_t* dst, uint64_t cap, uint64_t* jpeg_bytes) {
+    jpgenc_huff_table tables[4];
+    uint64_t scan = 0;
+    const int rc = run_entropy_stages(c, tables, &scan);             // its first synchronisation also covers the copies
+    if (rc) return rc;
+    const size_t hdr = jpgenc_write_headers(c->real_w, c->real_h, c->qy, c->qc, tables, nullptr);
+    if (jpeg_bytes) *jpeg_bytes = hdr + scan + 2;
+    if (!dst) return JPGENC_OK;
+    return assemble(c, tables, scan, dst, cap);
+}
+
 int jpgenc_encode_image(jpgenc_ctx* c, const void* host, uint32_t w, uint32_t h, uint32_t row_pitch, int format, uint32_t maxval,
                         uint8_t* dst, uint64_t cap, uint64_t* jpeg_bytes) try {
     if (!c) return JPGENC_ERR_ARG;
@@ -1028,13 +1074,21 @@ int jpgenc_encode_image(jpgenc_ctx* c, const void* host, uint32_t w, uint32_t h,
     if (maxval && maxval < 255 && !samples_within_maxval(px, w, h, row_pitch, pixel_bytes(format), maxval))
         return fail(c, JPGENC_ERR_FORMAT, "a sample exceeds maxval");
     if ((rc = upload_and_forward(c, px, w, h, maxval, nullptr, format, row_pitch))) return rc;
-    jpgenc_huff_table tables[4];
-    uint64_t scan = 0;
-    if ((rc = run_entropy_stages(c, tables, &scan))) return rc;       // its first synchronisation also covers the copies
-    const size_t hdr = jpgenc_write_headers(c->real_w, c->real_h, c->qy, c->qc, tables, nullptr);
-    if (jpeg_bytes) *jpeg_bytes = hdr + scan + 2;
-    if (!dst) return JPGENC_OK;
-    return assemble(c, tables, scan, dst, cap);
+    return finish_upload_encode(c, dst, cap, jpeg_bytes);
+} JPGENC_CATCH(c)
+
+int jpgenc_encode_planar(jpgenc_ctx* c, const void* r, const void* g, const void* b, uint32_t w, uint32_t h, uint32_t row_pitch, uint32_t maxval,
+                         uint8_t* dst, uint64_t cap, uint64_t* jpeg_bytes) try {
+    if (!c) return JPGENC_ERR_ARG;
+    if (!r || !g || !b) return fail(c, JPGENC_ERR_ARG, "null plane pointer");
+    int rc = check_layout(c, w, h, &row_pitch, JPGENC_PIXEL_GRAY);         // every plane: one byte per pixel
+    if (rc) return rc;
+    const uint8_t* plane[3] = {static_cast<const uint8_t*>(r), static_cast<const uint8_t*>(g), static_cast<const uint8_t*>(b)};
+    for (const uint8_t* px : plane)
+        if (maxval && maxval < 255 && !samples_within_maxval(px, w, h, row_pitch, 1, maxval))
+            return fail(c, JPGENC_ERR_FORMAT, "a sample exceeds maxval");
+    if ((rc = upload_and_forward(c, plane[0], w, h, maxval, nullptr, kPixelPlanar, row_pitch, plane[1], plane[2]))) return rc;
+    return finish_upload_encode(c, dst, cap, jpeg_bytes);
 } JPGENC_CATCH(c)
 
 // Image::writeJPEG for an image that is not (or no longer) a set of 8-bit samples: planes a caller edited after loadPPM,

@@ -107,17 +107,28 @@ struct ForwardParams {
     // pixels in another layout than tight RGB (forward_layout_kernel, forward_mixed_layout_kernel; the format is their template
     // parameter): bytes from one row to the next of the single image (images of individual sizes: FrameGeom::pitch)
     uint32_t pitch;
+    // planar RGB (kPixelPlanar): the G and B planes of the single image (its R plane is `rgb`) / of image f of a pass at
+    // planes[2f], planes[2f + 1] (its R plane is FrameGeom::rgb)
+    const uint8_t* plane_g;
+    const uint8_t* plane_b;
+    const uint8_t* const* planes;
 };
 
-// bytes per pixel of a JPGENC_PIXEL_* format
-__host__ __device__ constexpr uint32_t pixel_bytes(int format) { return format >= JPGENC_PIXEL_RGBA ? 4u : 3u; }
+// Planar RGB: three planes of one byte per pixel, one row pitch.  It has no JPGENC_PIXEL_* code (the calls take three plane
+// pointers); inside the library it is this format.
+constexpr int kPixelPlanar = 17;
+
+// bytes per pixel of a JPGENC_PIXEL_* format (planar: of one plane)
+__host__ __device__ constexpr uint32_t pixel_bytes(int format) {
+    return format >= JPGENC_PIXEL_GRAY ? 1u : format >= JPGENC_PIXEL_RGBA ? 4u : 3u;
+}
 
 // host side: the totals of the pass of images of individual sizes bound to a context (the device reads them from the
 // entry behind the last image of FrameGeom)
 struct MixedPass {
     bool on = false;
     bool aligned = false;                 // every image has real_w % 16 == 0 and a 16-byte aligned pointer (K1's bulk copies)
-    int format = -1;                      // JPGENC_PIXEL_*: the pixel-layout kernels (with FrameGeom::pitch); -1 tight RGB
+    int format = -1;                      // JPGENC_PIXEL_* or kPixelPlanar: the pixel-layout kernels (with FrameGeom::pitch); -1 tight RGB
     uint32_t blocks = 0, strips = 0, tiles = 0, groups = 0, supers = 0;
     uint32_t split = 1;                   // K3 ranges per K2 tile, one choice for the whole pass (launch_entropy)
 };
@@ -184,6 +195,8 @@ __host__ __device__ inline unsigned long long raw_slot_bytes(unsigned long long 
 
 namespace jpgenc { class TablePool; class HostPool; }
 
+constexpr int kGraphKeyWords = 7;         // jpgenc_ctx::PhaseGraph: what a captured encode phase depends on
+
 struct jpgenc_ctx {
     int device = 0;
     jpgenc::TablePool* pool = nullptr;    // host worker threads that build the four Huffman tables side by side
@@ -215,8 +228,8 @@ struct jpgenc_ctx {
     // CUDA graphs, captured when the same configuration is encoded a second time
     struct PhaseGraph {
         cudaGraphExec_t exec = nullptr;
-        uint64_t key[5] = {0, 0, 0, 0, 0};
-        uint64_t seen[5] = {0, 0, 0, 0, 0};   // key of the previous encode (a graph is captured when it repeats)
+        uint64_t key[kGraphKeyWords] = {};
+        uint64_t seen[kGraphKeyWords] = {};   // key of the previous encode (a graph is captured when it repeats)
         uint32_t launches = 0;                // kernels per replay
         uint32_t publishes = 0;               // mailbox announcements per replay
     } graph_a, graph_b;
@@ -239,6 +252,8 @@ struct jpgenc_ctx {
     uint32_t real_w = 0, real_h = 0, maxval = 255, mcu_w = 0, mcu_h = 0;
     int pixel_format = JPGENC_PIXEL_RGB;  // layout of the single image bound (set_geometry: tight RGB)
     uint32_t row_pitch = 0;               // ... bytes from one row to the next
+    const uint8_t* d_plane_g = nullptr;   // ... planar RGB (kPixelPlanar): the G and B planes (d_rgb is the R plane)
+    const uint8_t* d_plane_b = nullptr;
     bool have_pixels = false, have_coef = false, have_scan = false, forward_pending = false, upload_pending = false;
 
     int16_t* d_coef = nullptr;

@@ -169,7 +169,8 @@ __device__ __forceinline__ bool quantize_pack_packed(const f2 (&v)[32], const Qu
 // (0x4B0000bb == 8388608 + b exactly), one packed subtraction removes the 2^23.  Runs on the ALU + FMA pipes; the
 // plain I2F.U8 conversion is a quarter-rate XU instruction (measured: routing one to three of the channels through
 // I2F instead changes K1's time by -0.6 % .. +4 %, so the single PRMT path is kept).
-__device__ __forceinline__ f2 bytes_to_f2(const uint32_t (&w)[6], int lo, int hi) {
+template <int N>
+__device__ __forceinline__ f2 bytes_to_f2(const uint32_t (&w)[N], int lo, int hi) {
     const uint32_t a = __byte_perm(w[lo >> 2], 0x4B000000u, 0x7650 | (lo & 3));
     const uint32_t b = __byte_perm(w[hi >> 2], 0x4B000000u, 0x7650 | (hi & 3));
     return add2(make_float2(__uint_as_float(a), __uint_as_float(b)), make_float2(-8388608.f, -8388608.f));
@@ -303,11 +304,105 @@ __device__ __forceinline__ void stage_layout(const ForwardParams& p, ForwardSmem
     __syncthreads();
 }
 
+// Staging of grey (kPlanes 1) and planar RGB (kPlanes 3) pixels: the tile holds the strip in the source's own layout, kPlanes
+// planes of 16 rows of kMcus * 16 bytes (planar: 24 KB, the whole tile), and the colour read in forward_body takes the three
+// channels from the planes (grey: one byte for all three).  Interleaving the planes here instead would cost what the 4-byte
+// formats' byte permutes cost above.  Each CTA picks its path from its own image:
+//  * every plane's base and the pitch 16-byte aligned, real_w % 16 == 0: one bulk copy per plane row (16 / 48 per CTA);
+//  * otherwise 16-byte chunks: a vector load where the chunk lies inside an aligned image, clamped byte loads elsewhere.
+// The L2 prefetch of the strip `prefetch_ahead` CTAs later covers every plane.
+template <int kMcus, int kPlanes, bool kMixed>
+__device__ __forceinline__ void stage_planes(const ForwardParams& p, ForwardSmem<kMcus>& sm, int tid, const uint8_t* const (&plane)[3],
+                                             uint32_t pitch, uint32_t real_w, uint32_t real_h, uint32_t my, uint32_t mcu0, int nm) {
+    using Smem = ForwardSmem<kMcus>;
+    constexpr int kThreads = kMcus * 4, kRow = kMcus * 16;
+    static_assert(kPlanes * 16 * kRow <= Smem::kTileBytes, "the planes fit the tile");
+    auto pick = [](const uint8_t* const (&pl)[3], int k) { return kPlanes == 1 || k == 0 ? pl[0] : k == 1 ? pl[1] : pl[2]; };
+    uintptr_t bits = pitch;
+#pragma unroll
+    for (int k = 0; k < kPlanes; ++k) bits |= reinterpret_cast<uintptr_t>(plane[k]);
+    const bool aligned = (bits & 15) == 0;
+    const bool bulk = aligned && real_w % 16 == 0;                         // the same for every thread of the CTA
+    if (bulk) {
+        if (tid == 0) {
+            ptx::mbar_init(&sm.bar, 1);
+            ptx::mbar_init_fence();
+        }
+        __syncthreads();
+        if (tid < 16 * kPlanes) {
+            const uint32_t row_bytes = nm * 16;
+            if (tid == 0) ptx::mbar_expect_tx(&sm.bar, 16 * kPlanes * row_bytes);
+            const uint32_t sy = min(my * 16 + (tid & 15), real_h - 1);
+            ptx::bulk_g2s(sm.tile + tid * kRow, pick(plane, tid >> 4) + static_cast<size_t>(sy) * pitch + mcu0 * 16, row_bytes, &sm.bar);
+        }
+    }
+    if (p.prefetch_ahead && tid >= 32 && tid < 64) {
+        const uint8_t* pp[3] = {nullptr, nullptr, nullptr};
+        uint32_t ppitch = 0, pw = 0, ph = 0, pm0 = 0, pnm = 0, pby = 0;
+        if constexpr (kMixed) {
+            const uint32_t t = blockIdx.x + p.prefetch_ahead;
+            if (t < p.strips) {                                             // uniform over the warp (geom_find_warp needs all lanes)
+                const uint32_t gi = geom_find_warp(p.geom, p.nframes, t, &FrameGeom::strip0);
+                const FrameGeom& g = p.geom[gi];
+                const uint32_t per_row = (g.mcu_w + kMcus - 1) / kMcus, s = t - g.strip0;
+                pby = s / per_row;
+                pm0 = (s - pby * per_row) * kMcus;
+                pnm = min(static_cast<uint32_t>(kMcus), g.mcu_w - pm0);
+                pp[0] = g.rgb; ppitch = g.pitch; pw = g.real_w; ph = g.real_h;
+                if (kPlanes == 3) { pp[1] = p.planes[2 * gi]; pp[2] = p.planes[2 * gi + 1]; }
+            }
+        } else {
+            const uint32_t lin = blockIdx.y * gridDim.x + blockIdx.x + p.prefetch_ahead, y = lin / gridDim.x;
+            if (y < gridDim.y) {
+                pby = p.mcu_y0 + y;
+                pm0 = (lin - y * gridDim.x) * kMcus;
+                pnm = min(static_cast<uint32_t>(kMcus), p.mcu_w - pm0);
+                pp[0] = p.rgb; ppitch = pitch; pw = real_w; ph = real_h;
+                if (kPlanes == 3) { pp[1] = p.plane_g; pp[2] = p.plane_b; }
+            }
+        }
+        if (pp[0])
+            for (int i = tid - 32; i < 16 * kPlanes; i += 32) {
+                const uint8_t* src = pick(pp, i >> 4);
+                if (((reinterpret_cast<uintptr_t>(src) | ppitch | pw) & 15) == 0) {
+                    const uint32_t sy = min(pby * 16 + (i & 15), ph - 1);
+                    ptx::bulk_prefetch_l2(src + static_cast<size_t>(sy) * ppitch + pm0 * 16, pnm * 16);
+                }
+            }
+    }
+    if (bulk) {
+        ptx::mbar_wait(&sm.bar, 0);
+        return;
+    }
+    const int chunks = kPlanes * 16 * nm;                                   // 16 pixels of one plane row each
+    for (int i = tid; i < chunks; i += kThreads) {
+        const int k = i / (16 * nm), rm = i - k * 16 * nm, r = rm / nm, m = rm - r * nm;
+        const uint8_t* row = pick(plane, k) + static_cast<size_t>(min(my * 16 + r, real_h - 1)) * pitch;
+        const uint32_t x0 = (mcu0 + m) * 16;
+        uint4 v;
+        if (aligned && x0 + 16 <= real_w) {
+            v = __ldg(reinterpret_cast<const uint4*>(row + x0));
+        } else {                                                            // right edge replication, src/Image.cpp:491-530
+            uint32_t q[4];
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                const uint32_t x = x0 + 4 * j;
+                q[j] = row[min(x, real_w - 1)] | (row[min(x + 1, real_w - 1)] << 8) | (row[min(x + 2, real_w - 1)] << 16) |
+                       (static_cast<uint32_t>(row[min(x + 3, real_w - 1)]) << 24);
+            }
+            v = make_uint4(q[0], q[1], q[2], q[3]);
+        }
+        *reinterpret_cast<uint4*>(sm.tile + (k * 16 + r) * kRow + m * 16) = v;
+    }
+    __syncthreads();
+}
+
 // kAligned: real_w % 16 == 0 and 16-byte aligned base -> rows are staged with bulk copies; otherwise a clamped
 // byte loader fills the tile (odd sizes; right-edge replication, src/Image.cpp:491-530)
 // kMixed: images of individual sizes (p.geom): a 1-D grid over the strips of all images; a CTA finds its image by a search
 // over the first-strip prefix.  Otherwise one size: grid (strips of a row, rows, frames).
-// kFmt >= 0: pixels in that JPGENC_PIXEL_* format with a row pitch (stage_layout; kAligned is not used); -1: tight RGB
+// kFmt >= 0: pixels in that JPGENC_PIXEL_* format with a row pitch (stage_layout; grey and planar RGB: stage_planes; kAligned is
+// not used); -1: tight RGB
 template <int kMcus, bool kAligned, bool kBulkOut, bool kMixed, int kFmt = -1>
 // (shared memory and the thread index come from the kernel: there the compiler knows the alignment and, from the launch
 // bounds, the range of threadIdx.x)
@@ -315,10 +410,14 @@ __device__ __forceinline__ void forward_body(const ForwardParams& p, ForwardSmem
     using Smem = ForwardSmem<kMcus>;
     constexpr int kThreads = kMcus * 4;
     const int tid = thread;
+    constexpr bool kPlanar = kFmt == kPixelPlanar, kPlaneTile = kPlanar || kFmt == JPGENC_PIXEL_GRAY;   // stage_planes
     uint32_t my, mcu0, frame_block0, real_w, real_h, mcu_w, pitch;
     const uint8_t* __restrict__ rgb;
+    const uint8_t* plane_gb[2] = {nullptr, nullptr};                      // planar RGB: the G and B planes (rgb is R)
     if constexpr (kMixed) {
-        const FrameGeom& g = p.geom[geom_find_warp(p.geom, p.nframes, blockIdx.x, &FrameGeom::strip0)];
+        const uint32_t gi = geom_find_warp(p.geom, p.nframes, blockIdx.x, &FrameGeom::strip0);
+        const FrameGeom& g = p.geom[gi];
+        if constexpr (kPlanar) { plane_gb[0] = p.planes[2 * gi]; plane_gb[1] = p.planes[2 * gi + 1]; }
         mcu_w = g.mcu_w;
         const uint32_t per_row = (mcu_w + kMcus - 1) / kMcus, s = blockIdx.x - g.strip0;
         my = s / per_row;
@@ -337,11 +436,15 @@ __device__ __forceinline__ void forward_body(const ForwardParams& p, ForwardSmem
         real_h = p.real_h;
         mcu_w = p.mcu_w;
         pitch = p.pitch;
+        if constexpr (kPlanar) { plane_gb[0] = p.plane_g; plane_gb[1] = p.plane_b; }
     }
     const int nm = min(kMcus, static_cast<int>(mcu_w - mcu0));
 
     // ---- stage the 16-row RGB strip ----
-    if constexpr (kFmt >= 0) {
+    if constexpr (kPlaneTile) {
+        const uint8_t* const plane[3] = {rgb, plane_gb[0], plane_gb[1]};
+        stage_planes<kMcus, kPlanar ? 3 : 1, kMixed>(p, sm, tid, plane, pitch, real_w, real_h, my, mcu0, nm);
+    } else if constexpr (kFmt >= 0) {
         stage_layout<kMcus, kFmt, kMixed>(p, sm, tid, rgb, pitch, real_w, real_h, my, mcu0, nm);
     } else if constexpr (kAligned) {
         if (tid == 0) {
@@ -405,6 +508,25 @@ __device__ __forceinline__ void forward_body(const ForwardParams& p, ForwardSmem
 #pragma unroll
             for (int h = 0; h < 2; ++h) {
                 const int r = rp * 2 + h;
+                if constexpr (kPlaneTile) {                       // one 8-byte word per plane holds the thread's 8 pixels
+                    constexpr int kRow = kMcus * 16, kPlaneBytes = 16 * kRow;
+                    const uint8_t* src = sm.tile + (by * 8 + r) * kRow + bx * 8;
+                    const uint2 qr = *reinterpret_cast<const uint2*>(src);
+                    const uint32_t wr[2] = {qr.x, qr.y};
+                    uint32_t wg[2] = {qr.x, qr.y}, wb[2] = {qr.x, qr.y};
+                    if constexpr (kPlanar) {
+                        const uint2 qg = *reinterpret_cast<const uint2*>(src + kPlaneBytes), qb = *reinterpret_cast<const uint2*>(src + 2 * kPlaneBytes);
+                        wg[0] = qg.x; wg[1] = qg.y; wb[0] = qb.x; wb[1] = qb.y;
+                    }
+#pragma unroll
+                    for (int pp = 0; pp < 4; ++pp) {              // pixels 2pp, 2pp+1
+                        rr[h][pp] = bytes_to_f2(wr, 2 * pp, 2 * pp + 1);
+                        gg[h][pp] = kPlanar ? bytes_to_f2(wg, 2 * pp, 2 * pp + 1) : rr[h][pp];
+                        bb[h][pp] = kPlanar ? bytes_to_f2(wb, 2 * pp, 2 * pp + 1) : rr[h][pp];
+                        v[r * 4 + pp] = fma2s(rr[h][pp], cc.y[0], fma2s(gg[h][pp], cc.y[1], fma2s(bb[h][pp], cc.y[2], make_float2(-128.f, -128.f))));
+                    }
+                    continue;
+                }
                 const uint2* src = reinterpret_cast<const uint2*>(sm.tile + (by * 8 + r) * Smem::kPitch + bx * 24);
                 const uint2 q0 = src[0], q1 = src[1], q2 = src[2];
                 const uint32_t w[6] = {q0.x, q0.y, q1.x, q1.y, q2.x, q2.y};
@@ -524,11 +646,18 @@ __device__ __forceinline__ double exact_channel(int comp, double r, double g, do
     return dsub(dadd(128.0, dadd(dadd(dmul((double).5f, r), dmul((double)-.4186f, g)), dmul((double)-.0813f, b))), 128.0);
 }
 
-// kFmt: -1 tight RGB, otherwise the JPGENC_PIXEL_* format of pixels whose rows are `pitch` bytes apart
+// kFmt: -1 tight RGB, otherwise the JPGENC_PIXEL_* format (or kPixelPlanar, with the planes rgb, g, b) of pixels whose rows are
+// `pitch` bytes apart.  A grey pixel v is the pixel (v, v, v).
 template <int kFmt>
 __device__ __forceinline__ double exact_pixel(const uint8_t* rgb, uint32_t pitch, uint32_t real_w, uint32_t real_h, uint32_t x, uint32_t y,
-                                              int comp, double scale) {
+                                              int comp, double scale, const uint8_t* g = nullptr, const uint8_t* b = nullptr) {
     const uint32_t sx = min(x, real_w - 1), sy = min(y, real_h - 1);            // src/Image.cpp:491-530
+    if constexpr (kFmt == JPGENC_PIXEL_GRAY || kFmt == kPixelPlanar) {
+        const size_t at = static_cast<size_t>(sy) * pitch + sx;
+        const double r = dmul(static_cast<double>(rgb[at]), scale);
+        if constexpr (kFmt == JPGENC_PIXEL_GRAY) return exact_channel(comp, r, r, r);
+        else return exact_channel(comp, r, dmul(static_cast<double>(g[at]), scale), dmul(static_cast<double>(b[at]), scale));
+    }
     const uint8_t* px;
     if constexpr (kFmt < 0) px = rgb + (static_cast<size_t>(sy) * real_w + sx) * 3;
     else px = rgb + static_cast<size_t>(sy) * pitch + sx * pixel_bytes(kFmt);
@@ -550,14 +679,16 @@ __device__ __forceinline__ ExactColumn exact_locate(const uint8_t* rgb, uint32_t
     return ExactColumn{rgb, mx * 16 + 2 * c, my * 16, static_cast<int>(k) - 3};
 }
 // spatial sample of row r in the reference's arithmetic
+// (planar RGB: pg, pb are the G and B planes beside b.rgb)
 template <int kFmt = -1>
-__device__ __forceinline__ double exact_sample(const ExactColumn& b, uint32_t real_w, uint32_t real_h, int r, double scale, uint32_t pitch = 0) {
-    if (b.comp == 0) return exact_pixel<kFmt>(b.rgb, pitch, real_w, real_h, b.x, b.y + r, 0, scale);
+__device__ __forceinline__ double exact_sample(const ExactColumn& b, uint32_t real_w, uint32_t real_h, int r, double scale, uint32_t pitch = 0,
+                                               const uint8_t* pg = nullptr, const uint8_t* pb = nullptr) {
+    if (b.comp == 0) return exact_pixel<kFmt>(b.rgb, pitch, real_w, real_h, b.x, b.y + r, 0, scale, pg, pb);
     const uint32_t x = b.x, y = b.y + 2 * r;                                    // S420_m, src/Image.cpp:207-226
-    const double top = dadd(dadd(0.0, exact_pixel<kFmt>(b.rgb, pitch, real_w, real_h, x, y, b.comp, scale)),
-                            exact_pixel<kFmt>(b.rgb, pitch, real_w, real_h, x + 1, y, b.comp, scale));
-    const double bot = dadd(dadd(0.0, exact_pixel<kFmt>(b.rgb, pitch, real_w, real_h, x, y + 1, b.comp, scale)),
-                            exact_pixel<kFmt>(b.rgb, pitch, real_w, real_h, x + 1, y + 1, b.comp, scale));
+    const double top = dadd(dadd(0.0, exact_pixel<kFmt>(b.rgb, pitch, real_w, real_h, x, y, b.comp, scale, pg, pb)),
+                            exact_pixel<kFmt>(b.rgb, pitch, real_w, real_h, x + 1, y, b.comp, scale, pg, pb));
+    const double bot = dadd(dadd(0.0, exact_pixel<kFmt>(b.rgb, pitch, real_w, real_h, x, y + 1, b.comp, scale, pg, pb)),
+                            exact_pixel<kFmt>(b.rgb, pitch, real_w, real_h, x + 1, y + 1, b.comp, scale, pg, pb));
     return dmul(dadd(top, bot), 0.25);          // the reference divides by 4: the same double, bit for bit, without a division
 }
 
@@ -693,6 +824,44 @@ __global__ void __launch_bounds__(kRefineThreads) refine_mixed_kernel(const Fram
         return Column{exact_locate(g.rgb, g.mcu_w, id - g.block0, c), g.real_w, g.real_h, kFmt >= 0 ? g.pitch : 0u};
     };
     auto sample = [&](const Column& col, int r) { return exact_sample<kFmt>(col.col, col.real_w, col.real_h, r, e.scale, col.pitch); };
+    if constexpr (k64) refine_loop64(n0, n, list, false, coef, 0xFFFFFFFFu, e.qy, e.qc, e, locate, sample);
+    else refine_loop(n0, n, list, false, coef, 0xFFFFFFFFu, e.qy, e.qc, e, locate, sample);
+}
+
+// planar RGB, one image: the planes r, g, b with one row pitch (otherwise refine_kernel's single-image form)
+template <bool k64>
+__global__ void __launch_bounds__(kRefineThreads) refine_planar_kernel(const uint8_t* __restrict__ r, const uint8_t* __restrict__ g,
+                                                                           const uint8_t* __restrict__ b, int16_t* __restrict__ coef,
+                                                                           const uint32_t* __restrict__ list, const uint32_t* __restrict__ count,
+                                                                           uint32_t cap, int all, uint32_t nblocks, uint32_t real_w, uint32_t real_h,
+                                                                           uint32_t mcu_w, const __grid_constant__ ExactConsts e, uint32_t pitch) {
+    const uint32_t n = all ? nblocks : min(count[0], cap), n0 = all ? 0u : count[3];
+    auto locate = [&](uint32_t id, int c) { return exact_locate(r, mcu_w, id, c); };
+    auto sample = [&](const ExactColumn& col, int row) { return exact_sample<kPixelPlanar>(col, real_w, real_h, row, e.scale, pitch, g, b); };
+    if constexpr (k64) refine_loop64(n0, n, list, all != 0, coef, nblocks, e.qy, e.qc, e, locate, sample);
+    else refine_loop(n0, n, list, all != 0, coef, nblocks, e.qy, e.qc, e, locate, sample);
+}
+
+// planar RGB, images of individual sizes: image f's G and B planes at planes[2f], planes[2f + 1] (otherwise refine_mixed_kernel)
+template <bool k64>
+__global__ void __launch_bounds__(kRefineThreads) refine_mixed_planar_kernel(const FrameGeom* __restrict__ geom, const uint8_t* const* __restrict__ planes,
+                                                                                 uint32_t nframes, int16_t* __restrict__ coef,
+                                                                                 const uint32_t* __restrict__ list, const uint32_t* __restrict__ count,
+                                                                                 uint32_t cap, const __grid_constant__ ExactConsts e) {
+    const uint32_t n = min(count[0], cap), n0 = count[3];
+    struct Column { ExactColumn col; uint32_t real_w, real_h, pitch; const uint8_t *g, *b; };
+    auto locate = [&](uint32_t id, int c) {
+        uint32_t lo = 0, hi = nframes;
+        while (hi - lo > 1) {
+            const uint32_t mid = (lo + hi) >> 1;
+            if (geom[mid].block0 <= id) lo = mid; else hi = mid;
+        }
+        const FrameGeom& gm = geom[lo];
+        return Column{exact_locate(gm.rgb, gm.mcu_w, id - gm.block0, c), gm.real_w, gm.real_h, gm.pitch, planes[2 * lo], planes[2 * lo + 1]};
+    };
+    auto sample = [&](const Column& col, int r) {
+        return exact_sample<kPixelPlanar>(col.col, col.real_w, col.real_h, r, e.scale, col.pitch, col.g, col.b);
+    };
     if constexpr (k64) refine_loop64(n0, n, list, false, coef, 0xFFFFFFFFu, e.qy, e.qc, e, locate, sample);
     else refine_loop(n0, n, list, false, coef, 0xFFFFFFFFu, e.qy, e.qc, e, locate, sample);
 }
@@ -963,6 +1132,8 @@ static void with_format(int format, F&& f) {
         case JPGENC_PIXEL_RGB: f(std::integral_constant<int, JPGENC_PIXEL_RGB>{}); break;
         case JPGENC_PIXEL_BGR: f(std::integral_constant<int, JPGENC_PIXEL_BGR>{}); break;
         case JPGENC_PIXEL_RGBA: f(std::integral_constant<int, JPGENC_PIXEL_RGBA>{}); break;
+        case JPGENC_PIXEL_GRAY: f(std::integral_constant<int, JPGENC_PIXEL_GRAY>{}); break;
+        case kPixelPlanar: f(std::integral_constant<int, kPixelPlanar>{}); break;
         default: f(std::integral_constant<int, JPGENC_PIXEL_BGRA>{}); break;
     }
 }
@@ -987,7 +1158,16 @@ static int launch_refine(jpgenc_ctx* c, bool all) {
     if (layout_image(c)) {
         with_format(c->pixel_format, [&](auto fmt) {
             constexpr int kFmt = decltype(fmt)::value;
-            if (total < (3u << 19))
+            if constexpr (kFmt == kPixelPlanar) {
+                if (total < (3u << 19))
+                    refine_planar_kernel<true><<<grid, kRefineThreads, 0, c->stream>>>(c->d_rgb, c->d_plane_g, c->d_plane_b, c->d_coef, c->d_refine_list,
+                                                                                      c->d_counters, cap, all ? 1 : 0, bpf, c->real_w, c->real_h, c->mcu_w, e,
+                                                                                      c->row_pitch);
+                else
+                    refine_planar_kernel<false><<<grid, kRefineThreads, 0, c->stream>>>(c->d_rgb, c->d_plane_g, c->d_plane_b, c->d_coef, c->d_refine_list,
+                                                                                       c->d_counters, cap, all ? 1 : 0, bpf, c->real_w, c->real_h, c->mcu_w, e,
+                                                                                       c->row_pitch);
+            } else if (total < (3u << 19))
                 refine_kernel<true, kFmt><<<grid, kRefineThreads, 0, c->stream>>>(c->d_rgb, frames, bpf, c->d_coef, c->d_refine_list, c->d_counters, cap,
                                                                                   all ? 1 : 0, bpf * c->nframes, c->real_w, c->real_h, c->mcu_w, e, c->row_pitch);
             else
@@ -1026,6 +1206,8 @@ int launch_forward_rows(jpgenc_ctx* c, uint32_t y0, uint32_t rows, bool first, b
     if (layout_image(c)) {
         // each CTA picks its staging path from the image (stage_layout); the tensor store serves every full strip
         p.pitch = c->row_pitch;
+        p.plane_g = c->d_plane_g;
+        p.plane_b = c->d_plane_b;
         const bool bulk = make_block_map(c->d_coef, static_cast<uint64_t>(c->mcu_w) * c->mcu_h * kBlocksPerMcu, 32 * kBlocksPerMcu, &p.coef_map);
         with_format(c->pixel_format, [&](auto fmt) {
             constexpr int kFmt = decltype(fmt)::value;
@@ -1060,6 +1242,9 @@ int launch_forward_mixed(jpgenc_ctx* c) {
     c->stats_clear_valid = false;                                 // K2 clears the statistics and K3a's sums itself
     const bool layout = c->mixed.format >= 0;
     const bool aligned = c->mixed.aligned;
+    // planar RGB: the G and B plane pointers lie behind the geometry (enqueue_pass copies them in the same transfer)
+    const uint8_t* const* planes = c->mixed.format == kPixelPlanar ? reinterpret_cast<const uint8_t* const*>(c->d_geom + c->nframes + 1) : nullptr;
+    p.planes = planes;
     const bool bulk_out = (aligned || layout) && make_block_map(c->d_coef, c->mixed.blocks, 32 * kBlocksPerMcu, &p.coef_map);
     if (layout) {
         with_format(c->mixed.format, [&](auto fmt) {
@@ -1079,7 +1264,14 @@ int launch_forward_mixed(jpgenc_ctx* c) {
     if (layout) {
         with_format(c->mixed.format, [&](auto fmt) {
             constexpr int kFmt = decltype(fmt)::value;
-            if (total < (3u << 19))
+            if constexpr (kFmt == kPixelPlanar) {
+                if (total < (3u << 19))
+                    refine_mixed_planar_kernel<true><<<grid, kRefineThreads, 0, c->stream>>>(c->d_geom, planes, c->nframes, c->d_coef, c->d_refine_list,
+                                                                                            c->d_counters, cap, e);
+                else
+                    refine_mixed_planar_kernel<false><<<grid, kRefineThreads, 0, c->stream>>>(c->d_geom, planes, c->nframes, c->d_coef, c->d_refine_list,
+                                                                                             c->d_counters, cap, e);
+            } else if (total < (3u << 19))
                 refine_mixed_kernel<true, kFmt><<<grid, kRefineThreads, 0, c->stream>>>(c->d_geom, c->nframes, c->d_coef, c->d_refine_list, c->d_counters, cap, e);
             else
                 refine_mixed_kernel<false, kFmt><<<grid, kRefineThreads, 0, c->stream>>>(c->d_geom, c->nframes, c->d_coef, c->d_refine_list, c->d_counters, cap, e);

@@ -42,6 +42,7 @@ struct Job {
     const uint32_t* heights = nullptr;
     // pixels in another layout (jpgenc_encode_images_packed_layout; needs widths): JPGENC_PIXEL_* format, -1 tight RGB, and the
     // row pitch of every image as the caller holds it.  `staged`: host images, uploaded into tight rows of their format.
+    // kPixelPlanar (jpgenc_encode_images_packed_planar): three pointers per image, R, G, B; staged as three tight planes back to back.
     int format = -1;
     const uint32_t* pitches = nullptr;
     bool staged = false;
@@ -65,6 +66,8 @@ struct Pass {
 uint32_t job_w(const Job& job, uint32_t i) { return job.widths ? job.widths[i] : job.w; }
 uint32_t job_h(const Job& job, uint32_t i) { return job.heights ? job.heights[i] : job.h; }
 uint32_t job_bpp(const Job& job) { return job.format < 0 ? 3u : pixel_bytes(job.format); }
+// pointers (= planes) per image
+uint32_t job_planes(const Job& job) { return job.format == kPixelPlanar ? 3u : 1u; }
 // bytes from one row of image i to the next where the kernels read it
 uint32_t job_pitch(const Job& job, uint32_t i) { return job.pitches && !job.staged ? job.pitches[i] : job_w(job, i) * job_bpp(job); }
 uint64_t job_blocks(const Job& job, uint32_t i) {
@@ -129,8 +132,9 @@ std::vector<Pass> image_passes(const Job& job, uint32_t slots) {
 }
 
 // The geometry of a pass of images of individual sizes (FrameGeom, F + 1 entries) and its totals.  K3's split follows
-// launch_entropy's rule, applied to the pass's tiles.
-MixedPass image_geometry(const Job& job, const Pass& ps, const void* const* ptrs, FrameGeom* g) {
+// launch_entropy's rule, applied to the pass's tiles.  Planar RGB: ptrs holds R, G, B of every image; FrameGeom::rgb is the R
+// plane, gb[2f], gb[2f + 1] receive the G and B planes.
+MixedPass image_geometry(const Job& job, const Pass& ps, const void* const* ptrs, FrameGeom* g, const void** gb) {
     MixedPass m;
     m.on = true;
     m.aligned = true;
@@ -143,7 +147,9 @@ MixedPass image_geometry(const Job& job, const Pass& ps, const void* const* ptrs
         g[f].block0 = m.blocks; g[f].strip0 = m.strips; g[f].tile0 = m.tiles; g[f].group0 = m.groups; g[f].super0 = m.supers;
         if (f == ps.F) break;
         const uint32_t w = job_w(job, ps.f0 + f), h = job_h(job, ps.f0 + f);
-        g[f].rgb = static_cast<const uint8_t*>(ptrs[f]);
+        const uint32_t np = job_planes(job);
+        g[f].rgb = static_cast<const uint8_t*>(ptrs[np * f]);
+        if (np == 3) { gb[2 * f] = ptrs[3 * f + 1]; gb[2 * f + 1] = ptrs[3 * f + 2]; }
         g[f].real_w = w; g[f].real_h = h; g[f].mcu_w = (w + 15) / 16; g[f].mcu_h = (h + 15) / 16;
         if (job.format >= 0) g[f].pitch = job_pitch(job, ps.f0 + f);
         const uint32_t blocks = g[f].mcu_w * g[f].mcu_h * kBlocksPerMcu, tiles = (blocks + 383) / 384, groups = (tiles * m.split + 7) / 8;
@@ -152,7 +158,7 @@ MixedPass image_geometry(const Job& job, const Pass& ps, const void* const* ptrs
         m.tiles += tiles;
         m.groups += groups;
         m.supers += (groups + 255) / 256;
-        m.aligned = m.aligned && w % 16 == 0 && reinterpret_cast<uintptr_t>(ptrs[f]) % 16 == 0;
+        m.aligned = m.aligned && w % 16 == 0 && reinterpret_cast<uintptr_t>(g[f].rgb) % 16 == 0;
     }
     return m;
 }
@@ -220,17 +226,21 @@ int enqueue_pass(jpgenc_ctx* root, jpgenc_ctx* l, const Job& job, Pass& ps, cons
     l->d_rgb = static_cast<const uint8_t*>(dev_frames[0]);
     l->have_pixels = true;
     std::vector<FrameGeom> geom;
+    std::vector<const void*> gb;
     if (job.widths) {
         geom.resize(F + 1);
-        l->mixed = image_geometry(job, ps, dev_frames, geom.data());
+        gb.resize(job_planes(job) == 3 ? 2 * F : 0);
+        l->mixed = image_geometry(job, ps, dev_frames, geom.data(), gb.data());
     }
     if ((rc = ensure_coef(l))) return rc;
     if ((rc = ensure_stats_buffers(l))) return rc;               // also sizes the pinned staging (stage_bytes(F))
     if (job.widths) {
-        // the geometry (with the frame pointers) travels through pinned memory like the pointer array below
-        const size_t bytes = geom.size() * sizeof(FrameGeom);
+        // the geometry (with the frame pointers; planar RGB: and the G and B planes behind it) travels through pinned memory like
+        // the pointer array below
+        const size_t gbytes = geom.size() * sizeof(FrameGeom), bytes = gbytes + gb.size() * sizeof(void*);
         if ((rc = ensure(l, &l->d_geom, &l->geom_cap, bytes))) return rc;
-        std::memcpy(l->h_pinned, geom.data(), bytes);
+        std::memcpy(l->h_pinned, geom.data(), gbytes);
+        if (!gb.empty()) std::memcpy(static_cast<uint8_t*>(l->h_pinned) + gbytes, gb.data(), gb.size() * sizeof(void*));
         JPGENC_CUDA(l, cudaMemcpyAsync(l->d_geom, l->h_pinned, bytes, cudaMemcpyHostToDevice, l->stream));
     } else {
         size_t cap = l->frame_ptrs_cap;
@@ -447,7 +457,7 @@ int encode_device_frames(jpgenc_ctx* c, Job& job, const void* const* dev_frames)
     const uint32_t nslots = slots_for(pass.size());
     return run_passes(c, job, pass, nslots,
                       [&](uint32_t p, jpgenc_ctx*, const void* const** ptrs, cudaEvent_t* ready) {
-                          *ptrs = dev_frames + pass[p].f0;
+                          *ptrs = dev_frames + static_cast<size_t>(pass[p].f0) * job_planes(job);
                           *ready = nullptr;
                           return JPGENC_OK;
                       },
@@ -472,7 +482,9 @@ int encode_host_frames(jpgenc_ctx* c, Job& job, const uint8_t* const* frames) {
     const uint32_t npasses = static_cast<uint32_t>(pass.size());
     constexpr uint32_t kRingMax = sizeof(c->ev_band) / sizeof(c->ev_band[0]);
     const uint32_t ring = std::min({nslots + 2, npasses, kRingMax});
-    auto fbytes = [&](uint32_t i) { return static_cast<size_t>(job_w(job, i)) * job_h(job, i) * job_bpp(job); };
+    const uint32_t np = job_planes(job);
+    auto plane_bytes = [&](uint32_t i) { return static_cast<size_t>(job_w(job, i)) * job_h(job, i) * job_bpp(job); };
+    auto fbytes = [&](uint32_t i) { return plane_bytes(i) * np; };
     auto fstride = [&](uint32_t i) { return (fbytes(i) + 255) & ~static_cast<size_t>(255); };
     // frame f of pass p sits at slice (p % ring) + at[f0 + f]
     std::vector<size_t> at(job.n);
@@ -491,7 +503,17 @@ int encode_host_frames(jpgenc_ctx* c, Job& job, const uint8_t* const* frames) {
             while (!job.widths && f + run < F && frames[f0 + f + run] == frames[f0 + f + run - 1] + fbytes(0)) ++run;
             uint8_t* dst = c->d_rgb_owned + static_cast<size_t>(s) * slice + at[f0 + f];
             const size_t row = static_cast<size_t>(job_w(job, f0 + f)) * job_bpp(job);
-            if (job.pitches && job.pitches[f0 + f] != row)
+            if (np == 3) {
+                // planar RGB: one copy per plane, or one strided copy when the planes lie back to back with tight rows
+                const uint8_t* const* pl = frames + 3 * static_cast<size_t>(f0 + f);
+                const size_t pb = plane_bytes(f0 + f), h = job_h(job, f0 + f), pitch = job.pitches[f0 + f];
+                const uintptr_t gap = reinterpret_cast<uintptr_t>(pl[1]) - reinterpret_cast<uintptr_t>(pl[0]);
+                if (pitch == row && gap >= pb && gap <= (uintptr_t{1} << 48) && reinterpret_cast<uintptr_t>(pl[2]) - reinterpret_cast<uintptr_t>(pl[1]) == gap)
+                    JPGENC_CUDA(c, cudaMemcpy2DAsync(dst, pb, pl[0], gap, pb, 3, cudaMemcpyHostToDevice, c->copy_stream));
+                else
+                    for (uint32_t k = 0; k < 3; ++k)
+                        JPGENC_CUDA(c, cudaMemcpy2DAsync(dst + k * pb, row, pl[k], pitch, row, h, cudaMemcpyHostToDevice, c->copy_stream));
+            } else if (job.pitches && job.pitches[f0 + f] != row)
                 JPGENC_CUDA(c, cudaMemcpy2DAsync(dst, row, frames[f0 + f], job.pitches[f0 + f], row, job_h(job, f0 + f), cudaMemcpyHostToDevice, c->copy_stream));
             else if (run == 1) JPGENC_CUDA(c, cudaMemcpyAsync(dst, frames[f0 + f], fbytes(f0 + f), cudaMemcpyHostToDevice, c->copy_stream));
             else JPGENC_CUDA(c, cudaMemcpy2DAsync(dst, fstride(0), frames[f0 + f], fbytes(0), fbytes(0), run, cudaMemcpyHostToDevice, c->copy_stream));
@@ -509,8 +531,10 @@ int encode_host_frames(jpgenc_ctx* c, Job& job, const uint8_t* const* frames) {
                     [&](uint32_t p, jpgenc_ctx*, const void* const** out, cudaEvent_t* ready) {
                         const uint32_t f0 = pass[p].f0, F = pass[p].F, s = p % ring;
                         std::vector<const void*>& v = ptrs[p % nslots];
-                        v.resize(F);
-                        for (uint32_t f = 0; f < F; ++f) v[f] = c->d_rgb_owned + static_cast<size_t>(s) * slice + at[f0 + f];
+                        v.resize(static_cast<size_t>(F) * np);
+                        for (uint32_t f = 0; f < F; ++f)
+                            for (uint32_t k = 0; k < np; ++k)
+                                v[f * np + k] = c->d_rgb_owned + static_cast<size_t>(s) * slice + at[f0 + f] + k * plane_bytes(f0 + f);
                         *out = v.data();
                         *ready = c->ev_band[s];
                         return JPGENC_OK;
@@ -593,7 +617,7 @@ int jpgenc_encode_images_packed_layout(jpgenc_ctx* c, uint32_t n, const void* co
                                        uint64_t cap, uint64_t* offsets, uint64_t* sizes, uint64_t* total_bytes) try {
     if (!c) return JPGENC_ERR_ARG;
     if (total_bytes) *total_bytes = 0;
-    if (format < JPGENC_PIXEL_RGB || format > JPGENC_PIXEL_BGRA) return fail(c, JPGENC_ERR_ARG, "unknown pixel format");
+    if ((format < JPGENC_PIXEL_RGB || format > JPGENC_PIXEL_BGRA) && format != JPGENC_PIXEL_GRAY) return fail(c, JPGENC_ERR_ARG, "unknown pixel format");
     if (maxval == 0 || maxval > 255) return fail(c, JPGENC_ERR_ARG, "maxval out of range");
     if (n == 0) return JPGENC_OK;                                // an empty batch is legal and touches nothing
     if (!images || !widths || !heights || !offsets || !sizes) return fail(c, JPGENC_ERR_ARG, "null argument");
@@ -617,6 +641,35 @@ int jpgenc_encode_images_packed_layout(jpgenc_ctx* c, uint32_t n, const void* co
     job.format = format; job.pitches = pitch.data();
     job.packed_mode = true; job.packed = out; job.packed_cap = cap; job.offsets = offsets; job.sizes = sizes;
     const int rc = images_on_device ? encode_device_frames(c, job, images) : encode_host_frames(c, job, reinterpret_cast<const uint8_t* const*>(images));
+    if (total_bytes) *total_bytes = job.packed_at;
+    return rc;
+} JPGENC_CATCH(c)
+
+int jpgenc_encode_images_packed_planar(jpgenc_ctx* c, uint32_t n, const void* const* planes, int images_on_device, const uint32_t* widths,
+                                       const uint32_t* heights, const uint32_t* row_pitches, uint32_t maxval, uint8_t* out, uint64_t cap,
+                                       uint64_t* offsets, uint64_t* sizes, uint64_t* total_bytes) try {
+    if (!c) return JPGENC_ERR_ARG;
+    if (total_bytes) *total_bytes = 0;
+    if (maxval == 0 || maxval > 255) return fail(c, JPGENC_ERR_ARG, "maxval out of range");
+    if (n == 0) return JPGENC_OK;                                // an empty batch is legal and touches nothing
+    if (!planes || !widths || !heights || !offsets || !sizes) return fail(c, JPGENC_ERR_ARG, "null argument");
+    std::vector<uint32_t> pitch(n);
+    for (uint32_t i = 0; i < n; ++i) {
+        if (!planes[3 * i] || !planes[3 * i + 1] || !planes[3 * i + 2]) return fail(c, JPGENC_ERR_ARG, "null plane pointer");
+        pitch[i] = row_pitches ? row_pitches[i] : 0;
+        const int rc = check_layout(c, widths[i], heights[i], &pitch[i], JPGENC_PIXEL_GRAY);   // every plane: one byte per pixel
+        if (rc) return rc;
+    }
+    if (!images_on_device && maxval < 255)
+        for (uint32_t i = 0; i < 3 * n; ++i)
+            if (!samples_within_maxval(static_cast<const uint8_t*>(planes[i]), widths[i / 3], heights[i / 3], pitch[i / 3], 1, maxval))
+                return fail(c, JPGENC_ERR_FORMAT, "a sample exceeds maxval");
+    Job job;
+    job.n = n; job.w = widths[0]; job.h = heights[0]; job.maxval = maxval;
+    job.widths = widths; job.heights = heights;
+    job.format = kPixelPlanar; job.pitches = pitch.data();
+    job.packed_mode = true; job.packed = out; job.packed_cap = cap; job.offsets = offsets; job.sizes = sizes;
+    const int rc = images_on_device ? encode_device_frames(c, job, planes) : encode_host_frames(c, job, reinterpret_cast<const uint8_t* const*>(planes));
     if (total_bytes) *total_bytes = job.packed_at;
     return rc;
 } JPGENC_CATCH(c)

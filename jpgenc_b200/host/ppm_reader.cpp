@@ -96,9 +96,9 @@ bool samples_within_maxval(const uint8_t* px, size_t count, uint32_t maxval) {
 
 bool samples_within_maxval(const uint8_t* px, uint32_t w, uint32_t h, size_t pitch, uint32_t bpp, uint32_t maxval) {
     if (maxval >= 255) return true;
-    if (bpp == 3) {
+    if (bpp == 3 || bpp == 1) {
         for (uint32_t y = 0; y < h; ++y)
-            if (!samples_within_maxval(px + y * pitch, static_cast<size_t>(w) * 3, maxval)) return false;
+            if (!samples_within_maxval(px + y * pitch, static_cast<size_t>(w) * bpp, maxval)) return false;
         return true;
     }
     uint8_t over = 0;

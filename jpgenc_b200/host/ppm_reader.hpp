@@ -22,8 +22,8 @@ int ppm_samples(const uint8_t* file, size_t n, const PpmHeader& h, std::vector<u
 // false when a sample exceeds maxval (< 255): such a file is refused (JPGENC_ERR_FORMAT) -- the reference would scale the sample past 255,
 // which the 8-bit device path is not exact for; jpgenc_encode_planes takes such data as planes of doubles
 bool samples_within_maxval(const uint8_t* px, size_t count, uint32_t maxval);
-// the same for h rows of w pixels, `pitch` bytes apart, `bpp` bytes per pixel of which the first three are colour: a 4th byte and
-// the bytes between rows are not samples and are not read
+// the same for h rows of w pixels, `pitch` bytes apart, `bpp` bytes per pixel of which the first three are colour (bpp 1: a grey
+// pixel or one plane of planar RGB): a 4th byte and the bytes between rows are not samples and are not read
 bool samples_within_maxval(const uint8_t* px, uint32_t w, uint32_t h, size_t pitch, uint32_t bpp, uint32_t maxval);
 // whole file into memory; JPGENC_ERR_IO when it cannot be opened
 int slurp_file(const std::string& path, std::vector<uint8_t>* out);
