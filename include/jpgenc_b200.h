@@ -119,6 +119,20 @@ int jpgenc_bind_device_image(jpgenc_ctx* ctx, const void* dev, uint32_t real_w, 
  * A null plane, pitch below real_w, sides outside 1..65535: JPGENC_ERR_ARG. */
 int jpgenc_bind_device_planar(jpgenc_ctx* ctx, const void* r, const void* g, const void* b, uint32_t real_w, uint32_t real_h,
                               uint32_t row_pitch, uint32_t maxval);
+/* YUV 4:2:0 frames with 8-bit samples, as video decoders leave them.  A w x h frame has a Y plane of h rows of w bytes, y_pitch
+ * apart (0 = w), and chroma planes of ch = ceil(h/2) rows of cw = ceil(w/2) samples, c_pitch apart:
+ *   JPGENC_YUV_I420: U and V planes of cw bytes per row (0 = cw); YV12 is I420 with the u and v pointers swapped;
+ *   JPGENC_YUV_NV12: one plane of cw (U, V) byte pairs per row (0 = 2 cw), passed as u; v must be NULL.
+ * The samples are the file's Y, Cb and Cr as they are (JFIF reads them as full-range BT.601; no range or matrix conversion is
+ * done, and there is no maxval): the file is jpgenc_encode_planes(..., ycbcr = 1) of the planes Y - 128, Cb - 128, Cr - 128
+ * with every chroma sample repeated over its 2x2 pixels and the frame padded to whole MCUs by edge replication -- the
+ * reference's own 4:2:0 file of that YCbCr image, byte for byte.  Then jpgenc_color_dct_quant / jpgenc_encode_bound as after
+ * any other bind.  Unknown layout, a null Y or U plane, a null V plane for I420 or a non-null one for NV12, a pitch below its
+ * row size, sides outside 1..65535: JPGENC_ERR_ARG. */
+#define JPGENC_YUV_I420 0   /* Y, U, V planes */
+#define JPGENC_YUV_NV12 1   /* Y plane, interleaved UV plane (passed as u; v must be NULL) */
+int jpgenc_bind_device_yuv420(jpgenc_ctx* ctx, const void* y, const void* u, const void* v, uint32_t w, uint32_t h, uint32_t y_pitch,
+                              uint32_t c_pitch, int layout);
 
 /* ---- K1: convertToColorSpace(YCbCr) + applySubsampling(S420_m) + applyDCT(Arai) + applyQuantization
  *      + zigzag (src/Image.cpp:112-148, 198-235, 540-595, 597-636; Dct.hpp:47-215; Coding.hpp:57-97) -- */
@@ -185,6 +199,11 @@ int jpgenc_encode_image(jpgenc_ctx* ctx, const void* host, uint32_t real_w, uint
  * 255, in all three planes. */
 int jpgenc_encode_planar(jpgenc_ctx* ctx, const void* r, const void* g, const void* b, uint32_t real_w, uint32_t real_h,
                          uint32_t row_pitch, uint32_t maxval, uint8_t* dst, uint64_t cap, uint64_t* jpeg_bytes);
+/* the same for a YUV 4:2:0 frame in host memory (see jpgenc_bind_device_yuv420): every plane travels as it is, 1.5 bytes per
+ * pixel in all, the pitch gaps dropped by the copy engine; the upload of each band of MCU rows overlaps the kernels of the
+ * bands before it. */
+int jpgenc_encode_yuv420(jpgenc_ctx* ctx, const void* y, const void* u, const void* v, uint32_t w, uint32_t h, uint32_t y_pitch,
+                         uint32_t c_pitch, int layout, uint8_t* dst, uint64_t cap, uint64_t* jpeg_bytes);
 /* Image::writeJPEG (src/Image.cpp:831-976) for an image given as the reference holds it: three row-major planes of doubles
  * (Image::R/G/B, include/Image.hpp:104-114), `width` x `height` = the image padded to whole 16x16 MCUs (src/Image.cpp:479-530),
  * real_w x real_h = what SOF0 reports.  ycbcr != 0: the planes already are level-shifted Y, Cb, Cr and are not converted
@@ -257,6 +276,13 @@ int jpgenc_encode_images_packed_layout(jpgenc_ctx* ctx, uint32_t n, const void* 
 int jpgenc_encode_images_packed_planar(jpgenc_ctx* ctx, uint32_t n, const void* const* planes, int images_on_device,
                                        const uint32_t* widths, const uint32_t* heights, const uint32_t* row_pitches, uint32_t maxval,
                                        uint8_t* out, uint64_t cap, uint64_t* offsets, uint64_t* sizes, uint64_t* total_bytes);
+/* jpgenc_encode_images_packed_layout for YUV 4:2:0 frames of one layout (see jpgenc_bind_device_yuv420): planes[3i],
+ * planes[3i + 1], planes[3i + 2] are Y, U and V of image i (NV12: Y, UV, NULL), y_pitches[i] / c_pitches[i] its pitches (either
+ * array may be NULL: all tight; an entry of 0 is tight too).  Host frames are uploaded plane by plane in tight rows. */
+int jpgenc_encode_images_packed_yuv420(jpgenc_ctx* ctx, uint32_t n, const void* const* planes, int images_on_device,
+                                       const uint32_t* widths, const uint32_t* heights, const uint32_t* y_pitches,
+                                       const uint32_t* c_pitches, int layout, uint8_t* out, uint64_t cap, uint64_t* offsets,
+                                       uint64_t* sizes, uint64_t* total_bytes);
 
 /* ---- stage methods for the modes writeJPEG does not use (SURVEY.md 8(f)4) ------------------------------------------ */
 /* Image::applySubsampling(mode) on one chroma plane (src/Image.cpp:198-319): `plane` = height x width doubles (host), mode =

@@ -18,6 +18,8 @@ ERR_CUDA, ERR_ARG, ERR_NO_DEVICE, ERR_FORMAT, ERR_IO, ERR_CAPACITY, ERR_NOMEM = 
 
 # JPGENC_PIXEL_*: name -> (code, bytes per pixel); a GRAY pixel v is encoded as the pixel (v, v, v)
 PIXEL_FORMATS = {"RGB": (0, 3), "BGR": (1, 3), "RGBA": (2, 4), "BGRA": (3, 4), "GRAY": (16, 1)}
+# YUV 4:2:0 frames (JPGENC_YUV_*): Y, U, V planes / Y plane and interleaved UV plane
+YUV_LAYOUTS = {"I420": 0, "NV12": 1}
 
 u8p = C.POINTER(C.c_uint8)
 i16p = C.POINTER(C.c_int16)
@@ -65,6 +67,10 @@ _SIGNATURES = {
     "jpgenc_bind_device_image": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int, C.c_uint32]),
     "jpgenc_bind_device_planar": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32]),
     "jpgenc_encode_planar": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32,
+                                       C.c_void_p, C.c_uint64, u64p]),
+    "jpgenc_bind_device_yuv420": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32,
+                                            C.c_int]),
+    "jpgenc_encode_yuv420": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int,
                                        C.c_void_p, C.c_uint64, u64p]),
     "jpgenc_encode_image": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int, C.c_uint32, C.c_void_p, C.c_uint64,
                                       u64p]),
@@ -118,6 +124,8 @@ _SIGNATURES = {
     "jpgenc_encode_images_packed_layout": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(C.c_void_p), C.c_int, u32p, u32p, u32p, C.c_int,
                                                      C.c_uint32, C.c_void_p, C.c_uint64, u64p, u64p, u64p]),
     "jpgenc_encode_images_packed_planar": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(C.c_void_p), C.c_int, u32p, u32p, u32p, C.c_uint32,
+                                                     C.c_void_p, C.c_uint64, u64p, u64p, u64p]),
+    "jpgenc_encode_images_packed_yuv420": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(C.c_void_p), C.c_int, u32p, u32p, u32p, u32p, C.c_int,
                                                      C.c_void_p, C.c_uint64, u64p, u64p, u64p]),
     "jpgenc_batch_create": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "jpgenc_batch_destroy": (None, [C.c_void_p]),
@@ -241,6 +249,65 @@ def tensor_layout(t, order: str = "RGB"):
                      "channels_last, (H, W, 3|4) with strides (pitch, C, 1), or (H, W) / (1, H, W) grey")
 
 
+def _u8_plane(a, what: str):
+    """(pointer, shape, strides in bytes) of a uint8 numpy array or torch tensor (metadata only)"""
+    if isinstance(a, np.ndarray):
+        if a.dtype != np.uint8:
+            raise ValueError(f"{what} must be uint8, not {a.dtype}")
+        ptr, shape, strides = a.ctypes.data, tuple(a.shape), tuple(a.strides)
+    elif type(a).__module__.split(".")[0] == "torch" and hasattr(a, "stride"):
+        if str(a.dtype) != "torch.uint8":
+            raise ValueError(f"{what} must be uint8, not {a.dtype}")
+        ptr, shape, strides = a.data_ptr(), tuple(a.shape), tuple(a.stride())
+    else:
+        raise ValueError(f"{what} must be a numpy array or a torch tensor")
+    if 0 in shape:
+        raise ValueError(f"{what} is empty")
+    return ptr, shape, strides
+
+
+def yuv420_layout(y, u, v=None):
+    """How a YUV 4:2:0 frame is read in place: (layout, (y, u, v or 0) pointers, width, height, y_pitch, c_pitch).
+
+    y, u, v are uint8 numpy arrays or torch tensors.  Accepted, for a frame of H x W and ch = ceil(H/2), cw = ceil(W/2):
+      Y                        (H, W) with strides (y_pitch, 1)
+      I420 (v given)           U and V (ch, cw), strides (c_pitch, 1) with one c_pitch for both
+      NV12 (v is None)         UV (ch, cw, 2) with strides (c_pitch, 2, 1), or (ch, 2 cw) with strides (c_pitch, 1)
+    Anything else raises ValueError; nothing is ever copied.  Pure: only the metadata is read."""
+    yp, ys, yst = _u8_plane(y, "Y")
+    if len(ys) != 2:
+        raise ValueError(f"Y must be (H, W), not {ys}")
+    h, w = ys
+    y_pitch = yst[0] if h > 1 else w
+    if (w > 1 and yst[1] != 1) or y_pitch < w:
+        raise ValueError(f"Y must have strides (pitch, 1) with pitch >= {w}; got {yst}")
+    ch, cw = (h + 1) // 2, (w + 1) // 2
+    up, us, ust = _u8_plane(u, "U")
+    if v is None:
+        if us == (ch, cw, 2):
+            ok = (cw == 1 or ust[1] == 2) and ust[2] == 1
+        elif us == (ch, 2 * cw):
+            ok = ust[1] == 1
+        else:
+            raise ValueError(f"NV12 UV must be ({ch}, {cw}, 2) or ({ch}, {2 * cw}) for a {h} x {w} frame, not {us}")
+        c_pitch = ust[0] if ch > 1 else 2 * cw
+        if not ok or c_pitch < 2 * cw:
+            raise ValueError(f"NV12 UV must have strides (pitch, 2, 1) or (pitch, 1) with pitch >= {2 * cw}; got {ust}")
+        return "NV12", (yp, up, 0), w, h, y_pitch, c_pitch
+    vp, vs, vst = _u8_plane(v, "V")
+    pitches = []
+    for name, shape, st in (("U", us, ust), ("V", vs, vst)):
+        if shape != (ch, cw):
+            raise ValueError(f"I420 {name} must be ({ch}, {cw}) for a {h} x {w} frame, not {shape}")
+        pitch = st[0] if ch > 1 else cw
+        if (cw > 1 and st[1] != 1) or pitch < cw:
+            raise ValueError(f"I420 {name} must have strides (pitch, 1) with pitch >= {cw}; got {st}")
+        pitches.append(pitch)
+    if pitches[0] != pitches[1]:
+        raise ValueError(f"I420 U and V must share one row stride; got {pitches[0]} and {pitches[1]}")
+    return "I420", (yp, up, vp), w, h, y_pitch, pitches[0]
+
+
 class Encoder:
     """One GPU context (= one CUDA stream + its device buffers).  Methods mirror the C-ABI one to one."""
 
@@ -300,6 +367,10 @@ class Encoder:
         self._check(self.lib.jpgenc_bind_device_planar(self.h, r, g, b, w, h, pitch, maxval))
 
     # ---- stages ---------------------------------------------------------------------------------
+    def bind_device_yuv420(self, y: int, u: int, v: int | None, w: int, h: int, y_pitch: int = 0, c_pitch: int = 0, layout: str = "I420"):
+        """a YUV 4:2:0 frame in device memory (plane pointers; NV12: v None, u the UV plane; pitches 0: tight)"""
+        self._check(self.lib.jpgenc_bind_device_yuv420(self.h, y, u, v or None, w, h, y_pitch, c_pitch, YUV_LAYOUTS[layout]))
+
     def color_dct_quant(self):
         self._check(self.lib.jpgenc_color_dct_quant(self.h))
 
@@ -415,6 +486,21 @@ class Encoder:
             self._check(rc)
             return out[: n.value].tobytes()
 
+    def encode_yuv420_ptr(self, y: int, u: int, v: int | None, w: int, h: int, y_pitch: int = 0, c_pitch: int = 0,
+                          layout: str = "I420") -> bytes:
+        """a YUV 4:2:0 frame in host memory (plane pointers, see bind_device_yuv420) -> JPEG bytes"""
+        cap = max(4096, w * h * 3 // 2 + 4096)
+        while True:
+            out = np.empty(cap, np.uint8)
+            n = C.c_uint64()
+            rc = self.lib.jpgenc_encode_yuv420(self.h, y, u, v or None, w, h, y_pitch, c_pitch, YUV_LAYOUTS[layout], out.ctypes.data, cap,
+                                               C.byref(n))
+            if rc == ERR_CAPACITY:
+                cap = int(n.value) + 16
+                continue
+            self._check(rc)
+            return out[: n.value].tobytes()
+
     def encode_planes(self, p0: np.ndarray, p1: np.ndarray, p2: np.ndarray, real_w: int, real_h: int, ycbcr: bool = False) -> bytes:
         """three (H16, W16) float64 planes as the reference's Image holds them -> JPEG bytes (exact FP64 path for every block)"""
         planes = [np.ascontiguousarray(p, np.float64) for p in (p0, p1, p2)]
@@ -516,6 +602,85 @@ class Encoder:
                                                                 _np_ptr(p, u32p) if p is not None else None, maxval, out_ptr, cap, offs,
                                                                 sizes, C.byref(total)))
         return [int(x) for x in offs], [int(x) for x in sizes], int(total.value)
+
+    def encode_images_packed_yuv420(self, planes, widths, heights, out_ptr: int | None, cap: int, layout: str = "I420", host_images=False,
+                                    y_pitches=None, c_pitches=None):
+        """YUV 4:2:0 frames of individual sizes: planes[3i:3i + 3] = the Y, U, V plane pointers of frame i (NV12: Y, UV, None;
+        device memory, or host memory with host_images=True), pitches per frame (None or 0: tight) -> files back to back as
+        encode_images_packed"""
+        n = len(widths)
+        pl = (C.c_void_p * (3 * n))(*planes)
+        w = np.ascontiguousarray(widths, np.uint32)
+        h = np.ascontiguousarray(heights, np.uint32)
+        yp = np.ascontiguousarray(y_pitches, np.uint32) if y_pitches is not None else None
+        cp = np.ascontiguousarray(c_pitches, np.uint32) if c_pitches is not None else None
+        sizes = (C.c_uint64 * n)()
+        offs = (C.c_uint64 * n)()
+        total = C.c_uint64()
+        self._check(self.lib.jpgenc_encode_images_packed_yuv420(self.h, n, pl, 0 if host_images else 1, _np_ptr(w, u32p), _np_ptr(h, u32p),
+                                                                _np_ptr(yp, u32p) if yp is not None else None,
+                                                                _np_ptr(cp, u32p) if cp is not None else None, YUV_LAYOUTS[layout], out_ptr,
+                                                                cap, offs, sizes, C.byref(total)))
+        return [int(x) for x in offs], [int(x) for x in sizes], int(total.value)
+
+    def _planes_on_host(self, planes) -> bool:
+        """True for numpy arrays and CPU tensors; False for tensors on this encoder's GPU, once the work queued on torch's current
+        stream has finished.  Anything else (a mix, another device) raises ValueError."""
+        kinds = set()
+        for a in planes:
+            if isinstance(a, np.ndarray):
+                kinds.add("cpu")
+            else:
+                dev = a.device
+                if dev.type == "cuda" and dev.index != self.device:
+                    raise ValueError(f"tensor on {dev}, encoder on cuda:{self.device}")
+                if dev.type not in ("cpu", "cuda"):
+                    raise ValueError(f"tensors on {dev} cannot be read")
+                kinds.add(dev.type)
+        if len(kinds) != 1:
+            raise ValueError("the planes of one call must all be in host memory or all on the encoder's GPU")
+        if kinds.pop() == "cpu":
+            return True
+        import torch
+
+        dev = torch.device("cuda", self.device)
+        ev = torch.cuda.Event()
+        ev.record(torch.cuda.current_stream(dev))
+        ev.synchronize()
+        return False
+
+    def encode_yuv420(self, y, u, v=None) -> bytes:
+        """one YUV 4:2:0 frame read in place (yuv420_layout: I420 with v, NV12 without) from numpy arrays, CPU tensors or tensors on
+        this encoder's GPU -> JPEG bytes"""
+        layout, (yp, up, vp), w, h, y_pitch, c_pitch = yuv420_layout(y, u, v)
+        if self._planes_on_host([a for a in (y, u, v) if a is not None]):
+            return self.encode_yuv420_ptr(yp, up, vp, w, h, y_pitch, c_pitch, layout)
+        self.bind_device_yuv420(yp, up, vp, w, h, y_pitch, c_pitch, layout)
+        n = self.encode_bound(None)
+        out = np.empty(n, np.uint8)
+        n = C.c_uint64()
+        self._check(self.lib.jpgenc_assemble_last(self.h, out.ctypes.data, out.size, C.byref(n)))
+        return out[: n.value].tobytes()
+
+    def encode_yuv420_many(self, frames):
+        """(y, u) NV12 or (y, u, v) I420 frames of any sizes, one layout per call, all in host memory or all on this encoder's GPU
+        (see encode_yuv420), through one batched call -> list of JPEG byte strings"""
+        frames = [tuple(f) for f in frames]
+        if not frames:
+            return []
+        layouts = [yuv420_layout(*f) for f in frames]
+        kinds = {x[0] for x in layouts}
+        if len(kinds) != 1:
+            raise ValueError(f"one YUV layout per call; got {sorted(kinds)}")
+        host = self._planes_on_host([a for f in frames for a in f if a is not None])
+        planes = [p or None for x in layouts for p in x[1]]
+        ws = [x[2] for x in layouts]
+        hs = [x[3] for x in layouts]
+        yps = [x[4] for x in layouts]
+        cps = [x[5] for x in layouts]
+        layout = layouts[0][0]
+        enc = lambda o, c: self.encode_images_packed_yuv420(planes, ws, hs, o, c, layout, host_images=host, y_pitches=yps, c_pitches=cps)
+        return self._files(enc, sum(w * h for w, h in zip(ws, hs)), len(frames))
 
     def _files(self, encode, pixels: int, n: int):
         """encode(out_ptr, cap) -> (offsets, sizes, total) into a host buffer, again with the reported size when the files

@@ -87,6 +87,22 @@ int check_layout(jpgenc_ctx* c, uint32_t w, uint32_t h, uint32_t* row_pitch, int
     return JPGENC_OK;
 }
 
+// a YUV 4:2:0 frame's planes and pitches (jpgenc_bind_device_yuv420): 0 pitches become tight; the internal format on success
+int check_yuv420(jpgenc_ctx* c, const void* y, const void* u, const void* v, uint32_t w, uint32_t h, uint32_t* y_pitch, uint32_t* c_pitch,
+                 int layout, int* format) {
+    if (layout != JPGENC_YUV_I420 && layout != JPGENC_YUV_NV12) return fail(c, JPGENC_ERR_ARG, "unknown YUV layout");
+    if (!y || !u) return fail(c, JPGENC_ERR_ARG, "null plane pointer");
+    if (layout == JPGENC_YUV_I420 && !v) return fail(c, JPGENC_ERR_ARG, "null V plane (I420)");
+    if (layout == JPGENC_YUV_NV12 && v) return fail(c, JPGENC_ERR_ARG, "NV12 takes its UV plane as u; v must be NULL");
+    int rc = check_layout(c, w, h, y_pitch, JPGENC_PIXEL_GRAY);           // the Y plane: one byte per pixel
+    if (rc) return rc;
+    const uint32_t crow = ((w + 1) / 2) * (layout == JPGENC_YUV_NV12 ? 2 : 1);
+    if (*c_pitch == 0) *c_pitch = crow;
+    if (*c_pitch < crow) return fail(c, JPGENC_ERR_ARG, "chroma pitch below the chroma row size");
+    *format = layout == JPGENC_YUV_NV12 ? kPixelNV12 : kPixelI420;
+    return JPGENC_OK;
+}
+
 // pinned host staging, grown on demand
 int ensure_pinned(jpgenc_ctx* c, size_t bytes) {
     if (c->pinned_bytes >= bytes) return JPGENC_OK;
@@ -431,6 +447,22 @@ int jpgenc_bind_device_planar(jpgenc_ctx* c, const void* r, const void* g, const
     c->d_rgb = static_cast<const uint8_t*>(r);
     c->d_plane_g = static_cast<const uint8_t*>(g);
     c->d_plane_b = static_cast<const uint8_t*>(b);
+    c->have_pixels = true;
+    return JPGENC_OK;
+} JPGENC_CATCH(c)
+
+int jpgenc_bind_device_yuv420(jpgenc_ctx* c, const void* y, const void* u, const void* v, uint32_t w, uint32_t h, uint32_t y_pitch,
+                              uint32_t c_pitch, int layout) try {
+    if (!c) return JPGENC_ERR_ARG;
+    int format = 0;
+    int rc = check_yuv420(c, y, u, v, w, h, &y_pitch, &c_pitch, layout, &format);
+    if (rc || (rc = set_geometry(c, w, h, 255))) return rc;
+    c->pixel_format = format;
+    c->row_pitch = y_pitch;
+    c->d_rgb = static_cast<const uint8_t*>(y);
+    c->d_plane_g = static_cast<const uint8_t*>(u);
+    c->d_plane_b = static_cast<const uint8_t*>(v);
+    c->chroma_pitch = c_pitch;
     c->have_pixels = true;
     return JPGENC_OK;
 } JPGENC_CATCH(c)
@@ -853,12 +885,13 @@ static int run_pipeline(jpgenc_ctx* c, jpgenc_huff_table tables[4], uint64_t* sc
     if ((rc = ensure_stats_buffers(c))) return rc;
     // ---- phase A: K1, refinement, K2, statistics into the mailbox ----
     c->k2_tiles_done = 0;
-    // (the pixel layout picks K1 and the refinement: it is part of the key)
-    const bool planar = c->pixel_format == kPixelPlanar;
+    // (the pixel layout picks K1, its thresholds and the refinement: it is part of the key, with every plane and pitch)
+    const bool planes = c->pixel_format == kPixelPlanar || is_yuv(c->pixel_format);
     const uint64_t key_a[kGraphKeyWords] = {c->alloc_gen, reinterpret_cast<uint64_t>(c->d_rgb), (static_cast<uint64_t>(c->real_w) << 32) | c->real_h,
                                             c->maxval | static_cast<uint64_t>(c->pixel_format) << 8 | static_cast<uint64_t>(c->row_pitch) << 32,
                                             1u | static_cast<uint64_t>(c->stage_timing) << 8,
-                                            planar ? reinterpret_cast<uint64_t>(c->d_plane_g) : 0, planar ? reinterpret_cast<uint64_t>(c->d_plane_b) : 0};
+                                            planes ? reinterpret_cast<uint64_t>(c->d_plane_g) : 0, planes ? reinterpret_cast<uint64_t>(c->d_plane_b) : 0,
+                                            is_yuv(c->pixel_format) ? c->chroma_pitch : 0};
     const bool pool = c->parallel_tables;
     if (pool) {
         if (!c->pool) c->pool = new TablePool(kTableWorkers);
@@ -896,7 +929,7 @@ static int run_pipeline(jpgenc_ctx* c, jpgenc_huff_table tables[4], uint64_t* sc
     if (k4_tiles > c->k4_grid_hint || k4_tiles < c->k4_grid_hint / 4) c->k4_grid_hint = k4_tiles + k4_tiles / 2 + 8;
     const uint32_t k4_grid = std::min(c->k4_grid_hint, static_cast<uint32_t>(c->raw_cap / kK4TileBytes + 1));   // raw_cap holds the scan: >= k4_tiles
     const uint64_t key_b[kGraphKeyWords] = {c->alloc_gen, k4_grid, (static_cast<uint64_t>(c->real_w) << 32) | c->real_h, 0,
-                                            1u | static_cast<uint64_t>(c->stage_timing) << 8, 0, 0};
+                                            1u | static_cast<uint64_t>(c->stage_timing) << 8, 0, 0, 0};
     if ((rc = run_phase(c, c->graph_b, key_b, [&]() -> int { return enqueue_entropy_phase(c, k4_grid); }))) return rc;
     if ((rc = wait_entropy(c))) return rc;
     if (scan) *scan = c->stats.scan_bytes;
@@ -924,21 +957,30 @@ static int ensure_file_staging(jpgenc_ctx* c, size_t bytes) {
 // Pixels in another layout (`format`, rows `pitch` bytes apart in host memory) travel as they are, in their own format, the
 // pitch gap dropped by the copy: on the device they are tight rows of that format, read by the pixel-layout kernels.
 // Planar RGB (kPixelPlanar; host_rgb, host_g, host_b are the planes) lands as three tight planes back to back.
+// YUV 4:2:0 (kPixelI420 / kPixelNV12; host_rgb is Y with `pitch`, host_g and host_b are U and V -- NV12: UV -- with `c_pitch`)
+// lands as tight planes, each starting on 256 bytes; a band carries its 16 Y rows and 8 chroma rows per MCU row.
 static int upload_and_forward(jpgenc_ctx* c, const uint8_t* host_rgb, uint32_t w, uint32_t h, uint32_t maxval,
                               const std::function<int(uint8_t*, size_t, size_t)>* fill = nullptr, int format = JPGENC_PIXEL_RGB,
-                              size_t pitch = 0, const uint8_t* host_g = nullptr, const uint8_t* host_b = nullptr) {
+                              size_t pitch = 0, const uint8_t* host_g = nullptr, const uint8_t* host_b = nullptr, size_t c_pitch = 0) {
     JPGENC_CUDA(c, cudaSetDevice(c->device));
     int rc = set_geometry(c, w, h, maxval);
     if (rc) return rc;
     const size_t row_bytes = static_cast<size_t>(w) * pixel_bytes(format), bytes = row_bytes * h;
+    const bool yuv = is_yuv(format);
     const uint32_t nplanes = format == kPixelPlanar ? 3 : 1;
     if (pitch == 0) pitch = row_bytes;
     c->pixel_format = format;
     c->row_pitch = static_cast<uint32_t>(row_bytes);
-    if ((rc = ensure(c, &c->d_rgb_owned, &c->rgb_cap, nplanes * bytes + 16))) return rc;
+    // YUV: chroma rows of crow bytes, ch of them, in ncp planes behind the Y plane
+    const size_t crow = static_cast<size_t>((w + 1) / 2) * (format == kPixelNV12 ? 2 : 1), ch = (h + 1) / 2;
+    const uint32_t ncp = format == kPixelI420 ? 2 : 1;
+    auto align256 = [](size_t x) { return (x + 255) & ~static_cast<size_t>(255); };
+    const size_t c_off = align256(bytes), c_plane = align256(crow * ch);
+    if ((rc = ensure(c, &c->d_rgb_owned, &c->rgb_cap, (yuv ? c_off + ncp * c_plane : nplanes * bytes) + 16))) return rc;
     c->d_rgb = c->d_rgb_owned;
-    c->d_plane_g = c->d_rgb_owned + bytes;
-    c->d_plane_b = c->d_rgb_owned + 2 * bytes;
+    c->d_plane_g = c->d_rgb_owned + (yuv ? c_off : bytes);
+    c->d_plane_b = yuv ? (ncp == 2 ? c->d_rgb_owned + c_off + c_plane : nullptr) : c->d_rgb_owned + 2 * bytes;
+    if (yuv) c->chroma_pitch = static_cast<uint32_t>(crow);
     c->have_pixels = true;
     if ((rc = ensure_coef(c))) return rc;
     const uint8_t* host_plane[3] = {host_rgb, host_g, host_b};
@@ -948,7 +990,8 @@ static int upload_and_forward(jpgenc_ctx* c, const uint8_t* host_rgb, uint32_t w
                           reinterpret_cast<uintptr_t>(host_b) - reinterpret_cast<uintptr_t>(host_g) == gap;
     constexpr uint32_t kMaxBands = sizeof(c->ev_band) / sizeof(c->ev_band[0]);
     // bands of at least ~8 MB (a copy that size already runs at full PCIe rate), at most kMaxBands of them
-    uint32_t rows_per_band = static_cast<uint32_t>(std::max<size_t>(1, (8u << 20) / (row_bytes * nplanes * 16)));
+    const size_t mcu_row_bytes = yuv ? row_bytes * 16 + crow * ncp * 8 : row_bytes * nplanes * 16;
+    uint32_t rows_per_band = static_cast<uint32_t>(std::max<size_t>(1, (8u << 20) / mcu_row_bytes));
     rows_per_band = std::max(rows_per_band, (c->mcu_h + kMaxBands - 1) / kMaxBands);
     if ((rc = ensure_stats_buffers(c))) return rc;
     const uint32_t tiles = (c->mcu_w * c->mcu_h * kBlocksPerMcu + 383) / 384;
@@ -970,7 +1013,19 @@ static int upload_and_forward(jpgenc_ctx* c, const uint8_t* host_rgb, uint32_t w
                 if ((rc = (*fill)(slot, px0 * row_bytes, (px1 - px0) * row_bytes))) return fail(c, rc, "truncated PPM payload, or a sample above maxval");
                 src = slot;
             }
-            if (one_copy)
+            if (yuv) {
+                // Y rows [px0, px1), chroma rows [px0 / 2, ceil(px1 / 2)): what K1 reads for these MCU rows
+                auto copy_rows = [&](uint8_t* dst, const uint8_t* from, size_t row, size_t from_pitch, size_t rows) -> int {
+                    if (from_pitch == row) JPGENC_CUDA(c, cudaMemcpyAsync(dst, from, rows * row, cudaMemcpyHostToDevice, c->copy_stream));
+                    else JPGENC_CUDA(c, cudaMemcpy2DAsync(dst, row, from, from_pitch, row, rows, cudaMemcpyHostToDevice, c->copy_stream));
+                    return JPGENC_OK;
+                };
+                if ((rc = copy_rows(c->d_rgb_owned + px0 * row_bytes, src, row_bytes, pitch, px1 - px0))) return rc;
+                const size_t c0 = px0 / 2, c1 = (px1 + 1) / 2;
+                for (uint32_t k = 0; k < ncp; ++k)
+                    if ((rc = copy_rows(c->d_rgb_owned + c_off + k * c_plane + c0 * crow, host_plane[1 + k] + c0 * c_pitch, crow, c_pitch, c1 - c0)))
+                        return rc;
+            } else if (one_copy)
                 JPGENC_CUDA(c, cudaMemcpy2DAsync(c->d_rgb_owned + px0 * row_bytes, bytes, src, gap, (px1 - px0) * row_bytes, 3, cudaMemcpyHostToDevice,
                                                  c->copy_stream));
             else
@@ -1088,6 +1143,18 @@ int jpgenc_encode_planar(jpgenc_ctx* c, const void* r, const void* g, const void
         if (maxval && maxval < 255 && !samples_within_maxval(px, w, h, row_pitch, 1, maxval))
             return fail(c, JPGENC_ERR_FORMAT, "a sample exceeds maxval");
     if ((rc = upload_and_forward(c, plane[0], w, h, maxval, nullptr, kPixelPlanar, row_pitch, plane[1], plane[2]))) return rc;
+    return finish_upload_encode(c, dst, cap, jpeg_bytes);
+} JPGENC_CATCH(c)
+
+int jpgenc_encode_yuv420(jpgenc_ctx* c, const void* y, const void* u, const void* v, uint32_t w, uint32_t h, uint32_t y_pitch,
+                         uint32_t c_pitch, int layout, uint8_t* dst, uint64_t cap, uint64_t* jpeg_bytes) try {
+    if (!c) return JPGENC_ERR_ARG;
+    int format = 0;
+    int rc = check_yuv420(c, y, u, v, w, h, &y_pitch, &c_pitch, layout, &format);
+    if (rc) return rc;
+    if ((rc = upload_and_forward(c, static_cast<const uint8_t*>(y), w, h, 255, nullptr, format, y_pitch, static_cast<const uint8_t*>(u),
+                                 static_cast<const uint8_t*>(v), c_pitch)))
+        return rc;
     return finish_upload_encode(c, dst, cap, jpeg_bytes);
 } JPGENC_CATCH(c)
 

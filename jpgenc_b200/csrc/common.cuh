@@ -68,6 +68,13 @@ struct FrameGeom {
 };
 static_assert(sizeof(FrameGeom) == 48, "FrameGeom is copied as an array");
 
+// the chroma planes of one YUV image of a pass: they follow the FrameGeom array in the same copy (v is null for NV12)
+struct ChromaPlanes {
+    const uint8_t* u;
+    const uint8_t* v;
+    uint64_t pitch;
+};
+
 // the image f (0 <= f < F) whose units [geom[f].*key, geom[f + 1].*key) contain unit x, found by a whole warp in two rounds of
 // 32 parallel probes for F <= 1024 (every lane must take part; every lane returns f)
 __device__ __forceinline__ uint32_t geom_find_warp(const FrameGeom* geom, uint32_t F, uint32_t x, uint32_t FrameGeom::*key) {
@@ -112,13 +119,23 @@ struct ForwardParams {
     const uint8_t* plane_g;
     const uint8_t* plane_b;
     const uint8_t* const* planes;
+    // YUV 4:2:0 (kPixelI420, kPixelNV12): the single image's U and V planes are plane_g and plane_b (NV12: the UV plane is
+    // plane_g), its Y plane is `rgb` with `pitch`; chroma_pitch: bytes from one chroma row to the next.  Images of individual
+    // sizes: image f's chroma planes at yuv_chroma[f] (its Y plane is FrameGeom::rgb with FrameGeom::pitch)
+    uint32_t chroma_pitch;
+    const ChromaPlanes* yuv_chroma;
 };
 
 // Planar RGB: three planes of one byte per pixel, one row pitch.  It has no JPGENC_PIXEL_* code (the calls take three plane
 // pointers); inside the library it is this format.
 constexpr int kPixelPlanar = 17;
+// YUV 4:2:0 frames (jpgenc_*_yuv420; JPGENC_YUV_I420 / JPGENC_YUV_NV12 inside the library): a Y plane of one byte per pixel and
+// chroma planes of ceil(w/2) x ceil(h/2) samples -- U and V apart (I420) or interleaved U, V pairs (NV12)
+constexpr int kPixelI420 = 18;
+constexpr int kPixelNV12 = 19;
+__host__ __device__ constexpr bool is_yuv(int format) { return format == kPixelI420 || format == kPixelNV12; }
 
-// bytes per pixel of a JPGENC_PIXEL_* format (planar: of one plane)
+// bytes per pixel of a JPGENC_PIXEL_* format (planar: of one plane; YUV: of the Y plane)
 __host__ __device__ constexpr uint32_t pixel_bytes(int format) {
     return format >= JPGENC_PIXEL_GRAY ? 1u : format >= JPGENC_PIXEL_RGBA ? 4u : 3u;
 }
@@ -128,7 +145,8 @@ __host__ __device__ constexpr uint32_t pixel_bytes(int format) {
 struct MixedPass {
     bool on = false;
     bool aligned = false;                 // every image has real_w % 16 == 0 and a 16-byte aligned pointer (K1's bulk copies)
-    int format = -1;                      // JPGENC_PIXEL_* or kPixelPlanar: the pixel-layout kernels (with FrameGeom::pitch); -1 tight RGB
+    int format = -1;                      // JPGENC_PIXEL_*, kPixelPlanar, kPixelI420 or kPixelNV12: the pixel-layout kernels (with
+                                          // FrameGeom::pitch); -1 tight RGB
     uint32_t blocks = 0, strips = 0, tiles = 0, groups = 0, supers = 0;
     uint32_t split = 1;                   // K3 ranges per K2 tile, one choice for the whole pass (launch_entropy)
 };
@@ -195,7 +213,7 @@ __host__ __device__ inline unsigned long long raw_slot_bytes(unsigned long long 
 
 namespace jpgenc { class TablePool; class HostPool; }
 
-constexpr int kGraphKeyWords = 7;         // jpgenc_ctx::PhaseGraph: what a captured encode phase depends on
+constexpr int kGraphKeyWords = 8;         // jpgenc_ctx::PhaseGraph: what a captured encode phase depends on
 
 struct jpgenc_ctx {
     int device = 0;
@@ -254,6 +272,8 @@ struct jpgenc_ctx {
     uint32_t row_pitch = 0;               // ... bytes from one row to the next
     const uint8_t* d_plane_g = nullptr;   // ... planar RGB (kPixelPlanar): the G and B planes (d_rgb is the R plane)
     const uint8_t* d_plane_b = nullptr;
+    uint32_t chroma_pitch = 0;            // ... YUV 4:2:0 (kPixelI420 / kPixelNV12): d_plane_g, d_plane_b are the U and V planes
+                                          // (NV12: d_plane_g is the UV plane), rows chroma_pitch bytes apart; d_rgb is the Y plane
     bool have_pixels = false, have_coef = false, have_scan = false, forward_pending = false, upload_pending = false;
 
     int16_t* d_coef = nullptr;

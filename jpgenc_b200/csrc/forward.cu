@@ -176,6 +176,14 @@ __device__ __forceinline__ f2 bytes_to_f2(const uint32_t (&w)[N], int lo, int hi
     return add2(make_float2(__uint_as_float(a), __uint_as_float(b)), make_float2(-8388608.f, -8388608.f));
 }
 
+// the same with the level shift of YUV samples folded in: 8388608 + b - 8388736 == b - 128, exact
+template <int N>
+__device__ __forceinline__ f2 bytes_to_f2_centred(const uint32_t (&w)[N], int lo, int hi) {
+    const uint32_t a = __byte_perm(w[lo >> 2], 0x4B000000u, 0x7650 | (lo & 3));
+    const uint32_t b = __byte_perm(w[hi >> 2], 0x4B000000u, 0x7650 | (hi & 3));
+    return add2(make_float2(__uint_as_float(a), __uint_as_float(b)), make_float2(-8388736.f, -8388736.f));
+}
+
 // staging slot layout: 128 B per block, 16-byte chunk c of slot s lives at chunk (c ^ (s & 7)) — conflict-free
 // both for the per-thread 16-byte writes and for the linear copy-out
 __device__ __forceinline__ void stage_block(uint8_t* staging, int slot, const uint32_t (&w)[32]) {
@@ -397,12 +405,127 @@ __device__ __forceinline__ void stage_planes(const ForwardParams& p, ForwardSmem
     __syncthreads();
 }
 
+// Staging of YUV 4:2:0 frames: the tile holds the strip's 16 Y rows of kMcus * 16 bytes (8 KB at kMcus 32) and behind them its
+// 8 chroma rows, in the source's own layout: I420 a U and a V plane of rows of kMcus * 8 bytes, NV12 one plane of rows of
+// kMcus * 16 (U, V) bytes -- 12 KB in all, half the tile.  Each CTA picks its path from its own image:
+//  * every plane's base and pitch 16-byte aligned, real_w % 16 == 0 (so no chroma row needs padding either) and, for I420, an
+//    even number of MCUs (a bulk copy moves whole 16-byte units): one bulk copy per plane row (24 / 32 per CTA);
+//  * otherwise 16-byte chunks, per plane: a vector load where the chunk lies inside the plane's row and the plane is aligned,
+//    clamped byte loads elsewhere (edge replication, each plane clamped to its own size; NV12 clamps whole U, V pairs).
+// The L2 prefetch of the strip `prefetch_ahead` CTAs later covers every plane.
+template <int kMcus, bool kNV12, bool kMixed>
+__device__ __forceinline__ void stage_yuv(const ForwardParams& p, ForwardSmem<kMcus>& sm, int tid, const uint8_t* y, const uint8_t* u,
+                                          const uint8_t* v, uint32_t y_pitch, uint32_t c_pitch, uint32_t real_w, uint32_t real_h,
+                                          uint32_t my, uint32_t mcu0, int nm) {
+    constexpr int kThreads = kMcus * 4, kRow = kMcus * 16, kCRow = kNV12 ? kMcus * 16 : kMcus * 8, kCPlanes = kNV12 ? 1 : 2;
+    constexpr int kMcuC = kNV12 ? 16 : 8;                                  // chroma bytes of one MCU in one row
+    static_assert(16 * kRow + kCPlanes * 8 * kCRow <= ForwardSmem<kMcus>::kTileBytes, "the planes fit the tile");
+    const uint32_t cw_bytes = ((real_w + 1) / 2) * (kNV12 ? 2 : 1), ch = (real_h + 1) / 2;
+    const bool y_aligned = ((reinterpret_cast<uintptr_t>(y) | y_pitch) & 15) == 0;
+    const bool c_aligned = ((reinterpret_cast<uintptr_t>(u) | (kNV12 ? 0 : reinterpret_cast<uintptr_t>(v)) | c_pitch) & 15) == 0;
+    const bool bulk = y_aligned && c_aligned && real_w % 16 == 0 && (kNV12 || nm % 2 == 0);   // the same for every thread of the CTA
+    uint8_t* const ctile = sm.tile + 16 * kRow;
+    if (bulk) {
+        if (tid == 0) {
+            ptx::mbar_init(&sm.bar, 1);
+            ptx::mbar_init_fence();
+        }
+        __syncthreads();
+        if (tid < 16 + 8 * kCPlanes) {
+            if (tid == 0) ptx::mbar_expect_tx(&sm.bar, 16 * nm * 16 + kCPlanes * 8 * nm * kMcuC);
+            if (tid < 16) {
+                const uint32_t sy = min(my * 16 + tid, real_h - 1);
+                ptx::bulk_g2s(sm.tile + tid * kRow, y + static_cast<size_t>(sy) * y_pitch + mcu0 * 16, nm * 16, &sm.bar);
+            } else {
+                const int k = (tid - 16) >> 3, r = (tid - 16) & 7;
+                const uint32_t sy = min(my * 8 + r, ch - 1);
+                ptx::bulk_g2s(ctile + (k * 8 + r) * kCRow, (k ? v : u) + static_cast<size_t>(sy) * c_pitch + mcu0 * kMcuC, nm * kMcuC, &sm.bar);
+            }
+        }
+    }
+    if (p.prefetch_ahead && tid >= 32 && tid < 64) {
+        const uint8_t *py = nullptr, *pu = nullptr, *pv = nullptr;
+        uint32_t pyp = 0, pcp = 0, pw = 0, ph = 0, pm0 = 0, pnm = 0, pby = 0;
+        if constexpr (kMixed) {
+            const uint32_t t = blockIdx.x + p.prefetch_ahead;
+            if (t < p.strips) {                                             // uniform over the warp (geom_find_warp needs all lanes)
+                const uint32_t gi = geom_find_warp(p.geom, p.nframes, t, &FrameGeom::strip0);
+                const FrameGeom& g = p.geom[gi];
+                const uint32_t per_row = (g.mcu_w + kMcus - 1) / kMcus, s = t - g.strip0;
+                pby = s / per_row;
+                pm0 = (s - pby * per_row) * kMcus;
+                pnm = min(static_cast<uint32_t>(kMcus), g.mcu_w - pm0);
+                py = g.rgb; pyp = g.pitch; pw = g.real_w; ph = g.real_h;
+                const ChromaPlanes& cp = p.yuv_chroma[gi];
+                pu = cp.u; pv = cp.v; pcp = static_cast<uint32_t>(cp.pitch);
+            }
+        } else {
+            const uint32_t lin = blockIdx.y * gridDim.x + blockIdx.x + p.prefetch_ahead, yy = lin / gridDim.x;
+            if (yy < gridDim.y) {
+                pby = p.mcu_y0 + yy;
+                pm0 = (lin - yy * gridDim.x) * kMcus;
+                pnm = min(static_cast<uint32_t>(kMcus), p.mcu_w - pm0);
+                py = p.rgb; pyp = y_pitch; pw = real_w; ph = real_h;
+                pu = p.plane_g; pv = p.plane_b; pcp = c_pitch;
+            }
+        }
+        // whole 16-byte units inside the rows only (the range must not pass the end of a row): real_w % 16 == 0 makes every
+        // plane's strip end on its row's end
+        const int i = tid - 32;
+        if (py && pw % 16 == 0 && i < 16 + 8 * kCPlanes) {
+            const uint8_t* src = i < 16 ? py : i < 24 ? pu : pv;
+            const uint32_t pitch = i < 16 ? pyp : pcp;
+            if (((reinterpret_cast<uintptr_t>(src) | pitch) & 15) == 0) {
+                const uint32_t sy = i < 16 ? min(pby * 16 + i, ph - 1) : min(pby * 8 + ((i - 16) & 7), (ph + 1) / 2 - 1);
+                const uint32_t x0 = i < 16 ? pm0 * 16 : pm0 * kMcuC, n = (i < 16 ? pnm * 16 : pnm * kMcuC) & ~15u;
+                if (n) ptx::bulk_prefetch_l2(src + static_cast<size_t>(sy) * pitch + x0, n);
+            }
+        }
+    }
+    if (bulk) {
+        ptx::mbar_wait(&sm.bar, 0);
+        return;
+    }
+    // one plane: `rows` rows of `chunks` 16-byte chunks from x0 on; es: bytes of one sample (NV12 chroma: a U, V pair)
+    auto stage_plane = [&](const uint8_t* src, uint32_t pitch, bool aligned, uint32_t row0, uint32_t last_row, uint32_t width, uint32_t es,
+                           uint32_t x0, int rows, int chunks, uint8_t* dst, int dst_row) {
+        for (int i = tid; i < rows * chunks; i += kThreads) {
+            const int r = i / chunks, m = i - r * chunks;
+            const uint8_t* row = src + static_cast<size_t>(min(row0 + r, last_row)) * pitch;
+            const uint32_t x = x0 + m * 16;
+            uint4 q;
+            if (aligned && x + 16 <= width) {
+                q = __ldg(reinterpret_cast<const uint4*>(row + x));
+            } else {                                                        // right edge replication
+                uint32_t b[4];
+#pragma unroll
+                for (int j = 0; j < 4; ++j) {
+                    uint32_t word = 0;
+#pragma unroll
+                    for (int t = 0; t < 4; ++t) {
+                        const uint32_t xx = x + 4 * j + t, sx = xx < width ? xx : width - es + (xx & (es - 1));
+                        word |= static_cast<uint32_t>(row[sx]) << (8 * t);
+                    }
+                    b[j] = word;
+                }
+                q = make_uint4(b[0], b[1], b[2], b[3]);
+            }
+            *reinterpret_cast<uint4*>(dst + r * dst_row + m * 16) = q;
+        }
+    };
+    stage_plane(y, y_pitch, y_aligned, my * 16, real_h - 1, real_w, 1, mcu0 * 16, 16, nm, sm.tile, kRow);
+    const int cchunks = (nm * kMcuC + 15) / 16;                             // I420, odd nm: the last chunk's upper half is not read
+    stage_plane(u, c_pitch, c_aligned, my * 8, ch - 1, cw_bytes, kNV12 ? 2 : 1, mcu0 * kMcuC, 8, cchunks, ctile, kCRow);
+    if constexpr (!kNV12) stage_plane(v, c_pitch, c_aligned, my * 8, ch - 1, cw_bytes, 1, mcu0 * kMcuC, 8, cchunks, ctile + 8 * kCRow, kCRow);
+    __syncthreads();
+}
+
 // kAligned: real_w % 16 == 0 and 16-byte aligned base -> rows are staged with bulk copies; otherwise a clamped
 // byte loader fills the tile (odd sizes; right-edge replication, src/Image.cpp:491-530)
 // kMixed: images of individual sizes (p.geom): a 1-D grid over the strips of all images; a CTA finds its image by a search
 // over the first-strip prefix.  Otherwise one size: grid (strips of a row, rows, frames).
-// kFmt >= 0: pixels in that JPGENC_PIXEL_* format with a row pitch (stage_layout; grey and planar RGB: stage_planes; kAligned is
-// not used); -1: tight RGB
+// kFmt >= 0: pixels in that JPGENC_PIXEL_* format with a row pitch (stage_layout; grey and planar RGB: stage_planes; YUV 4:2:0:
+// stage_yuv; kAligned is not used); -1: tight RGB
 template <int kMcus, bool kAligned, bool kBulkOut, bool kMixed, int kFmt = -1>
 // (shared memory and the thread index come from the kernel: there the compiler knows the alignment and, from the launch
 // bounds, the range of threadIdx.x)
@@ -411,13 +534,18 @@ __device__ __forceinline__ void forward_body(const ForwardParams& p, ForwardSmem
     constexpr int kThreads = kMcus * 4;
     const int tid = thread;
     constexpr bool kPlanar = kFmt == kPixelPlanar, kPlaneTile = kPlanar || kFmt == JPGENC_PIXEL_GRAY;   // stage_planes
-    uint32_t my, mcu0, frame_block0, real_w, real_h, mcu_w, pitch;
+    constexpr bool kYuv = is_yuv(kFmt), kNV12 = kFmt == kPixelNV12;                                // stage_yuv
+    uint32_t my, mcu0, frame_block0, real_w, real_h, mcu_w, pitch, c_pitch = 0;
     const uint8_t* __restrict__ rgb;
-    const uint8_t* plane_gb[2] = {nullptr, nullptr};                      // planar RGB: the G and B planes (rgb is R)
+    const uint8_t* plane_gb[2] = {nullptr, nullptr};                      // planar RGB: the G and B planes (rgb is R); YUV: U and V
     if constexpr (kMixed) {
         const uint32_t gi = geom_find_warp(p.geom, p.nframes, blockIdx.x, &FrameGeom::strip0);
         const FrameGeom& g = p.geom[gi];
         if constexpr (kPlanar) { plane_gb[0] = p.planes[2 * gi]; plane_gb[1] = p.planes[2 * gi + 1]; }
+        if constexpr (kYuv) {
+            const ChromaPlanes& cp = p.yuv_chroma[gi];
+            plane_gb[0] = cp.u; plane_gb[1] = cp.v; c_pitch = static_cast<uint32_t>(cp.pitch);
+        }
         mcu_w = g.mcu_w;
         const uint32_t per_row = (mcu_w + kMcus - 1) / kMcus, s = blockIdx.x - g.strip0;
         my = s / per_row;
@@ -436,12 +564,15 @@ __device__ __forceinline__ void forward_body(const ForwardParams& p, ForwardSmem
         real_h = p.real_h;
         mcu_w = p.mcu_w;
         pitch = p.pitch;
-        if constexpr (kPlanar) { plane_gb[0] = p.plane_g; plane_gb[1] = p.plane_b; }
+        if constexpr (kPlanar || kYuv) { plane_gb[0] = p.plane_g; plane_gb[1] = p.plane_b; }
+        if constexpr (kYuv) c_pitch = p.chroma_pitch;
     }
     const int nm = min(kMcus, static_cast<int>(mcu_w - mcu0));
 
     // ---- stage the 16-row RGB strip ----
-    if constexpr (kPlaneTile) {
+    if constexpr (kYuv) {
+        stage_yuv<kMcus, kNV12, kMixed>(p, sm, tid, rgb, plane_gb[0], plane_gb[1], pitch, c_pitch, real_w, real_h, my, mcu0, nm);
+    } else if constexpr (kPlaneTile) {
         const uint8_t* const plane[3] = {rgb, plane_gb[0], plane_gb[1]};
         stage_planes<kMcus, kPlanar ? 3 : 1, kMixed>(p, sm, tid, plane, pitch, real_w, real_h, my, mcu0, nm);
     } else if constexpr (kFmt >= 0) {
@@ -500,7 +631,42 @@ __device__ __forceinline__ void forward_body(const ForwardParams& p, ForwardSmem
     const bool active = (bx >> 1) < nm;
     f2 v[32];                                     // v[r*4+p] = samples (r, 2p) and (r, 2p+1)
     constexpr int kR = (kFmt == JPGENC_PIXEL_BGR || kFmt == JPGENC_PIXEL_BGRA) ? 2 : 0, kB = 2 - kR;   // tile bytes of R and B
-    if (active) {
+    if constexpr (kYuv) {
+        if (active) {
+            // The samples themselves, level-shifted: no colour conversion and no 2x2 means.  The chroma sample of an MCU position
+            // is the stored one: the reference's S420_m averages four equal values there ((a + a) + (a + a), then / 4, gives
+            // exactly a), see exact_yuv_sample.  Every value is an integer in [-128, 127], exact in FP32.  The chroma goes first,
+            // before the luma block fills its registers.
+            constexpr int kRow = kMcus * 16;
+            const uint8_t* ctile = sm.tile + 16 * kRow;
+#pragma unroll
+            for (int rp = 0; rp < 4; ++rp) {          // chroma row by * 4 + rp, columns bx * 4 .. bx * 4 + 3 (this thread's 2x2 cells)
+                const int cr = by * 4 + rp;
+                f2 cb[2], crr[2];
+                if constexpr (kNV12) {
+                    const uint2 q = *reinterpret_cast<const uint2*>(ctile + cr * kRow + bx * 8);          // U V U V U V U V
+                    const uint32_t w[2] = {q.x, q.y};
+                    cb[0] = bytes_to_f2_centred(w, 0, 2); cb[1] = bytes_to_f2_centred(w, 4, 6);
+                    crr[0] = bytes_to_f2_centred(w, 1, 3); crr[1] = bytes_to_f2_centred(w, 5, 7);
+                } else {
+                    constexpr int kCRow = kMcus * 8;
+                    const uint32_t wu[1] = {*reinterpret_cast<const uint32_t*>(ctile + cr * kCRow + bx * 4)};
+                    const uint32_t wv[1] = {*reinterpret_cast<const uint32_t*>(ctile + (8 + cr) * kCRow + bx * 4)};
+                    cb[0] = bytes_to_f2_centred(wu, 0, 1); cb[1] = bytes_to_f2_centred(wu, 2, 3);
+                    crr[0] = bytes_to_f2_centred(wv, 0, 1); crr[1] = bytes_to_f2_centred(wv, 2, 3);
+                }
+                *reinterpret_cast<float4*>(&sm.chroma[0][cr][bx * 4]) = make_float4(cb[0].x, cb[0].y, cb[1].x, cb[1].y);
+                *reinterpret_cast<float4*>(&sm.chroma[1][cr][bx * 4]) = make_float4(crr[0].x, crr[0].y, crr[1].x, crr[1].y);
+            }
+#pragma unroll
+            for (int r = 0; r < 8; ++r) {
+                const uint2 q = *reinterpret_cast<const uint2*>(sm.tile + (by * 8 + r) * kRow + bx * 8);
+                const uint32_t w[2] = {q.x, q.y};
+#pragma unroll
+                for (int pp = 0; pp < 4; ++pp) v[r * 4 + pp] = bytes_to_f2_centred(w, 2 * pp, 2 * pp + 1);
+            }
+        }
+    } else if (active) {
         const ColorConsts& cc = p.color;
 #pragma unroll
         for (int rp = 0; rp < 4; ++rp) {
@@ -866,6 +1032,66 @@ __global__ void __launch_bounds__(kRefineThreads) refine_mixed_planar_kernel(con
     else refine_loop(n0, n, list, false, coef, 0xFFFFFFFFu, e.qy, e.qc, e, locate, sample);
 }
 
+// YUV 4:2:0, sample of row r of a column: what Image::writeJPEG computes for the image whose level-shifted Y, Cb, Cr planes are
+// the clamped bytes minus 128 (the frame padded to whole MCUs by edge replication, every chroma sample repeated over its 2x2
+// pixels; jpgenc_encode_planes(..., ycbcr = 1)), bit for bit: such an image skips the colour conversion (src/Image.cpp:
+// 112-115); a luma sample is (double)byte - 128, exact; S420_m (src/Image.cpp:207-226) sums the four pixels of a cell as
+// (0 + a + a) + (0 + a + a) -- a cell's four clamped pixels map to one chroma sample a (x, x + 1 with x even, or both clamped to
+// the last column; the same for rows) -- and quarters the sum: every step is exact on these small integers and gives a again.
+// So the chroma sample of cell (x / 2, y / 2) is U[min(y / 2, ch - 1)][min(x / 2, cw - 1)] - 128 (V for Cr; NV12: the pair's
+// first / second byte).
+template <bool kNV12>
+__device__ __forceinline__ double exact_yuv_sample(const ExactColumn& b, const uint8_t* u, const uint8_t* v, uint32_t y_pitch, uint32_t c_pitch,
+                                                   uint32_t real_w, uint32_t real_h, int r) {
+    if (b.comp == 0) {
+        const uint32_t sx = min(b.x, real_w - 1), sy = min(b.y + r, real_h - 1);
+        return dsub(static_cast<double>(b.rgb[static_cast<size_t>(sy) * y_pitch + sx]), 128.0);
+    }
+    const uint32_t cx = min(b.x / 2, (real_w + 1) / 2 - 1), cy = min(b.y / 2 + r, (real_h + 1) / 2 - 1);
+    const size_t row = static_cast<size_t>(cy) * c_pitch;
+    const uint8_t s = kNV12 ? u[row + 2 * cx + (b.comp - 1)] : (b.comp == 1 ? u : v)[row + cx];
+    return dsub(static_cast<double>(s), 128.0);
+}
+
+// YUV 4:2:0, one image: Y plane y (rows y_pitch apart), chroma planes u, v (NV12: u is the UV plane) with rows c_pitch apart
+template <bool k64, bool kNV12>
+__global__ void __launch_bounds__(kRefineThreads) refine_yuv_kernel(const uint8_t* __restrict__ y, const uint8_t* __restrict__ u,
+                                                                        const uint8_t* __restrict__ v, int16_t* __restrict__ coef,
+                                                                        const uint32_t* __restrict__ list, const uint32_t* __restrict__ count,
+                                                                        uint32_t cap, int all, uint32_t nblocks, uint32_t real_w, uint32_t real_h,
+                                                                        uint32_t mcu_w, const __grid_constant__ ExactConsts e, uint32_t y_pitch,
+                                                                        uint32_t c_pitch) {
+    const uint32_t n = all ? nblocks : min(count[0], cap), n0 = all ? 0u : count[3];
+    auto locate = [&](uint32_t id, int c) { return exact_locate(y, mcu_w, id, c); };
+    auto sample = [&](const ExactColumn& col, int row) { return exact_yuv_sample<kNV12>(col, u, v, y_pitch, c_pitch, real_w, real_h, row); };
+    if constexpr (k64) refine_loop64(n0, n, list, all != 0, coef, nblocks, e.qy, e.qc, e, locate, sample);
+    else refine_loop(n0, n, list, all != 0, coef, nblocks, e.qy, e.qc, e, locate, sample);
+}
+
+// YUV 4:2:0, images of individual sizes: image f's chroma planes at chroma[f] (otherwise refine_mixed_kernel)
+template <bool k64, bool kNV12>
+__global__ void __launch_bounds__(kRefineThreads) refine_mixed_yuv_kernel(const FrameGeom* __restrict__ geom, const ChromaPlanes* __restrict__ chroma,
+                                                                              uint32_t nframes, int16_t* __restrict__ coef,
+                                                                              const uint32_t* __restrict__ list, const uint32_t* __restrict__ count,
+                                                                              uint32_t cap, const __grid_constant__ ExactConsts e) {
+    const uint32_t n = min(count[0], cap), n0 = count[3];
+    struct Column { ExactColumn col; uint32_t real_w, real_h, pitch; ChromaPlanes cp; };
+    auto locate = [&](uint32_t id, int c) {
+        uint32_t lo = 0, hi = nframes;
+        while (hi - lo > 1) {
+            const uint32_t mid = (lo + hi) >> 1;
+            if (geom[mid].block0 <= id) lo = mid; else hi = mid;
+        }
+        const FrameGeom& gm = geom[lo];
+        return Column{exact_locate(gm.rgb, gm.mcu_w, id - gm.block0, c), gm.real_w, gm.real_h, gm.pitch, chroma[lo]};
+    };
+    auto sample = [&](const Column& col, int r) {
+        return exact_yuv_sample<kNV12>(col.col, col.cp.u, col.cp.v, col.pitch, static_cast<uint32_t>(col.cp.pitch), col.real_w, col.real_h, r);
+    };
+    if constexpr (k64) refine_loop64(n0, n, list, false, coef, 0xFFFFFFFFu, e.qy, e.qc, e, locate, sample);
+    else refine_loop(n0, n, list, false, coef, 0xFFFFFFFFu, e.qy, e.qc, e, locate, sample);
+}
+
 // Images that are not 8-bit samples: three planes of doubles as the reference holds them (Image::R/G/B after loadPPM, or
 // planes a caller computed; already YCbCr when `ycbcr`: Image::writeJPEG converts only an RGB image, src/Image.cpp:112-115,
 // 839).  Every block takes the exact path; width x height are the padded plane dimensions (multiples of 16).
@@ -1119,7 +1345,12 @@ static void fill_forward_params(const jpgenc_ctx* c, ForwardParams* p) {
         p->color.cb[i] = static_cast<float>(fcb[i] * scale / 4);
         p->color.cr[i] = static_cast<float>(fcr[i] * scale / 4);
     }
-    const double colour_err = c->maxval == 255 ? kColourErr255 : kColourErrScaled;
+    // YUV 4:2:0 samples reach the transform unconverted: byte - 128, exact integers in [-128, 127], inside the [-128, 128] that
+    // aan2d_bounds assumes, with no input error -- the stand-alone block kernel's case.  Their thresholds are tighter than the
+    // RGB ones, so an RGB encode must never take them (nor a YUV encode the RGB ones, which would only flag more blocks): they
+    // follow the layout of the image(s) bound, computed anew for every launch.
+    const int format = c->mixed.on ? c->mixed.format : c->pixel_format;
+    const double colour_err = is_yuv(format) ? 0.0 : c->maxval == 255 ? kColourErr255 : kColourErrScaled;
     fill_quant_consts2(c->qy, c->dct_s, &p->luma, colour_err);
     fill_quant_consts2(c->qc, c->dct_s, &p->chroma, colour_err);
 }
@@ -1134,6 +1365,8 @@ static void with_format(int format, F&& f) {
         case JPGENC_PIXEL_RGBA: f(std::integral_constant<int, JPGENC_PIXEL_RGBA>{}); break;
         case JPGENC_PIXEL_GRAY: f(std::integral_constant<int, JPGENC_PIXEL_GRAY>{}); break;
         case kPixelPlanar: f(std::integral_constant<int, kPixelPlanar>{}); break;
+        case kPixelI420: f(std::integral_constant<int, kPixelI420>{}); break;
+        case kPixelNV12: f(std::integral_constant<int, kPixelNV12>{}); break;
         default: f(std::integral_constant<int, JPGENC_PIXEL_BGRA>{}); break;
     }
 }
@@ -1167,6 +1400,16 @@ static int launch_refine(jpgenc_ctx* c, bool all) {
                     refine_planar_kernel<false><<<grid, kRefineThreads, 0, c->stream>>>(c->d_rgb, c->d_plane_g, c->d_plane_b, c->d_coef, c->d_refine_list,
                                                                                        c->d_counters, cap, all ? 1 : 0, bpf, c->real_w, c->real_h, c->mcu_w, e,
                                                                                        c->row_pitch);
+            } else if constexpr (is_yuv(kFmt)) {
+                constexpr bool kNV12 = kFmt == kPixelNV12;
+                if (total < (3u << 19))
+                    refine_yuv_kernel<true, kNV12><<<grid, kRefineThreads, 0, c->stream>>>(c->d_rgb, c->d_plane_g, c->d_plane_b, c->d_coef, c->d_refine_list,
+                                                                                          c->d_counters, cap, all ? 1 : 0, bpf, c->real_w, c->real_h, c->mcu_w,
+                                                                                          e, c->row_pitch, c->chroma_pitch);
+                else
+                    refine_yuv_kernel<false, kNV12><<<grid, kRefineThreads, 0, c->stream>>>(c->d_rgb, c->d_plane_g, c->d_plane_b, c->d_coef, c->d_refine_list,
+                                                                                           c->d_counters, cap, all ? 1 : 0, bpf, c->real_w, c->real_h, c->mcu_w,
+                                                                                           e, c->row_pitch, c->chroma_pitch);
             } else if (total < (3u << 19))
                 refine_kernel<true, kFmt><<<grid, kRefineThreads, 0, c->stream>>>(c->d_rgb, frames, bpf, c->d_coef, c->d_refine_list, c->d_counters, cap,
                                                                                   all ? 1 : 0, bpf * c->nframes, c->real_w, c->real_h, c->mcu_w, e, c->row_pitch);
@@ -1208,6 +1451,7 @@ int launch_forward_rows(jpgenc_ctx* c, uint32_t y0, uint32_t rows, bool first, b
         p.pitch = c->row_pitch;
         p.plane_g = c->d_plane_g;
         p.plane_b = c->d_plane_b;
+        p.chroma_pitch = c->chroma_pitch;
         const bool bulk = make_block_map(c->d_coef, static_cast<uint64_t>(c->mcu_w) * c->mcu_h * kBlocksPerMcu, 32 * kBlocksPerMcu, &p.coef_map);
         with_format(c->pixel_format, [&](auto fmt) {
             constexpr int kFmt = decltype(fmt)::value;
@@ -1245,6 +1489,9 @@ int launch_forward_mixed(jpgenc_ctx* c) {
     // planar RGB: the G and B plane pointers lie behind the geometry (enqueue_pass copies them in the same transfer)
     const uint8_t* const* planes = c->mixed.format == kPixelPlanar ? reinterpret_cast<const uint8_t* const*>(c->d_geom + c->nframes + 1) : nullptr;
     p.planes = planes;
+    // YUV 4:2:0: each image's chroma planes lie there instead (ChromaPlanes)
+    const ChromaPlanes* chroma = is_yuv(c->mixed.format) ? reinterpret_cast<const ChromaPlanes*>(c->d_geom + c->nframes + 1) : nullptr;
+    p.yuv_chroma = chroma;
     const bool bulk_out = (aligned || layout) && make_block_map(c->d_coef, c->mixed.blocks, 32 * kBlocksPerMcu, &p.coef_map);
     if (layout) {
         with_format(c->mixed.format, [&](auto fmt) {
@@ -1271,6 +1518,14 @@ int launch_forward_mixed(jpgenc_ctx* c) {
                 else
                     refine_mixed_planar_kernel<false><<<grid, kRefineThreads, 0, c->stream>>>(c->d_geom, planes, c->nframes, c->d_coef, c->d_refine_list,
                                                                                              c->d_counters, cap, e);
+            } else if constexpr (is_yuv(kFmt)) {
+                constexpr bool kNV12 = kFmt == kPixelNV12;
+                if (total < (3u << 19))
+                    refine_mixed_yuv_kernel<true, kNV12><<<grid, kRefineThreads, 0, c->stream>>>(c->d_geom, chroma, c->nframes, c->d_coef, c->d_refine_list,
+                                                                                                c->d_counters, cap, e);
+                else
+                    refine_mixed_yuv_kernel<false, kNV12><<<grid, kRefineThreads, 0, c->stream>>>(c->d_geom, chroma, c->nframes, c->d_coef, c->d_refine_list,
+                                                                                                 c->d_counters, cap, e);
             } else if (total < (3u << 19))
                 refine_mixed_kernel<true, kFmt><<<grid, kRefineThreads, 0, c->stream>>>(c->d_geom, c->nframes, c->d_coef, c->d_refine_list, c->d_counters, cap, e);
             else

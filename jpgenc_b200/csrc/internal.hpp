@@ -25,6 +25,8 @@ int ensure(jpgenc_ctx* c, T** ptr, size_t* cap, size_t need_bytes, bool headroom
 int set_geometry(jpgenc_ctx* c, uint32_t w, uint32_t h, uint32_t maxval);
 // a JPGENC_PIXEL_* format, sides 1..65535 and a row pitch (0 -> the row size, set in *row_pitch) that holds a row; JPGENC_ERR_ARG otherwise
 int check_layout(jpgenc_ctx* c, uint32_t w, uint32_t h, uint32_t* row_pitch, int format);
+int check_yuv420(jpgenc_ctx* c, const void* y, const void* u, const void* v, uint32_t w, uint32_t h, uint32_t* y_pitch, uint32_t* c_pitch,
+                 int layout, int* format);
 int ensure_pinned(jpgenc_ctx* c, size_t bytes);                 // c->h_pinned, grown on demand
 int ensure_coef(jpgenc_ctx* c);                                  // coefficients + refinement list of the bound frames
 int ensure_stats_buffers(jpgenc_ctx* c);                         // K2's outputs for the bound frames (+ pinned staging)

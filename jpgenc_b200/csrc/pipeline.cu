@@ -43,8 +43,11 @@ struct Job {
     // pixels in another layout (jpgenc_encode_images_packed_layout; needs widths): JPGENC_PIXEL_* format, -1 tight RGB, and the
     // row pitch of every image as the caller holds it.  `staged`: host images, uploaded into tight rows of their format.
     // kPixelPlanar (jpgenc_encode_images_packed_planar): three pointers per image, R, G, B; staged as three tight planes back to back.
+    // kPixelI420 / kPixelNV12 (jpgenc_encode_images_packed_yuv420): three pointers per image, Y, U, V (NV12: Y, UV, null), Y rows
+    // `pitches` apart, chroma rows `c_pitches` apart; staged as tight planes, each starting on 256 bytes.
     int format = -1;
     const uint32_t* pitches = nullptr;
+    const uint32_t* c_pitches = nullptr;
     bool staged = false;
     double raw_per_block = 0;              // ... raw-scan bytes reserved per block: 1.5 x the most this call has seen (0: nothing yet)
     // output: per-frame buffers (legacy), one packed buffer, or none (sizes only)
@@ -67,9 +70,12 @@ uint32_t job_w(const Job& job, uint32_t i) { return job.widths ? job.widths[i] :
 uint32_t job_h(const Job& job, uint32_t i) { return job.heights ? job.heights[i] : job.h; }
 uint32_t job_bpp(const Job& job) { return job.format < 0 ? 3u : pixel_bytes(job.format); }
 // pointers (= planes) per image
-uint32_t job_planes(const Job& job) { return job.format == kPixelPlanar ? 3u : 1u; }
+uint32_t job_planes(const Job& job) { return job.format == kPixelPlanar || is_yuv(job.format) ? 3u : 1u; }
 // bytes from one row of image i to the next where the kernels read it
 uint32_t job_pitch(const Job& job, uint32_t i) { return job.pitches && !job.staged ? job.pitches[i] : job_w(job, i) * job_bpp(job); }
+// YUV 4:2:0: bytes of one chroma row of image i (tight), and from one chroma row to the next where the kernels read it
+uint32_t job_crow(const Job& job, uint32_t i) { return (job_w(job, i) + 1) / 2 * (job.format == kPixelNV12 ? 2u : 1u); }
+uint32_t job_c_pitch(const Job& job, uint32_t i) { return job.staged ? job_crow(job, i) : job.c_pitches[i]; }
 uint64_t job_blocks(const Job& job, uint32_t i) {
     return static_cast<uint64_t>((job_w(job, i) + 15) / 16) * ((job_h(job, i) + 15) / 16) * kBlocksPerMcu;
 }
@@ -133,8 +139,9 @@ std::vector<Pass> image_passes(const Job& job, uint32_t slots) {
 
 // The geometry of a pass of images of individual sizes (FrameGeom, F + 1 entries) and its totals.  K3's split follows
 // launch_entropy's rule, applied to the pass's tiles.  Planar RGB: ptrs holds R, G, B of every image; FrameGeom::rgb is the R
-// plane, gb[2f], gb[2f + 1] receive the G and B planes.
-MixedPass image_geometry(const Job& job, const Pass& ps, const void* const* ptrs, FrameGeom* g, const void** gb) {
+// plane, gb[2f], gb[2f + 1] receive the G and B planes.  YUV 4:2:0: ptrs holds Y, U, V; FrameGeom::rgb is the Y plane, cp[f]
+// receives the chroma planes and pitch.
+MixedPass image_geometry(const Job& job, const Pass& ps, const void* const* ptrs, FrameGeom* g, const void** gb, ChromaPlanes* cp) {
     MixedPass m;
     m.on = true;
     m.aligned = true;
@@ -149,7 +156,9 @@ MixedPass image_geometry(const Job& job, const Pass& ps, const void* const* ptrs
         const uint32_t w = job_w(job, ps.f0 + f), h = job_h(job, ps.f0 + f);
         const uint32_t np = job_planes(job);
         g[f].rgb = static_cast<const uint8_t*>(ptrs[np * f]);
-        if (np == 3) { gb[2 * f] = ptrs[3 * f + 1]; gb[2 * f + 1] = ptrs[3 * f + 2]; }
+        if (is_yuv(job.format))
+            cp[f] = ChromaPlanes{static_cast<const uint8_t*>(ptrs[3 * f + 1]), static_cast<const uint8_t*>(ptrs[3 * f + 2]), job_c_pitch(job, ps.f0 + f)};
+        else if (np == 3) { gb[2 * f] = ptrs[3 * f + 1]; gb[2 * f + 1] = ptrs[3 * f + 2]; }
         g[f].real_w = w; g[f].real_h = h; g[f].mcu_w = (w + 15) / 16; g[f].mcu_h = (h + 15) / 16;
         if (job.format >= 0) g[f].pitch = job_pitch(job, ps.f0 + f);
         const uint32_t blocks = g[f].mcu_w * g[f].mcu_h * kBlocksPerMcu, tiles = (blocks + 383) / 384, groups = (tiles * m.split + 7) / 8;
@@ -227,20 +236,23 @@ int enqueue_pass(jpgenc_ctx* root, jpgenc_ctx* l, const Job& job, Pass& ps, cons
     l->have_pixels = true;
     std::vector<FrameGeom> geom;
     std::vector<const void*> gb;
+    std::vector<ChromaPlanes> cp;
     if (job.widths) {
         geom.resize(F + 1);
-        gb.resize(job_planes(job) == 3 ? 2 * F : 0);
-        l->mixed = image_geometry(job, ps, dev_frames, geom.data(), gb.data());
+        gb.resize(job.format == kPixelPlanar ? 2 * F : 0);
+        cp.resize(is_yuv(job.format) ? F : 0);
+        l->mixed = image_geometry(job, ps, dev_frames, geom.data(), gb.data(), cp.data());
     }
     if ((rc = ensure_coef(l))) return rc;
     if ((rc = ensure_stats_buffers(l))) return rc;               // also sizes the pinned staging (stage_bytes(F))
     if (job.widths) {
-        // the geometry (with the frame pointers; planar RGB: and the G and B planes behind it) travels through pinned memory like
-        // the pointer array below
-        const size_t gbytes = geom.size() * sizeof(FrameGeom), bytes = gbytes + gb.size() * sizeof(void*);
+        // the geometry (with the frame pointers; planar RGB: and the G and B planes behind it; YUV: the chroma planes) travels
+        // through pinned memory like the pointer array below
+        const size_t gbytes = geom.size() * sizeof(FrameGeom), bytes = gbytes + gb.size() * sizeof(void*) + cp.size() * sizeof(ChromaPlanes);
         if ((rc = ensure(l, &l->d_geom, &l->geom_cap, bytes))) return rc;
         std::memcpy(l->h_pinned, geom.data(), gbytes);
         if (!gb.empty()) std::memcpy(static_cast<uint8_t*>(l->h_pinned) + gbytes, gb.data(), gb.size() * sizeof(void*));
+        if (!cp.empty()) std::memcpy(static_cast<uint8_t*>(l->h_pinned) + gbytes, cp.data(), cp.size() * sizeof(ChromaPlanes));
         JPGENC_CUDA(l, cudaMemcpyAsync(l->d_geom, l->h_pinned, bytes, cudaMemcpyHostToDevice, l->stream));
     } else {
         size_t cap = l->frame_ptrs_cap;
@@ -483,8 +495,15 @@ int encode_host_frames(jpgenc_ctx* c, Job& job, const uint8_t* const* frames) {
     constexpr uint32_t kRingMax = sizeof(c->ev_band) / sizeof(c->ev_band[0]);
     const uint32_t ring = std::min({nslots + 2, npasses, kRingMax});
     const uint32_t np = job_planes(job);
+    const bool yuv = is_yuv(job.format);
     auto plane_bytes = [&](uint32_t i) { return static_cast<size_t>(job_w(job, i)) * job_h(job, i) * job_bpp(job); };
-    auto fbytes = [&](uint32_t i) { return plane_bytes(i) * np; };
+    // YUV: plane k of image i starts at yuv_off(i, k) of its slot (on 256 bytes), behind the last plane lies yuv_off(i, 3)
+    auto yuv_off = [&](uint32_t i, uint32_t k) {
+        const size_t y = (plane_bytes(i) + 255) & ~static_cast<size_t>(255);
+        const size_t cplane = (static_cast<size_t>(job_crow(job, i)) * ((job_h(job, i) + 1) / 2) + 255) & ~static_cast<size_t>(255);
+        return k == 0 ? 0 : y + std::min(k - 1, job.format == kPixelNV12 ? 1u : 2u) * cplane;
+    };
+    auto fbytes = [&](uint32_t i) { return yuv ? yuv_off(i, 3) : plane_bytes(i) * np; };
     auto fstride = [&](uint32_t i) { return (fbytes(i) + 255) & ~static_cast<size_t>(255); };
     // frame f of pass p sits at slice (p % ring) + at[f0 + f]
     std::vector<size_t> at(job.n);
@@ -503,7 +522,15 @@ int encode_host_frames(jpgenc_ctx* c, Job& job, const uint8_t* const* frames) {
             while (!job.widths && f + run < F && frames[f0 + f + run] == frames[f0 + f + run - 1] + fbytes(0)) ++run;
             uint8_t* dst = c->d_rgb_owned + static_cast<size_t>(s) * slice + at[f0 + f];
             const size_t row = static_cast<size_t>(job_w(job, f0 + f)) * job_bpp(job);
-            if (np == 3) {
+            if (yuv) {
+                // YUV 4:2:0: one copy per plane, the pitch gaps dropped
+                const uint8_t* const* pl = frames + 3 * static_cast<size_t>(f0 + f);
+                const size_t h = job_h(job, f0 + f), crow = job_crow(job, f0 + f);
+                JPGENC_CUDA(c, cudaMemcpy2DAsync(dst, row, pl[0], job.pitches[f0 + f], row, h, cudaMemcpyHostToDevice, c->copy_stream));
+                for (uint32_t k = 1; k < 3 && pl[k]; ++k)
+                    JPGENC_CUDA(c, cudaMemcpy2DAsync(dst + yuv_off(f0 + f, k), crow, pl[k], job.c_pitches[f0 + f], crow, (h + 1) / 2,
+                                                     cudaMemcpyHostToDevice, c->copy_stream));
+            } else if (np == 3) {
                 // planar RGB: one copy per plane, or one strided copy when the planes lie back to back with tight rows
                 const uint8_t* const* pl = frames + 3 * static_cast<size_t>(f0 + f);
                 const size_t pb = plane_bytes(f0 + f), h = job_h(job, f0 + f), pitch = job.pitches[f0 + f];
@@ -533,8 +560,11 @@ int encode_host_frames(jpgenc_ctx* c, Job& job, const uint8_t* const* frames) {
                         std::vector<const void*>& v = ptrs[p % nslots];
                         v.resize(static_cast<size_t>(F) * np);
                         for (uint32_t f = 0; f < F; ++f)
-                            for (uint32_t k = 0; k < np; ++k)
-                                v[f * np + k] = c->d_rgb_owned + static_cast<size_t>(s) * slice + at[f0 + f] + k * plane_bytes(f0 + f);
+                            for (uint32_t k = 0; k < np; ++k) {
+                                const size_t off = yuv ? yuv_off(f0 + f, k) : k * plane_bytes(f0 + f);
+                                const bool none = yuv && k == 2 && job.format == kPixelNV12;            // NV12 has no V plane
+                                v[f * np + k] = none ? nullptr : c->d_rgb_owned + static_cast<size_t>(s) * slice + at[f0 + f] + off;
+                            }
                         *out = v.data();
                         *ready = c->ev_band[s];
                         return JPGENC_OK;
@@ -668,6 +698,32 @@ int jpgenc_encode_images_packed_planar(jpgenc_ctx* c, uint32_t n, const void* co
     job.n = n; job.w = widths[0]; job.h = heights[0]; job.maxval = maxval;
     job.widths = widths; job.heights = heights;
     job.format = kPixelPlanar; job.pitches = pitch.data();
+    job.packed_mode = true; job.packed = out; job.packed_cap = cap; job.offsets = offsets; job.sizes = sizes;
+    const int rc = images_on_device ? encode_device_frames(c, job, planes) : encode_host_frames(c, job, reinterpret_cast<const uint8_t* const*>(planes));
+    if (total_bytes) *total_bytes = job.packed_at;
+    return rc;
+} JPGENC_CATCH(c)
+
+int jpgenc_encode_images_packed_yuv420(jpgenc_ctx* c, uint32_t n, const void* const* planes, int images_on_device, const uint32_t* widths,
+                                       const uint32_t* heights, const uint32_t* y_pitches, const uint32_t* c_pitches, int layout, uint8_t* out,
+                                       uint64_t cap, uint64_t* offsets, uint64_t* sizes, uint64_t* total_bytes) try {
+    if (!c) return JPGENC_ERR_ARG;
+    if (total_bytes) *total_bytes = 0;
+    if (layout != JPGENC_YUV_I420 && layout != JPGENC_YUV_NV12) return fail(c, JPGENC_ERR_ARG, "unknown YUV layout");
+    if (n == 0) return JPGENC_OK;                                // an empty batch is legal and touches nothing
+    if (!planes || !widths || !heights || !offsets || !sizes) return fail(c, JPGENC_ERR_ARG, "null argument");
+    std::vector<uint32_t> pitch(n), c_pitch(n);
+    int format = 0;
+    for (uint32_t i = 0; i < n; ++i) {
+        pitch[i] = y_pitches ? y_pitches[i] : 0;
+        c_pitch[i] = c_pitches ? c_pitches[i] : 0;
+        const int rc = check_yuv420(c, planes[3 * i], planes[3 * i + 1], planes[3 * i + 2], widths[i], heights[i], &pitch[i], &c_pitch[i], layout, &format);
+        if (rc) return rc;
+    }
+    Job job;
+    job.n = n; job.w = widths[0]; job.h = heights[0]; job.maxval = 255;
+    job.widths = widths; job.heights = heights;
+    job.format = format; job.pitches = pitch.data(); job.c_pitches = c_pitch.data();
     job.packed_mode = true; job.packed = out; job.packed_cap = cap; job.offsets = offsets; job.sizes = sizes;
     const int rc = images_on_device ? encode_device_frames(c, job, planes) : encode_host_frames(c, job, reinterpret_cast<const uint8_t* const*>(planes));
     if (total_bytes) *total_bytes = job.packed_at;
