@@ -186,7 +186,7 @@ size_t jpgenc_write_headers(uint32_t real_w, uint32_t real_h, const uint8_t qy[6
 int jpgenc_encode_bound(jpgenc_ctx* ctx, uint8_t* dst, uint64_t cap, uint64_t* jpeg_bytes);
 /* headers + scan of the LAST jpgenc_encode_bound on this context + EOI into dst, without re-running the pipeline */
 int jpgenc_assemble_last(jpgenc_ctx* ctx, uint8_t* dst, uint64_t cap, uint64_t* jpeg_bytes);
-/* upload + encode (host pixels in, JPEG bytes out) */
+/* upload + encode (host pixels in, JPEG bytes out).  Sides outside 1..65535: JPGENC_ERR_ARG. */
 int jpgenc_encode_rgb(jpgenc_ctx* ctx, const uint8_t* host_rgb, uint32_t real_w, uint32_t real_h, uint32_t maxval,
                       uint8_t* dst, uint64_t cap, uint64_t* jpeg_bytes);
 /* the same for host pixels in any JPGENC_PIXEL_* format with a row pitch (0 = tight).  The rows travel as they are, in their

@@ -443,63 +443,44 @@ class Encoder:
             self._check(self.lib.jpgenc_encode_bound(self.h, out.ctypes.data, out.size, C.byref(n)))
         return n.value
 
-    def encode_rgb(self, rgb: np.ndarray, maxval: int = 255) -> bytes:
-        rgb = np.ascontiguousarray(rgb, np.uint8)
-        h, w, _ = rgb.shape
-        cap = max(4096, rgb.size // 2 + 4096)
+    def _file(self, encode, cap: int) -> bytes:
+        """encode(out_ptr, cap, byref(size)) -> rc of a call that writes one file; the buffer grows to the size it reports when
+        it is too small"""
         while True:
             out = np.empty(cap, np.uint8)
             n = C.c_uint64()
-            rc = self.lib.jpgenc_encode_rgb(self.h, rgb.ctypes.data, w, h, maxval, out.ctypes.data, cap, C.byref(n))
+            rc = encode(out.ctypes.data, cap, C.byref(n))
             if rc == ERR_CAPACITY:
                 cap = int(n.value) + 16
                 continue
             self._check(rc)
             return out[: n.value].tobytes()
+
+    def encode_rgb(self, rgb: np.ndarray, maxval: int = 255) -> bytes:
+        rgb = np.ascontiguousarray(rgb, np.uint8)
+        h, w, _ = rgb.shape
+        return self._file(lambda out, cap, n: self.lib.jpgenc_encode_rgb(self.h, rgb.ctypes.data, w, h, maxval, out, cap, n),
+                          max(4096, rgb.size // 2 + 4096))
 
     def encode_image(self, arr: np.ndarray, fmt: str = "RGB", maxval: int = 255) -> bytes:
         """host pixels in format fmt: a uint8 (H, W, 3 or 4) array with strides (pitch, C, 1), e.g. a crop view of a larger
         image (see image_layout) -> JPEG bytes"""
         ptr, w, h, pitch = image_layout(arr, fmt)
         code = _format_code(fmt)
-        cap = max(4096, w * h * 3 // 2 + 4096)
-        while True:
-            out = np.empty(cap, np.uint8)
-            n = C.c_uint64()
-            rc = self.lib.jpgenc_encode_image(self.h, ptr, w, h, pitch, code, maxval, out.ctypes.data, cap, C.byref(n))
-            if rc == ERR_CAPACITY:
-                cap = int(n.value) + 16
-                continue
-            self._check(rc)
-            return out[: n.value].tobytes()
+        return self._file(lambda out, cap, n: self.lib.jpgenc_encode_image(self.h, ptr, w, h, pitch, code, maxval, out, cap, n),
+                          max(4096, w * h * 3 // 2 + 4096))
 
     def encode_planar(self, r: int, g: int, b: int, w: int, h: int, pitch: int = 0, maxval: int = 255) -> bytes:
         """planar RGB in host memory (three plane pointers, one row pitch; 0: tight) -> JPEG bytes"""
-        cap = max(4096, w * h * 3 // 2 + 4096)
-        while True:
-            out = np.empty(cap, np.uint8)
-            n = C.c_uint64()
-            rc = self.lib.jpgenc_encode_planar(self.h, r, g, b, w, h, pitch, maxval, out.ctypes.data, cap, C.byref(n))
-            if rc == ERR_CAPACITY:
-                cap = int(n.value) + 16
-                continue
-            self._check(rc)
-            return out[: n.value].tobytes()
+        return self._file(lambda out, cap, n: self.lib.jpgenc_encode_planar(self.h, r, g, b, w, h, pitch, maxval, out, cap, n),
+                          max(4096, w * h * 3 // 2 + 4096))
 
     def encode_yuv420_ptr(self, y: int, u: int, v: int | None, w: int, h: int, y_pitch: int = 0, c_pitch: int = 0,
                           layout: str = "I420") -> bytes:
         """a YUV 4:2:0 frame in host memory (plane pointers, see bind_device_yuv420) -> JPEG bytes"""
-        cap = max(4096, w * h * 3 // 2 + 4096)
-        while True:
-            out = np.empty(cap, np.uint8)
-            n = C.c_uint64()
-            rc = self.lib.jpgenc_encode_yuv420(self.h, y, u, v or None, w, h, y_pitch, c_pitch, YUV_LAYOUTS[layout], out.ctypes.data, cap,
-                                               C.byref(n))
-            if rc == ERR_CAPACITY:
-                cap = int(n.value) + 16
-                continue
-            self._check(rc)
-            return out[: n.value].tobytes()
+        code = YUV_LAYOUTS[layout]
+        return self._file(lambda out, cap, n: self.lib.jpgenc_encode_yuv420(self.h, y, u, v or None, w, h, y_pitch, c_pitch, code, out, cap, n),
+                          max(4096, w * h * 3 // 2 + 4096))
 
     def encode_planes(self, p0: np.ndarray, p1: np.ndarray, p2: np.ndarray, real_w: int, real_h: int, ycbcr: bool = False) -> bytes:
         """three (H16, W16) float64 planes as the reference's Image holds them -> JPEG bytes (exact FP64 path for every block)"""
@@ -564,64 +545,51 @@ class Encoder:
                                                          offs, sizes, C.byref(total)))
         return [int(x) for x in offs], [int(x) for x in sizes], int(total.value)
 
+    def _packed(self, fn, n: int, per_image: int, ptrs, host_images: bool, widths, heights, *args):
+        """the marshalling the encode_images_packed* calls share: fn(handle, n, pointers, on_device, widths, heights, *args,
+        offsets, sizes, &total); optional per-image arrays in args are lists or None; returns (offsets, sizes, total bytes).
+        The pointer array holds per_image * n entries, as the C side reads them; missing ones are NULL."""
+        arrays = [np.ascontiguousarray(a, np.uint32) for a in (widths, heights)]
+        conv = []
+        for a in args:
+            if isinstance(a, (list, tuple, np.ndarray)):
+                arrays.append(np.ascontiguousarray(a, np.uint32))
+                conv.append(_np_ptr(arrays[-1], u32p))
+            else:
+                conv.append(a)
+        sizes = (C.c_uint64 * n)()
+        offs = (C.c_uint64 * n)()
+        total = C.c_uint64()
+        self._check(fn(self.h, n, (C.c_void_p * (per_image * n))(*ptrs), 0 if host_images else 1, _np_ptr(arrays[0], u32p), _np_ptr(arrays[1], u32p),
+                       *conv, offs, sizes, C.byref(total)))
+        return [int(x) for x in offs], [int(x) for x in sizes], int(total.value)
+
     def encode_images_packed(self, ptrs, widths, heights, out_ptr: int | None, cap: int, maxval: int = 255, host_images=False,
                              pitches=None, fmt=None):
         """images of individual sizes (device memory, or host memory with host_images=True) -> complete files back to back in
         ONE buffer, in input order; returns (offsets, sizes, total bytes).  pitches (bytes from row to row, per image; None or 0:
         tight) and fmt ('RGB', 'BGR', 'RGBA', 'BGRA') describe pixels in another layout than tight RGB."""
         n = len(ptrs)
-        imgs = (C.c_void_p * n)(*ptrs)
-        w = np.ascontiguousarray(widths, np.uint32)
-        h = np.ascontiguousarray(heights, np.uint32)
-        sizes = (C.c_uint64 * n)()
-        offs = (C.c_uint64 * n)()
-        total = C.c_uint64()
         if pitches is None and fmt is None:
-            self._check(self.lib.jpgenc_encode_images_packed(self.h, n, imgs, 0 if host_images else 1, _np_ptr(w, u32p), _np_ptr(h, u32p), maxval,
-                                                             out_ptr, cap, offs, sizes, C.byref(total)))
-        else:
-            p = np.ascontiguousarray(pitches, np.uint32) if pitches is not None else None
-            self._check(self.lib.jpgenc_encode_images_packed_layout(self.h, n, imgs, 0 if host_images else 1, _np_ptr(w, u32p), _np_ptr(h, u32p),
-                                                                    _np_ptr(p, u32p) if p is not None else None, _format_code(fmt or "RGB"),
-                                                                    maxval, out_ptr, cap, offs, sizes, C.byref(total)))
-        return [int(x) for x in offs], [int(x) for x in sizes], int(total.value)
+            return self._packed(self.lib.jpgenc_encode_images_packed, n, 1, ptrs, host_images, widths, heights, maxval, out_ptr, cap)
+        return self._packed(self.lib.jpgenc_encode_images_packed_layout, n, 1, ptrs, host_images, widths, heights,
+                            None if pitches is None else list(pitches), _format_code(fmt or "RGB"), maxval, out_ptr, cap)
 
     def encode_images_packed_planar(self, planes, widths, heights, out_ptr: int | None, cap: int, maxval: int = 255, host_images=False,
                                     pitches=None):
         """planar RGB images of individual sizes: planes[3i:3i + 3] = the R, G, B plane pointers of image i (device memory, or host
         memory with host_images=True), pitches per image (None or 0: tight) -> files back to back as encode_images_packed"""
-        n = len(widths)
-        pl = (C.c_void_p * (3 * n))(*planes)
-        w = np.ascontiguousarray(widths, np.uint32)
-        h = np.ascontiguousarray(heights, np.uint32)
-        p = np.ascontiguousarray(pitches, np.uint32) if pitches is not None else None
-        sizes = (C.c_uint64 * n)()
-        offs = (C.c_uint64 * n)()
-        total = C.c_uint64()
-        self._check(self.lib.jpgenc_encode_images_packed_planar(self.h, n, pl, 0 if host_images else 1, _np_ptr(w, u32p), _np_ptr(h, u32p),
-                                                                _np_ptr(p, u32p) if p is not None else None, maxval, out_ptr, cap, offs,
-                                                                sizes, C.byref(total)))
-        return [int(x) for x in offs], [int(x) for x in sizes], int(total.value)
+        return self._packed(self.lib.jpgenc_encode_images_packed_planar, len(widths), 3, planes, host_images, widths, heights,
+                            None if pitches is None else list(pitches), maxval, out_ptr, cap)
 
     def encode_images_packed_yuv420(self, planes, widths, heights, out_ptr: int | None, cap: int, layout: str = "I420", host_images=False,
                                     y_pitches=None, c_pitches=None):
         """YUV 4:2:0 frames of individual sizes: planes[3i:3i + 3] = the Y, U, V plane pointers of frame i (NV12: Y, UV, None;
         device memory, or host memory with host_images=True), pitches per frame (None or 0: tight) -> files back to back as
         encode_images_packed"""
-        n = len(widths)
-        pl = (C.c_void_p * (3 * n))(*planes)
-        w = np.ascontiguousarray(widths, np.uint32)
-        h = np.ascontiguousarray(heights, np.uint32)
-        yp = np.ascontiguousarray(y_pitches, np.uint32) if y_pitches is not None else None
-        cp = np.ascontiguousarray(c_pitches, np.uint32) if c_pitches is not None else None
-        sizes = (C.c_uint64 * n)()
-        offs = (C.c_uint64 * n)()
-        total = C.c_uint64()
-        self._check(self.lib.jpgenc_encode_images_packed_yuv420(self.h, n, pl, 0 if host_images else 1, _np_ptr(w, u32p), _np_ptr(h, u32p),
-                                                                _np_ptr(yp, u32p) if yp is not None else None,
-                                                                _np_ptr(cp, u32p) if cp is not None else None, YUV_LAYOUTS[layout], out_ptr,
-                                                                cap, offs, sizes, C.byref(total)))
-        return [int(x) for x in offs], [int(x) for x in sizes], int(total.value)
+        return self._packed(self.lib.jpgenc_encode_images_packed_yuv420, len(widths), 3, planes, host_images, widths, heights,
+                            None if y_pitches is None else list(y_pitches), None if c_pitches is None else list(c_pitches),
+                            YUV_LAYOUTS[layout], out_ptr, cap)
 
     def _planes_on_host(self, planes) -> bool:
         """True for numpy arrays and CPU tensors; False for tensors on this encoder's GPU, once the work queued on torch's current

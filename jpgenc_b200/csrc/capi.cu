@@ -69,8 +69,8 @@ int set_geometry(jpgenc_ctx* c, uint32_t w, uint32_t h, uint32_t maxval) {
     if (w == 0 || h == 0 || maxval == 0 || maxval > 255) return fail(c, JPGENC_ERR_ARG, "width/height/maxval out of range");
     c->real_w = w; c->real_h = h; c->maxval = maxval;
     c->mcu_w = (w + 15) / 16; c->mcu_h = (h + 15) / 16;        // src/Image.cpp:479-489
-    c->pixel_format = JPGENC_PIXEL_RGB;
-    c->row_pitch = w * 3;
+    c->src = PixelSource{};                                      // tight RGB until a bind sets its source
+    c->src.pitch = w * 3;
     c->nframes = 1;
     c->mixed.on = false;
     c->have_pixels = false;                                      // whoever changes the geometry binds its pixels afterwards
@@ -78,29 +78,83 @@ int set_geometry(jpgenc_ctx* c, uint32_t w, uint32_t h, uint32_t maxval) {
     return JPGENC_OK;
 }
 
-int check_layout(jpgenc_ctx* c, uint32_t w, uint32_t h, uint32_t* row_pitch, int format) {
-    if ((format < JPGENC_PIXEL_RGB || format > JPGENC_PIXEL_BGRA) && format != JPGENC_PIXEL_GRAY) return fail(c, JPGENC_ERR_ARG, "unknown pixel format");
+int check_source(jpgenc_ctx* c, PixelSource* s, uint32_t w, uint32_t h) {
+    const int f = s->format;
+    if ((f < JPGENC_PIXEL_RGB || f > JPGENC_PIXEL_BGRA) && f != JPGENC_PIXEL_GRAY && f != kPixelPlanar && !is_yuv(f))
+        return fail(c, JPGENC_ERR_ARG, "unknown pixel format");
+    for (uint32_t k = 0; k < source_planes(f); ++k)
+        if (!s->plane[k] && !(f == kPixelNV12 && k == 2)) return fail(c, JPGENC_ERR_ARG, "null plane pointer");
+    if (f == kPixelNV12 && s->plane[2]) return fail(c, JPGENC_ERR_ARG, "NV12 takes its UV plane as u; v must be NULL");
     if (w == 0 || h == 0 || w > 65535 || h > 65535) return fail(c, JPGENC_ERR_ARG, "image side out of range (1..65535)");
-    const uint32_t row = w * pixel_bytes(format);
-    if (*row_pitch == 0) *row_pitch = row;
-    if (*row_pitch < row) return fail(c, JPGENC_ERR_ARG, "row pitch below the row size");
+    const uint32_t row = w * pixel_bytes(f);
+    if (s->pitch == 0) s->pitch = row;
+    if (s->pitch < row) return fail(c, JPGENC_ERR_ARG, "row pitch below the row size");
+    if (f == kPixelPlanar) s->pitch2 = s->pitch;
+    if (is_yuv(f)) {
+        const uint32_t crow = chroma_row_bytes(f, w);
+        if (s->pitch2 == 0) s->pitch2 = crow;
+        if (s->pitch2 < crow) return fail(c, JPGENC_ERR_ARG, "chroma pitch below the chroma row size");
+    }
     return JPGENC_OK;
 }
 
-// a YUV 4:2:0 frame's planes and pitches (jpgenc_bind_device_yuv420): 0 pitches become tight; the internal format on success
-int check_yuv420(jpgenc_ctx* c, const void* y, const void* u, const void* v, uint32_t w, uint32_t h, uint32_t* y_pitch, uint32_t* c_pitch,
-                 int layout, int* format) {
-    if (layout != JPGENC_YUV_I420 && layout != JPGENC_YUV_NV12) return fail(c, JPGENC_ERR_ARG, "unknown YUV layout");
-    if (!y || !u) return fail(c, JPGENC_ERR_ARG, "null plane pointer");
-    if (layout == JPGENC_YUV_I420 && !v) return fail(c, JPGENC_ERR_ARG, "null V plane (I420)");
-    if (layout == JPGENC_YUV_NV12 && v) return fail(c, JPGENC_ERR_ARG, "NV12 takes its UV plane as u; v must be NULL");
-    int rc = check_layout(c, w, h, y_pitch, JPGENC_PIXEL_GRAY);           // the Y plane: one byte per pixel
-    if (rc) return rc;
-    const uint32_t crow = ((w + 1) / 2) * (layout == JPGENC_YUV_NV12 ? 2 : 1);
-    if (*c_pitch == 0) *c_pitch = crow;
-    if (*c_pitch < crow) return fail(c, JPGENC_ERR_ARG, "chroma pitch below the chroma row size");
-    *format = layout == JPGENC_YUV_NV12 ? kPixelNV12 : kPixelI420;
-    return JPGENC_OK;
+bool source_within_maxval(const PixelSource& s, uint32_t w, uint32_t h, uint32_t maxval) {
+    if (maxval == 0 || maxval >= 255 || is_yuv(s.format)) return true;
+    for (uint32_t k = 0; k < source_planes(s.format); ++k)
+        if (!samples_within_maxval(s.plane[k], w, h, s.pitch, pixel_bytes(s.format), maxval)) return false;
+    return true;
+}
+
+PixelSource yuv420_source(const void* y, const void* u, const void* v, uint32_t y_pitch, uint32_t c_pitch, int layout) {
+    PixelSource s;
+    s.format = layout == JPGENC_YUV_I420 ? kPixelI420 : layout == JPGENC_YUV_NV12 ? kPixelNV12 : -1;
+    s.pitch = y_pitch;
+    s.pitch2 = c_pitch;
+    s.plane[0] = static_cast<const uint8_t*>(y); s.plane[1] = static_cast<const uint8_t*>(u); s.plane[2] = static_cast<const uint8_t*>(v);
+    return s;
+}
+
+PixelSource planar_source(const void* r, const void* g, const void* b, uint32_t pitch) {
+    PixelSource s;
+    s.format = kPixelPlanar;
+    s.pitch = pitch;
+    s.plane[0] = static_cast<const uint8_t*>(r); s.plane[1] = static_cast<const uint8_t*>(g); s.plane[2] = static_cast<const uint8_t*>(b);
+    return s;
+}
+
+PixelSource image_source(const void* px, uint32_t pitch, int format) {
+    PixelSource s;
+    s.format = (format >= JPGENC_PIXEL_RGB && format <= JPGENC_PIXEL_BGRA) || format == JPGENC_PIXEL_GRAY ? format : -1;   // public codes only
+    s.pitch = pitch;
+    s.plane[0] = static_cast<const uint8_t*>(px);
+    return s;
+}
+
+uint32_t staged_planes(const PixelSource& s, uint32_t w, uint32_t h, StagedPlane pl[3]) {
+    const bool yuv = is_yuv(s.format);
+    const uint32_t np = s.format == kPixelNV12 ? 2u : source_planes(s.format);
+    size_t off = 0;
+    for (uint32_t k = 0; k < np; ++k) {
+        const bool chroma = yuv && k > 0;
+        pl[k].host = s.plane[k];
+        pl[k].pitch = chroma ? s.pitch2 : s.pitch;
+        pl[k].row = chroma ? chroma_row_bytes(s.format, w) : static_cast<size_t>(w) * pixel_bytes(s.format);
+        pl[k].vsub = chroma ? 1u : 0u;
+        pl[k].rows = (h + pl[k].vsub) >> pl[k].vsub;
+        pl[k].dev_off = off;
+        off += pl[k].row * pl[k].rows;
+        if (yuv) off = (off + 255) & ~static_cast<size_t>(255);
+    }
+    return np;
+}
+
+size_t staged_bytes(const StagedPlane* pl, uint32_t np) { return pl[np - 1].dev_off + pl[np - 1].row * pl[np - 1].rows; }
+
+size_t planes_gap(const StagedPlane* pl, uint32_t np) {
+    if (np != 3 || pl[1].vsub || pl[0].pitch != pl[0].row) return 0;
+    const uintptr_t gap = reinterpret_cast<uintptr_t>(pl[1].host) - reinterpret_cast<uintptr_t>(pl[0].host);
+    const bool equal = reinterpret_cast<uintptr_t>(pl[2].host) - reinterpret_cast<uintptr_t>(pl[1].host) == gap;
+    return equal && gap >= pl[0].row * pl[0].rows && gap <= (uintptr_t{1} << 48) ? gap : 0;
 }
 
 // pinned host staging, grown on demand
@@ -396,10 +450,18 @@ int jpgenc_set_dct_constants(jpgenc_ctx* c, const double a[5], const double s[8]
     return JPGENC_OK;
 } JPGENC_CATCH(c)
 
+// binds device pixels: the source is checked, then replaces whatever was bound
+static int bind_source(jpgenc_ctx* c, PixelSource src, uint32_t w, uint32_t h, uint32_t maxval) {
+    int rc = check_source(c, &src, w, h);
+    if (rc || (rc = set_geometry(c, w, h, maxval))) return rc;
+    c->src = src;
+    c->have_pixels = true;
+    return JPGENC_OK;
+}
+
 int jpgenc_upload_rgb(jpgenc_ctx* c, const uint8_t* host_rgb, uint32_t w, uint32_t h, uint32_t maxval) try {
     if (!c || !host_rgb) return JPGENC_ERR_ARG;
-    if (maxval && maxval < 255 && !samples_within_maxval(host_rgb, static_cast<size_t>(w) * h * 3, maxval))
-        return fail(c, JPGENC_ERR_FORMAT, "a sample exceeds maxval");
+    if (!source_within_maxval(image_source(host_rgb, w * 3, JPGENC_PIXEL_RGB), w, h, maxval)) return fail(c, JPGENC_ERR_FORMAT, "a sample exceeds maxval");
     JPGENC_CUDA(c, cudaSetDevice(c->device));
     int rc = set_geometry(c, w, h, maxval);
     if (rc) return rc;
@@ -410,7 +472,7 @@ int jpgenc_upload_rgb(jpgenc_ctx* c, const uint8_t* host_rgb, uint32_t w, uint32
     JPGENC_CUDA(c, jpgenc_record(c, c->ev_b));
     JPGENC_CUDA(c, cudaStreamSynchronize(c->stream));            // the caller may reuse host_rgb as soon as we return
     JPGENC_CUDA(c, cudaEventElapsedTime(&c->stats.ms_h2d, c->ev_a, c->ev_b));
-    c->d_rgb = c->d_rgb_owned;
+    c->src.plane[0] = c->d_rgb_owned;
     c->have_pixels = true;
     return JPGENC_OK;
 } JPGENC_CATCH(c)
@@ -419,52 +481,26 @@ int jpgenc_bind_device_rgb(jpgenc_ctx* c, const void* dev_rgb, uint32_t w, uint3
     if (!c || !dev_rgb) return JPGENC_ERR_ARG;
     const int rc = set_geometry(c, w, h, maxval);
     if (rc) return rc;
-    c->d_rgb = static_cast<const uint8_t*>(dev_rgb);
+    c->src.plane[0] = static_cast<const uint8_t*>(dev_rgb);
     c->have_pixels = true;
     return JPGENC_OK;
 } JPGENC_CATCH(c)
 
 int jpgenc_bind_device_image(jpgenc_ctx* c, const void* dev, uint32_t w, uint32_t h, uint32_t row_pitch, int format, uint32_t maxval) try {
     if (!c) return JPGENC_ERR_ARG;
-    if (!dev) return fail(c, JPGENC_ERR_ARG, "null image pointer");
-    int rc = check_layout(c, w, h, &row_pitch, format);
-    if (rc || (rc = set_geometry(c, w, h, maxval))) return rc;
-    c->pixel_format = format;
-    c->row_pitch = row_pitch;
-    c->d_rgb = static_cast<const uint8_t*>(dev);
-    c->have_pixels = true;
-    return JPGENC_OK;
+    return bind_source(c, image_source(dev, row_pitch, format), w, h, maxval);
 } JPGENC_CATCH(c)
 
 int jpgenc_bind_device_planar(jpgenc_ctx* c, const void* r, const void* g, const void* b, uint32_t w, uint32_t h, uint32_t row_pitch,
                               uint32_t maxval) try {
     if (!c) return JPGENC_ERR_ARG;
-    if (!r || !g || !b) return fail(c, JPGENC_ERR_ARG, "null plane pointer");
-    int rc = check_layout(c, w, h, &row_pitch, JPGENC_PIXEL_GRAY);        // every plane: one byte per pixel
-    if (rc || (rc = set_geometry(c, w, h, maxval))) return rc;
-    c->pixel_format = kPixelPlanar;
-    c->row_pitch = row_pitch;
-    c->d_rgb = static_cast<const uint8_t*>(r);
-    c->d_plane_g = static_cast<const uint8_t*>(g);
-    c->d_plane_b = static_cast<const uint8_t*>(b);
-    c->have_pixels = true;
-    return JPGENC_OK;
+    return bind_source(c, planar_source(r, g, b, row_pitch), w, h, maxval);
 } JPGENC_CATCH(c)
 
 int jpgenc_bind_device_yuv420(jpgenc_ctx* c, const void* y, const void* u, const void* v, uint32_t w, uint32_t h, uint32_t y_pitch,
                               uint32_t c_pitch, int layout) try {
     if (!c) return JPGENC_ERR_ARG;
-    int format = 0;
-    int rc = check_yuv420(c, y, u, v, w, h, &y_pitch, &c_pitch, layout, &format);
-    if (rc || (rc = set_geometry(c, w, h, 255))) return rc;
-    c->pixel_format = format;
-    c->row_pitch = y_pitch;
-    c->d_rgb = static_cast<const uint8_t*>(y);
-    c->d_plane_g = static_cast<const uint8_t*>(u);
-    c->d_plane_b = static_cast<const uint8_t*>(v);
-    c->chroma_pitch = c_pitch;
-    c->have_pixels = true;
-    return JPGENC_OK;
+    return bind_source(c, yuv420_source(y, u, v, y_pitch, c_pitch, layout), w, h, 255);
 } JPGENC_CATCH(c)
 
 static int enqueue_forward(jpgenc_ctx* c);
@@ -886,12 +922,11 @@ static int run_pipeline(jpgenc_ctx* c, jpgenc_huff_table tables[4], uint64_t* sc
     // ---- phase A: K1, refinement, K2, statistics into the mailbox ----
     c->k2_tiles_done = 0;
     // (the pixel layout picks K1, its thresholds and the refinement: it is part of the key, with every plane and pitch)
-    const bool planes = c->pixel_format == kPixelPlanar || is_yuv(c->pixel_format);
-    const uint64_t key_a[kGraphKeyWords] = {c->alloc_gen, reinterpret_cast<uint64_t>(c->d_rgb), (static_cast<uint64_t>(c->real_w) << 32) | c->real_h,
-                                            c->maxval | static_cast<uint64_t>(c->pixel_format) << 8 | static_cast<uint64_t>(c->row_pitch) << 32,
-                                            1u | static_cast<uint64_t>(c->stage_timing) << 8,
-                                            planes ? reinterpret_cast<uint64_t>(c->d_plane_g) : 0, planes ? reinterpret_cast<uint64_t>(c->d_plane_b) : 0,
-                                            is_yuv(c->pixel_format) ? c->chroma_pitch : 0};
+    const PixelSource& src = c->src;
+    const uint64_t key_a[kGraphKeyWords] = {c->alloc_gen, reinterpret_cast<uint64_t>(src.plane[0]), (static_cast<uint64_t>(c->real_w) << 32) | c->real_h,
+                                            c->maxval | static_cast<uint64_t>(src.format) << 8 | static_cast<uint64_t>(src.pitch) << 32,
+                                            1u | static_cast<uint64_t>(c->stage_timing) << 8, reinterpret_cast<uint64_t>(src.plane[1]),
+                                            reinterpret_cast<uint64_t>(src.plane[2]), src.pitch2};
     const bool pool = c->parallel_tables;
     if (pool) {
         if (!c->pool) c->pool = new TablePool(kTableWorkers);
@@ -954,43 +989,29 @@ static int ensure_file_staging(jpgenc_ctx* c, size_t bytes) {
 // `fill` (optional): instead of reading the pixels from `host_rgb`, every band is first produced by fill(dst, byte offset in
 // the image, bytes) into one of two pinned staging buffers (a file read, for instance) and uploaded from there: bounded
 // pinned memory, full PCIe rate, and the production of band b+1 overlaps the upload of band b.
-// Pixels in another layout (`format`, rows `pitch` bytes apart in host memory) travel as they are, in their own format, the
-// pitch gap dropped by the copy: on the device they are tight rows of that format, read by the pixel-layout kernels.
-// Planar RGB (kPixelPlanar; host_rgb, host_g, host_b are the planes) lands as three tight planes back to back.
-// YUV 4:2:0 (kPixelI420 / kPixelNV12; host_rgb is Y with `pitch`, host_g and host_b are U and V -- NV12: UV -- with `c_pitch`)
-// lands as tight planes, each starting on 256 bytes; a band carries its 16 Y rows and 8 chroma rows per MCU row.
-static int upload_and_forward(jpgenc_ctx* c, const uint8_t* host_rgb, uint32_t w, uint32_t h, uint32_t maxval,
-                              const std::function<int(uint8_t*, size_t, size_t)>* fill = nullptr, int format = JPGENC_PIXEL_RGB,
-                              size_t pitch = 0, const uint8_t* host_g = nullptr, const uint8_t* host_b = nullptr, size_t c_pitch = 0) {
+// Pixels in another layout travel as they are, in their own format, plane by plane (staged_planes), the pitch gaps dropped by
+// the copy: on the device they are tight rows of that format, read by the pixel-layout kernels; a band carries every plane's
+// rows of its MCU rows.  `host` is checked (check_source); with `fill` its plane is not read.
+static int upload_and_forward(jpgenc_ctx* c, const PixelSource& host, uint32_t w, uint32_t h, uint32_t maxval,
+                              const std::function<int(uint8_t*, size_t, size_t)>* fill = nullptr) {
     JPGENC_CUDA(c, cudaSetDevice(c->device));
     int rc = set_geometry(c, w, h, maxval);
     if (rc) return rc;
-    const size_t row_bytes = static_cast<size_t>(w) * pixel_bytes(format), bytes = row_bytes * h;
-    const bool yuv = is_yuv(format);
-    const uint32_t nplanes = format == kPixelPlanar ? 3 : 1;
-    if (pitch == 0) pitch = row_bytes;
-    c->pixel_format = format;
-    c->row_pitch = static_cast<uint32_t>(row_bytes);
-    // YUV: chroma rows of crow bytes, ch of them, in ncp planes behind the Y plane
-    const size_t crow = static_cast<size_t>((w + 1) / 2) * (format == kPixelNV12 ? 2 : 1), ch = (h + 1) / 2;
-    const uint32_t ncp = format == kPixelI420 ? 2 : 1;
-    auto align256 = [](size_t x) { return (x + 255) & ~static_cast<size_t>(255); };
-    const size_t c_off = align256(bytes), c_plane = align256(crow * ch);
-    if ((rc = ensure(c, &c->d_rgb_owned, &c->rgb_cap, (yuv ? c_off + ncp * c_plane : nplanes * bytes) + 16))) return rc;
-    c->d_rgb = c->d_rgb_owned;
-    c->d_plane_g = c->d_rgb_owned + (yuv ? c_off : bytes);
-    c->d_plane_b = yuv ? (ncp == 2 ? c->d_rgb_owned + c_off + c_plane : nullptr) : c->d_rgb_owned + 2 * bytes;
-    if (yuv) c->chroma_pitch = static_cast<uint32_t>(crow);
+    StagedPlane pl[3];
+    const uint32_t np = staged_planes(host, w, h, pl);
+    const size_t row_bytes = pl[0].row;
+    if ((rc = ensure(c, &c->d_rgb_owned, &c->rgb_cap, staged_bytes(pl, np) + 16))) return rc;
+    c->src = host;
+    for (uint32_t k = 0; k < 3; ++k) c->src.plane[k] = k < np ? c->d_rgb_owned + pl[k].dev_off : nullptr;
+    c->src.pitch = static_cast<uint32_t>(row_bytes);
+    if (np > 1) c->src.pitch2 = static_cast<uint32_t>(pl[1].row);
     c->have_pixels = true;
     if ((rc = ensure_coef(c))) return rc;
-    const uint8_t* host_plane[3] = {host_rgb, host_g, host_b};
-    // planes that lie `gap` bytes apart with tight rows (a (3, H, W) buffer) travel as ONE strided copy per band
-    const uintptr_t gap = reinterpret_cast<uintptr_t>(host_g) - reinterpret_cast<uintptr_t>(host_rgb);
-    const bool one_copy = nplanes == 3 && pitch == row_bytes && gap >= bytes && gap <= (uintptr_t{1} << 48) &&
-                          reinterpret_cast<uintptr_t>(host_b) - reinterpret_cast<uintptr_t>(host_g) == gap;
+    const size_t gap = planes_gap(pl, np);                       // planes equally spaced with tight rows: one strided copy per band
     constexpr uint32_t kMaxBands = sizeof(c->ev_band) / sizeof(c->ev_band[0]);
     // bands of at least ~8 MB (a copy that size already runs at full PCIe rate), at most kMaxBands of them
-    const size_t mcu_row_bytes = yuv ? row_bytes * 16 + crow * ncp * 8 : row_bytes * nplanes * 16;
+    size_t mcu_row_bytes = 0;
+    for (uint32_t k = 0; k < np; ++k) mcu_row_bytes += pl[k].row * (16 >> pl[k].vsub);
     uint32_t rows_per_band = static_cast<uint32_t>(std::max<size_t>(1, (8u << 20) / mcu_row_bytes));
     rows_per_band = std::max(rows_per_band, (c->mcu_h + kMaxBands - 1) / kMaxBands);
     if ((rc = ensure_stats_buffers(c))) return rc;
@@ -1001,7 +1022,8 @@ static int upload_and_forward(jpgenc_ctx* c, const uint8_t* host_rgb, uint32_t w
         const uint32_t rows = std::min(rows_per_band, c->mcu_h - y0);
         const size_t px0 = static_cast<size_t>(y0) * 16, px1 = std::min<size_t>(h, static_cast<size_t>(y0 + rows) * 16);
         if (px1 > px0) {
-            const uint8_t* src = host_rgb ? host_rgb + px0 * pitch : nullptr;
+            const uint8_t* src = fill ? nullptr : pl[0].host + px0 * pl[0].pitch;
+            size_t src_pitch = pl[0].pitch;
             if (fill) {
                 const size_t band_bytes = static_cast<size_t>(rows_per_band) * 16 * row_bytes;
                 if (band == 0) {
@@ -1012,30 +1034,22 @@ static int upload_and_forward(jpgenc_ctx* c, const uint8_t* host_rgb, uint32_t w
                 uint8_t* slot = static_cast<uint8_t*>(c->h_file_pinned) + (band & 1) * band_bytes;
                 if ((rc = (*fill)(slot, px0 * row_bytes, (px1 - px0) * row_bytes))) return fail(c, rc, "truncated PPM payload, or a sample above maxval");
                 src = slot;
+                src_pitch = row_bytes;
             }
-            if (yuv) {
-                // Y rows [px0, px1), chroma rows [px0 / 2, ceil(px1 / 2)): what K1 reads for these MCU rows
-                auto copy_rows = [&](uint8_t* dst, const uint8_t* from, size_t row, size_t from_pitch, size_t rows) -> int {
-                    if (from_pitch == row) JPGENC_CUDA(c, cudaMemcpyAsync(dst, from, rows * row, cudaMemcpyHostToDevice, c->copy_stream));
-                    else JPGENC_CUDA(c, cudaMemcpy2DAsync(dst, row, from, from_pitch, row, rows, cudaMemcpyHostToDevice, c->copy_stream));
-                    return JPGENC_OK;
-                };
-                if ((rc = copy_rows(c->d_rgb_owned + px0 * row_bytes, src, row_bytes, pitch, px1 - px0))) return rc;
-                const size_t c0 = px0 / 2, c1 = (px1 + 1) / 2;
-                for (uint32_t k = 0; k < ncp; ++k)
-                    if ((rc = copy_rows(c->d_rgb_owned + c_off + k * c_plane + c0 * crow, host_plane[1 + k] + c0 * c_pitch, crow, c_pitch, c1 - c0)))
-                        return rc;
-            } else if (one_copy)
-                JPGENC_CUDA(c, cudaMemcpy2DAsync(c->d_rgb_owned + px0 * row_bytes, bytes, src, gap, (px1 - px0) * row_bytes, 3, cudaMemcpyHostToDevice,
-                                                 c->copy_stream));
+            if (gap)
+                JPGENC_CUDA(c, cudaMemcpy2DAsync(c->d_rgb_owned + px0 * row_bytes, pl[1].dev_off, src, gap, (px1 - px0) * row_bytes, np,
+                                                 cudaMemcpyHostToDevice, c->copy_stream));
             else
-                for (uint32_t k = 0; k < nplanes; ++k) {
-                    if (k) src = host_plane[k] + px0 * pitch;
-                    uint8_t* dst = c->d_rgb_owned + k * bytes + px0 * row_bytes;
-                    if (pitch == row_bytes)
-                        JPGENC_CUDA(c, cudaMemcpyAsync(dst, src, (px1 - px0) * row_bytes, cudaMemcpyHostToDevice, c->copy_stream));
+                for (uint32_t k = 0; k < np; ++k) {
+                    // the rows of plane k under MCU rows [y0, y0 + rows): [px0, px1) at full height, [px0 / 2, ceil(px1 / 2)) subsampled
+                    const size_t r0 = px0 >> pl[k].vsub, r1 = (px1 + pl[k].vsub) >> pl[k].vsub;
+                    const uint8_t* from = k ? pl[k].host + r0 * pl[k].pitch : src;
+                    const size_t from_pitch = k ? pl[k].pitch : src_pitch;
+                    uint8_t* dst = c->d_rgb_owned + pl[k].dev_off + r0 * pl[k].row;
+                    if (from_pitch == pl[k].row)
+                        JPGENC_CUDA(c, cudaMemcpyAsync(dst, from, (r1 - r0) * pl[k].row, cudaMemcpyHostToDevice, c->copy_stream));
                     else
-                        JPGENC_CUDA(c, cudaMemcpy2DAsync(dst, row_bytes, src, pitch, row_bytes, px1 - px0, cudaMemcpyHostToDevice, c->copy_stream));
+                        JPGENC_CUDA(c, cudaMemcpy2DAsync(dst, pl[k].row, from, from_pitch, pl[k].row, r1 - r0, cudaMemcpyHostToDevice, c->copy_stream));
                 }
         }
         JPGENC_CUDA(c, cudaEventRecord(c->ev_band[band], c->copy_stream));
@@ -1091,71 +1105,56 @@ int jpgenc_assemble_last(jpgenc_ctx* c, uint8_t* dst, uint64_t cap, uint64_t* jp
     return assemble(c, c->last_tables, c->stats.scan_bytes, dst, cap);
 } JPGENC_CATCH(c)
 
-int jpgenc_encode_rgb(jpgenc_ctx* c, const uint8_t* host_rgb, uint32_t w, uint32_t h, uint32_t maxval, uint8_t* dst,
-                      uint64_t cap, uint64_t* jpeg_bytes) try {
-    if (!c || !host_rgb) return JPGENC_ERR_ARG;
-    if (maxval && maxval < 255 && !samples_within_maxval(host_rgb, static_cast<size_t>(w) * h * 3, maxval))
-        return fail(c, JPGENC_ERR_FORMAT, "a sample exceeds maxval");
-    int rc = upload_and_forward(c, host_rgb, w, h, maxval);
-    if (rc) return rc;
-    jpgenc_huff_table tables[4];
-    uint64_t scan = 0;
-    if ((rc = run_entropy_stages(c, tables, &scan))) return rc;       // its first synchronisation also covers the copies
-    const size_t hdr = jpgenc_write_headers(c->real_w, c->real_h, c->qy, c->qc, tables, nullptr);
-    if (jpeg_bytes) *jpeg_bytes = hdr + scan + 2;
-    if (!dst) return JPGENC_OK;
-    return assemble(c, tables, scan, dst, cap);
-} JPGENC_CATCH(c)
-
-// the rest of an encode after upload_and_forward: K2 .. K4, then the file into dst (NULL: the size only)
-static int finish_upload_encode(jpgenc_ctx* c, uint8_t* dst, uint64_t cap, uint64_t* jpeg_bytes) {
+// the rest of an encode whose coefficients are on their way: K2 .. K4, then the file into dst (NULL: the size only) or, with
+// `out`, into *out, resized to the file
+static int finish_encode(jpgenc_ctx* c, uint8_t* dst, uint64_t cap, uint64_t* jpeg_bytes, std::vector<uint8_t>* out = nullptr) {
     jpgenc_huff_table tables[4];
     uint64_t scan = 0;
     const int rc = run_entropy_stages(c, tables, &scan);             // its first synchronisation also covers the copies
     if (rc) return rc;
     const size_t hdr = jpgenc_write_headers(c->real_w, c->real_h, c->qy, c->qc, tables, nullptr);
     if (jpeg_bytes) *jpeg_bytes = hdr + scan + 2;
+    if (out) {
+        out->resize(hdr + scan + 2);
+        dst = out->data();
+        cap = out->size();
+    }
     if (!dst) return JPGENC_OK;
     return assemble(c, tables, scan, dst, cap);
 }
 
+// host pixels: checked, uploaded band by band behind K1, encoded
+static int encode_host_source(jpgenc_ctx* c, PixelSource src, uint32_t w, uint32_t h, uint32_t maxval, uint8_t* dst, uint64_t cap,
+                              uint64_t* jpeg_bytes) {
+    int rc = check_source(c, &src, w, h);
+    if (rc) return rc;
+    if (!source_within_maxval(src, w, h, maxval)) return fail(c, JPGENC_ERR_FORMAT, "a sample exceeds maxval");
+    if ((rc = upload_and_forward(c, src, w, h, maxval))) return rc;
+    return finish_encode(c, dst, cap, jpeg_bytes);
+}
+
+int jpgenc_encode_rgb(jpgenc_ctx* c, const uint8_t* host_rgb, uint32_t w, uint32_t h, uint32_t maxval, uint8_t* dst,
+                      uint64_t cap, uint64_t* jpeg_bytes) try {
+    if (!c || !host_rgb) return JPGENC_ERR_ARG;
+    return encode_host_source(c, image_source(host_rgb, 0, JPGENC_PIXEL_RGB), w, h, maxval, dst, cap, jpeg_bytes);
+} JPGENC_CATCH(c)
+
 int jpgenc_encode_image(jpgenc_ctx* c, const void* host, uint32_t w, uint32_t h, uint32_t row_pitch, int format, uint32_t maxval,
                         uint8_t* dst, uint64_t cap, uint64_t* jpeg_bytes) try {
     if (!c) return JPGENC_ERR_ARG;
-    if (!host) return fail(c, JPGENC_ERR_ARG, "null image pointer");
-    int rc = check_layout(c, w, h, &row_pitch, format);
-    if (rc) return rc;
-    const uint8_t* px = static_cast<const uint8_t*>(host);
-    if (maxval && maxval < 255 && !samples_within_maxval(px, w, h, row_pitch, pixel_bytes(format), maxval))
-        return fail(c, JPGENC_ERR_FORMAT, "a sample exceeds maxval");
-    if ((rc = upload_and_forward(c, px, w, h, maxval, nullptr, format, row_pitch))) return rc;
-    return finish_upload_encode(c, dst, cap, jpeg_bytes);
+    return encode_host_source(c, image_source(host, row_pitch, format), w, h, maxval, dst, cap, jpeg_bytes);
 } JPGENC_CATCH(c)
 
 int jpgenc_encode_planar(jpgenc_ctx* c, const void* r, const void* g, const void* b, uint32_t w, uint32_t h, uint32_t row_pitch, uint32_t maxval,
                          uint8_t* dst, uint64_t cap, uint64_t* jpeg_bytes) try {
     if (!c) return JPGENC_ERR_ARG;
-    if (!r || !g || !b) return fail(c, JPGENC_ERR_ARG, "null plane pointer");
-    int rc = check_layout(c, w, h, &row_pitch, JPGENC_PIXEL_GRAY);         // every plane: one byte per pixel
-    if (rc) return rc;
-    const uint8_t* plane[3] = {static_cast<const uint8_t*>(r), static_cast<const uint8_t*>(g), static_cast<const uint8_t*>(b)};
-    for (const uint8_t* px : plane)
-        if (maxval && maxval < 255 && !samples_within_maxval(px, w, h, row_pitch, 1, maxval))
-            return fail(c, JPGENC_ERR_FORMAT, "a sample exceeds maxval");
-    if ((rc = upload_and_forward(c, plane[0], w, h, maxval, nullptr, kPixelPlanar, row_pitch, plane[1], plane[2]))) return rc;
-    return finish_upload_encode(c, dst, cap, jpeg_bytes);
+    return encode_host_source(c, planar_source(r, g, b, row_pitch), w, h, maxval, dst, cap, jpeg_bytes);
 } JPGENC_CATCH(c)
 
 int jpgenc_encode_yuv420(jpgenc_ctx* c, const void* y, const void* u, const void* v, uint32_t w, uint32_t h, uint32_t y_pitch,
                          uint32_t c_pitch, int layout, uint8_t* dst, uint64_t cap, uint64_t* jpeg_bytes) try {
     if (!c) return JPGENC_ERR_ARG;
-    int format = 0;
-    int rc = check_yuv420(c, y, u, v, w, h, &y_pitch, &c_pitch, layout, &format);
-    if (rc) return rc;
-    if ((rc = upload_and_forward(c, static_cast<const uint8_t*>(y), w, h, 255, nullptr, format, y_pitch, static_cast<const uint8_t*>(u),
-                                 static_cast<const uint8_t*>(v), c_pitch)))
-        return rc;
-    return finish_upload_encode(c, dst, cap, jpeg_bytes);
+    return encode_host_source(c, yuv420_source(y, u, v, y_pitch, c_pitch, layout), w, h, 255, dst, cap, jpeg_bytes);
 } JPGENC_CATCH(c)
 
 // Image::writeJPEG for an image that is not (or no longer) a set of 8-bit samples: planes a caller edited after loadPPM,
@@ -1184,13 +1183,7 @@ int jpgenc_encode_planes(jpgenc_ctx* c, const double* p0, const double* p1, cons
     c->stats.refined_blocks = static_cast<uint64_t>(c->mcu_w) * c->mcu_h * kBlocksPerMcu;
     c->have_coef = true;
     c->have_scan = c->have_items = false; c->k2_tiles_done = 0;
-    jpgenc_huff_table tables[4];
-    uint64_t scan = 0;
-    if ((rc = run_entropy_stages(c, tables, &scan))) return rc;
-    const size_t hdr = jpgenc_write_headers(c->real_w, c->real_h, c->qy, c->qc, tables, nullptr);
-    if (jpeg_bytes) *jpeg_bytes = hdr + scan + 2;
-    if (!dst) return JPGENC_OK;
-    return assemble(c, tables, scan, dst, cap);
+    return finish_encode(c, dst, cap, jpeg_bytes);
 } JPGENC_CATCH(c)
 
 // main.cpp:8-32.  A binary (P6) payload is streamed: the header is parsed from the first bytes, then every band of rows is
@@ -1230,7 +1223,7 @@ int jpgenc_encode_ppm_file(jpgenc_ctx* c, const char* ppm_path, const char* jpg_
             if (!bad.load() && !samples_within_maxval(dst, n, h.maxval)) bad.store(1);     // only scans when maxval < 255
             return bad.load() ? JPGENC_ERR_FORMAT : JPGENC_OK;
         };
-        if ((rc = upload_and_forward(c, nullptr, h.width, h.height, h.maxval, &fill))) return rc;
+        if ((rc = upload_and_forward(c, image_source(nullptr, h.width * 3, JPGENC_PIXEL_RGB), h.width, h.height, h.maxval, &fill))) return rc;
     } else {
         std::vector<uint8_t> file, p3;
         std::fclose(in);
@@ -1238,14 +1231,10 @@ int jpgenc_encode_ppm_file(jpgenc_ctx* c, const char* ppm_path, const char* jpg_
         if ((rc = slurp_file(ppm_path, &file))) return fail(c, rc, "Failed to open input file");
         const uint8_t* samples = nullptr;
         if ((rc = ppm_samples(file.data(), file.size(), h, &p3, &samples))) return fail(c, rc, "truncated PPM payload, or a sample above maxval");
-        if ((rc = upload_and_forward(c, samples, h.width, h.height, h.maxval))) return rc;
+        if ((rc = upload_and_forward(c, image_source(samples, h.width * 3, JPGENC_PIXEL_RGB), h.width, h.height, h.maxval))) return rc;
     }
-    jpgenc_huff_table tables[4];
-    uint64_t scan = 0;
-    if ((rc = run_entropy_stages(c, tables, &scan))) return rc;
-    const size_t hdr = jpgenc_write_headers(c->real_w, c->real_h, c->qy, c->qc, tables, nullptr);
-    std::vector<uint8_t> out(hdr + scan + 2);
-    if ((rc = assemble(c, tables, scan, out.data(), out.size()))) return rc;
+    std::vector<uint8_t> out;
+    if ((rc = finish_encode(c, nullptr, 0, nullptr, &out))) return rc;
     std::FILE* f = std::fopen(jpg_path, "wb");
     if (!f) return fail(c, JPGENC_ERR_IO, "Failed to open output file");
     const size_t wrote = std::fwrite(out.data(), 1, out.size(), f);

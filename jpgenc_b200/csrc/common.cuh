@@ -52,6 +52,42 @@ struct ColorConsts {                      // FP32 fast path; sample scale folded
     float y[3], cb[3], cr[3];
 };
 
+// Planar RGB: three planes of one byte per pixel, one row pitch.  It has no JPGENC_PIXEL_* code (the calls take three plane
+// pointers); inside the library it is this format.
+constexpr int kPixelPlanar = 17;
+// YUV 4:2:0 frames (jpgenc_*_yuv420; JPGENC_YUV_I420 / JPGENC_YUV_NV12 inside the library): a Y plane of one byte per pixel and
+// chroma planes of ceil(w/2) x ceil(h/2) samples -- U and V apart (I420) or interleaved U, V pairs (NV12)
+constexpr int kPixelI420 = 18;
+constexpr int kPixelNV12 = 19;
+__host__ __device__ constexpr bool is_yuv(int format) { return format == kPixelI420 || format == kPixelNV12; }
+
+// bytes of one chroma row of a YUV 4:2:0 image w pixels wide (NV12: U, V pairs)
+__host__ __device__ constexpr uint32_t chroma_row_bytes(int format, uint32_t w) { return (w + 1) / 2 * (format == kPixelNV12 ? 2u : 1u); }
+
+// bytes per pixel of a JPGENC_PIXEL_* format (planar: of one plane; YUV: of the Y plane)
+__host__ __device__ constexpr uint32_t pixel_bytes(int format) {
+    return format >= JPGENC_PIXEL_GRAY ? 1u : format >= JPGENC_PIXEL_RGBA ? 4u : 3u;
+}
+
+// Where an image's bytes are and how they are laid out: up to three planes, the format, the row pitch of the first plane and
+// a second pitch (YUV: of the chroma planes; planar RGB: equal to `pitch`; unused otherwise).  Tight RGB is {{p}, RGB, w * 3,
+// 0}.  Planar RGB: planes R, G, B; YUV: Y, U, V (NV12: Y, UV, null).
+struct PixelSource {
+    const uint8_t* plane[3] = {nullptr, nullptr, nullptr};
+    int format = JPGENC_PIXEL_RGB;        // JPGENC_PIXEL_*, kPixelPlanar, kPixelI420 or kPixelNV12
+    uint32_t pitch = 0;
+    uint32_t pitch2 = 0;
+};
+// pointers (= planes) a caller passes for an image of this format
+__host__ __device__ constexpr uint32_t source_planes(int format) { return format == kPixelPlanar || is_yuv(format) ? 3u : 1u; }
+
+// the second and third plane of one image of a pass and its second pitch: one entry per image follows the FrameGeom array in
+// the same copy for the formats of several planes (planar RGB, YUV)
+struct ExtraPlanes {
+    const uint8_t* plane[2];
+    uint64_t pitch2;
+};
+
 // ---- a pass of images of individual sizes (jpgenc_encode_images_packed), device resident -------------------------
 // One entry per image of the pass and one behind the last, whose prefix fields hold the pass totals: the images' work
 // units are numbered through the whole pass, and a CTA finds its image by a search over the prefix of its own unit.
@@ -67,13 +103,6 @@ struct FrameGeom {
     uint32_t pitch;                       // bytes from one pixel row to the next (read only by the kernels of other pixel layouts)
 };
 static_assert(sizeof(FrameGeom) == 48, "FrameGeom is copied as an array");
-
-// the chroma planes of one YUV image of a pass: they follow the FrameGeom array in the same copy (v is null for NV12)
-struct ChromaPlanes {
-    const uint8_t* u;
-    const uint8_t* v;
-    uint64_t pitch;
-};
 
 // the image f (0 <= f < F) whose units [geom[f].*key, geom[f + 1].*key) contain unit x, found by a whole warp in two rounds of
 // 32 parallel probes for F <= 1024 (every lane must take part; every lane returns f)
@@ -91,7 +120,8 @@ __device__ __forceinline__ uint32_t geom_find_warp(const FrameGeom* geom, uint32
 }
 
 struct ForwardParams {
-    const uint8_t* rgb;                   // one image ...
+    const uint8_t* rgb;                   // src.plane[0] of one image (K1 reads it here: at this offset the tight-RGB kernels compile
+                                          // to the code they were measured with) ...
     const uint8_t* const* frames;         // ... or (non-null) one device pointer per frame of a batch of equally sized frames
     uint32_t blocks_per_frame;            // frame f owns coefficient blocks [f * blocks_per_frame, (f + 1) * blocks_per_frame)
     int16_t* coef;
@@ -107,38 +137,14 @@ struct ForwardParams {
     QuantConsts2 chroma;
     alignas(64) CUtensorMap coef_map;     // coefficient array as rows of 128 bytes, for the tensor store of full strips
     // images of individual sizes (forward_mixed_kernel): geom[nframes + 1], `strips` CTAs in all; the fields above that
-    // describe one size (rgb, frames, blocks_per_frame, real_w .. mcu_y0) are unused there
+    // describe one size (frames, blocks_per_frame, real_w .. mcu_y0) and `src` are unused there
     const FrameGeom* geom;
     uint32_t nframes;
     uint32_t strips;
-    // pixels in another layout than tight RGB (forward_layout_kernel, forward_mixed_layout_kernel; the format is their template
-    // parameter): bytes from one row to the next of the single image (images of individual sizes: FrameGeom::pitch)
-    uint32_t pitch;
-    // planar RGB (kPixelPlanar): the G and B planes of the single image (its R plane is `rgb`) / of image f of a pass at
-    // planes[2f], planes[2f + 1] (its R plane is FrameGeom::rgb)
-    const uint8_t* plane_g;
-    const uint8_t* plane_b;
-    const uint8_t* const* planes;
-    // YUV 4:2:0 (kPixelI420, kPixelNV12): the single image's U and V planes are plane_g and plane_b (NV12: the UV plane is
-    // plane_g), its Y plane is `rgb` with `pitch`; chroma_pitch: bytes from one chroma row to the next.  Images of individual
-    // sizes: image f's chroma planes at yuv_chroma[f] (its Y plane is FrameGeom::rgb with FrameGeom::pitch)
-    uint32_t chroma_pitch;
-    const ChromaPlanes* yuv_chroma;
+    PixelSource src;                      // the single image: its other planes and pitches (the format is the kernels' template parameter)
+    // images of individual sizes in a format of several planes: extra[f] (plane 0 and `pitch` are in FrameGeom)
+    const ExtraPlanes* extra;
 };
-
-// Planar RGB: three planes of one byte per pixel, one row pitch.  It has no JPGENC_PIXEL_* code (the calls take three plane
-// pointers); inside the library it is this format.
-constexpr int kPixelPlanar = 17;
-// YUV 4:2:0 frames (jpgenc_*_yuv420; JPGENC_YUV_I420 / JPGENC_YUV_NV12 inside the library): a Y plane of one byte per pixel and
-// chroma planes of ceil(w/2) x ceil(h/2) samples -- U and V apart (I420) or interleaved U, V pairs (NV12)
-constexpr int kPixelI420 = 18;
-constexpr int kPixelNV12 = 19;
-__host__ __device__ constexpr bool is_yuv(int format) { return format == kPixelI420 || format == kPixelNV12; }
-
-// bytes per pixel of a JPGENC_PIXEL_* format (planar: of one plane; YUV: of the Y plane)
-__host__ __device__ constexpr uint32_t pixel_bytes(int format) {
-    return format >= JPGENC_PIXEL_GRAY ? 1u : format >= JPGENC_PIXEL_RGBA ? 4u : 3u;
-}
 
 // host side: the totals of the pass of images of individual sizes bound to a context (the device reads them from the
 // entry behind the last image of FrameGeom)
@@ -146,7 +152,7 @@ struct MixedPass {
     bool on = false;
     bool aligned = false;                 // every image has real_w % 16 == 0 and a 16-byte aligned pointer (K1's bulk copies)
     int format = -1;                      // JPGENC_PIXEL_*, kPixelPlanar, kPixelI420 or kPixelNV12: the pixel-layout kernels (with
-                                          // FrameGeom::pitch); -1 tight RGB
+                                          // FrameGeom::pitch and, for several planes, ExtraPlanes); -1 tight RGB
     uint32_t blocks = 0, strips = 0, tiles = 0, groups = 0, supers = 0;
     uint32_t split = 1;                   // K3 ranges per K2 tile, one choice for the whole pass (launch_entropy)
 };
@@ -264,16 +270,10 @@ struct jpgenc_ctx {
     jpgenc::MixedPass mixed;              // on: the frames bound are images of individual sizes, described by d_geom
     jpgenc::FrameGeom* d_geom = nullptr;  // [nframes + 1]
     size_t geom_cap = 0;
-    const uint8_t* d_rgb = nullptr;       // bound or owned
+    jpgenc::PixelSource src;              // the single image bound (set whole by every bind; plane 0 is also a batch's first frame)
     uint8_t* d_rgb_owned = nullptr;
     size_t rgb_cap = 0;
     uint32_t real_w = 0, real_h = 0, maxval = 255, mcu_w = 0, mcu_h = 0;
-    int pixel_format = JPGENC_PIXEL_RGB;  // layout of the single image bound (set_geometry: tight RGB)
-    uint32_t row_pitch = 0;               // ... bytes from one row to the next
-    const uint8_t* d_plane_g = nullptr;   // ... planar RGB (kPixelPlanar): the G and B planes (d_rgb is the R plane)
-    const uint8_t* d_plane_b = nullptr;
-    uint32_t chroma_pitch = 0;            // ... YUV 4:2:0 (kPixelI420 / kPixelNV12): d_plane_g, d_plane_b are the U and V planes
-                                          // (NV12: d_plane_g is the UV plane), rows chroma_pitch bytes apart; d_rgb is the Y plane
     bool have_pixels = false, have_coef = false, have_scan = false, forward_pending = false, upload_pending = false;
 
     int16_t* d_coef = nullptr;

@@ -215,6 +215,81 @@ struct ForwardSmem {
     alignas(8) uint64_t bar;
 };
 
+// The image of a K1 strip and where the strip lies in it
+struct StripImage {
+    PixelSource src;                      // planes and pitches (the format is the kernel's template parameter)
+    uint32_t real_w, real_h, mcu_w;
+    uint32_t block0;                      // the image's first coefficient block
+    uint32_t my, mcu0;                    // the strip's MCU row and first MCU column
+};
+
+// A strip's position in the grid: the CTA's own (ThisCta; each coordinate is read where it is used, which keeps the scheduling
+// of the tight-RGB kernels) or another one (GridPos)
+struct ThisCta {
+    __device__ uint32_t x() const { return blockIdx.x; }
+    __device__ uint32_t y() const { return blockIdx.y; }
+    __device__ uint32_t z() const { return blockIdx.z; }
+};
+struct GridPos {
+    uint32_t x_, y_, z_;
+    __device__ uint32_t x() const { return x_; }
+    __device__ uint32_t y() const { return y_; }
+    __device__ uint32_t z() const { return z_; }
+};
+
+// The image of strip (x, y, z) of the one-size grid (strip of the row, MCU row of the launch, frame), or of strip x of the grid
+// over images of individual sizes: there the image is found by a search over the first-strip prefix, in which every lane of
+// the warp takes part.
+template <int kMcus, bool kMixed, int kFmt, class Pos>
+__device__ __forceinline__ StripImage strip_image(const ForwardParams& p, Pos at) {
+    StripImage s;
+    if constexpr (kMixed) {
+        const uint32_t gi = geom_find_warp(p.geom, p.nframes, at.x(), &FrameGeom::strip0);
+        const FrameGeom& g = p.geom[gi];
+        if constexpr (source_planes(kFmt) == 3) {
+            const ExtraPlanes& e = p.extra[gi];
+            s.src.plane[1] = e.plane[0];
+            s.src.plane[2] = e.plane[1];
+            s.src.pitch2 = static_cast<uint32_t>(e.pitch2);
+        }
+        s.mcu_w = g.mcu_w;
+        const uint32_t per_row = (s.mcu_w + kMcus - 1) / kMcus, k = at.x() - g.strip0;
+        s.my = k / per_row;
+        s.mcu0 = (k - s.my * per_row) * kMcus;
+        s.src.plane[0] = g.rgb;
+        s.block0 = g.block0;
+        s.real_w = g.real_w;
+        s.real_h = g.real_h;
+        s.src.pitch = g.pitch;
+    } else {
+        s.my = p.mcu_y0 + at.y();
+        s.mcu0 = at.x() * kMcus;
+        s.src = p.src;
+        s.src.plane[0] = p.frames ? p.frames[at.z()] : p.rgb;             // batch: grid.z walks over the frames
+        s.block0 = at.z() * p.blocks_per_frame;
+        s.real_w = p.real_w;
+        s.real_h = p.real_h;
+        s.mcu_w = p.mcu_w;
+    }
+    return s;
+}
+
+// The image of the strip `prefetch_ahead` CTAs after this one, for the L2 prefetch of the pixel-layout kernels; false past the
+// end of the grid (the one-size grid of these kernels holds one image).  Called by a whole warp.
+template <int kMcus, bool kMixed, int kFmt>
+__device__ __forceinline__ bool ahead_image(const ForwardParams& p, StripImage& s) {
+    if constexpr (kMixed) {
+        const uint32_t t = blockIdx.x + p.prefetch_ahead;
+        if (t >= p.strips) return false;                                    // uniform over the warp
+        s = strip_image<kMcus, true, kFmt>(p, GridPos{t, 0, 0});
+    } else {
+        const uint32_t lin = blockIdx.y * gridDim.x + blockIdx.x + p.prefetch_ahead, y = lin / gridDim.x;
+        if (y >= gridDim.y) return false;
+        s = strip_image<kMcus, false, kFmt>(p, GridPos{lin - y * gridDim.x, y, blockIdx.z});
+    }
+    return true;
+}
+
 // Staging of the pixel-layout kernels: the same 16-row tile of 3 bytes per pixel, in the byte order of the source (the colour
 // read below swaps R and B of BGR / BGRA at compile time).  Each CTA picks its path from its own image:
 //  * 3 bytes per pixel, base and pitch 16-byte aligned, real_w % 16 == 0: one bulk copy per row, as forward_kernel;
@@ -223,11 +298,12 @@ struct ForwardSmem {
 //    K1 its 5 CTAs per SM.  Chunks past the right edge, and every chunk of an unaligned image, take clamped byte loads;
 //  * otherwise a clamped byte loader with the pitch.
 template <int kMcus, int kFmt, bool kMixed>
-__device__ __forceinline__ void stage_layout(const ForwardParams& p, ForwardSmem<kMcus>& sm, int tid, const uint8_t* __restrict__ rgb,
-                                             uint32_t pitch, uint32_t real_w, uint32_t real_h, uint32_t my, uint32_t mcu0, int nm) {
+__device__ __forceinline__ void stage_layout(const ForwardParams& p, ForwardSmem<kMcus>& sm, int tid, const StripImage& s, int nm) {
     using Smem = ForwardSmem<kMcus>;
     constexpr int kThreads = kMcus * 4;
     constexpr uint32_t kBpp = pixel_bytes(kFmt);
+    const uint8_t* __restrict__ rgb = s.src.plane[0];
+    const uint32_t pitch = s.src.pitch, real_w = s.real_w, real_h = s.real_h, my = s.my, mcu0 = s.mcu0;
     const bool aligned = ((reinterpret_cast<uintptr_t>(rgb) | pitch) & 15) == 0;
     const bool bulk = kBpp == 3 && aligned && real_w % 16 == 0;           // the same for every thread of the CTA
     if (bulk) {
@@ -246,30 +322,11 @@ __device__ __forceinline__ void stage_layout(const ForwardParams& p, ForwardSmem
     // the strip `prefetch_ahead` CTAs later into L2, when its rows are whole 16-byte multiples inside the image (the range must
     // not pass the end of a row)
     if (p.prefetch_ahead && tid >= 32 && tid < 64) {
-        const uint8_t* prgb = nullptr;
-        uint32_t ppitch = 0, pw = 0, ph = 0, pm0 = 0, pnm = 0, pby = 0;
-        if constexpr (kMixed) {
-            const uint32_t t = blockIdx.x + p.prefetch_ahead;
-            if (t < p.strips) {                                             // uniform over the warp (geom_find_warp needs all lanes)
-                const FrameGeom& g = p.geom[geom_find_warp(p.geom, p.nframes, t, &FrameGeom::strip0)];
-                const uint32_t per_row = (g.mcu_w + kMcus - 1) / kMcus, s = t - g.strip0;
-                pby = s / per_row;
-                pm0 = (s - pby * per_row) * kMcus;
-                pnm = min(static_cast<uint32_t>(kMcus), g.mcu_w - pm0);
-                prgb = g.rgb; ppitch = g.pitch; pw = g.real_w; ph = g.real_h;
-            }
-        } else {
-            const uint32_t lin = blockIdx.y * gridDim.x + blockIdx.x + p.prefetch_ahead, y = lin / gridDim.x;
-            if (y < gridDim.y) {
-                pby = p.mcu_y0 + y;
-                pm0 = (lin - y * gridDim.x) * kMcus;
-                pnm = min(static_cast<uint32_t>(kMcus), p.mcu_w - pm0);
-                prgb = p.rgb; ppitch = pitch; pw = real_w; ph = real_h;
-            }
-        }
-        if (prgb && tid < 48 && ((reinterpret_cast<uintptr_t>(prgb) | ppitch | pw) & 15) == 0) {
-            const uint32_t sy = min(pby * 16 + (tid - 32), ph - 1);
-            ptx::bulk_prefetch_l2(prgb + static_cast<size_t>(sy) * ppitch + pm0 * 16 * kBpp, pnm * 16 * kBpp);
+        StripImage a;
+        if (ahead_image<kMcus, kMixed, kFmt>(p, a) && tid < 48 && ((reinterpret_cast<uintptr_t>(a.src.plane[0]) | a.src.pitch | a.real_w) & 15) == 0) {
+            const uint32_t pnm = min(static_cast<uint32_t>(kMcus), a.mcu_w - a.mcu0);
+            const uint32_t sy = min(a.my * 16 + (tid - 32), a.real_h - 1);
+            ptx::bulk_prefetch_l2(a.src.plane[0] + static_cast<size_t>(sy) * a.src.pitch + a.mcu0 * 16 * kBpp, pnm * 16 * kBpp);
         }
     }
     if (bulk) {
@@ -312,20 +369,21 @@ __device__ __forceinline__ void stage_layout(const ForwardParams& p, ForwardSmem
     __syncthreads();
 }
 
-// Staging of grey (kPlanes 1) and planar RGB (kPlanes 3) pixels: the tile holds the strip in the source's own layout, kPlanes
+// Staging of grey (one plane) and planar RGB (three planes) pixels: the tile holds the strip in the source's own layout, kPlanes
 // planes of 16 rows of kMcus * 16 bytes (planar: 24 KB, the whole tile), and the colour read in forward_body takes the three
 // channels from the planes (grey: one byte for all three).  Interleaving the planes here instead would cost what the 4-byte
 // formats' byte permutes cost above.  Each CTA picks its path from its own image:
 //  * every plane's base and the pitch 16-byte aligned, real_w % 16 == 0: one bulk copy per plane row (16 / 48 per CTA);
 //  * otherwise 16-byte chunks: a vector load where the chunk lies inside an aligned image, clamped byte loads elsewhere.
 // The L2 prefetch of the strip `prefetch_ahead` CTAs later covers every plane.
-template <int kMcus, int kPlanes, bool kMixed>
-__device__ __forceinline__ void stage_planes(const ForwardParams& p, ForwardSmem<kMcus>& sm, int tid, const uint8_t* const (&plane)[3],
-                                             uint32_t pitch, uint32_t real_w, uint32_t real_h, uint32_t my, uint32_t mcu0, int nm) {
+template <int kMcus, int kFmt, bool kMixed>
+__device__ __forceinline__ void stage_planes(const ForwardParams& p, ForwardSmem<kMcus>& sm, int tid, const StripImage& s, int nm) {
     using Smem = ForwardSmem<kMcus>;
-    constexpr int kThreads = kMcus * 4, kRow = kMcus * 16;
+    constexpr int kThreads = kMcus * 4, kRow = kMcus * 16, kPlanes = source_planes(kFmt);
     static_assert(kPlanes * 16 * kRow <= Smem::kTileBytes, "the planes fit the tile");
-    auto pick = [](const uint8_t* const (&pl)[3], int k) { return kPlanes == 1 || k == 0 ? pl[0] : k == 1 ? pl[1] : pl[2]; };
+    const auto& plane = s.src.plane;
+    const uint32_t pitch = s.src.pitch, real_w = s.real_w, real_h = s.real_h, my = s.my, mcu0 = s.mcu0;
+    auto pick = [](const auto& pl, int k) { return kPlanes == 1 || k == 0 ? pl[0] : k == 1 ? pl[1] : pl[2]; };
     uintptr_t bits = pitch;
 #pragma unroll
     for (int k = 0; k < kPlanes; ++k) bits |= reinterpret_cast<uintptr_t>(plane[k]);
@@ -345,38 +403,17 @@ __device__ __forceinline__ void stage_planes(const ForwardParams& p, ForwardSmem
         }
     }
     if (p.prefetch_ahead && tid >= 32 && tid < 64) {
-        const uint8_t* pp[3] = {nullptr, nullptr, nullptr};
-        uint32_t ppitch = 0, pw = 0, ph = 0, pm0 = 0, pnm = 0, pby = 0;
-        if constexpr (kMixed) {
-            const uint32_t t = blockIdx.x + p.prefetch_ahead;
-            if (t < p.strips) {                                             // uniform over the warp (geom_find_warp needs all lanes)
-                const uint32_t gi = geom_find_warp(p.geom, p.nframes, t, &FrameGeom::strip0);
-                const FrameGeom& g = p.geom[gi];
-                const uint32_t per_row = (g.mcu_w + kMcus - 1) / kMcus, s = t - g.strip0;
-                pby = s / per_row;
-                pm0 = (s - pby * per_row) * kMcus;
-                pnm = min(static_cast<uint32_t>(kMcus), g.mcu_w - pm0);
-                pp[0] = g.rgb; ppitch = g.pitch; pw = g.real_w; ph = g.real_h;
-                if (kPlanes == 3) { pp[1] = p.planes[2 * gi]; pp[2] = p.planes[2 * gi + 1]; }
-            }
-        } else {
-            const uint32_t lin = blockIdx.y * gridDim.x + blockIdx.x + p.prefetch_ahead, y = lin / gridDim.x;
-            if (y < gridDim.y) {
-                pby = p.mcu_y0 + y;
-                pm0 = (lin - y * gridDim.x) * kMcus;
-                pnm = min(static_cast<uint32_t>(kMcus), p.mcu_w - pm0);
-                pp[0] = p.rgb; ppitch = pitch; pw = real_w; ph = real_h;
-                if (kPlanes == 3) { pp[1] = p.plane_g; pp[2] = p.plane_b; }
-            }
-        }
-        if (pp[0])
+        StripImage a;
+        if (ahead_image<kMcus, kMixed, kFmt>(p, a)) {
+            const uint32_t pnm = min(static_cast<uint32_t>(kMcus), a.mcu_w - a.mcu0);
             for (int i = tid - 32; i < 16 * kPlanes; i += 32) {
-                const uint8_t* src = pick(pp, i >> 4);
-                if (((reinterpret_cast<uintptr_t>(src) | ppitch | pw) & 15) == 0) {
-                    const uint32_t sy = min(pby * 16 + (i & 15), ph - 1);
-                    ptx::bulk_prefetch_l2(src + static_cast<size_t>(sy) * ppitch + pm0 * 16, pnm * 16);
+                const uint8_t* src = pick(a.src.plane, i >> 4);
+                if (((reinterpret_cast<uintptr_t>(src) | a.src.pitch | a.real_w) & 15) == 0) {
+                    const uint32_t sy = min(a.my * 16 + (i & 15), a.real_h - 1);
+                    ptx::bulk_prefetch_l2(src + static_cast<size_t>(sy) * a.src.pitch + a.mcu0 * 16, pnm * 16);
                 }
             }
+        }
     }
     if (bulk) {
         ptx::mbar_wait(&sm.bar, 0);
@@ -413,13 +450,14 @@ __device__ __forceinline__ void stage_planes(const ForwardParams& p, ForwardSmem
 //  * otherwise 16-byte chunks, per plane: a vector load where the chunk lies inside the plane's row and the plane is aligned,
 //    clamped byte loads elsewhere (edge replication, each plane clamped to its own size; NV12 clamps whole U, V pairs).
 // The L2 prefetch of the strip `prefetch_ahead` CTAs later covers every plane.
-template <int kMcus, bool kNV12, bool kMixed>
-__device__ __forceinline__ void stage_yuv(const ForwardParams& p, ForwardSmem<kMcus>& sm, int tid, const uint8_t* y, const uint8_t* u,
-                                          const uint8_t* v, uint32_t y_pitch, uint32_t c_pitch, uint32_t real_w, uint32_t real_h,
-                                          uint32_t my, uint32_t mcu0, int nm) {
+template <int kMcus, int kFmt, bool kMixed>
+__device__ __forceinline__ void stage_yuv(const ForwardParams& p, ForwardSmem<kMcus>& sm, int tid, const StripImage& s, int nm) {
+    constexpr bool kNV12 = kFmt == kPixelNV12;
     constexpr int kThreads = kMcus * 4, kRow = kMcus * 16, kCRow = kNV12 ? kMcus * 16 : kMcus * 8, kCPlanes = kNV12 ? 1 : 2;
     constexpr int kMcuC = kNV12 ? 16 : 8;                                  // chroma bytes of one MCU in one row
     static_assert(16 * kRow + kCPlanes * 8 * kCRow <= ForwardSmem<kMcus>::kTileBytes, "the planes fit the tile");
+    const uint8_t *y = s.src.plane[0], *u = s.src.plane[1], *v = s.src.plane[2];
+    const uint32_t y_pitch = s.src.pitch, c_pitch = s.src.pitch2, real_w = s.real_w, real_h = s.real_h, my = s.my, mcu0 = s.mcu0;
     const uint32_t cw_bytes = ((real_w + 1) / 2) * (kNV12 ? 2 : 1), ch = (real_h + 1) / 2;
     const bool y_aligned = ((reinterpret_cast<uintptr_t>(y) | y_pitch) & 15) == 0;
     const bool c_aligned = ((reinterpret_cast<uintptr_t>(u) | (kNV12 ? 0 : reinterpret_cast<uintptr_t>(v)) | c_pitch) & 15) == 0;
@@ -444,40 +482,17 @@ __device__ __forceinline__ void stage_yuv(const ForwardParams& p, ForwardSmem<kM
         }
     }
     if (p.prefetch_ahead && tid >= 32 && tid < 64) {
-        const uint8_t *py = nullptr, *pu = nullptr, *pv = nullptr;
-        uint32_t pyp = 0, pcp = 0, pw = 0, ph = 0, pm0 = 0, pnm = 0, pby = 0;
-        if constexpr (kMixed) {
-            const uint32_t t = blockIdx.x + p.prefetch_ahead;
-            if (t < p.strips) {                                             // uniform over the warp (geom_find_warp needs all lanes)
-                const uint32_t gi = geom_find_warp(p.geom, p.nframes, t, &FrameGeom::strip0);
-                const FrameGeom& g = p.geom[gi];
-                const uint32_t per_row = (g.mcu_w + kMcus - 1) / kMcus, s = t - g.strip0;
-                pby = s / per_row;
-                pm0 = (s - pby * per_row) * kMcus;
-                pnm = min(static_cast<uint32_t>(kMcus), g.mcu_w - pm0);
-                py = g.rgb; pyp = g.pitch; pw = g.real_w; ph = g.real_h;
-                const ChromaPlanes& cp = p.yuv_chroma[gi];
-                pu = cp.u; pv = cp.v; pcp = static_cast<uint32_t>(cp.pitch);
-            }
-        } else {
-            const uint32_t lin = blockIdx.y * gridDim.x + blockIdx.x + p.prefetch_ahead, yy = lin / gridDim.x;
-            if (yy < gridDim.y) {
-                pby = p.mcu_y0 + yy;
-                pm0 = (lin - yy * gridDim.x) * kMcus;
-                pnm = min(static_cast<uint32_t>(kMcus), p.mcu_w - pm0);
-                py = p.rgb; pyp = y_pitch; pw = real_w; ph = real_h;
-                pu = p.plane_g; pv = p.plane_b; pcp = c_pitch;
-            }
-        }
+        StripImage a;
         // whole 16-byte units inside the rows only (the range must not pass the end of a row): real_w % 16 == 0 makes every
         // plane's strip end on its row's end
         const int i = tid - 32;
-        if (py && pw % 16 == 0 && i < 16 + 8 * kCPlanes) {
-            const uint8_t* src = i < 16 ? py : i < 24 ? pu : pv;
-            const uint32_t pitch = i < 16 ? pyp : pcp;
+        if (ahead_image<kMcus, kMixed, kFmt>(p, a) && a.real_w % 16 == 0 && i < 16 + 8 * kCPlanes) {
+            const uint8_t* src = a.src.plane[i < 16 ? 0 : i < 24 ? 1 : 2];
+            const uint32_t pitch = i < 16 ? a.src.pitch : a.src.pitch2;
             if (((reinterpret_cast<uintptr_t>(src) | pitch) & 15) == 0) {
-                const uint32_t sy = i < 16 ? min(pby * 16 + i, ph - 1) : min(pby * 8 + ((i - 16) & 7), (ph + 1) / 2 - 1);
-                const uint32_t x0 = i < 16 ? pm0 * 16 : pm0 * kMcuC, n = (i < 16 ? pnm * 16 : pnm * kMcuC) & ~15u;
+                const uint32_t pnm = min(static_cast<uint32_t>(kMcus), a.mcu_w - a.mcu0);
+                const uint32_t sy = i < 16 ? min(a.my * 16 + i, a.real_h - 1) : min(a.my * 8 + ((i - 16) & 7), (a.real_h + 1) / 2 - 1);
+                const uint32_t x0 = i < 16 ? a.mcu0 * 16 : a.mcu0 * kMcuC, n = (i < 16 ? pnm * 16 : pnm * kMcuC) & ~15u;
                 if (n) ptx::bulk_prefetch_l2(src + static_cast<size_t>(sy) * pitch + x0, n);
             }
         }
@@ -535,48 +550,18 @@ __device__ __forceinline__ void forward_body(const ForwardParams& p, ForwardSmem
     const int tid = thread;
     constexpr bool kPlanar = kFmt == kPixelPlanar, kPlaneTile = kPlanar || kFmt == JPGENC_PIXEL_GRAY;   // stage_planes
     constexpr bool kYuv = is_yuv(kFmt), kNV12 = kFmt == kPixelNV12;                                // stage_yuv
-    uint32_t my, mcu0, frame_block0, real_w, real_h, mcu_w, pitch, c_pitch = 0;
-    const uint8_t* __restrict__ rgb;
-    const uint8_t* plane_gb[2] = {nullptr, nullptr};                      // planar RGB: the G and B planes (rgb is R); YUV: U and V
-    if constexpr (kMixed) {
-        const uint32_t gi = geom_find_warp(p.geom, p.nframes, blockIdx.x, &FrameGeom::strip0);
-        const FrameGeom& g = p.geom[gi];
-        if constexpr (kPlanar) { plane_gb[0] = p.planes[2 * gi]; plane_gb[1] = p.planes[2 * gi + 1]; }
-        if constexpr (kYuv) {
-            const ChromaPlanes& cp = p.yuv_chroma[gi];
-            plane_gb[0] = cp.u; plane_gb[1] = cp.v; c_pitch = static_cast<uint32_t>(cp.pitch);
-        }
-        mcu_w = g.mcu_w;
-        const uint32_t per_row = (mcu_w + kMcus - 1) / kMcus, s = blockIdx.x - g.strip0;
-        my = s / per_row;
-        mcu0 = (s - my * per_row) * kMcus;
-        rgb = g.rgb;
-        frame_block0 = g.block0;
-        real_w = g.real_w;
-        real_h = g.real_h;
-        pitch = g.pitch;
-    } else {
-        my = p.mcu_y0 + blockIdx.y;
-        mcu0 = blockIdx.x * kMcus;
-        rgb = p.frames ? p.frames[blockIdx.z] : p.rgb;      // batch: grid.z walks over the frames
-        frame_block0 = blockIdx.z * p.blocks_per_frame;
-        real_w = p.real_w;
-        real_h = p.real_h;
-        mcu_w = p.mcu_w;
-        pitch = p.pitch;
-        if constexpr (kPlanar || kYuv) { plane_gb[0] = p.plane_g; plane_gb[1] = p.plane_b; }
-        if constexpr (kYuv) c_pitch = p.chroma_pitch;
-    }
+    const StripImage s = strip_image<kMcus, kMixed, kFmt>(p, ThisCta{});
+    const uint8_t* __restrict__ rgb = s.src.plane[0];
+    const uint32_t my = s.my, mcu0 = s.mcu0, frame_block0 = s.block0, real_w = s.real_w, real_h = s.real_h, mcu_w = s.mcu_w;
     const int nm = min(kMcus, static_cast<int>(mcu_w - mcu0));
 
     // ---- stage the 16-row RGB strip ----
     if constexpr (kYuv) {
-        stage_yuv<kMcus, kNV12, kMixed>(p, sm, tid, rgb, plane_gb[0], plane_gb[1], pitch, c_pitch, real_w, real_h, my, mcu0, nm);
+        stage_yuv<kMcus, kFmt, kMixed>(p, sm, tid, s, nm);
     } else if constexpr (kPlaneTile) {
-        const uint8_t* const plane[3] = {rgb, plane_gb[0], plane_gb[1]};
-        stage_planes<kMcus, kPlanar ? 3 : 1, kMixed>(p, sm, tid, plane, pitch, real_w, real_h, my, mcu0, nm);
+        stage_planes<kMcus, kFmt, kMixed>(p, sm, tid, s, nm);
     } else if constexpr (kFmt >= 0) {
-        stage_layout<kMcus, kFmt, kMixed>(p, sm, tid, rgb, pitch, real_w, real_h, my, mcu0, nm);
+        stage_layout<kMcus, kFmt, kMixed>(p, sm, tid, s, nm);
     } else if constexpr (kAligned) {
         if (tid == 0) {
             ptx::mbar_init(&sm.bar, 1);
@@ -635,7 +620,7 @@ __device__ __forceinline__ void forward_body(const ForwardParams& p, ForwardSmem
         if (active) {
             // The samples themselves, level-shifted: no colour conversion and no 2x2 means.  The chroma sample of an MCU position
             // is the stored one: the reference's S420_m averages four equal values there ((a + a) + (a + a), then / 4, gives
-            // exactly a), see exact_yuv_sample.  Every value is an integer in [-128, 127], exact in FP32.  The chroma goes first,
+            // exactly a), see exact_sample.  Every value is an integer in [-128, 127], exact in FP32.  The chroma goes first,
             // before the luma block fills its registers.
             constexpr int kRow = kMcus * 16;
             const uint8_t* ctile = sm.tile + 16 * kRow;
@@ -784,7 +769,7 @@ __global__ void __launch_bounds__(kMcus * 4, 640 / (kMcus * 4)) forward_mixed_ke
     forward_body<kMcus, kAligned, kBulkOut, true>(p, sm, threadIdx.x);
 }
 
-// pixels in another layout (JPGENC_PIXEL_* kFmt, row pitch): one image (p.rgb, p.pitch) / images of individual sizes
+// pixels in another layout (kFmt): one image (p.rgb, p.src) / images of individual sizes
 template <int kMcus, int kFmt, bool kBulkOut>
 __global__ void __launch_bounds__(kMcus * 4, 640 / (kMcus * 4)) forward_layout_kernel(const __grid_constant__ ForwardParams p) {
     __shared__ ForwardSmem<kMcus> sm;
@@ -812,21 +797,21 @@ __device__ __forceinline__ double exact_channel(int comp, double r, double g, do
     return dsub(dadd(128.0, dadd(dadd(dmul((double).5f, r), dmul((double)-.4186f, g)), dmul((double)-.0813f, b))), 128.0);
 }
 
-// kFmt: -1 tight RGB, otherwise the JPGENC_PIXEL_* format (or kPixelPlanar, with the planes rgb, g, b) of pixels whose rows are
-// `pitch` bytes apart.  A grey pixel v is the pixel (v, v, v).
+// kFmt: -1 tight RGB, otherwise the JPGENC_PIXEL_* format (or kPixelPlanar) of pixels whose rows are s.pitch bytes apart; `rgb` is
+// the first plane, s.plane[1] and s.plane[2] are the G and B planes of planar RGB.  A grey pixel v is the pixel (v, v, v).
 template <int kFmt>
-__device__ __forceinline__ double exact_pixel(const uint8_t* rgb, uint32_t pitch, uint32_t real_w, uint32_t real_h, uint32_t x, uint32_t y,
-                                              int comp, double scale, const uint8_t* g = nullptr, const uint8_t* b = nullptr) {
+__device__ __forceinline__ double exact_pixel(const uint8_t* rgb, const PixelSource& s, uint32_t real_w, uint32_t real_h, uint32_t x, uint32_t y,
+                                              int comp, double scale) {
     const uint32_t sx = min(x, real_w - 1), sy = min(y, real_h - 1);            // src/Image.cpp:491-530
     if constexpr (kFmt == JPGENC_PIXEL_GRAY || kFmt == kPixelPlanar) {
-        const size_t at = static_cast<size_t>(sy) * pitch + sx;
+        const size_t at = static_cast<size_t>(sy) * s.pitch + sx;
         const double r = dmul(static_cast<double>(rgb[at]), scale);
         if constexpr (kFmt == JPGENC_PIXEL_GRAY) return exact_channel(comp, r, r, r);
-        else return exact_channel(comp, r, dmul(static_cast<double>(g[at]), scale), dmul(static_cast<double>(b[at]), scale));
+        else return exact_channel(comp, r, dmul(static_cast<double>(s.plane[1][at]), scale), dmul(static_cast<double>(s.plane[2][at]), scale));
     }
     const uint8_t* px;
     if constexpr (kFmt < 0) px = rgb + (static_cast<size_t>(sy) * real_w + sx) * 3;
-    else px = rgb + static_cast<size_t>(sy) * pitch + sx * pixel_bytes(kFmt);
+    else px = rgb + static_cast<size_t>(sy) * s.pitch + sx * pixel_bytes(kFmt);
     constexpr int kR = (kFmt == JPGENC_PIXEL_BGR || kFmt == JPGENC_PIXEL_BGRA) ? 2 : 0, kB = 2 - kR;
     return exact_channel(comp, dmul(static_cast<double>(px[kR]), scale), dmul(static_cast<double>(px[1]), scale),
                          dmul(static_cast<double>(px[kB]), scale));
@@ -844,18 +829,35 @@ __device__ __forceinline__ ExactColumn exact_locate(const uint8_t* rgb, uint32_t
     if (k < 4) return ExactColumn{rgb, mx * 16 + (k & 1) * 8 + c, my * 16 + (k >> 1) * 8, 0};
     return ExactColumn{rgb, mx * 16 + 2 * c, my * 16, static_cast<int>(k) - 3};
 }
-// spatial sample of row r in the reference's arithmetic
-// (planar RGB: pg, pb are the G and B planes beside b.rgb)
-template <int kFmt = -1>
-__device__ __forceinline__ double exact_sample(const ExactColumn& b, uint32_t real_w, uint32_t real_h, int r, double scale, uint32_t pitch = 0,
-                                               const uint8_t* pg = nullptr, const uint8_t* pb = nullptr) {
-    if (b.comp == 0) return exact_pixel<kFmt>(b.rgb, pitch, real_w, real_h, b.x, b.y + r, 0, scale, pg, pb);
-    const uint32_t x = b.x, y = b.y + 2 * r;                                    // S420_m, src/Image.cpp:207-226
-    const double top = dadd(dadd(0.0, exact_pixel<kFmt>(b.rgb, pitch, real_w, real_h, x, y, b.comp, scale, pg, pb)),
-                            exact_pixel<kFmt>(b.rgb, pitch, real_w, real_h, x + 1, y, b.comp, scale, pg, pb));
-    const double bot = dadd(dadd(0.0, exact_pixel<kFmt>(b.rgb, pitch, real_w, real_h, x, y + 1, b.comp, scale, pg, pb)),
-                            exact_pixel<kFmt>(b.rgb, pitch, real_w, real_h, x + 1, y + 1, b.comp, scale, pg, pb));
-    return dmul(dadd(top, bot), 0.25);          // the reference divides by 4: the same double, bit for bit, without a division
+// Spatial sample of row r in the reference's arithmetic, of the image whose first plane is b.rgb and whose other planes and
+// pitches are those of `s`.
+// YUV 4:2:0: what Image::writeJPEG computes for the image whose level-shifted Y, Cb, Cr planes are the clamped bytes minus 128
+// (the frame padded to whole MCUs by edge replication, every chroma sample repeated over its 2x2 pixels; jpgenc_encode_planes(...,
+// ycbcr = 1)), bit for bit: such an image skips the colour conversion (src/Image.cpp:112-115); a luma sample is (double)byte -
+// 128, exact; S420_m (src/Image.cpp:207-226) sums the four pixels of a cell as (0 + a + a) + (0 + a + a) -- a cell's four
+// clamped pixels map to one chroma sample a (x, x + 1 with x even, or both clamped to the last column; the same for rows) -- and
+// quarters the sum: every step is exact on these small integers and gives a again.  So the chroma sample of cell (x / 2, y / 2)
+// is U[min(y / 2, ch - 1)][min(x / 2, cw - 1)] - 128 (V for Cr; NV12: the pair's first / second byte).
+template <int kFmt>
+__device__ __forceinline__ double exact_sample(const ExactColumn& b, const PixelSource& s, uint32_t real_w, uint32_t real_h, int r, double scale) {
+    if constexpr (is_yuv(kFmt)) {
+        if (b.comp == 0) {
+            const uint32_t sx = min(b.x, real_w - 1), sy = min(b.y + r, real_h - 1);
+            return dsub(static_cast<double>(b.rgb[static_cast<size_t>(sy) * s.pitch + sx]), 128.0);
+        }
+        const uint32_t cx = min(b.x / 2, (real_w + 1) / 2 - 1), cy = min(b.y / 2 + r, (real_h + 1) / 2 - 1);
+        const size_t row = static_cast<size_t>(cy) * s.pitch2;
+        const uint8_t v = kFmt == kPixelNV12 ? s.plane[1][row + 2 * cx + (b.comp - 1)] : (b.comp == 1 ? s.plane[1] : s.plane[2])[row + cx];
+        return dsub(static_cast<double>(v), 128.0);
+    } else {
+        if (b.comp == 0) return exact_pixel<kFmt>(b.rgb, s, real_w, real_h, b.x, b.y + r, 0, scale);
+        const uint32_t x = b.x, y = b.y + 2 * r;                                // S420_m, src/Image.cpp:207-226
+        const double top = dadd(dadd(0.0, exact_pixel<kFmt>(b.rgb, s, real_w, real_h, x, y, b.comp, scale)),
+                                exact_pixel<kFmt>(b.rgb, s, real_w, real_h, x + 1, y, b.comp, scale));
+        const double bot = dadd(dadd(0.0, exact_pixel<kFmt>(b.rgb, s, real_w, real_h, x, y + 1, b.comp, scale)),
+                                exact_pixel<kFmt>(b.rgb, s, real_w, real_h, x + 1, y + 1, b.comp, scale));
+        return dmul(dadd(top, bot), 0.25);      // the reference divides by 4: the same double, bit for bit, without a division
+    }
 }
 
 // Exact 8x8 transform, 8 threads per block (4 blocks per warp), everything in registers: thread c fetches column c
@@ -951,35 +953,38 @@ __device__ __forceinline__ void refine_loop64(uint32_t n0, uint32_t n, const uin
     }
 }
 
-// ids are global block indices; with `frames` (a batch) block id belongs to frame id / blocks_per_frame
-// kFmt >= 0: pixels in that JPGENC_PIXEL_* format, rows `pitch` bytes apart (-1: tight RGB, pitch unused)
-template <bool k64, int kFmt = -1>
+// ids are global block indices; with `frames` (a batch) block id belongs to frame id / blocks_per_frame, whose first plane is
+// frames[id / blocks_per_frame]; otherwise the image is `src`, whose first plane `rgb` also is (a parameter of its own: as a
+// restricted pointer its bytes take the read-only load path).  kFmt: -1 tight RGB, otherwise src.format.
+template <bool k64, int kFmt>
 __global__ void __launch_bounds__(kRefineThreads) refine_kernel(const uint8_t* __restrict__ rgb, const uint8_t* const* __restrict__ frames,
                                                                     uint32_t blocks_per_frame, int16_t* __restrict__ coef,
                                                                     const uint32_t* __restrict__ list,
                                                                     const uint32_t* __restrict__ count, uint32_t cap, int all,
                                                                     uint32_t nblocks, uint32_t real_w, uint32_t real_h,
-                                                                    uint32_t mcu_w, const __grid_constant__ ExactConsts e, uint32_t pitch) {
+                                                                    uint32_t mcu_w, const __grid_constant__ ExactConsts e,
+                                                                    const __grid_constant__ PixelSource src) {
     // count[0] = entries in the list, count[3] = entries already refined (band-wise encodes refine after every band)
     const uint32_t n = all ? nblocks : min(count[0], cap), n0 = all ? 0u : count[3];
     auto locate = [&](uint32_t id, int c) {
         const uint32_t f = frames ? id / blocks_per_frame : 0u;
         return exact_locate(frames ? frames[f] : rgb, mcu_w, id - f * blocks_per_frame, c);
     };
-    auto sample = [&](const ExactColumn& col, int r) { return exact_sample<kFmt>(col, real_w, real_h, r, e.scale, pitch); };
+    auto sample = [&](const ExactColumn& col, int r) { return exact_sample<kFmt>(col, src, real_w, real_h, r, e.scale); };
     if constexpr (k64) refine_loop64(n0, n, list, all != 0, coef, blocks_per_frame, e.qy, e.qc, e, locate, sample);
     else refine_loop(n0, n, list, all != 0, coef, blocks_per_frame, e.qy, e.qc, e, locate, sample);
 }
 
 // images of individual sizes: block id -> image by a search over the first-block prefix (every image starts on an MCU, so
-// id % 6 still tells luma from chroma: blocks_per_frame = 2^32 - 1 leaves ids < 2^31 as they are)
-template <bool k64, int kFmt = -1>
+// id % 6 still tells luma from chroma: blocks_per_frame = 2^32 - 1 leaves ids < 2^31 as they are).  Formats of several planes:
+// image f's other planes at extra[f].
+template <bool k64, int kFmt>
 __global__ void __launch_bounds__(kRefineThreads) refine_mixed_kernel(const FrameGeom* __restrict__ geom, uint32_t nframes,
                                                                           int16_t* __restrict__ coef, const uint32_t* __restrict__ list,
                                                                           const uint32_t* __restrict__ count, uint32_t cap,
-                                                                          const __grid_constant__ ExactConsts e) {
+                                                                          const __grid_constant__ ExactConsts e, const ExtraPlanes* __restrict__ extra) {
     const uint32_t n = min(count[0], cap), n0 = count[3];
-    struct Column { ExactColumn col; uint32_t real_w, real_h, pitch; };
+    struct Column { ExactColumn col; uint32_t real_w, real_h; PixelSource src; };
     auto locate = [&](uint32_t id, int c) {
         uint32_t lo = 0, hi = nframes;
         while (hi - lo > 1) {
@@ -987,107 +992,16 @@ __global__ void __launch_bounds__(kRefineThreads) refine_mixed_kernel(const Fram
             if (geom[mid].block0 <= id) lo = mid; else hi = mid;
         }
         const FrameGeom& g = geom[lo];
-        return Column{exact_locate(g.rgb, g.mcu_w, id - g.block0, c), g.real_w, g.real_h, kFmt >= 0 ? g.pitch : 0u};
-    };
-    auto sample = [&](const Column& col, int r) { return exact_sample<kFmt>(col.col, col.real_w, col.real_h, r, e.scale, col.pitch); };
-    if constexpr (k64) refine_loop64(n0, n, list, false, coef, 0xFFFFFFFFu, e.qy, e.qc, e, locate, sample);
-    else refine_loop(n0, n, list, false, coef, 0xFFFFFFFFu, e.qy, e.qc, e, locate, sample);
-}
-
-// planar RGB, one image: the planes r, g, b with one row pitch (otherwise refine_kernel's single-image form)
-template <bool k64>
-__global__ void __launch_bounds__(kRefineThreads) refine_planar_kernel(const uint8_t* __restrict__ r, const uint8_t* __restrict__ g,
-                                                                           const uint8_t* __restrict__ b, int16_t* __restrict__ coef,
-                                                                           const uint32_t* __restrict__ list, const uint32_t* __restrict__ count,
-                                                                           uint32_t cap, int all, uint32_t nblocks, uint32_t real_w, uint32_t real_h,
-                                                                           uint32_t mcu_w, const __grid_constant__ ExactConsts e, uint32_t pitch) {
-    const uint32_t n = all ? nblocks : min(count[0], cap), n0 = all ? 0u : count[3];
-    auto locate = [&](uint32_t id, int c) { return exact_locate(r, mcu_w, id, c); };
-    auto sample = [&](const ExactColumn& col, int row) { return exact_sample<kPixelPlanar>(col, real_w, real_h, row, e.scale, pitch, g, b); };
-    if constexpr (k64) refine_loop64(n0, n, list, all != 0, coef, nblocks, e.qy, e.qc, e, locate, sample);
-    else refine_loop(n0, n, list, all != 0, coef, nblocks, e.qy, e.qc, e, locate, sample);
-}
-
-// planar RGB, images of individual sizes: image f's G and B planes at planes[2f], planes[2f + 1] (otherwise refine_mixed_kernel)
-template <bool k64>
-__global__ void __launch_bounds__(kRefineThreads) refine_mixed_planar_kernel(const FrameGeom* __restrict__ geom, const uint8_t* const* __restrict__ planes,
-                                                                                 uint32_t nframes, int16_t* __restrict__ coef,
-                                                                                 const uint32_t* __restrict__ list, const uint32_t* __restrict__ count,
-                                                                                 uint32_t cap, const __grid_constant__ ExactConsts e) {
-    const uint32_t n = min(count[0], cap), n0 = count[3];
-    struct Column { ExactColumn col; uint32_t real_w, real_h, pitch; const uint8_t *g, *b; };
-    auto locate = [&](uint32_t id, int c) {
-        uint32_t lo = 0, hi = nframes;
-        while (hi - lo > 1) {
-            const uint32_t mid = (lo + hi) >> 1;
-            if (geom[mid].block0 <= id) lo = mid; else hi = mid;
+        Column col{exact_locate(g.rgb, g.mcu_w, id - g.block0, c), g.real_w, g.real_h, {}};
+        if constexpr (kFmt >= 0) col.src.pitch = g.pitch;
+        if constexpr (source_planes(kFmt) == 3) {
+            col.src.plane[1] = extra[lo].plane[0];
+            col.src.plane[2] = extra[lo].plane[1];
+            col.src.pitch2 = static_cast<uint32_t>(extra[lo].pitch2);
         }
-        const FrameGeom& gm = geom[lo];
-        return Column{exact_locate(gm.rgb, gm.mcu_w, id - gm.block0, c), gm.real_w, gm.real_h, gm.pitch, planes[2 * lo], planes[2 * lo + 1]};
+        return col;
     };
-    auto sample = [&](const Column& col, int r) {
-        return exact_sample<kPixelPlanar>(col.col, col.real_w, col.real_h, r, e.scale, col.pitch, col.g, col.b);
-    };
-    if constexpr (k64) refine_loop64(n0, n, list, false, coef, 0xFFFFFFFFu, e.qy, e.qc, e, locate, sample);
-    else refine_loop(n0, n, list, false, coef, 0xFFFFFFFFu, e.qy, e.qc, e, locate, sample);
-}
-
-// YUV 4:2:0, sample of row r of a column: what Image::writeJPEG computes for the image whose level-shifted Y, Cb, Cr planes are
-// the clamped bytes minus 128 (the frame padded to whole MCUs by edge replication, every chroma sample repeated over its 2x2
-// pixels; jpgenc_encode_planes(..., ycbcr = 1)), bit for bit: such an image skips the colour conversion (src/Image.cpp:
-// 112-115); a luma sample is (double)byte - 128, exact; S420_m (src/Image.cpp:207-226) sums the four pixels of a cell as
-// (0 + a + a) + (0 + a + a) -- a cell's four clamped pixels map to one chroma sample a (x, x + 1 with x even, or both clamped to
-// the last column; the same for rows) -- and quarters the sum: every step is exact on these small integers and gives a again.
-// So the chroma sample of cell (x / 2, y / 2) is U[min(y / 2, ch - 1)][min(x / 2, cw - 1)] - 128 (V for Cr; NV12: the pair's
-// first / second byte).
-template <bool kNV12>
-__device__ __forceinline__ double exact_yuv_sample(const ExactColumn& b, const uint8_t* u, const uint8_t* v, uint32_t y_pitch, uint32_t c_pitch,
-                                                   uint32_t real_w, uint32_t real_h, int r) {
-    if (b.comp == 0) {
-        const uint32_t sx = min(b.x, real_w - 1), sy = min(b.y + r, real_h - 1);
-        return dsub(static_cast<double>(b.rgb[static_cast<size_t>(sy) * y_pitch + sx]), 128.0);
-    }
-    const uint32_t cx = min(b.x / 2, (real_w + 1) / 2 - 1), cy = min(b.y / 2 + r, (real_h + 1) / 2 - 1);
-    const size_t row = static_cast<size_t>(cy) * c_pitch;
-    const uint8_t s = kNV12 ? u[row + 2 * cx + (b.comp - 1)] : (b.comp == 1 ? u : v)[row + cx];
-    return dsub(static_cast<double>(s), 128.0);
-}
-
-// YUV 4:2:0, one image: Y plane y (rows y_pitch apart), chroma planes u, v (NV12: u is the UV plane) with rows c_pitch apart
-template <bool k64, bool kNV12>
-__global__ void __launch_bounds__(kRefineThreads) refine_yuv_kernel(const uint8_t* __restrict__ y, const uint8_t* __restrict__ u,
-                                                                        const uint8_t* __restrict__ v, int16_t* __restrict__ coef,
-                                                                        const uint32_t* __restrict__ list, const uint32_t* __restrict__ count,
-                                                                        uint32_t cap, int all, uint32_t nblocks, uint32_t real_w, uint32_t real_h,
-                                                                        uint32_t mcu_w, const __grid_constant__ ExactConsts e, uint32_t y_pitch,
-                                                                        uint32_t c_pitch) {
-    const uint32_t n = all ? nblocks : min(count[0], cap), n0 = all ? 0u : count[3];
-    auto locate = [&](uint32_t id, int c) { return exact_locate(y, mcu_w, id, c); };
-    auto sample = [&](const ExactColumn& col, int row) { return exact_yuv_sample<kNV12>(col, u, v, y_pitch, c_pitch, real_w, real_h, row); };
-    if constexpr (k64) refine_loop64(n0, n, list, all != 0, coef, nblocks, e.qy, e.qc, e, locate, sample);
-    else refine_loop(n0, n, list, all != 0, coef, nblocks, e.qy, e.qc, e, locate, sample);
-}
-
-// YUV 4:2:0, images of individual sizes: image f's chroma planes at chroma[f] (otherwise refine_mixed_kernel)
-template <bool k64, bool kNV12>
-__global__ void __launch_bounds__(kRefineThreads) refine_mixed_yuv_kernel(const FrameGeom* __restrict__ geom, const ChromaPlanes* __restrict__ chroma,
-                                                                              uint32_t nframes, int16_t* __restrict__ coef,
-                                                                              const uint32_t* __restrict__ list, const uint32_t* __restrict__ count,
-                                                                              uint32_t cap, const __grid_constant__ ExactConsts e) {
-    const uint32_t n = min(count[0], cap), n0 = count[3];
-    struct Column { ExactColumn col; uint32_t real_w, real_h, pitch; ChromaPlanes cp; };
-    auto locate = [&](uint32_t id, int c) {
-        uint32_t lo = 0, hi = nframes;
-        while (hi - lo > 1) {
-            const uint32_t mid = (lo + hi) >> 1;
-            if (geom[mid].block0 <= id) lo = mid; else hi = mid;
-        }
-        const FrameGeom& gm = geom[lo];
-        return Column{exact_locate(gm.rgb, gm.mcu_w, id - gm.block0, c), gm.real_w, gm.real_h, gm.pitch, chroma[lo]};
-    };
-    auto sample = [&](const Column& col, int r) {
-        return exact_yuv_sample<kNV12>(col.col, col.cp.u, col.cp.v, col.pitch, static_cast<uint32_t>(col.cp.pitch), col.real_w, col.real_h, r);
-    };
+    auto sample = [&](const Column& col, int r) { return exact_sample<kFmt>(col.col, col.src, col.real_w, col.real_h, r, e.scale); };
     if constexpr (k64) refine_loop64(n0, n, list, false, coef, 0xFFFFFFFFu, e.qy, e.qc, e, locate, sample);
     else refine_loop(n0, n, list, false, coef, 0xFFFFFFFFu, e.qy, e.qc, e, locate, sample);
 }
@@ -1330,7 +1244,8 @@ static bool make_block_map(void* base, uint64_t nblocks, uint32_t box_blocks, CU
 }
 // Everything K1 needs to know about the image(s) bound to the context
 static void fill_forward_params(const jpgenc_ctx* c, ForwardParams* p) {
-    p->rgb = c->d_rgb;
+    p->rgb = c->src.plane[0];
+    p->src = c->src;
     p->frames = c->nframes > 1 ? c->d_frame_ptrs : nullptr;
     p->blocks_per_frame = c->mcu_w * c->mcu_h * kBlocksPerMcu;
     p->coef = c->d_coef;
@@ -1349,17 +1264,18 @@ static void fill_forward_params(const jpgenc_ctx* c, ForwardParams* p) {
     // aan2d_bounds assumes, with no input error -- the stand-alone block kernel's case.  Their thresholds are tighter than the
     // RGB ones, so an RGB encode must never take them (nor a YUV encode the RGB ones, which would only flag more blocks): they
     // follow the layout of the image(s) bound, computed anew for every launch.
-    const int format = c->mixed.on ? c->mixed.format : c->pixel_format;
+    const int format = c->mixed.on ? c->mixed.format : c->src.format;
     const double colour_err = is_yuv(format) ? 0.0 : c->maxval == 255 ? kColourErr255 : kColourErrScaled;
     fill_quant_consts2(c->qy, c->dct_s, &p->luma, colour_err);
     fill_quant_consts2(c->qc, c->dct_s, &p->chroma, colour_err);
 }
 
-// calls f(std::integral_constant<int, format>) for a JPGENC_PIXEL_* format: the kernels of the other pixel layouts take the
-// format as a template parameter
+// calls f(std::integral_constant<int, format>) for an internal format, or -1 for tight RGB: the kernels take the format as a
+// template parameter
 template <class F>
 static void with_format(int format, F&& f) {
     switch (format) {
+        case -1: f(std::integral_constant<int, -1>{}); break;
         case JPGENC_PIXEL_RGB: f(std::integral_constant<int, JPGENC_PIXEL_RGB>{}); break;
         case JPGENC_PIXEL_BGR: f(std::integral_constant<int, JPGENC_PIXEL_BGR>{}); break;
         case JPGENC_PIXEL_RGBA: f(std::integral_constant<int, JPGENC_PIXEL_RGBA>{}); break;
@@ -1371,9 +1287,19 @@ static void with_format(int format, F&& f) {
     }
 }
 
-// the single image bound is not tight RGB: K1 and the refinement take the pixel-layout kernels
-static bool layout_image(const jpgenc_ctx* c) {
-    return c->pixel_format != JPGENC_PIXEL_RGB || c->row_pitch != c->real_w * 3;
+// the format the kernels of the single image bound take: its own, or -1 when it is tight RGB
+static int kernel_format(const jpgenc_ctx* c) {
+    return c->src.format != JPGENC_PIXEL_RGB || c->src.pitch != c->real_w * 3 ? c->src.format : -1;
+}
+
+// The refinement over `total` blocks: grid-stride over the list; a small image does not need (and should not wait for) 2368
+// mostly empty CTAs.  64 threads per block where the flagged blocks are few (latency: 3840x2160 15 -> 6 us), 8 per block where
+// they are many (throughput: at 16384^2 the 64-thread form's barriers cost 42 us against 28).  f(std::bool_constant<k64>, grid).
+template <class F>
+static void with_refine_grid(const jpgenc_ctx* c, uint64_t total, F&& f) {
+    const unsigned grid = static_cast<unsigned>(std::max<uint64_t>(c->sm_count, std::min<uint64_t>(c->sm_count * 16, total / 256 + 1)));
+    if (total < (3u << 19)) f(std::true_type{}, grid);
+    else f(std::false_type{}, grid);
 }
 
 // exact FP64 pass over the blocks K1 flagged (all == false) or over every block (all == true)
@@ -1381,50 +1307,15 @@ static int launch_refine(jpgenc_ctx* c, bool all) {
     ExactConsts e;
     fill_exact(c, c->qy, c->qc, 255. / c->maxval, &e);
     const uint32_t bpf = c->mcu_w * c->mcu_h * kBlocksPerMcu;
-    // grid-stride over the list; a small image does not need (and should not wait for) 2368 mostly empty CTAs
-    const uint64_t total = static_cast<uint64_t>(bpf) * c->nframes;
-    const unsigned grid = static_cast<unsigned>(std::max<uint64_t>(c->sm_count, std::min<uint64_t>(c->sm_count * 16, total / 256 + 1)));
-    // 64 threads per block where the flagged blocks are few (latency: 3840x2160 15 -> 6 us), 8 per block where they are many
-    // (throughput: at 16384^2 the 64-thread form's barriers cost 42 us against 28)
     const uint32_t cap = all ? 0u : static_cast<uint32_t>(c->refine_cap);
     const uint8_t* const* frames = c->nframes > 1 ? c->d_frame_ptrs : nullptr;
-    if (layout_image(c)) {
-        with_format(c->pixel_format, [&](auto fmt) {
-            constexpr int kFmt = decltype(fmt)::value;
-            if constexpr (kFmt == kPixelPlanar) {
-                if (total < (3u << 19))
-                    refine_planar_kernel<true><<<grid, kRefineThreads, 0, c->stream>>>(c->d_rgb, c->d_plane_g, c->d_plane_b, c->d_coef, c->d_refine_list,
-                                                                                      c->d_counters, cap, all ? 1 : 0, bpf, c->real_w, c->real_h, c->mcu_w, e,
-                                                                                      c->row_pitch);
-                else
-                    refine_planar_kernel<false><<<grid, kRefineThreads, 0, c->stream>>>(c->d_rgb, c->d_plane_g, c->d_plane_b, c->d_coef, c->d_refine_list,
-                                                                                       c->d_counters, cap, all ? 1 : 0, bpf, c->real_w, c->real_h, c->mcu_w, e,
-                                                                                       c->row_pitch);
-            } else if constexpr (is_yuv(kFmt)) {
-                constexpr bool kNV12 = kFmt == kPixelNV12;
-                if (total < (3u << 19))
-                    refine_yuv_kernel<true, kNV12><<<grid, kRefineThreads, 0, c->stream>>>(c->d_rgb, c->d_plane_g, c->d_plane_b, c->d_coef, c->d_refine_list,
-                                                                                          c->d_counters, cap, all ? 1 : 0, bpf, c->real_w, c->real_h, c->mcu_w,
-                                                                                          e, c->row_pitch, c->chroma_pitch);
-                else
-                    refine_yuv_kernel<false, kNV12><<<grid, kRefineThreads, 0, c->stream>>>(c->d_rgb, c->d_plane_g, c->d_plane_b, c->d_coef, c->d_refine_list,
-                                                                                           c->d_counters, cap, all ? 1 : 0, bpf, c->real_w, c->real_h, c->mcu_w,
-                                                                                           e, c->row_pitch, c->chroma_pitch);
-            } else if (total < (3u << 19))
-                refine_kernel<true, kFmt><<<grid, kRefineThreads, 0, c->stream>>>(c->d_rgb, frames, bpf, c->d_coef, c->d_refine_list, c->d_counters, cap,
-                                                                                  all ? 1 : 0, bpf * c->nframes, c->real_w, c->real_h, c->mcu_w, e, c->row_pitch);
-            else
-                refine_kernel<false, kFmt><<<grid, kRefineThreads, 0, c->stream>>>(c->d_rgb, frames, bpf, c->d_coef, c->d_refine_list, c->d_counters, cap,
-                                                                                   all ? 1 : 0, bpf * c->nframes, c->real_w, c->real_h, c->mcu_w, e, c->row_pitch);
+    with_format(kernel_format(c), [&](auto fmt) {
+        with_refine_grid(c, static_cast<uint64_t>(bpf) * c->nframes, [&](auto k64, unsigned grid) {
+            refine_kernel<decltype(k64)::value, decltype(fmt)::value><<<grid, kRefineThreads, 0, c->stream>>>(
+                c->src.plane[0], frames, bpf, c->d_coef, c->d_refine_list, c->d_counters, cap, all ? 1 : 0, bpf * c->nframes, c->real_w, c->real_h, c->mcu_w, e,
+                c->src);
         });
-    } else if (total < (3u << 19))
-        refine_kernel<true><<<grid, kRefineThreads, 0, c->stream>>>(
-            c->d_rgb, frames, bpf, c->d_coef, c->d_refine_list, c->d_counters,
-            cap, all ? 1 : 0, bpf * c->nframes, c->real_w, c->real_h, c->mcu_w, e, 0u);
-    else
-        refine_kernel<false><<<grid, kRefineThreads, 0, c->stream>>>(
-            c->d_rgb, frames, bpf, c->d_coef, c->d_refine_list, c->d_counters,
-            cap, all ? 1 : 0, bpf * c->nframes, c->real_w, c->real_h, c->mcu_w, e, 0u);
+    });
     JPGENC_CUDA(c, cudaGetLastError());
     c->launches += 1;
     return JPGENC_OK;
@@ -1441,22 +1332,20 @@ int launch_forward_rows(jpgenc_ctx* c, uint32_t y0, uint32_t rows, bool first, b
     p.prefetch_ahead = 256;
     if (first && !launch_encode_clear(c))                                                          // counters + K2's / K3a's accumulators in one kernel
         JPGENC_CUDA(c, cudaMemsetAsync(c->d_counters, 0, 4 * sizeof(uint32_t), c->stream));          // (no statistics buffers yet) list length .. refined so far
-    bool aligned = (c->real_w % 16 == 0) && (reinterpret_cast<uintptr_t>(c->d_rgb) % 16 == 0);
+    bool aligned = (c->real_w % 16 == 0) && (reinterpret_cast<uintptr_t>(c->src.plane[0]) % 16 == 0);
     if (c->nframes > 1) aligned = (c->real_w % 16 == 0) && c->frames_aligned;
     // (strips of 24 and of 40 MCUs, which divide 1920- and 3840-pixel rows evenly, were measured: no gain on those frames
     // -- the partial fourth strip is not what costs -- and 24 is 7 % slower where 32 divides the row)
     const dim3 grid((c->mcu_w + 31) / 32, rows, c->nframes);
-    if (layout_image(c)) {
+    if (kernel_format(c) >= 0) {
         // each CTA picks its staging path from the image (stage_layout); the tensor store serves every full strip
-        p.pitch = c->row_pitch;
-        p.plane_g = c->d_plane_g;
-        p.plane_b = c->d_plane_b;
-        p.chroma_pitch = c->chroma_pitch;
         const bool bulk = make_block_map(c->d_coef, static_cast<uint64_t>(c->mcu_w) * c->mcu_h * kBlocksPerMcu, 32 * kBlocksPerMcu, &p.coef_map);
-        with_format(c->pixel_format, [&](auto fmt) {
+        with_format(c->src.format, [&](auto fmt) {
             constexpr int kFmt = decltype(fmt)::value;
-            if (bulk) forward_layout_kernel<32, kFmt, true><<<grid, 128, 0, c->stream>>>(p);
-            else forward_layout_kernel<32, kFmt, false><<<grid, 128, 0, c->stream>>>(p);
+            if constexpr (kFmt >= 0) {
+                if (bulk) forward_layout_kernel<32, kFmt, true><<<grid, 128, 0, c->stream>>>(p);
+                else forward_layout_kernel<32, kFmt, false><<<grid, 128, 0, c->stream>>>(p);
+            }
         });
         JPGENC_CUDA(c, cudaGetLastError());
         c->launches += 1;
@@ -1486,18 +1375,16 @@ int launch_forward_mixed(jpgenc_ctx* c) {
     c->stats_clear_valid = false;                                 // K2 clears the statistics and K3a's sums itself
     const bool layout = c->mixed.format >= 0;
     const bool aligned = c->mixed.aligned;
-    // planar RGB: the G and B plane pointers lie behind the geometry (enqueue_pass copies them in the same transfer)
-    const uint8_t* const* planes = c->mixed.format == kPixelPlanar ? reinterpret_cast<const uint8_t* const*>(c->d_geom + c->nframes + 1) : nullptr;
-    p.planes = planes;
-    // YUV 4:2:0: each image's chroma planes lie there instead (ChromaPlanes)
-    const ChromaPlanes* chroma = is_yuv(c->mixed.format) ? reinterpret_cast<const ChromaPlanes*>(c->d_geom + c->nframes + 1) : nullptr;
-    p.yuv_chroma = chroma;
+    // formats of several planes: each image's other planes lie behind the geometry (enqueue_pass copies them in the same transfer)
+    p.extra = source_planes(c->mixed.format) == 3 ? reinterpret_cast<const ExtraPlanes*>(c->d_geom + c->nframes + 1) : nullptr;
     const bool bulk_out = (aligned || layout) && make_block_map(c->d_coef, c->mixed.blocks, 32 * kBlocksPerMcu, &p.coef_map);
     if (layout) {
         with_format(c->mixed.format, [&](auto fmt) {
             constexpr int kFmt = decltype(fmt)::value;
-            if (bulk_out) forward_mixed_layout_kernel<32, kFmt, true><<<c->mixed.strips, 128, 0, c->stream>>>(p);
-            else forward_mixed_layout_kernel<32, kFmt, false><<<c->mixed.strips, 128, 0, c->stream>>>(p);
+            if constexpr (kFmt >= 0) {
+                if (bulk_out) forward_mixed_layout_kernel<32, kFmt, true><<<c->mixed.strips, 128, 0, c->stream>>>(p);
+                else forward_mixed_layout_kernel<32, kFmt, false><<<c->mixed.strips, 128, 0, c->stream>>>(p);
+            }
         });
     } else if (bulk_out) forward_mixed_kernel<32, true, true><<<c->mixed.strips, 128, 0, c->stream>>>(p);
     else if (aligned) forward_mixed_kernel<32, true, false><<<c->mixed.strips, 128, 0, c->stream>>>(p);
@@ -1505,36 +1392,13 @@ int launch_forward_mixed(jpgenc_ctx* c) {
     JPGENC_CUDA(c, cudaGetLastError());
     ExactConsts e;
     fill_exact(c, c->qy, c->qc, 255. / c->maxval, &e);
-    const uint64_t total = c->mixed.blocks;                       // the same grid and thread layout rules as launch_refine
-    const unsigned grid = static_cast<unsigned>(std::max<uint64_t>(c->sm_count, std::min<uint64_t>(c->sm_count * 16, total / 256 + 1)));
     const uint32_t cap = static_cast<uint32_t>(c->refine_cap);
-    if (layout) {
-        with_format(c->mixed.format, [&](auto fmt) {
-            constexpr int kFmt = decltype(fmt)::value;
-            if constexpr (kFmt == kPixelPlanar) {
-                if (total < (3u << 19))
-                    refine_mixed_planar_kernel<true><<<grid, kRefineThreads, 0, c->stream>>>(c->d_geom, planes, c->nframes, c->d_coef, c->d_refine_list,
-                                                                                            c->d_counters, cap, e);
-                else
-                    refine_mixed_planar_kernel<false><<<grid, kRefineThreads, 0, c->stream>>>(c->d_geom, planes, c->nframes, c->d_coef, c->d_refine_list,
-                                                                                             c->d_counters, cap, e);
-            } else if constexpr (is_yuv(kFmt)) {
-                constexpr bool kNV12 = kFmt == kPixelNV12;
-                if (total < (3u << 19))
-                    refine_mixed_yuv_kernel<true, kNV12><<<grid, kRefineThreads, 0, c->stream>>>(c->d_geom, chroma, c->nframes, c->d_coef, c->d_refine_list,
-                                                                                                c->d_counters, cap, e);
-                else
-                    refine_mixed_yuv_kernel<false, kNV12><<<grid, kRefineThreads, 0, c->stream>>>(c->d_geom, chroma, c->nframes, c->d_coef, c->d_refine_list,
-                                                                                                 c->d_counters, cap, e);
-            } else if (total < (3u << 19))
-                refine_mixed_kernel<true, kFmt><<<grid, kRefineThreads, 0, c->stream>>>(c->d_geom, c->nframes, c->d_coef, c->d_refine_list, c->d_counters, cap, e);
-            else
-                refine_mixed_kernel<false, kFmt><<<grid, kRefineThreads, 0, c->stream>>>(c->d_geom, c->nframes, c->d_coef, c->d_refine_list, c->d_counters, cap, e);
+    with_format(c->mixed.format, [&](auto fmt) {
+        with_refine_grid(c, c->mixed.blocks, [&](auto k64, unsigned grid) {
+            refine_mixed_kernel<decltype(k64)::value, decltype(fmt)::value><<<grid, kRefineThreads, 0, c->stream>>>(
+                c->d_geom, c->nframes, c->d_coef, c->d_refine_list, c->d_counters, cap, e, p.extra);
         });
-    } else if (total < (3u << 19))
-        refine_mixed_kernel<true><<<grid, kRefineThreads, 0, c->stream>>>(c->d_geom, c->nframes, c->d_coef, c->d_refine_list, c->d_counters, cap, e);
-    else
-        refine_mixed_kernel<false><<<grid, kRefineThreads, 0, c->stream>>>(c->d_geom, c->nframes, c->d_coef, c->d_refine_list, c->d_counters, cap, e);
+    });
     JPGENC_CUDA(c, cudaGetLastError());
     c->launches += 2;
     return JPGENC_OK;

@@ -23,10 +23,30 @@ int ensure(jpgenc_ctx* c, T** ptr, size_t* cap, size_t need_bytes, bool headroom
 }
 
 int set_geometry(jpgenc_ctx* c, uint32_t w, uint32_t h, uint32_t maxval);
-// a JPGENC_PIXEL_* format, sides 1..65535 and a row pitch (0 -> the row size, set in *row_pitch) that holds a row; JPGENC_ERR_ARG otherwise
-int check_layout(jpgenc_ctx* c, uint32_t w, uint32_t h, uint32_t* row_pitch, int format);
-int check_yuv420(jpgenc_ctx* c, const void* y, const void* u, const void* v, uint32_t w, uint32_t h, uint32_t* y_pitch, uint32_t* c_pitch,
-                 int layout, int* format);
+// A caller's image: a known format, its planes (NV12: v must be NULL), sides 1..65535 and pitches that hold a row (0 -> the row
+// size, filled in; planar RGB: pitch2 = pitch); JPGENC_ERR_ARG otherwise
+int check_source(jpgenc_ctx* c, PixelSource* s, uint32_t w, uint32_t h);
+// every colour sample of a host source is <= maxval (maxval 0 or 255: true): a 4th byte and the bytes between rows are not read;
+// planar RGB: all three planes; YUV frames have no maxval
+bool source_within_maxval(const PixelSource& s, uint32_t w, uint32_t h, uint32_t maxval);
+// the sources of the C entry points (a format code they do not take becomes -1, which check_source refuses)
+PixelSource image_source(const void* px, uint32_t pitch, int format);
+PixelSource planar_source(const void* r, const void* g, const void* b, uint32_t pitch);
+PixelSource yuv420_source(const void* y, const void* u, const void* v, uint32_t y_pitch, uint32_t c_pitch, int layout);
+
+// One plane of a checked host source as it is uploaded: `rows` host rows of `row` bytes, `pitch` bytes apart (vsub 1: the chroma
+// planes of YUV, half the image's rows rounded up), staged as tight rows at `dev_off` of the device copy; YUV planes start on
+// 256 bytes
+struct StagedPlane {
+    const uint8_t* host;
+    size_t pitch, row, rows, dev_off;
+    uint32_t vsub;
+};
+uint32_t staged_planes(const PixelSource& s, uint32_t w, uint32_t h, StagedPlane pl[3]);   // the number of planes
+size_t staged_bytes(const StagedPlane* pl, uint32_t np);
+// the three planes of planar RGB lie equally spaced in host memory with tight rows: their spacing (one strided copy moves them
+// all); 0 otherwise
+size_t planes_gap(const StagedPlane* pl, uint32_t np);
 int ensure_pinned(jpgenc_ctx* c, size_t bytes);                 // c->h_pinned, grown on demand
 int ensure_coef(jpgenc_ctx* c);                                  // coefficients + refinement list of the bound frames
 int ensure_stats_buffers(jpgenc_ctx* c);                         // K2's outputs for the bound frames (+ pinned staging)

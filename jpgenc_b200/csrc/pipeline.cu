@@ -40,15 +40,10 @@ struct Job {
     // null: every frame is w x h
     const uint32_t* widths = nullptr;
     const uint32_t* heights = nullptr;
-    // pixels in another layout (jpgenc_encode_images_packed_layout; needs widths): JPGENC_PIXEL_* format, -1 tight RGB, and the
-    // row pitch of every image as the caller holds it.  `staged`: host images, uploaded into tight rows of their format.
-    // kPixelPlanar (jpgenc_encode_images_packed_planar): three pointers per image, R, G, B; staged as three tight planes back to back.
-    // kPixelI420 / kPixelNV12 (jpgenc_encode_images_packed_yuv420): three pointers per image, Y, U, V (NV12: Y, UV, null), Y rows
-    // `pitches` apart, chroma rows `c_pitches` apart; staged as tight planes, each starting on 256 bytes.
+    // image i as the caller holds it (checked: pitches filled in), and the format the kernels take: -1 tight RGB, otherwise that
+    // of every image (needs widths)
+    std::vector<PixelSource> src;
     int format = -1;
-    const uint32_t* pitches = nullptr;
-    const uint32_t* c_pitches = nullptr;
-    bool staged = false;
     double raw_per_block = 0;              // ... raw-scan bytes reserved per block: 1.5 x the most this call has seen (0: nothing yet)
     // output: per-frame buffers (legacy), one packed buffer, or none (sizes only)
     uint8_t* const* out_ptrs = nullptr;
@@ -68,14 +63,6 @@ struct Pass {
 
 uint32_t job_w(const Job& job, uint32_t i) { return job.widths ? job.widths[i] : job.w; }
 uint32_t job_h(const Job& job, uint32_t i) { return job.heights ? job.heights[i] : job.h; }
-uint32_t job_bpp(const Job& job) { return job.format < 0 ? 3u : pixel_bytes(job.format); }
-// pointers (= planes) per image
-uint32_t job_planes(const Job& job) { return job.format == kPixelPlanar || is_yuv(job.format) ? 3u : 1u; }
-// bytes from one row of image i to the next where the kernels read it
-uint32_t job_pitch(const Job& job, uint32_t i) { return job.pitches && !job.staged ? job.pitches[i] : job_w(job, i) * job_bpp(job); }
-// YUV 4:2:0: bytes of one chroma row of image i (tight), and from one chroma row to the next where the kernels read it
-uint32_t job_crow(const Job& job, uint32_t i) { return (job_w(job, i) + 1) / 2 * (job.format == kPixelNV12 ? 2u : 1u); }
-uint32_t job_c_pitch(const Job& job, uint32_t i) { return job.staged ? job_crow(job, i) : job.c_pitches[i]; }
 uint64_t job_blocks(const Job& job, uint32_t i) {
     return static_cast<uint64_t>((job_w(job, i) + 15) / 16) * ((job_h(job, i) + 15) / 16) * kBlocksPerMcu;
 }
@@ -138,10 +125,9 @@ std::vector<Pass> image_passes(const Job& job, uint32_t slots) {
 }
 
 // The geometry of a pass of images of individual sizes (FrameGeom, F + 1 entries) and its totals.  K3's split follows
-// launch_entropy's rule, applied to the pass's tiles.  Planar RGB: ptrs holds R, G, B of every image; FrameGeom::rgb is the R
-// plane, gb[2f], gb[2f + 1] receive the G and B planes.  YUV 4:2:0: ptrs holds Y, U, V; FrameGeom::rgb is the Y plane, cp[f]
-// receives the chroma planes and pitch.
-MixedPass image_geometry(const Job& job, const Pass& ps, const void* const* ptrs, FrameGeom* g, const void** gb, ChromaPlanes* cp) {
+// launch_entropy's rule, applied to the pass's tiles.  FrameGeom holds each image's first plane and pitch; formats of several
+// planes put the others in extra[f].
+MixedPass image_geometry(const Job& job, const Pass& ps, const PixelSource* src, FrameGeom* g, ExtraPlanes* extra) {
     MixedPass m;
     m.on = true;
     m.aligned = true;
@@ -154,13 +140,10 @@ MixedPass image_geometry(const Job& job, const Pass& ps, const void* const* ptrs
         g[f].block0 = m.blocks; g[f].strip0 = m.strips; g[f].tile0 = m.tiles; g[f].group0 = m.groups; g[f].super0 = m.supers;
         if (f == ps.F) break;
         const uint32_t w = job_w(job, ps.f0 + f), h = job_h(job, ps.f0 + f);
-        const uint32_t np = job_planes(job);
-        g[f].rgb = static_cast<const uint8_t*>(ptrs[np * f]);
-        if (is_yuv(job.format))
-            cp[f] = ChromaPlanes{static_cast<const uint8_t*>(ptrs[3 * f + 1]), static_cast<const uint8_t*>(ptrs[3 * f + 2]), job_c_pitch(job, ps.f0 + f)};
-        else if (np == 3) { gb[2 * f] = ptrs[3 * f + 1]; gb[2 * f + 1] = ptrs[3 * f + 2]; }
+        g[f].rgb = src[f].plane[0];
+        if (source_planes(job.format) == 3) extra[f] = ExtraPlanes{{src[f].plane[1], src[f].plane[2]}, src[f].pitch2};
         g[f].real_w = w; g[f].real_h = h; g[f].mcu_w = (w + 15) / 16; g[f].mcu_h = (h + 15) / 16;
-        if (job.format >= 0) g[f].pitch = job_pitch(job, ps.f0 + f);
+        if (job.format >= 0) g[f].pitch = src[f].pitch;
         const uint32_t blocks = g[f].mcu_w * g[f].mcu_h * kBlocksPerMcu, tiles = (blocks + 383) / 384, groups = (tiles * m.split + 7) / 8;
         m.blocks += blocks;
         m.strips += (g[f].mcu_w + 31) / 32 * g[f].mcu_h;
@@ -220,9 +203,9 @@ int enqueue_entropy(jpgenc_ctx* l, Pass& ps, cudaEvent_t prev_k4 = nullptr) {
     return JPGENC_OK;
 }
 
-// the whole chain of one pass on slot `l`; `ready` (optional): event after which the pixels are valid
-// `after` (optional): the event after the previous pass's K1 (see run_passes)
-int enqueue_pass(jpgenc_ctx* root, jpgenc_ctx* l, const Job& job, Pass& ps, const void* const* dev_frames, cudaEvent_t ready, cudaEvent_t after,
+// the whole chain of one pass on slot `l` over the device images src[0 .. F); `ready` (optional): event after which the pixels are
+// valid; `after` (optional): the event after the previous pass's K1 (see run_passes)
+int enqueue_pass(jpgenc_ctx* root, jpgenc_ctx* l, const Job& job, Pass& ps, const PixelSource* src, cudaEvent_t ready, cudaEvent_t after,
                  cudaEvent_t prev_k4) {
     const uint32_t F = ps.F;
     int rc;
@@ -230,29 +213,26 @@ int enqueue_pass(jpgenc_ctx* root, jpgenc_ctx* l, const Job& job, Pass& ps, cons
     l->have_coef = l->have_scan = l->have_items = false; l->k2_tiles_done = 0;
     l->file_mode = true;
     bool aligned = true;
-    for (uint32_t f = 0; f < F; ++f) aligned = aligned && (reinterpret_cast<uintptr_t>(dev_frames[f]) % 16 == 0);
+    for (uint32_t f = 0; f < F; ++f) aligned = aligned && (reinterpret_cast<uintptr_t>(src[f].plane[0]) % 16 == 0);
     l->frames_aligned = aligned;
-    l->d_rgb = static_cast<const uint8_t*>(dev_frames[0]);
+    l->src.plane[0] = src[0].plane[0];
     l->have_pixels = true;
     std::vector<FrameGeom> geom;
-    std::vector<const void*> gb;
-    std::vector<ChromaPlanes> cp;
+    std::vector<ExtraPlanes> extra;
     if (job.widths) {
         geom.resize(F + 1);
-        gb.resize(job.format == kPixelPlanar ? 2 * F : 0);
-        cp.resize(is_yuv(job.format) ? F : 0);
-        l->mixed = image_geometry(job, ps, dev_frames, geom.data(), gb.data(), cp.data());
+        extra.resize(source_planes(job.format) == 3 ? F : 0);
+        l->mixed = image_geometry(job, ps, src, geom.data(), extra.data());
     }
     if ((rc = ensure_coef(l))) return rc;
     if ((rc = ensure_stats_buffers(l))) return rc;               // also sizes the pinned staging (stage_bytes(F))
     if (job.widths) {
-        // the geometry (with the frame pointers; planar RGB: and the G and B planes behind it; YUV: the chroma planes) travels
-        // through pinned memory like the pointer array below
-        const size_t gbytes = geom.size() * sizeof(FrameGeom), bytes = gbytes + gb.size() * sizeof(void*) + cp.size() * sizeof(ChromaPlanes);
+        // the geometry (with the frame pointers, and the extra planes behind it) travels through pinned memory like the pointer
+        // array below
+        const size_t gbytes = geom.size() * sizeof(FrameGeom), bytes = gbytes + extra.size() * sizeof(ExtraPlanes);
         if ((rc = ensure(l, &l->d_geom, &l->geom_cap, bytes))) return rc;
         std::memcpy(l->h_pinned, geom.data(), gbytes);
-        if (!gb.empty()) std::memcpy(static_cast<uint8_t*>(l->h_pinned) + gbytes, gb.data(), gb.size() * sizeof(void*));
-        if (!cp.empty()) std::memcpy(static_cast<uint8_t*>(l->h_pinned) + gbytes, cp.data(), cp.size() * sizeof(ChromaPlanes));
+        if (!extra.empty()) std::memcpy(static_cast<uint8_t*>(l->h_pinned) + gbytes, extra.data(), extra.size() * sizeof(ExtraPlanes));
         JPGENC_CUDA(l, cudaMemcpyAsync(l->d_geom, l->h_pinned, bytes, cudaMemcpyHostToDevice, l->stream));
     } else {
         size_t cap = l->frame_ptrs_cap;
@@ -262,7 +242,8 @@ int enqueue_pass(jpgenc_ctx* root, jpgenc_ctx* l, const Job& job, Pass& ps, cons
         l->frame_ptrs_cap = cap;
         // the pointer array travels through pinned memory (the statistics' staging area is unused in this path), so that the
         // copy is asynchronous and the caller's array need not outlive the call
-        std::memcpy(l->h_pinned, dev_frames, F * sizeof(void*));
+        const uint8_t** ptrs = static_cast<const uint8_t**>(l->h_pinned);
+        for (uint32_t f = 0; f < F; ++f) ptrs[f] = src[f].plane[0];
         JPGENC_CUDA(l, cudaMemcpyAsync(l->d_frame_ptrs, l->h_pinned, F * sizeof(void*), cudaMemcpyHostToDevice, l->stream));
     }
     if (ready) JPGENC_CUDA(l, cudaStreamWaitEvent(l->stream, ready, 0));
@@ -364,8 +345,8 @@ int finish_pass(jpgenc_ctx* root, jpgenc_ctx* l, Pass& ps, Job& job) {
     }
 }
 
-// Runs the passes over the slots.  frames_of(p, slot context) -> device pointers of pass p's frames and the event after
-// which they are valid; done_with(p) is called when pass p's pixels are no longer needed.
+// Runs the passes over the slots.  frames_of(p, slot context) -> device sources of pass p's images and the event after which
+// they are valid; done_with(p) is called when pass p's pixels are no longer needed.
 template <class FramesOf, class DoneWith>
 int run_passes(jpgenc_ctx* c, Job& job, std::vector<Pass>& pass, uint32_t nslots, FramesOf&& frames_of, DoneWith&& done_with) {
     const uint32_t npasses = static_cast<uint32_t>(pass.size());
@@ -406,7 +387,7 @@ int run_passes(jpgenc_ctx* c, Job& job, std::vector<Pass>& pass, uint32_t nslots
         }
         if (p < npasses) {
             jpgenc_ctx* l = slot[p % nslots];
-            const void* const* ptrs = nullptr;
+            const PixelSource* ptrs = nullptr;
             cudaEvent_t ready = nullptr;
             rc = frames_of(p, l, &ptrs, &ready);
             // Staggering: the wide kernels of pass p start when pass p - 1's K1 is through.  Left alone, the streams run the
@@ -456,7 +437,7 @@ int check_job(jpgenc_ctx* c, const Job& job, const void* frames) {
     return JPGENC_OK;
 }
 
-int encode_device_frames(jpgenc_ctx* c, Job& job, const void* const* dev_frames) {
+int encode_device_frames(jpgenc_ctx* c, Job& job) {
     // an empty batch is legal and touches nothing: an image bound to the context keeps its geometry
     if (job.n == 0) return (job.w && job.h && job.maxval && job.maxval <= 255) ? JPGENC_OK : fail(c, JPGENC_ERR_ARG, "width/height/maxval out of range");
     JPGENC_CUDA(c, cudaSetDevice(c->device));
@@ -468,8 +449,8 @@ int encode_device_frames(jpgenc_ctx* c, Job& job, const void* const* dev_frames)
     std::vector<Pass> pass = plan_passes(c, job);
     const uint32_t nslots = slots_for(pass.size());
     return run_passes(c, job, pass, nslots,
-                      [&](uint32_t p, jpgenc_ctx*, const void* const** ptrs, cudaEvent_t* ready) {
-                          *ptrs = dev_frames + static_cast<size_t>(pass[p].f0) * job_planes(job);
+                      [&](uint32_t p, jpgenc_ctx*, const PixelSource** src, cudaEvent_t* ready) {
+                          *src = job.src.data() + pass[p].f0;
                           *ready = nullptr;
                           return JPGENC_OK;
                       },
@@ -480,7 +461,7 @@ int encode_device_frames(jpgenc_ctx* c, Job& job, const void* const* dev_frames)
 // of device memory, always a few passes ahead of the kernels; when pass p is finished its slice is re-filled with the
 // frames of pass p + ring.  A slice holds the bytes of the largest pass (passes of images of individual sizes differ);
 // every frame starts on 256 bytes.  Pixels in another layout travel in their own format, the pitch gap dropped by the copy.
-int encode_host_frames(jpgenc_ctx* c, Job& job, const uint8_t* const* frames) {
+int encode_host_frames(jpgenc_ctx* c, Job& job) {
     // an empty batch is legal and touches nothing: an image bound to the context keeps its geometry
     if (job.n == 0) return (job.w && job.h && job.maxval && job.maxval <= 255) ? JPGENC_OK : fail(c, JPGENC_ERR_ARG, "width/height/maxval out of range");
     JPGENC_CUDA(c, cudaSetDevice(c->device));
@@ -494,77 +475,67 @@ int encode_host_frames(jpgenc_ctx* c, Job& job, const uint8_t* const* frames) {
     const uint32_t npasses = static_cast<uint32_t>(pass.size());
     constexpr uint32_t kRingMax = sizeof(c->ev_band) / sizeof(c->ev_band[0]);
     const uint32_t ring = std::min({nslots + 2, npasses, kRingMax});
-    const uint32_t np = job_planes(job);
-    const bool yuv = is_yuv(job.format);
-    auto plane_bytes = [&](uint32_t i) { return static_cast<size_t>(job_w(job, i)) * job_h(job, i) * job_bpp(job); };
-    // YUV: plane k of image i starts at yuv_off(i, k) of its slot (on 256 bytes), behind the last plane lies yuv_off(i, 3)
-    auto yuv_off = [&](uint32_t i, uint32_t k) {
-        const size_t y = (plane_bytes(i) + 255) & ~static_cast<size_t>(255);
-        const size_t cplane = (static_cast<size_t>(job_crow(job, i)) * ((job_h(job, i) + 1) / 2) + 255) & ~static_cast<size_t>(255);
-        return k == 0 ? 0 : y + std::min(k - 1, job.format == kPixelNV12 ? 1u : 2u) * cplane;
-    };
-    auto fbytes = [&](uint32_t i) { return yuv ? yuv_off(i, 3) : plane_bytes(i) * np; };
-    auto fstride = [&](uint32_t i) { return (fbytes(i) + 255) & ~static_cast<size_t>(255); };
-    // frame f of pass p sits at slice (p % ring) + at[f0 + f]
+    // image i: its planes as they are uploaded (staged_planes), at slice (p % ring) + at[i] of the ring
+    std::vector<StagedPlane> pl(3 * static_cast<size_t>(job.n));
+    std::vector<uint32_t> np(job.n);
     std::vector<size_t> at(job.n);
+    auto fstride = [&](uint32_t i) { return (staged_bytes(&pl[3 * i], np[i]) + 255) & ~static_cast<size_t>(255); };
     size_t slice = 0;
     for (const Pass& ps : pass) {
         size_t o = 0;
-        for (uint32_t f = 0; f < ps.F; ++f) { at[ps.f0 + f] = o; o += fstride(ps.f0 + f); }
+        for (uint32_t i = ps.f0; i < ps.f0 + ps.F; ++i) {
+            np[i] = staged_planes(job.src[i], job_w(job, i), job_h(job, i), &pl[3 * i]);
+            at[i] = o;
+            o += fstride(i);
+        }
         slice = std::max(slice, o);
     }
     if ((rc = ensure(c, &c->d_rgb_owned, &c->rgb_cap, static_cast<size_t>(ring) * slice + 16))) return rc;
     auto upload = [&](uint32_t p) -> int {
         const uint32_t f0 = pass[p].f0, F = pass[p].F, s = p % ring;
-        // equal frames that follow each other in host memory (a video buffer) travel as one strided copy
         for (uint32_t f = 0; f < F;) {
+            const uint32_t i = f0 + f;
+            const StagedPlane* q = &pl[3 * i];
+            uint8_t* dst = c->d_rgb_owned + static_cast<size_t>(s) * slice + at[i];
+            // equal frames that follow each other in host memory (a video buffer) travel as one strided copy
+            const size_t fbytes = staged_bytes(q, np[i]);
             uint32_t run = 1;
-            while (!job.widths && f + run < F && frames[f0 + f + run] == frames[f0 + f + run - 1] + fbytes(0)) ++run;
-            uint8_t* dst = c->d_rgb_owned + static_cast<size_t>(s) * slice + at[f0 + f];
-            const size_t row = static_cast<size_t>(job_w(job, f0 + f)) * job_bpp(job);
-            if (yuv) {
-                // YUV 4:2:0: one copy per plane, the pitch gaps dropped
-                const uint8_t* const* pl = frames + 3 * static_cast<size_t>(f0 + f);
-                const size_t h = job_h(job, f0 + f), crow = job_crow(job, f0 + f);
-                JPGENC_CUDA(c, cudaMemcpy2DAsync(dst, row, pl[0], job.pitches[f0 + f], row, h, cudaMemcpyHostToDevice, c->copy_stream));
-                for (uint32_t k = 1; k < 3 && pl[k]; ++k)
-                    JPGENC_CUDA(c, cudaMemcpy2DAsync(dst + yuv_off(f0 + f, k), crow, pl[k], job.c_pitches[f0 + f], crow, (h + 1) / 2,
-                                                     cudaMemcpyHostToDevice, c->copy_stream));
-            } else if (np == 3) {
-                // planar RGB: one copy per plane, or one strided copy when the planes lie back to back with tight rows
-                const uint8_t* const* pl = frames + 3 * static_cast<size_t>(f0 + f);
-                const size_t pb = plane_bytes(f0 + f), h = job_h(job, f0 + f), pitch = job.pitches[f0 + f];
-                const uintptr_t gap = reinterpret_cast<uintptr_t>(pl[1]) - reinterpret_cast<uintptr_t>(pl[0]);
-                if (pitch == row && gap >= pb && gap <= (uintptr_t{1} << 48) && reinterpret_cast<uintptr_t>(pl[2]) - reinterpret_cast<uintptr_t>(pl[1]) == gap)
-                    JPGENC_CUDA(c, cudaMemcpy2DAsync(dst, pb, pl[0], gap, pb, 3, cudaMemcpyHostToDevice, c->copy_stream));
-                else
-                    for (uint32_t k = 0; k < 3; ++k)
-                        JPGENC_CUDA(c, cudaMemcpy2DAsync(dst + k * pb, row, pl[k], pitch, row, h, cudaMemcpyHostToDevice, c->copy_stream));
-            } else if (job.pitches && job.pitches[f0 + f] != row)
-                JPGENC_CUDA(c, cudaMemcpy2DAsync(dst, row, frames[f0 + f], job.pitches[f0 + f], row, job_h(job, f0 + f), cudaMemcpyHostToDevice, c->copy_stream));
-            else if (run == 1) JPGENC_CUDA(c, cudaMemcpyAsync(dst, frames[f0 + f], fbytes(f0 + f), cudaMemcpyHostToDevice, c->copy_stream));
-            else JPGENC_CUDA(c, cudaMemcpy2DAsync(dst, fstride(0), frames[f0 + f], fbytes(0), fbytes(0), run, cudaMemcpyHostToDevice, c->copy_stream));
+            while (!job.widths && f + run < F && job.src[i + run].plane[0] == job.src[i + run - 1].plane[0] + fbytes) ++run;
+            if (run > 1) {
+                JPGENC_CUDA(c, cudaMemcpy2DAsync(dst, fstride(i), q[0].host, fbytes, fbytes, run, cudaMemcpyHostToDevice, c->copy_stream));
+            } else if (const size_t gap = planes_gap(q, np[i])) {
+                JPGENC_CUDA(c, cudaMemcpy2DAsync(dst, q[1].dev_off, q[0].host, gap, q[1].dev_off, np[i], cudaMemcpyHostToDevice, c->copy_stream));
+            } else {
+                for (uint32_t k = 0; k < np[i]; ++k) {
+                    if (q[k].pitch == q[k].row)
+                        JPGENC_CUDA(c, cudaMemcpyAsync(dst + q[k].dev_off, q[k].host, q[k].row * q[k].rows, cudaMemcpyHostToDevice, c->copy_stream));
+                    else
+                        JPGENC_CUDA(c, cudaMemcpy2DAsync(dst + q[k].dev_off, q[k].row, q[k].host, q[k].pitch, q[k].row, q[k].rows, cudaMemcpyHostToDevice,
+                                                         c->copy_stream));
+                }
+            }
             f += run;
         }
         JPGENC_CUDA(c, cudaEventRecord(c->ev_band[s], c->copy_stream));
         return JPGENC_OK;
     };
-    job.staged = true;
     for (uint32_t p = 0; p < ring; ++p)
         if ((rc = upload(p))) return rc;
-    std::vector<std::vector<const void*>> ptrs(nslots);
+    std::vector<std::vector<PixelSource>> staged(nslots);
     int upload_rc = JPGENC_OK;
     rc = run_passes(c, job, pass, nslots,
-                    [&](uint32_t p, jpgenc_ctx*, const void* const** out, cudaEvent_t* ready) {
+                    [&](uint32_t p, jpgenc_ctx*, const PixelSource** out, cudaEvent_t* ready) {
                         const uint32_t f0 = pass[p].f0, F = pass[p].F, s = p % ring;
-                        std::vector<const void*>& v = ptrs[p % nslots];
-                        v.resize(static_cast<size_t>(F) * np);
-                        for (uint32_t f = 0; f < F; ++f)
-                            for (uint32_t k = 0; k < np; ++k) {
-                                const size_t off = yuv ? yuv_off(f0 + f, k) : k * plane_bytes(f0 + f);
-                                const bool none = yuv && k == 2 && job.format == kPixelNV12;            // NV12 has no V plane
-                                v[f * np + k] = none ? nullptr : c->d_rgb_owned + static_cast<size_t>(s) * slice + at[f0 + f] + off;
-                            }
+                        std::vector<PixelSource>& v = staged[p % nslots];
+                        v.resize(F);
+                        for (uint32_t f = 0; f < F; ++f) {
+                            const StagedPlane* q = &pl[3 * (f0 + f)];
+                            v[f] = job.src[f0 + f];
+                            for (uint32_t k = 0; k < 3; ++k)
+                                v[f].plane[k] = k < np[f0 + f] ? c->d_rgb_owned + static_cast<size_t>(s) * slice + at[f0 + f] + q[k].dev_off : nullptr;
+                            v[f].pitch = static_cast<uint32_t>(q[0].row);
+                            if (np[f0 + f] > 1) v[f].pitch2 = static_cast<uint32_t>(q[1].row);
+                        }
                         *out = v.data();
                         *ready = c->ev_band[s];
                         return JPGENC_OK;
@@ -577,7 +548,39 @@ int encode_host_frames(jpgenc_ctx* c, Job& job, const uint8_t* const* frames) {
     if (rc == JPGENC_OK) rc = upload_rc;
     const cudaError_t e = cudaStreamSynchronize(c->copy_stream);
     if (e != cudaSuccess && rc == JPGENC_OK) rc = fail(c, JPGENC_ERR_CUDA, "host-to-device copy of a frame failed");
-    c->d_rgb = c->d_rgb_owned;
+    c->src.plane[0] = c->d_rgb_owned;
+    return rc;
+}
+
+// equal tight RGB frames of one call (the pointers are not checked one by one)
+void rgb_frames(Job& job, const void* const* frames) {
+    job.src.resize(job.n);
+    for (uint32_t i = 0; i < job.n; ++i) job.src[i] = image_source(frames[i], job.w * 3, JPGENC_PIXEL_RGB);
+}
+
+// The packed calls: images of individual sizes in any source.  Every source is checked (from host memory: its samples against
+// maxval too).  Tight RGB takes the kernels of tight RGB, and when every image has one size, the batched-frame path as it is.
+int encode_packed(jpgenc_ctx* c, std::vector<PixelSource>& src, int images_on_device, const uint32_t* widths, const uint32_t* heights,
+                  uint32_t maxval, uint8_t* out, uint64_t cap, uint64_t* offsets, uint64_t* sizes, uint64_t* total_bytes) {
+    const uint32_t n = static_cast<uint32_t>(src.size());
+    bool same = true, tight_rgb = true;
+    for (uint32_t i = 0; i < n; ++i) {
+        const int rc = check_source(c, &src[i], widths[i], heights[i]);
+        if (rc) return rc;
+        same = same && widths[i] == widths[0] && heights[i] == heights[0];
+        tight_rgb = tight_rgb && src[i].format == JPGENC_PIXEL_RGB && src[i].pitch == widths[i] * 3;
+    }
+    if (!images_on_device)
+        for (uint32_t i = 0; i < n; ++i)
+            if (!source_within_maxval(src[i], widths[i], heights[i], maxval)) return fail(c, JPGENC_ERR_FORMAT, "a sample exceeds maxval");
+    Job job;
+    job.n = n; job.w = widths[0]; job.h = heights[0]; job.maxval = maxval;
+    if (!tight_rgb || !same) { job.widths = widths; job.heights = heights; }   // the pass pipeline of images of individual sizes
+    job.format = tight_rgb ? -1 : src[0].format;
+    job.src = std::move(src);
+    job.packed_mode = true; job.packed = out; job.packed_cap = cap; job.offsets = offsets; job.sizes = sizes;
+    const int rc = images_on_device ? encode_device_frames(c, job) : encode_host_frames(c, job);
+    if (total_bytes) *total_bytes = job.packed_at;
     return rc;
 }
 
@@ -591,7 +594,9 @@ int jpgenc_encode_frames_device(jpgenc_ctx* c, uint32_t n, const void* const* de
     job.n = n; job.w = w; job.h = h; job.maxval = maxval;
     job.out_ptrs = out; job.caps = caps; job.sizes = sizes;
     const int rc = check_job(c, job, dev_frames);
-    return rc ? rc : encode_device_frames(c, job, dev_frames);
+    if (rc) return rc;
+    rgb_frames(job, dev_frames);
+    return encode_device_frames(c, job);
 } JPGENC_CATCH(c)
 
 int jpgenc_encode_frames(jpgenc_ctx* c, uint32_t n, const uint8_t* const* frames, uint32_t w, uint32_t h, uint32_t maxval,
@@ -600,7 +605,9 @@ int jpgenc_encode_frames(jpgenc_ctx* c, uint32_t n, const uint8_t* const* frames
     job.n = n; job.w = w; job.h = h; job.maxval = maxval;
     job.out_ptrs = out; job.caps = caps; job.sizes = sizes;
     const int rc = check_job(c, job, frames);
-    return rc ? rc : encode_host_frames(c, job, frames);
+    if (rc) return rc;
+    rgb_frames(job, reinterpret_cast<const void* const*>(frames));
+    return encode_host_frames(c, job);
 } JPGENC_CATCH(c)
 
 int jpgenc_encode_frames_packed(jpgenc_ctx* c, uint32_t n, const void* const* frames, int frames_on_device, uint32_t w, uint32_t h,
@@ -610,7 +617,8 @@ int jpgenc_encode_frames_packed(jpgenc_ctx* c, uint32_t n, const void* const* fr
     job.packed_mode = true; job.packed = out; job.packed_cap = cap; job.offsets = offsets; job.sizes = sizes;
     int rc = check_job(c, job, frames);
     if (rc) return rc;
-    rc = frames_on_device ? encode_device_frames(c, job, frames) : encode_host_frames(c, job, reinterpret_cast<const uint8_t* const*>(frames));
+    rgb_frames(job, frames);
+    rc = frames_on_device ? encode_device_frames(c, job) : encode_host_frames(c, job);
     if (total_bytes) *total_bytes = job.packed_at;
     return rc;
 } JPGENC_CATCH(c)
@@ -623,23 +631,9 @@ int jpgenc_encode_images_packed(jpgenc_ctx* c, uint32_t n, const void* const* im
     if (maxval == 0 || maxval > 255) return fail(c, JPGENC_ERR_ARG, "maxval out of range");
     if (n == 0) return JPGENC_OK;                                // an empty batch is legal and touches nothing
     if (!images || !widths || !heights || !offsets || !sizes) return fail(c, JPGENC_ERR_ARG, "null argument");
-    bool same = true;
-    for (uint32_t i = 0; i < n; ++i) {
-        if (!images[i]) return fail(c, JPGENC_ERR_ARG, "null image pointer");
-        if (widths[i] == 0 || heights[i] == 0 || widths[i] > 65535 || heights[i] > 65535) return fail(c, JPGENC_ERR_ARG, "image side out of range (1..65535)");
-        same = same && widths[i] == widths[0] && heights[i] == heights[0];
-    }
-    if (!images_on_device && maxval < 255)
-        for (uint32_t i = 0; i < n; ++i)
-            if (!samples_within_maxval(static_cast<const uint8_t*>(images[i]), static_cast<size_t>(widths[i]) * heights[i] * 3, maxval))
-                return fail(c, JPGENC_ERR_FORMAT, "a sample exceeds maxval");
-    Job job;
-    job.n = n; job.w = widths[0]; job.h = heights[0]; job.maxval = maxval;
-    if (!same) { job.widths = widths; job.heights = heights; }   // one size: the batched-frame path as it is
-    job.packed_mode = true; job.packed = out; job.packed_cap = cap; job.offsets = offsets; job.sizes = sizes;
-    const int rc = images_on_device ? encode_device_frames(c, job, images) : encode_host_frames(c, job, reinterpret_cast<const uint8_t* const*>(images));
-    if (total_bytes) *total_bytes = job.packed_at;
-    return rc;
+    std::vector<PixelSource> src(n);
+    for (uint32_t i = 0; i < n; ++i) src[i] = image_source(images[i], 0, JPGENC_PIXEL_RGB);
+    return encode_packed(c, src, images_on_device, widths, heights, maxval, out, cap, offsets, sizes, total_bytes);
 } JPGENC_CATCH(c)
 
 int jpgenc_encode_images_packed_layout(jpgenc_ctx* c, uint32_t n, const void* const* images, int images_on_device, const uint32_t* widths,
@@ -647,32 +641,13 @@ int jpgenc_encode_images_packed_layout(jpgenc_ctx* c, uint32_t n, const void* co
                                        uint64_t cap, uint64_t* offsets, uint64_t* sizes, uint64_t* total_bytes) try {
     if (!c) return JPGENC_ERR_ARG;
     if (total_bytes) *total_bytes = 0;
-    if ((format < JPGENC_PIXEL_RGB || format > JPGENC_PIXEL_BGRA) && format != JPGENC_PIXEL_GRAY) return fail(c, JPGENC_ERR_ARG, "unknown pixel format");
+    if (image_source(nullptr, 0, format).format < 0) return fail(c, JPGENC_ERR_ARG, "unknown pixel format");
     if (maxval == 0 || maxval > 255) return fail(c, JPGENC_ERR_ARG, "maxval out of range");
     if (n == 0) return JPGENC_OK;                                // an empty batch is legal and touches nothing
     if (!images || !widths || !heights || !offsets || !sizes) return fail(c, JPGENC_ERR_ARG, "null argument");
-    std::vector<uint32_t> pitch(n);
-    bool tight_rgb = format == JPGENC_PIXEL_RGB;
-    for (uint32_t i = 0; i < n; ++i) {
-        if (!images[i]) return fail(c, JPGENC_ERR_ARG, "null image pointer");
-        pitch[i] = row_pitches ? row_pitches[i] : 0;
-        const int rc = check_layout(c, widths[i], heights[i], &pitch[i], format);
-        if (rc) return rc;
-        tight_rgb = tight_rgb && pitch[i] == widths[i] * 3;
-    }
-    if (tight_rgb) return jpgenc_encode_images_packed(c, n, images, images_on_device, widths, heights, maxval, out, cap, offsets, sizes, total_bytes);
-    if (!images_on_device && maxval < 255)
-        for (uint32_t i = 0; i < n; ++i)
-            if (!samples_within_maxval(static_cast<const uint8_t*>(images[i]), widths[i], heights[i], pitch[i], pixel_bytes(format), maxval))
-                return fail(c, JPGENC_ERR_FORMAT, "a sample exceeds maxval");
-    Job job;
-    job.n = n; job.w = widths[0]; job.h = heights[0]; job.maxval = maxval;
-    job.widths = widths; job.heights = heights;                  // the pass pipeline of images of individual sizes, equal sizes too
-    job.format = format; job.pitches = pitch.data();
-    job.packed_mode = true; job.packed = out; job.packed_cap = cap; job.offsets = offsets; job.sizes = sizes;
-    const int rc = images_on_device ? encode_device_frames(c, job, images) : encode_host_frames(c, job, reinterpret_cast<const uint8_t* const*>(images));
-    if (total_bytes) *total_bytes = job.packed_at;
-    return rc;
+    std::vector<PixelSource> src(n);
+    for (uint32_t i = 0; i < n; ++i) src[i] = image_source(images[i], row_pitches ? row_pitches[i] : 0, format);
+    return encode_packed(c, src, images_on_device, widths, heights, maxval, out, cap, offsets, sizes, total_bytes);
 } JPGENC_CATCH(c)
 
 int jpgenc_encode_images_packed_planar(jpgenc_ctx* c, uint32_t n, const void* const* planes, int images_on_device, const uint32_t* widths,
@@ -683,25 +658,9 @@ int jpgenc_encode_images_packed_planar(jpgenc_ctx* c, uint32_t n, const void* co
     if (maxval == 0 || maxval > 255) return fail(c, JPGENC_ERR_ARG, "maxval out of range");
     if (n == 0) return JPGENC_OK;                                // an empty batch is legal and touches nothing
     if (!planes || !widths || !heights || !offsets || !sizes) return fail(c, JPGENC_ERR_ARG, "null argument");
-    std::vector<uint32_t> pitch(n);
-    for (uint32_t i = 0; i < n; ++i) {
-        if (!planes[3 * i] || !planes[3 * i + 1] || !planes[3 * i + 2]) return fail(c, JPGENC_ERR_ARG, "null plane pointer");
-        pitch[i] = row_pitches ? row_pitches[i] : 0;
-        const int rc = check_layout(c, widths[i], heights[i], &pitch[i], JPGENC_PIXEL_GRAY);   // every plane: one byte per pixel
-        if (rc) return rc;
-    }
-    if (!images_on_device && maxval < 255)
-        for (uint32_t i = 0; i < 3 * n; ++i)
-            if (!samples_within_maxval(static_cast<const uint8_t*>(planes[i]), widths[i / 3], heights[i / 3], pitch[i / 3], 1, maxval))
-                return fail(c, JPGENC_ERR_FORMAT, "a sample exceeds maxval");
-    Job job;
-    job.n = n; job.w = widths[0]; job.h = heights[0]; job.maxval = maxval;
-    job.widths = widths; job.heights = heights;
-    job.format = kPixelPlanar; job.pitches = pitch.data();
-    job.packed_mode = true; job.packed = out; job.packed_cap = cap; job.offsets = offsets; job.sizes = sizes;
-    const int rc = images_on_device ? encode_device_frames(c, job, planes) : encode_host_frames(c, job, reinterpret_cast<const uint8_t* const*>(planes));
-    if (total_bytes) *total_bytes = job.packed_at;
-    return rc;
+    std::vector<PixelSource> src(n);
+    for (uint32_t i = 0; i < n; ++i) src[i] = planar_source(planes[3 * i], planes[3 * i + 1], planes[3 * i + 2], row_pitches ? row_pitches[i] : 0);
+    return encode_packed(c, src, images_on_device, widths, heights, maxval, out, cap, offsets, sizes, total_bytes);
 } JPGENC_CATCH(c)
 
 int jpgenc_encode_images_packed_yuv420(jpgenc_ctx* c, uint32_t n, const void* const* planes, int images_on_device, const uint32_t* widths,
@@ -712,22 +671,10 @@ int jpgenc_encode_images_packed_yuv420(jpgenc_ctx* c, uint32_t n, const void* co
     if (layout != JPGENC_YUV_I420 && layout != JPGENC_YUV_NV12) return fail(c, JPGENC_ERR_ARG, "unknown YUV layout");
     if (n == 0) return JPGENC_OK;                                // an empty batch is legal and touches nothing
     if (!planes || !widths || !heights || !offsets || !sizes) return fail(c, JPGENC_ERR_ARG, "null argument");
-    std::vector<uint32_t> pitch(n), c_pitch(n);
-    int format = 0;
-    for (uint32_t i = 0; i < n; ++i) {
-        pitch[i] = y_pitches ? y_pitches[i] : 0;
-        c_pitch[i] = c_pitches ? c_pitches[i] : 0;
-        const int rc = check_yuv420(c, planes[3 * i], planes[3 * i + 1], planes[3 * i + 2], widths[i], heights[i], &pitch[i], &c_pitch[i], layout, &format);
-        if (rc) return rc;
-    }
-    Job job;
-    job.n = n; job.w = widths[0]; job.h = heights[0]; job.maxval = 255;
-    job.widths = widths; job.heights = heights;
-    job.format = format; job.pitches = pitch.data(); job.c_pitches = c_pitch.data();
-    job.packed_mode = true; job.packed = out; job.packed_cap = cap; job.offsets = offsets; job.sizes = sizes;
-    const int rc = images_on_device ? encode_device_frames(c, job, planes) : encode_host_frames(c, job, reinterpret_cast<const uint8_t* const*>(planes));
-    if (total_bytes) *total_bytes = job.packed_at;
-    return rc;
+    std::vector<PixelSource> src(n);
+    for (uint32_t i = 0; i < n; ++i)
+        src[i] = yuv420_source(planes[3 * i], planes[3 * i + 1], planes[3 * i + 2], y_pitches ? y_pitches[i] : 0, c_pitches ? c_pitches[i] : 0, layout);
+    return encode_packed(c, src, images_on_device, widths, heights, 255, out, cap, offsets, sizes, total_bytes);
 } JPGENC_CATCH(c)
 
 }  // extern "C"
