@@ -133,6 +133,29 @@ int jpgenc_bind_device_planar(jpgenc_ctx* ctx, const void* r, const void* g, con
 #define JPGENC_YUV_NV12 1   /* Y plane, interleaved UV plane (passed as u; v must be NULL) */
 int jpgenc_bind_device_yuv420(jpgenc_ctx* ctx, const void* y, const void* u, const void* v, uint32_t w, uint32_t h, uint32_t y_pitch,
                               uint32_t c_pitch, int layout);
+/* YUV frames with 8-bit samples in any of these layouts (and the two above), as cameras, capture cards and decoders leave them.
+ * With cw = ceil(w/2), a frame has:
+ *   JPGENC_YUV_I422: a Y plane of h rows of w bytes, U and V planes of h rows of cw bytes, c_pitch apart (0 = cw); YV16 is I422
+ *                    with the u and v pointers swapped (ffmpeg yuv422p / yuvj422p);
+ *   JPGENC_YUV_NV16: a Y plane and one plane of h rows of cw (U, V) byte pairs (0 = 2 cw), passed as u; v must be NULL;
+ *   JPGENC_YUV_I444: Y, U and V planes of h rows of w bytes; U and V share c_pitch (0 = w) (ffmpeg yuv444p);
+ *   JPGENC_YUV_YUYV: one packed plane of h rows of cw groups Y0 U Y1 V (4 cw bytes, y_pitch apart; V4L2_PIX_FMT_YUYV), passed as
+ *                    y; u and v must be NULL and c_pitch 0.  For an odd w the second Y of the last group is never read;
+ *   JPGENC_YUV_UYVY: the same with groups U Y0 V Y1 (8-bit YUV of SDI capture cards).
+ * The colour contract is that of the 4:2:0 layouts: the samples are the file's Y, Cb and Cr as they are.  The file is always the
+ * reference's 4:2:0 file: jpgenc_encode_planes(..., ycbcr = 1) of the planes Y - 128, U - 128, V - 128 at full resolution
+ * (every 4:2:2 chroma sample repeated over its two pixels), padded to whole MCUs by edge replication -- so the chroma of a 2x2
+ * cell is the mean of its four (clamped) samples, as S420_m takes it.  These three calls take all seven JPGENC_YUV_* codes;
+ * jpgenc_bind_device_yuv420 / jpgenc_encode_yuv420 / jpgenc_encode_images_packed_yuv420 only the two 4:2:0 ones.  Unknown
+ * layout, a null Y plane, a null chroma plane where one is needed or a non-null one where it must be NULL, c_pitch != 0 for the
+ * packed layouts, a pitch below its row size, sides outside 1..65535: JPGENC_ERR_ARG. */
+#define JPGENC_YUV_I422 2   /* Y, U, V planes, chroma of cw x h */
+#define JPGENC_YUV_NV16 3   /* Y plane, interleaved UV plane of cw pairs x h (passed as u; v must be NULL) */
+#define JPGENC_YUV_I444 4   /* Y, U, V planes, all w x h */
+#define JPGENC_YUV_YUYV 5   /* one packed plane of Y0 U Y1 V groups (passed as y) */
+#define JPGENC_YUV_UYVY 6   /* one packed plane of U Y0 V Y1 groups (passed as y) */
+int jpgenc_bind_device_yuv(jpgenc_ctx* ctx, const void* y, const void* u, const void* v, uint32_t w, uint32_t h, uint32_t y_pitch,
+                           uint32_t c_pitch, int layout);
 
 /* ---- K1: convertToColorSpace(YCbCr) + applySubsampling(S420_m) + applyDCT(Arai) + applyQuantization
  *      + zigzag (src/Image.cpp:112-148, 198-235, 540-595, 597-636; Dct.hpp:47-215; Coding.hpp:57-97) -- */
@@ -204,6 +227,9 @@ int jpgenc_encode_planar(jpgenc_ctx* ctx, const void* r, const void* g, const vo
  * bands before it. */
 int jpgenc_encode_yuv420(jpgenc_ctx* ctx, const void* y, const void* u, const void* v, uint32_t w, uint32_t h, uint32_t y_pitch,
                          uint32_t c_pitch, int layout, uint8_t* dst, uint64_t cap, uint64_t* jpeg_bytes);
+/* the same for a frame in any JPGENC_YUV_* layout (see jpgenc_bind_device_yuv): 4:2:2 travels at 2 bytes per pixel, 4:4:4 at 3 */
+int jpgenc_encode_yuv(jpgenc_ctx* ctx, const void* y, const void* u, const void* v, uint32_t w, uint32_t h, uint32_t y_pitch,
+                      uint32_t c_pitch, int layout, uint8_t* dst, uint64_t cap, uint64_t* jpeg_bytes);
 /* Image::writeJPEG (src/Image.cpp:831-976) for an image given as the reference holds it: three row-major planes of doubles
  * (Image::R/G/B, include/Image.hpp:104-114), `width` x `height` = the image padded to whole 16x16 MCUs (src/Image.cpp:479-530),
  * real_w x real_h = what SOF0 reports.  ycbcr != 0: the planes already are level-shifted Y, Cb, Cr and are not converted
@@ -283,6 +309,12 @@ int jpgenc_encode_images_packed_yuv420(jpgenc_ctx* ctx, uint32_t n, const void* 
                                        const uint32_t* widths, const uint32_t* heights, const uint32_t* y_pitches,
                                        const uint32_t* c_pitches, int layout, uint8_t* out, uint64_t cap, uint64_t* offsets,
                                        uint64_t* sizes, uint64_t* total_bytes);
+/* the same for frames in any JPGENC_YUV_* layout (see jpgenc_bind_device_yuv), one layout per call: planes[3i .. 3i + 2] are
+ * Y, U, V of frame i (NV12 / NV16: Y, UV, NULL; YUYV / UYVY: the packed plane, NULL, NULL) */
+int jpgenc_encode_images_packed_yuv(jpgenc_ctx* ctx, uint32_t n, const void* const* planes, int images_on_device,
+                                    const uint32_t* widths, const uint32_t* heights, const uint32_t* y_pitches,
+                                    const uint32_t* c_pitches, int layout, uint8_t* out, uint64_t cap, uint64_t* offsets,
+                                    uint64_t* sizes, uint64_t* total_bytes);
 
 /* ---- stage methods for the modes writeJPEG does not use (SURVEY.md 8(f)4) ------------------------------------------ */
 /* Image::applySubsampling(mode) on one chroma plane (src/Image.cpp:198-319): `plane` = height x width doubles (host), mode =

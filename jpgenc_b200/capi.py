@@ -20,6 +20,8 @@ ERR_CUDA, ERR_ARG, ERR_NO_DEVICE, ERR_FORMAT, ERR_IO, ERR_CAPACITY, ERR_NOMEM = 
 PIXEL_FORMATS = {"RGB": (0, 3), "BGR": (1, 3), "RGBA": (2, 4), "BGRA": (3, 4), "GRAY": (16, 1)}
 # YUV 4:2:0 frames (JPGENC_YUV_*): Y, U, V planes / Y plane and interleaved UV plane
 YUV_LAYOUTS = {"I420": 0, "NV12": 1}
+# every JPGENC_YUV_* layout: 4:2:0 as above; 4:2:2 planar (I422), semi-planar (NV16) and packed (YUYV, UYVY); 4:4:4 planar (I444)
+YUV_FORMATS = {"I420": 0, "NV12": 1, "I422": 2, "NV16": 3, "I444": 4, "YUYV": 5, "UYVY": 6}
 
 u8p = C.POINTER(C.c_uint8)
 i16p = C.POINTER(C.c_int16)
@@ -72,6 +74,10 @@ _SIGNATURES = {
                                             C.c_int]),
     "jpgenc_encode_yuv420": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int,
                                        C.c_void_p, C.c_uint64, u64p]),
+    "jpgenc_bind_device_yuv": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32,
+                                         C.c_int]),
+    "jpgenc_encode_yuv": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int,
+                                    C.c_void_p, C.c_uint64, u64p]),
     "jpgenc_encode_image": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int, C.c_uint32, C.c_void_p, C.c_uint64,
                                       u64p]),
     "jpgenc_color_dct_quant": (C.c_int, [C.c_void_p]),
@@ -127,6 +133,8 @@ _SIGNATURES = {
                                                      C.c_void_p, C.c_uint64, u64p, u64p, u64p]),
     "jpgenc_encode_images_packed_yuv420": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(C.c_void_p), C.c_int, u32p, u32p, u32p, u32p, C.c_int,
                                                      C.c_void_p, C.c_uint64, u64p, u64p, u64p]),
+    "jpgenc_encode_images_packed_yuv": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(C.c_void_p), C.c_int, u32p, u32p, u32p, u32p, C.c_int,
+                                                  C.c_void_p, C.c_uint64, u64p, u64p, u64p]),
     "jpgenc_batch_create": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "jpgenc_batch_destroy": (None, [C.c_void_p]),
     "jpgenc_batch_last_error": (C.c_char_p, [C.c_void_p]),
@@ -308,6 +316,93 @@ def yuv420_layout(y, u, v=None):
     return "I420", (yp, up, vp), w, h, y_pitch, pitches[0]
 
 
+def _pitched(name, shape, st, rows, row):
+    """the row pitch of a (rows, row) uint8 plane with strides (pitch, 1); ValueError otherwise"""
+    if shape != (rows, row):
+        raise ValueError(f"{name} must be ({rows}, {row}), not {shape}")
+    pitch = st[0] if rows > 1 else row
+    if (row > 1 and st[1] != 1) or pitch < row:
+        raise ValueError(f"{name} must have strides (pitch, 1) with pitch >= {row}; got {st}")
+    return pitch
+
+
+def _pairs(name, shape, st, rows, n, k):
+    """the row pitch of a plane of `rows` rows of n groups of k bytes: (rows, n, k) with strides (pitch, k, 1) or (rows, n k) with
+    strides (pitch, 1); ValueError otherwise"""
+    if shape == (rows, n, k):
+        ok = (n == 1 or st[1] == k) and st[2] == 1
+    elif shape == (rows, n * k):
+        ok = st[1] == 1
+    else:
+        raise ValueError(f"{name} must be ({rows}, {n}, {k}) or ({rows}, {n * k}), not {shape}")
+    pitch = st[0] if rows > 1 else n * k
+    if not ok or pitch < n * k:
+        raise ValueError(f"{name} must have strides (pitch, {k}, 1) or (pitch, 1) with pitch >= {n * k}; got {st}")
+    return pitch
+
+
+def yuv_layout(layout, y, u=None, v=None, w=None):
+    """How a YUV frame in the named layout (a YUV_FORMATS key) is read in place: (layout, (y, u or 0, v or 0) pointers, width,
+    height, y_pitch, c_pitch).
+
+    y, u, v are uint8 numpy arrays or torch tensors.  For a frame of H x W and cw = ceil(W/2):
+      I420, NV12               as yuv420_layout (NV12: v is None)
+      I422 (YV16: u, v swapped) Y (H, W), U and V (H, cw), strides (pitch, 1), one c_pitch for U and V
+      NV16                     Y (H, W); UV (H, cw, 2) with strides (c_pitch, 2, 1), or (H, 2 cw) with strides (c_pitch, 1); v None
+      I444                     Y, U, V (H, W), strides (pitch, 1), one c_pitch for U and V
+      YUYV, UYVY               one packed plane y, (H, 4 cw) with strides (pitch, 1) or (H, cw, 4) with strides (pitch, 4, 1);
+                               u and v None; c_pitch 0.  The width is 2 cw unless w says 2 cw - 1 (the last group's second Y
+                               is then not read).
+    w, where given, must be the width the planes describe.  Anything else raises ValueError; nothing is ever copied.  Pure: only
+    the metadata is read."""
+    if layout not in YUV_FORMATS:
+        raise ValueError(f"unknown YUV layout {layout!r}; expected one of {sorted(YUV_FORMATS)}")
+    if layout in ("YUYV", "UYVY"):
+        if u is not None or v is not None:
+            raise ValueError(f"{layout} is one packed plane: u and v must be None")
+        yp, ys, yst = _u8_plane(y, layout)
+        if len(ys) not in (2, 3):
+            raise ValueError(f"{layout} must be (H, 4 cw) or (H, cw, 4), not {ys}")
+        cw = ys[1] if len(ys) == 3 else ys[1] // 4
+        if cw == 0 or (len(ys) == 2 and ys[1] % 4):
+            raise ValueError(f"{layout} rows must be whole groups of 4 bytes; got {ys}")
+        h = ys[0]
+        pitch = _pairs(layout, ys, yst, h, cw, 4)
+        width = 2 * cw if w is None else w
+        if width not in (2 * cw, 2 * cw - 1):
+            raise ValueError(f"{layout} rows of {cw} groups hold {2 * cw - 1} or {2 * cw} pixels, not {width}")
+        return layout, (yp, 0, 0), width, h, pitch, 0
+    if layout in ("I420", "NV12"):
+        if (layout == "NV12") != (v is None):
+            raise ValueError(f"{layout} takes {'Y and UV (v None)' if layout == 'NV12' else 'Y, U and V'}")
+        got = yuv420_layout(y, u, v)
+    else:
+        yp, ys, yst = _u8_plane(y, "Y")
+        if len(ys) != 2:
+            raise ValueError(f"Y must be (H, W), not {ys}")
+        h, width = ys
+        y_pitch = _pitched("Y", ys, yst, h, width)
+        cw = width if layout == "I444" else (width + 1) // 2
+        if u is None:
+            raise ValueError(f"{layout} needs its chroma plane(s)")
+        up, us, ust = _u8_plane(u, "U")
+        if layout == "NV16":
+            if v is not None:
+                raise ValueError("NV16 takes its UV plane as u; v must be None")
+            got = ("NV16", (yp, up, 0), width, h, y_pitch, _pairs("NV16 UV", us, ust, h, cw, 2))
+        else:
+            if v is None:
+                raise ValueError(f"{layout} takes Y, U and V")
+            vp, vs, vst = _u8_plane(v, "V")
+            pu, pv = _pitched(f"{layout} U", us, ust, h, cw), _pitched(f"{layout} V", vs, vst, h, cw)
+            if pu != pv:
+                raise ValueError(f"{layout} U and V must share one row stride; got {pu} and {pv}")
+            got = (layout, (yp, up, vp), width, h, y_pitch, pu)
+    if w is not None and w != got[2]:
+        raise ValueError(f"w = {w}, but the planes describe a frame {got[2]} wide")
+    return got
+
+
 class Encoder:
     """One GPU context (= one CUDA stream + its device buffers).  Methods mirror the C-ABI one to one."""
 
@@ -367,6 +462,10 @@ class Encoder:
         self._check(self.lib.jpgenc_bind_device_planar(self.h, r, g, b, w, h, pitch, maxval))
 
     # ---- stages ---------------------------------------------------------------------------------
+    def bind_device_yuv(self, layout: str, y: int, u: int | None, v: int | None, w: int, h: int, y_pitch: int = 0, c_pitch: int = 0):
+        """a YUV frame of any YUV_FORMATS layout in device memory (plane pointers; None where the layout has no such plane)"""
+        self._check(self.lib.jpgenc_bind_device_yuv(self.h, y, u or None, v or None, w, h, y_pitch, c_pitch, YUV_FORMATS[layout]))
+
     def bind_device_yuv420(self, y: int, u: int, v: int | None, w: int, h: int, y_pitch: int = 0, c_pitch: int = 0, layout: str = "I420"):
         """a YUV 4:2:0 frame in device memory (plane pointers; NV12: v None, u the UV plane; pitches 0: tight)"""
         self._check(self.lib.jpgenc_bind_device_yuv420(self.h, y, u, v or None, w, h, y_pitch, c_pitch, YUV_LAYOUTS[layout]))
@@ -482,6 +581,12 @@ class Encoder:
         return self._file(lambda out, cap, n: self.lib.jpgenc_encode_yuv420(self.h, y, u, v or None, w, h, y_pitch, c_pitch, code, out, cap, n),
                           max(4096, w * h * 3 // 2 + 4096))
 
+    def encode_yuv_ptr(self, layout: str, y: int, u: int | None, v: int | None, w: int, h: int, y_pitch: int = 0, c_pitch: int = 0) -> bytes:
+        """a YUV frame of any YUV_FORMATS layout in host memory (plane pointers, see bind_device_yuv) -> JPEG bytes"""
+        code = YUV_FORMATS[layout]
+        return self._file(lambda out, cap, n: self.lib.jpgenc_encode_yuv(self.h, y, u or None, v or None, w, h, y_pitch, c_pitch, code, out, cap, n),
+                          max(4096, w * h * 3 // 2 + 4096))
+
     def encode_planes(self, p0: np.ndarray, p1: np.ndarray, p2: np.ndarray, real_w: int, real_h: int, ycbcr: bool = False) -> bytes:
         """three (H16, W16) float64 planes as the reference's Image holds them -> JPEG bytes (exact FP64 path for every block)"""
         planes = [np.ascontiguousarray(p, np.float64) for p in (p0, p1, p2)]
@@ -591,6 +696,14 @@ class Encoder:
                             None if y_pitches is None else list(y_pitches), None if c_pitches is None else list(c_pitches),
                             YUV_LAYOUTS[layout], out_ptr, cap)
 
+    def encode_images_packed_yuv(self, planes, widths, heights, out_ptr: int | None, cap: int, layout: str, host_images=False,
+                                 y_pitches=None, c_pitches=None):
+        """YUV frames of one YUV_FORMATS layout and individual sizes: planes[3i:3i + 3] = the plane pointers of frame i (None where
+        the layout has no such plane) -> files back to back as encode_images_packed"""
+        return self._packed(self.lib.jpgenc_encode_images_packed_yuv, len(widths), 3, planes, host_images, widths, heights,
+                            None if y_pitches is None else list(y_pitches), None if c_pitches is None else list(c_pitches),
+                            YUV_FORMATS[layout], out_ptr, cap)
+
     def _planes_on_host(self, planes) -> bool:
         """True for numpy arrays and CPU tensors; False for tensors on this encoder's GPU, once the work queued on torch's current
         stream has finished.  Anything else (a mix, another device) raises ValueError."""
@@ -648,6 +761,33 @@ class Encoder:
         cps = [x[5] for x in layouts]
         layout = layouts[0][0]
         enc = lambda o, c: self.encode_images_packed_yuv420(planes, ws, hs, o, c, layout, host_images=host, y_pitches=yps, c_pitches=cps)
+        return self._files(enc, sum(w * h for w, h in zip(ws, hs)), len(frames))
+
+    def encode_yuv(self, layout: str, y, u=None, v=None, w=None) -> bytes:
+        """one YUV frame in the named layout read in place (see yuv_layout) from numpy arrays, CPU tensors or tensors on this
+        encoder's GPU -> JPEG bytes"""
+        layout, (yp, up, vp), w, h, y_pitch, c_pitch = yuv_layout(layout, y, u, v, w)
+        if self._planes_on_host([a for a in (y, u, v) if a is not None]):
+            return self.encode_yuv_ptr(layout, yp, up, vp, w, h, y_pitch, c_pitch)
+        self.bind_device_yuv(layout, yp, up, vp, w, h, y_pitch, c_pitch)
+        n = self.encode_bound(None)
+        out = np.empty(n, np.uint8)
+        n = C.c_uint64()
+        self._check(self.lib.jpgenc_assemble_last(self.h, out.ctypes.data, out.size, C.byref(n)))
+        return out[: n.value].tobytes()
+
+    def encode_yuv_many(self, layout: str, frames):
+        """frames of one named layout and any sizes, each a tuple (y, u, v, w) or a prefix of it (see yuv_layout), all in host
+        memory or all on this encoder's GPU, through one batched call -> list of JPEG byte strings"""
+        frames = [tuple(f) for f in frames]
+        if not frames:
+            return []
+        layouts = [yuv_layout(layout, *f) for f in frames]
+        host = self._planes_on_host([a for f in frames for a in f[:3] if a is not None])
+        planes = [p or None for x in layouts for p in x[1]]
+        ws, hs = [x[2] for x in layouts], [x[3] for x in layouts]
+        yps, cps = [x[4] for x in layouts], [x[5] for x in layouts]
+        enc = lambda o, c: self.encode_images_packed_yuv(planes, ws, hs, o, c, layout, host_images=host, y_pitches=yps, c_pitches=cps)
         return self._files(enc, sum(w * h for w, h in zip(ws, hs)), len(frames))
 
     def _files(self, encode, pixels: int, n: int):

@@ -82,15 +82,18 @@ int check_source(jpgenc_ctx* c, PixelSource* s, uint32_t w, uint32_t h) {
     const int f = s->format;
     if ((f < JPGENC_PIXEL_RGB || f > JPGENC_PIXEL_BGRA) && f != JPGENC_PIXEL_GRAY && f != kPixelPlanar && !is_yuv(f))
         return fail(c, JPGENC_ERR_ARG, "unknown pixel format");
+    const bool semi = f == kPixelNV12 || f == kPixelNV16;
     for (uint32_t k = 0; k < source_planes(f); ++k)
-        if (!s->plane[k] && !(f == kPixelNV12 && k == 2)) return fail(c, JPGENC_ERR_ARG, "null plane pointer");
-    if (f == kPixelNV12 && s->plane[2]) return fail(c, JPGENC_ERR_ARG, "NV12 takes its UV plane as u; v must be NULL");
+        if (!s->plane[k] && !(semi && k == 2)) return fail(c, JPGENC_ERR_ARG, "null plane pointer");
+    if (semi && s->plane[2]) return fail(c, JPGENC_ERR_ARG, "NV12 / NV16 take their UV plane as u; v must be NULL");
+    if (is_packed_yuv(f) && (s->plane[1] || s->plane[2] || s->pitch2))
+        return fail(c, JPGENC_ERR_ARG, "YUYV / UYVY take one packed plane as y; u and v must be NULL and c_pitch 0");
     if (w == 0 || h == 0 || w > 65535 || h > 65535) return fail(c, JPGENC_ERR_ARG, "image side out of range (1..65535)");
-    const uint32_t row = w * pixel_bytes(f);
+    const uint32_t row = row_bytes(f, w);
     if (s->pitch == 0) s->pitch = row;
     if (s->pitch < row) return fail(c, JPGENC_ERR_ARG, "row pitch below the row size");
     if (f == kPixelPlanar) s->pitch2 = s->pitch;
-    if (is_yuv(f)) {
+    if (is_yuv(f) && !is_packed_yuv(f)) {
         const uint32_t crow = chroma_row_bytes(f, w);
         if (s->pitch2 == 0) s->pitch2 = crow;
         if (s->pitch2 < crow) return fail(c, JPGENC_ERR_ARG, "chroma pitch below the chroma row size");
@@ -105,9 +108,10 @@ bool source_within_maxval(const PixelSource& s, uint32_t w, uint32_t h, uint32_t
     return true;
 }
 
-PixelSource yuv420_source(const void* y, const void* u, const void* v, uint32_t y_pitch, uint32_t c_pitch, int layout) {
+PixelSource yuv_source(const void* y, const void* u, const void* v, uint32_t y_pitch, uint32_t c_pitch, int layout) {
+    static_assert(kPixelI420 + JPGENC_YUV_UYVY == kPixelUYVY && kPixelI420 + JPGENC_YUV_NV16 == kPixelNV16, "JPGENC_YUV_* follow the formats");
     PixelSource s;
-    s.format = layout == JPGENC_YUV_I420 ? kPixelI420 : layout == JPGENC_YUV_NV12 ? kPixelNV12 : -1;
+    s.format = layout >= JPGENC_YUV_I420 && layout <= JPGENC_YUV_UYVY ? kPixelI420 + layout : -1;
     s.pitch = y_pitch;
     s.pitch2 = c_pitch;
     s.plane[0] = static_cast<const uint8_t*>(y); s.plane[1] = static_cast<const uint8_t*>(u); s.plane[2] = static_cast<const uint8_t*>(v);
@@ -132,14 +136,14 @@ PixelSource image_source(const void* px, uint32_t pitch, int format) {
 
 uint32_t staged_planes(const PixelSource& s, uint32_t w, uint32_t h, StagedPlane pl[3]) {
     const bool yuv = is_yuv(s.format);
-    const uint32_t np = s.format == kPixelNV12 ? 2u : source_planes(s.format);
+    const uint32_t np = s.format == kPixelNV12 || s.format == kPixelNV16 ? 2u : source_planes(s.format);
     size_t off = 0;
     for (uint32_t k = 0; k < np; ++k) {
         const bool chroma = yuv && k > 0;
         pl[k].host = s.plane[k];
         pl[k].pitch = chroma ? s.pitch2 : s.pitch;
-        pl[k].row = chroma ? chroma_row_bytes(s.format, w) : static_cast<size_t>(w) * pixel_bytes(s.format);
-        pl[k].vsub = chroma ? 1u : 0u;
+        pl[k].row = chroma ? chroma_row_bytes(s.format, w) : row_bytes(s.format, w);
+        pl[k].vsub = chroma ? chroma_vsub(s.format) : 0u;
         pl[k].rows = (h + pl[k].vsub) >> pl[k].vsub;
         pl[k].dev_off = off;
         off += pl[k].row * pl[k].rows;
@@ -151,7 +155,10 @@ uint32_t staged_planes(const PixelSource& s, uint32_t w, uint32_t h, StagedPlane
 size_t staged_bytes(const StagedPlane* pl, uint32_t np) { return pl[np - 1].dev_off + pl[np - 1].row * pl[np - 1].rows; }
 
 size_t planes_gap(const StagedPlane* pl, uint32_t np) {
-    if (np != 3 || pl[1].vsub || pl[0].pitch != pl[0].row) return 0;
+    // (planes of one row size, tight rows, and device planes as far apart as a plane is long: planar RGB and tight I444 planes)
+    if (np != 3 || pl[1].vsub || pl[0].pitch != pl[0].row || pl[1].row != pl[0].row || pl[1].pitch != pl[1].row ||
+        pl[1].dev_off != pl[0].row * pl[0].rows)
+        return 0;
     const uintptr_t gap = reinterpret_cast<uintptr_t>(pl[1].host) - reinterpret_cast<uintptr_t>(pl[0].host);
     const bool equal = reinterpret_cast<uintptr_t>(pl[2].host) - reinterpret_cast<uintptr_t>(pl[1].host) == gap;
     return equal && gap >= pl[0].row * pl[0].rows && gap <= (uintptr_t{1} << 48) ? gap : 0;
@@ -497,10 +504,17 @@ int jpgenc_bind_device_planar(jpgenc_ctx* c, const void* r, const void* g, const
     return bind_source(c, planar_source(r, g, b, row_pitch), w, h, maxval);
 } JPGENC_CATCH(c)
 
+int jpgenc_bind_device_yuv(jpgenc_ctx* c, const void* y, const void* u, const void* v, uint32_t w, uint32_t h, uint32_t y_pitch,
+                           uint32_t c_pitch, int layout) try {
+    if (!c) return JPGENC_ERR_ARG;
+    return bind_source(c, yuv_source(y, u, v, y_pitch, c_pitch, layout), w, h, 255);
+} JPGENC_CATCH(c)
+
 int jpgenc_bind_device_yuv420(jpgenc_ctx* c, const void* y, const void* u, const void* v, uint32_t w, uint32_t h, uint32_t y_pitch,
                               uint32_t c_pitch, int layout) try {
     if (!c) return JPGENC_ERR_ARG;
-    return bind_source(c, yuv420_source(y, u, v, y_pitch, c_pitch, layout), w, h, 255);
+    if (!is_yuv420_layout(layout)) return fail(c, JPGENC_ERR_ARG, "unknown YUV 4:2:0 layout");
+    return jpgenc_bind_device_yuv(c, y, u, v, w, h, y_pitch, c_pitch, layout);
 } JPGENC_CATCH(c)
 
 static int enqueue_forward(jpgenc_ctx* c);
@@ -1151,10 +1165,17 @@ int jpgenc_encode_planar(jpgenc_ctx* c, const void* r, const void* g, const void
     return encode_host_source(c, planar_source(r, g, b, row_pitch), w, h, maxval, dst, cap, jpeg_bytes);
 } JPGENC_CATCH(c)
 
+int jpgenc_encode_yuv(jpgenc_ctx* c, const void* y, const void* u, const void* v, uint32_t w, uint32_t h, uint32_t y_pitch,
+                      uint32_t c_pitch, int layout, uint8_t* dst, uint64_t cap, uint64_t* jpeg_bytes) try {
+    if (!c) return JPGENC_ERR_ARG;
+    return encode_host_source(c, yuv_source(y, u, v, y_pitch, c_pitch, layout), w, h, 255, dst, cap, jpeg_bytes);
+} JPGENC_CATCH(c)
+
 int jpgenc_encode_yuv420(jpgenc_ctx* c, const void* y, const void* u, const void* v, uint32_t w, uint32_t h, uint32_t y_pitch,
                          uint32_t c_pitch, int layout, uint8_t* dst, uint64_t cap, uint64_t* jpeg_bytes) try {
     if (!c) return JPGENC_ERR_ARG;
-    return encode_host_source(c, yuv420_source(y, u, v, y_pitch, c_pitch, layout), w, h, 255, dst, cap, jpeg_bytes);
+    if (!is_yuv420_layout(layout)) return fail(c, JPGENC_ERR_ARG, "unknown YUV 4:2:0 layout");
+    return jpgenc_encode_yuv(c, y, u, v, w, h, y_pitch, c_pitch, layout, dst, cap, jpeg_bytes);
 } JPGENC_CATCH(c)
 
 // Image::writeJPEG for an image that is not (or no longer) a set of 8-bit samples: planes a caller edited after loadPPM,

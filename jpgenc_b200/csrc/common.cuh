@@ -59,27 +59,45 @@ constexpr int kPixelPlanar = 17;
 // chroma planes of ceil(w/2) x ceil(h/2) samples -- U and V apart (I420) or interleaved U, V pairs (NV12)
 constexpr int kPixelI420 = 18;
 constexpr int kPixelNV12 = 19;
-__host__ __device__ constexpr bool is_yuv(int format) { return format == kPixelI420 || format == kPixelNV12; }
+// YUV 4:2:2 and 4:4:4 frames (jpgenc_*_yuv; JPGENC_YUV_I422 .. JPGENC_YUV_UYVY): chroma of ceil(w/2) x h samples -- U and V apart
+// (I422) or interleaved U, V pairs (NV16) --, of w x h samples (I444), or 4:2:2 packed into the Y plane as groups of two pixels
+// Y0 U Y1 V (YUYV) or U Y0 V Y1 (UYVY)
+constexpr int kPixelI422 = 20;
+constexpr int kPixelNV16 = 21;
+constexpr int kPixelI444 = 22;
+constexpr int kPixelYUYV = 23;
+constexpr int kPixelUYVY = 24;
+__host__ __device__ constexpr bool is_yuv(int format) { return format >= kPixelI420 && format <= kPixelUYVY; }
+__host__ __device__ constexpr bool is_packed_yuv(int format) { return format == kPixelYUYV || format == kPixelUYVY; }
+// chroma subsampling of a YUV format: vertical (4:2:0) and horizontal (all but 4:4:4), as shifts
+__host__ __device__ constexpr uint32_t chroma_vsub(int format) { return format == kPixelI420 || format == kPixelNV12 ? 1u : 0u; }
+__host__ __device__ constexpr uint32_t chroma_hsub(int format) { return format == kPixelI444 ? 0u : 1u; }
 
-// bytes of one chroma row of a YUV 4:2:0 image w pixels wide (NV12: U, V pairs)
-__host__ __device__ constexpr uint32_t chroma_row_bytes(int format, uint32_t w) { return (w + 1) / 2 * (format == kPixelNV12 ? 2u : 1u); }
-
-// bytes per pixel of a JPGENC_PIXEL_* format (planar: of one plane; YUV: of the Y plane)
-__host__ __device__ constexpr uint32_t pixel_bytes(int format) {
-    return format >= JPGENC_PIXEL_GRAY ? 1u : format >= JPGENC_PIXEL_RGBA ? 4u : 3u;
+// bytes of one chroma row of a YUV image w pixels wide (NV12 / NV16: U, V pairs; packed formats have no chroma plane)
+__host__ __device__ constexpr uint32_t chroma_row_bytes(int format, uint32_t w) {
+    return is_packed_yuv(format) ? 0u : format == kPixelI444 ? w : (w + 1) / 2 * (format == kPixelNV12 || format == kPixelNV16 ? 2u : 1u);
 }
+
+// bytes per pixel of a JPGENC_PIXEL_* format (planar: of one plane; YUV: of the Y plane, 2 for packed 4:2:2)
+__host__ __device__ constexpr uint32_t pixel_bytes(int format) {
+    return is_packed_yuv(format) ? 2u : format >= JPGENC_PIXEL_GRAY ? 1u : format >= JPGENC_PIXEL_RGBA ? 4u : 3u;
+}
+// bytes of one row of the first plane (packed 4:2:2: whole groups of two pixels, 4 ceil(w/2))
+__host__ __device__ constexpr uint32_t row_bytes(int format, uint32_t w) { return is_packed_yuv(format) ? (w + 1) / 2 * 4 : w * pixel_bytes(format); }
 
 // Where an image's bytes are and how they are laid out: up to three planes, the format, the row pitch of the first plane and
 // a second pitch (YUV: of the chroma planes; planar RGB: equal to `pitch`; unused otherwise).  Tight RGB is {{p}, RGB, w * 3,
-// 0}.  Planar RGB: planes R, G, B; YUV: Y, U, V (NV12: Y, UV, null).
+// 0}.  Planar RGB: planes R, G, B; YUV: Y, U, V (NV12 / NV16: Y, UV, null; YUYV / UYVY: the packed plane, null, null).
 struct PixelSource {
     const uint8_t* plane[3] = {nullptr, nullptr, nullptr};
-    int format = JPGENC_PIXEL_RGB;        // JPGENC_PIXEL_*, kPixelPlanar, kPixelI420 or kPixelNV12
+    int format = JPGENC_PIXEL_RGB;        // JPGENC_PIXEL_*, kPixelPlanar or kPixelI420 .. kPixelUYVY
     uint32_t pitch = 0;
     uint32_t pitch2 = 0;
 };
 // pointers (= planes) a caller passes for an image of this format
-__host__ __device__ constexpr uint32_t source_planes(int format) { return format == kPixelPlanar || is_yuv(format) ? 3u : 1u; }
+__host__ __device__ constexpr uint32_t source_planes(int format) {
+    return format == kPixelPlanar || (is_yuv(format) && !is_packed_yuv(format)) ? 3u : 1u;
+}
 
 // the second and third plane of one image of a pass and its second pitch: one entry per image follows the FrameGeom array in
 // the same copy for the formats of several planes (planar RGB, YUV)
@@ -151,7 +169,7 @@ struct ForwardParams {
 struct MixedPass {
     bool on = false;
     bool aligned = false;                 // every image has real_w % 16 == 0 and a 16-byte aligned pointer (K1's bulk copies)
-    int format = -1;                      // JPGENC_PIXEL_*, kPixelPlanar, kPixelI420 or kPixelNV12: the pixel-layout kernels (with
+    int format = -1;                      // JPGENC_PIXEL_*, kPixelPlanar or kPixelI420 .. kPixelUYVY: the pixel-layout kernels (with
                                           // FrameGeom::pitch and, for several planes, ExtraPlanes); -1 tight RGB
     uint32_t blocks = 0, strips = 0, tiles = 0, groups = 0, supers = 0;
     uint32_t split = 1;                   // K3 ranges per K2 tile, one choice for the whole pass (launch_entropy)

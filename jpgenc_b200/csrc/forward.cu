@@ -442,26 +442,33 @@ __device__ __forceinline__ void stage_planes(const ForwardParams& p, ForwardSmem
     __syncthreads();
 }
 
-// Staging of YUV 4:2:0 frames: the tile holds the strip's 16 Y rows of kMcus * 16 bytes (8 KB at kMcus 32) and behind them its
-// 8 chroma rows, in the source's own layout: I420 a U and a V plane of rows of kMcus * 8 bytes, NV12 one plane of rows of
-// kMcus * 16 (U, V) bytes -- 12 KB in all, half the tile.  Each CTA picks its path from its own image:
-//  * every plane's base and pitch 16-byte aligned, real_w % 16 == 0 (so no chroma row needs padding either) and, for I420, an
-//    even number of MCUs (a bulk copy moves whole 16-byte units): one bulk copy per plane row (24 / 32 per CTA);
+// Staging of YUV frames: the tile holds the strip's 16 rows of the first plane and behind them its chroma rows, in the source's own
+// layout.  kCRows chroma rows per MCU row (8 for 4:2:0, 16 for 4:2:2 and 4:4:4), kMcuC chroma bytes of one MCU in one row:
+//  * I420 / NV12: 16 Y rows of kMcus * 16 bytes (8 KB at kMcus 32) and 8 chroma rows, U and V planes of rows of kMcus * 8 bytes
+//    (I420) or one plane of rows of kMcus * 16 (U, V) bytes (NV12): 12 KB in all;
+//  * I422 / NV16: 16 Y rows and 16 chroma rows of the same sizes: 16 KB;  I444: three planes of 16 rows of kMcus * 16 bytes: 24 KB;
+//  * YUYV / UYVY: one plane of 16 rows of kMcus * 32 bytes (two bytes per pixel, the chroma inside): 16 KB.
+// Each CTA picks its path from its own image:
+//  * every plane's base and pitch 16-byte aligned, real_w % 16 == 0 (so no row needs padding either) and, with 8 chroma bytes
+//    per MCU, an even number of MCUs (a bulk copy moves whole 16-byte units): one bulk copy per plane row (16 to 48 per CTA);
 //  * otherwise 16-byte chunks, per plane: a vector load where the chunk lies inside the plane's row and the plane is aligned,
-//    clamped byte loads elsewhere (edge replication, each plane clamped to its own size; NV12 clamps whole U, V pairs).
+//    clamped byte loads elsewhere (edge replication, each plane clamped to its own size; NV12 / NV16 clamp whole U, V pairs, the
+//    packed layouts clamp a pixel's Y to the last pixel and its U, V to the last group).
 // The L2 prefetch of the strip `prefetch_ahead` CTAs later covers every plane.
 template <int kMcus, int kFmt, bool kMixed>
 __device__ __forceinline__ void stage_yuv(const ForwardParams& p, ForwardSmem<kMcus>& sm, int tid, const StripImage& s, int nm) {
-    constexpr bool kNV12 = kFmt == kPixelNV12;
-    constexpr int kThreads = kMcus * 4, kRow = kMcus * 16, kCRow = kNV12 ? kMcus * 16 : kMcus * 8, kCPlanes = kNV12 ? 1 : 2;
-    constexpr int kMcuC = kNV12 ? 16 : 8;                                  // chroma bytes of one MCU in one row
-    static_assert(16 * kRow + kCPlanes * 8 * kCRow <= ForwardSmem<kMcus>::kTileBytes, "the planes fit the tile");
+    constexpr bool kPacked = is_packed_yuv(kFmt), kSemi = kFmt == kPixelNV12 || kFmt == kPixelNV16;
+    constexpr int kYB = kPacked ? 32 : 16;                                 // bytes of one MCU in one row of the first plane
+    constexpr int kMcuC = kSemi || kFmt == kPixelI444 ? 16 : 8;           // chroma bytes of one MCU in one row
+    constexpr int kCRows = chroma_vsub(kFmt) ? 8 : 16, kCPlanes = kPacked ? 0 : kSemi ? 1 : 2;
+    constexpr int kThreads = kMcus * 4, kRow = kMcus * kYB, kCRow = kMcus * kMcuC, kRows = 16 + kCRows * kCPlanes;
+    static_assert(16 * kRow + kCPlanes * kCRows * kCRow <= ForwardSmem<kMcus>::kTileBytes, "the planes fit the tile");
     const uint8_t *y = s.src.plane[0], *u = s.src.plane[1], *v = s.src.plane[2];
     const uint32_t y_pitch = s.src.pitch, c_pitch = s.src.pitch2, real_w = s.real_w, real_h = s.real_h, my = s.my, mcu0 = s.mcu0;
-    const uint32_t cw_bytes = ((real_w + 1) / 2) * (kNV12 ? 2 : 1), ch = (real_h + 1) / 2;
+    const uint32_t cw_bytes = chroma_row_bytes(kFmt, real_w), ch = kCRows == 8 ? (real_h + 1) / 2 : real_h;
     const bool y_aligned = ((reinterpret_cast<uintptr_t>(y) | y_pitch) & 15) == 0;
-    const bool c_aligned = ((reinterpret_cast<uintptr_t>(u) | (kNV12 ? 0 : reinterpret_cast<uintptr_t>(v)) | c_pitch) & 15) == 0;
-    const bool bulk = y_aligned && c_aligned && real_w % 16 == 0 && (kNV12 || nm % 2 == 0);   // the same for every thread of the CTA
+    const bool c_aligned = kPacked || ((reinterpret_cast<uintptr_t>(u) | (kCPlanes == 1 ? 0 : reinterpret_cast<uintptr_t>(v)) | c_pitch) & 15) == 0;
+    const bool bulk = y_aligned && c_aligned && real_w % 16 == 0 && (kMcuC == 16 || nm % 2 == 0);   // the same for every thread of the CTA
     uint8_t* const ctile = sm.tile + 16 * kRow;
     if (bulk) {
         if (tid == 0) {
@@ -469,15 +476,15 @@ __device__ __forceinline__ void stage_yuv(const ForwardParams& p, ForwardSmem<kM
             ptx::mbar_init_fence();
         }
         __syncthreads();
-        if (tid < 16 + 8 * kCPlanes) {
-            if (tid == 0) ptx::mbar_expect_tx(&sm.bar, 16 * nm * 16 + kCPlanes * 8 * nm * kMcuC);
+        if (tid < kRows) {
+            if (tid == 0) ptx::mbar_expect_tx(&sm.bar, 16 * nm * kYB + kCPlanes * kCRows * nm * kMcuC);
             if (tid < 16) {
                 const uint32_t sy = min(my * 16 + tid, real_h - 1);
-                ptx::bulk_g2s(sm.tile + tid * kRow, y + static_cast<size_t>(sy) * y_pitch + mcu0 * 16, nm * 16, &sm.bar);
+                ptx::bulk_g2s(sm.tile + tid * kRow, y + static_cast<size_t>(sy) * y_pitch + mcu0 * kYB, nm * kYB, &sm.bar);
             } else {
-                const int k = (tid - 16) >> 3, r = (tid - 16) & 7;
-                const uint32_t sy = min(my * 8 + r, ch - 1);
-                ptx::bulk_g2s(ctile + (k * 8 + r) * kCRow, (k ? v : u) + static_cast<size_t>(sy) * c_pitch + mcu0 * kMcuC, nm * kMcuC, &sm.bar);
+                const int k = (tid - 16) >> (kCRows == 8 ? 3 : 4), r = (tid - 16) & (kCRows - 1);
+                const uint32_t sy = min(my * kCRows + r, ch - 1);
+                ptx::bulk_g2s(ctile + (k * kCRows + r) * kCRow, (k ? v : u) + static_cast<size_t>(sy) * c_pitch + mcu0 * kMcuC, nm * kMcuC, &sm.bar);
             }
         }
     }
@@ -485,15 +492,22 @@ __device__ __forceinline__ void stage_yuv(const ForwardParams& p, ForwardSmem<kM
         StripImage a;
         // whole 16-byte units inside the rows only (the range must not pass the end of a row): real_w % 16 == 0 makes every
         // plane's strip end on its row's end
-        const int i = tid - 32;
-        if (ahead_image<kMcus, kMixed, kFmt>(p, a) && a.real_w % 16 == 0 && i < 16 + 8 * kCPlanes) {
-            const uint8_t* src = a.src.plane[i < 16 ? 0 : i < 24 ? 1 : 2];
-            const uint32_t pitch = i < 16 ? a.src.pitch : a.src.pitch2;
-            if (((reinterpret_cast<uintptr_t>(src) | pitch) & 15) == 0) {
-                const uint32_t pnm = min(static_cast<uint32_t>(kMcus), a.mcu_w - a.mcu0);
-                const uint32_t sy = i < 16 ? min(a.my * 16 + i, a.real_h - 1) : min(a.my * 8 + ((i - 16) & 7), (a.real_h + 1) / 2 - 1);
-                const uint32_t x0 = i < 16 ? a.mcu0 * 16 : a.mcu0 * kMcuC, n = (i < 16 ? pnm * 16 : pnm * kMcuC) & ~15u;
-                if (n) ptx::bulk_prefetch_l2(src + static_cast<size_t>(sy) * pitch + x0, n);
+        // (one row per lane of the second warp, two for the 48 rows of I422 / I444)
+        if (ahead_image<kMcus, kMixed, kFmt>(p, a) && a.real_w % 16 == 0) {
+#pragma unroll
+            for (int j = 0; j < (kRows + 31) / 32; ++j) {
+                const int i = tid - 32 + 32 * j;
+                if (i < kRows) {
+                    const uint8_t* src = a.src.plane[i < 16 ? 0 : i < 16 + kCRows ? 1 : 2];
+                    const uint32_t pitch = i < 16 ? a.src.pitch : a.src.pitch2;
+                    if (((reinterpret_cast<uintptr_t>(src) | pitch) & 15) == 0) {
+                        const uint32_t pnm = min(static_cast<uint32_t>(kMcus), a.mcu_w - a.mcu0);
+                        const uint32_t sy = i < 16 ? min(a.my * 16 + i, a.real_h - 1)
+                                                   : min(a.my * kCRows + ((i - 16) & (kCRows - 1)), (kCRows == 8 ? (a.real_h + 1) / 2 : a.real_h) - 1);
+                        const uint32_t x0 = i < 16 ? a.mcu0 * kYB : a.mcu0 * kMcuC, n = (i < 16 ? pnm * kYB : pnm * kMcuC) & ~15u;
+                        if (n) ptx::bulk_prefetch_l2(src + static_cast<size_t>(sy) * pitch + x0, n);
+                    }
+                }
             }
         }
     }
@@ -501,7 +515,8 @@ __device__ __forceinline__ void stage_yuv(const ForwardParams& p, ForwardSmem<kM
         ptx::mbar_wait(&sm.bar, 0);
         return;
     }
-    // one plane: `rows` rows of `chunks` 16-byte chunks from x0 on; es: bytes of one sample (NV12 chroma: a U, V pair)
+    // one plane: `rows` rows of `chunks` 16-byte chunks from x0 on; es: bytes of one sample (NV12 / NV16 chroma: a U, V pair).  A
+    // chunk that ends past `width` takes clamped byte loads.
     auto stage_plane = [&](const uint8_t* src, uint32_t pitch, bool aligned, uint32_t row0, uint32_t last_row, uint32_t width, uint32_t es,
                            uint32_t x0, int rows, int chunks, uint8_t* dst, int dst_row) {
         for (int i = tid; i < rows * chunks; i += kThreads) {
@@ -518,7 +533,21 @@ __device__ __forceinline__ void stage_yuv(const ForwardParams& p, ForwardSmem<kM
                     uint32_t word = 0;
 #pragma unroll
                     for (int t = 0; t < 4; ++t) {
-                        const uint32_t xx = x + 4 * j + t, sx = xx < width ? xx : width - es + (xx & (es - 1));
+                        const uint32_t xx = x + 4 * j + t;
+                        uint32_t sx;
+                        if constexpr (kPacked) {
+                            // byte xx of the packed row: a Y sample of pixel 2g + k (group g = xx / 4) or the U / V of group g
+                            constexpr uint32_t kYOff = kFmt == kPixelYUYV ? 0 : 1;
+                            const uint32_t g = xx >> 2, pos = xx & 3;
+                            if ((pos & 1) == kYOff) {
+                                const uint32_t px = min(2 * g + (pos >> 1), real_w - 1);
+                                sx = (px >> 1) * 4 + (px & 1) * 2 + kYOff;
+                            } else {
+                                sx = min(g, (real_w - 1) >> 1) * 4 + pos;
+                            }
+                        } else {
+                            sx = xx < width ? xx : width - es + (xx & (es - 1));
+                        }
                         word |= static_cast<uint32_t>(row[sx]) << (8 * t);
                     }
                     b[j] = word;
@@ -528,10 +557,14 @@ __device__ __forceinline__ void stage_yuv(const ForwardParams& p, ForwardSmem<kM
             *reinterpret_cast<uint4*>(dst + r * dst_row + m * 16) = q;
         }
     };
-    stage_plane(y, y_pitch, y_aligned, my * 16, real_h - 1, real_w, 1, mcu0 * 16, 16, nm, sm.tile, kRow);
-    const int cchunks = (nm * kMcuC + 15) / 16;                             // I420, odd nm: the last chunk's upper half is not read
-    stage_plane(u, c_pitch, c_aligned, my * 8, ch - 1, cw_bytes, kNV12 ? 2 : 1, mcu0 * kMcuC, 8, cchunks, ctile, kCRow);
-    if constexpr (!kNV12) stage_plane(v, c_pitch, c_aligned, my * 8, ch - 1, cw_bytes, 1, mcu0 * kMcuC, 8, cchunks, ctile + 8 * kCRow, kCRow);
+    // (packed: a chunk lies inside the row when its 8 pixels are inside the image; for odd widths the last group's second Y is not)
+    stage_plane(y, y_pitch, y_aligned, my * 16, real_h - 1, kPacked ? 2 * real_w : real_w, 1, mcu0 * kYB, 16, kPacked ? 2 * nm : nm, sm.tile, kRow);
+    if constexpr (kCPlanes > 0) {
+        const int cchunks = (nm * kMcuC + 15) / 16;                         // 8 bytes per MCU, odd nm: the last chunk's upper half is not read
+        stage_plane(u, c_pitch, c_aligned, my * kCRows, ch - 1, cw_bytes, kSemi ? 2 : 1, mcu0 * kMcuC, kCRows, cchunks, ctile, kCRow);
+        if constexpr (kCPlanes == 2)
+            stage_plane(v, c_pitch, c_aligned, my * kCRows, ch - 1, cw_bytes, 1, mcu0 * kMcuC, kCRows, cchunks, ctile + kCRows * kCRow, kCRow);
+    }
     __syncthreads();
 }
 
@@ -539,7 +572,7 @@ __device__ __forceinline__ void stage_yuv(const ForwardParams& p, ForwardSmem<kM
 // byte loader fills the tile (odd sizes; right-edge replication, src/Image.cpp:491-530)
 // kMixed: images of individual sizes (p.geom): a 1-D grid over the strips of all images; a CTA finds its image by a search
 // over the first-strip prefix.  Otherwise one size: grid (strips of a row, rows, frames).
-// kFmt >= 0: pixels in that JPGENC_PIXEL_* format with a row pitch (stage_layout; grey and planar RGB: stage_planes; YUV 4:2:0:
+// kFmt >= 0: pixels in that JPGENC_PIXEL_* format with a row pitch (stage_layout; grey and planar RGB: stage_planes; YUV:
 // stage_yuv; kAligned is not used); -1: tight RGB
 template <int kMcus, bool kAligned, bool kBulkOut, bool kMixed, int kFmt = -1>
 // (shared memory and the thread index come from the kernel: there the compiler knows the alignment and, from the launch
@@ -550,6 +583,7 @@ __device__ __forceinline__ void forward_body(const ForwardParams& p, ForwardSmem
     const int tid = thread;
     constexpr bool kPlanar = kFmt == kPixelPlanar, kPlaneTile = kPlanar || kFmt == JPGENC_PIXEL_GRAY;   // stage_planes
     constexpr bool kYuv = is_yuv(kFmt), kNV12 = kFmt == kPixelNV12;                                // stage_yuv
+    constexpr bool kYuv420 = kYuv && chroma_vsub(kFmt), kPacked = is_packed_yuv(kFmt);
     const StripImage s = strip_image<kMcus, kMixed, kFmt>(p, ThisCta{});
     const uint8_t* __restrict__ rgb = s.src.plane[0];
     const uint32_t my = s.my, mcu0 = s.mcu0, frame_block0 = s.block0, real_w = s.real_w, real_h = s.real_h, mcu_w = s.mcu_w;
@@ -616,7 +650,7 @@ __device__ __forceinline__ void forward_body(const ForwardParams& p, ForwardSmem
     const bool active = (bx >> 1) < nm;
     f2 v[32];                                     // v[r*4+p] = samples (r, 2p) and (r, 2p+1)
     constexpr int kR = (kFmt == JPGENC_PIXEL_BGR || kFmt == JPGENC_PIXEL_BGRA) ? 2 : 0, kB = 2 - kR;   // tile bytes of R and B
-    if constexpr (kYuv) {
+    if constexpr (kYuv420) {
         if (active) {
             // The samples themselves, level-shifted: no colour conversion and no 2x2 means.  The chroma sample of an MCU position
             // is the stored one: the reference's S420_m averages four equal values there ((a + a) + (a + a), then / 4, gives
@@ -649,6 +683,92 @@ __device__ __forceinline__ void forward_body(const ForwardParams& p, ForwardSmem
                 const uint32_t w[2] = {q.x, q.y};
 #pragma unroll
                 for (int pp = 0; pp < 4; ++pp) v[r * 4 + pp] = bytes_to_f2_centred(w, 2 * pp, 2 * pp + 1);
+            }
+        }
+    } else if constexpr (kYuv) {
+        if (active) {
+            // 4:2:2 and 4:4:4: level-shifted samples, no colour conversion; the chroma of a 2x2 cell is the mean of its four samples
+            // as S420_m takes it (see exact_sample).  4:2:2: the two pixels of a cell share a sample, so the mean is that of the
+            // cell's two rows, (a + b) * 0.5; 4:4:4: 2x2 sums * 0.25.  Small integers and halves / quarters of them: exact in FP32.
+            constexpr int kRow = kMcus * (kPacked ? 32 : 16);
+            constexpr int kCRow = kMcus * (kFmt == kPixelI422 ? 8 : 16);
+            const uint8_t* ctile = sm.tile + 16 * kRow;
+#pragma unroll
+            for (int rp = 0; rp < 4; ++rp) {          // chroma row by * 4 + rp = tile rows r0, r0 + 1; columns bx * 4 .. bx * 4 + 3
+                const int r0 = by * 8 + rp * 2;
+                f2 cb[2], crr[2];
+                if constexpr (kPacked) {
+                    // a row's 16 bytes: the thread's 8 pixels as 4 groups, Y0 U Y1 V (YUYV) or U Y0 V Y1 (UYVY)
+                    constexpr int kY = kFmt == kPixelYUYV ? 0 : 1, kU = 1 - kY, kV = kU + 2;
+                    const uint4 q0 = *reinterpret_cast<const uint4*>(sm.tile + r0 * kRow + bx * 16);
+                    const uint4 q1 = *reinterpret_cast<const uint4*>(sm.tile + (r0 + 1) * kRow + bx * 16);
+                    const uint32_t w0[4] = {q0.x, q0.y, q0.z, q0.w}, w1[4] = {q1.x, q1.y, q1.z, q1.w};
+#pragma unroll
+                    for (int pp = 0; pp < 4; ++pp) {
+                        v[(rp * 2) * 4 + pp] = bytes_to_f2_centred(w0, 4 * pp + kY, 4 * pp + 2 + kY);
+                        v[(rp * 2 + 1) * 4 + pp] = bytes_to_f2_centred(w1, 4 * pp + kY, 4 * pp + 2 + kY);
+                    }
+#pragma unroll
+                    for (int j = 0; j < 2; ++j) {             // groups 2j, 2j + 1
+                        cb[j] = __fmul2_rn(add2(bytes_to_f2_centred(w0, 8 * j + kU, 8 * j + 4 + kU), bytes_to_f2_centred(w1, 8 * j + kU, 8 * j + 4 + kU)),
+                                           make_float2(0.5f, 0.5f));
+                        crr[j] = __fmul2_rn(add2(bytes_to_f2_centred(w0, 8 * j + kV, 8 * j + 4 + kV), bytes_to_f2_centred(w1, 8 * j + kV, 8 * j + 4 + kV)),
+                                            make_float2(0.5f, 0.5f));
+                    }
+                } else if constexpr (kFmt == kPixelI422) {
+                    const uint32_t u0[1] = {*reinterpret_cast<const uint32_t*>(ctile + r0 * kCRow + bx * 4)};
+                    const uint32_t u1[1] = {*reinterpret_cast<const uint32_t*>(ctile + (r0 + 1) * kCRow + bx * 4)};
+                    const uint32_t v0[1] = {*reinterpret_cast<const uint32_t*>(ctile + (16 + r0) * kCRow + bx * 4)};
+                    const uint32_t v1[1] = {*reinterpret_cast<const uint32_t*>(ctile + (17 + r0) * kCRow + bx * 4)};
+#pragma unroll
+                    for (int j = 0; j < 2; ++j) {
+                        cb[j] = __fmul2_rn(add2(bytes_to_f2_centred(u0, 2 * j, 2 * j + 1), bytes_to_f2_centred(u1, 2 * j, 2 * j + 1)), make_float2(0.5f, 0.5f));
+                        crr[j] = __fmul2_rn(add2(bytes_to_f2_centred(v0, 2 * j, 2 * j + 1), bytes_to_f2_centred(v1, 2 * j, 2 * j + 1)), make_float2(0.5f, 0.5f));
+                    }
+                } else if constexpr (kFmt == kPixelNV16) {
+                    const uint2 q0 = *reinterpret_cast<const uint2*>(ctile + r0 * kCRow + bx * 8);          // U V U V U V U V
+                    const uint2 q1 = *reinterpret_cast<const uint2*>(ctile + (r0 + 1) * kCRow + bx * 8);
+                    const uint32_t w0[2] = {q0.x, q0.y}, w1[2] = {q1.x, q1.y};
+#pragma unroll
+                    for (int j = 0; j < 2; ++j) {
+                        cb[j] = __fmul2_rn(add2(bytes_to_f2_centred(w0, 4 * j, 4 * j + 2), bytes_to_f2_centred(w1, 4 * j, 4 * j + 2)), make_float2(0.5f, 0.5f));
+                        crr[j] = __fmul2_rn(add2(bytes_to_f2_centred(w0, 4 * j + 1, 4 * j + 3), bytes_to_f2_centred(w1, 4 * j + 1, 4 * j + 3)),
+                                            make_float2(0.5f, 0.5f));
+                    }
+                } else {                                      // I444: 8 bytes per row and plane, 2x2 sums
+                    static_assert(kFmt == kPixelI444, "a YUV 4:2:2 / 4:4:4 layout");
+                    f2 c4[2][2];                              // [plane][j]: the sums of cells 2j, 2j + 1
+#pragma unroll
+                    for (int k = 0; k < 2; ++k) {
+                        const uint2 q0 = *reinterpret_cast<const uint2*>(ctile + (16 * k + r0) * kCRow + bx * 8);
+                        const uint2 q1 = *reinterpret_cast<const uint2*>(ctile + (16 * k + r0 + 1) * kCRow + bx * 8);
+                        const uint32_t w0[2] = {q0.x, q0.y}, w1[2] = {q1.x, q1.y};
+                        float s4[4];
+#pragma unroll
+                        for (int pp = 0; pp < 4; ++pp) {
+                            const f2 sc = add2(bytes_to_f2_centred(w0, 2 * pp, 2 * pp + 1), bytes_to_f2_centred(w1, 2 * pp, 2 * pp + 1));
+                            s4[pp] = sc.x + sc.y;
+                        }
+                        c4[k][0] = make_float2(s4[0], s4[1]);
+                        c4[k][1] = make_float2(s4[2], s4[3]);
+                    }
+#pragma unroll
+                    for (int j = 0; j < 2; ++j) {
+                        cb[j] = __fmul2_rn(c4[0][j], make_float2(0.25f, 0.25f));
+                        crr[j] = __fmul2_rn(c4[1][j], make_float2(0.25f, 0.25f));
+                    }
+                }
+                *reinterpret_cast<float4*>(&sm.chroma[0][by * 4 + rp][bx * 4]) = make_float4(cb[0].x, cb[0].y, cb[1].x, cb[1].y);
+                *reinterpret_cast<float4*>(&sm.chroma[1][by * 4 + rp][bx * 4]) = make_float4(crr[0].x, crr[0].y, crr[1].x, crr[1].y);
+            }
+            if constexpr (!kPacked) {
+#pragma unroll
+                for (int r = 0; r < 8; ++r) {
+                    const uint2 q = *reinterpret_cast<const uint2*>(sm.tile + (by * 8 + r) * kRow + bx * 8);
+                    const uint32_t w[2] = {q.x, q.y};
+#pragma unroll
+                    for (int pp = 0; pp < 4; ++pp) v[r * 4 + pp] = bytes_to_f2_centred(w, 2 * pp, 2 * pp + 1);
+                }
             }
         }
     } else if (active) {
@@ -838,9 +958,34 @@ __device__ __forceinline__ ExactColumn exact_locate(const uint8_t* rgb, uint32_t
 // clamped pixels map to one chroma sample a (x, x + 1 with x even, or both clamped to the last column; the same for rows) -- and
 // quarters the sum: every step is exact on these small integers and gives a again.  So the chroma sample of cell (x / 2, y / 2)
 // is U[min(y / 2, ch - 1)][min(x / 2, cw - 1)] - 128 (V for Cr; NV12: the pair's first / second byte).
+// YUV 4:2:2 and 4:4:4: the image whose level-shifted planes are the clamped bytes minus 128 at full resolution (a 4:2:2 chroma
+// sample at both pixels of its group); luma as above, chroma by S420_m over the four clamped pixels of the cell in the reference's
+// order, ((0 + p00) + p01) + ((0 + p10) + p11), times 0.25.
+template <int kFmt>
+__device__ __forceinline__ double exact_yuv_byte(const uint8_t* y, const PixelSource& s, uint32_t sx, uint32_t sy, int comp) {
+    if constexpr (is_packed_yuv(kFmt)) {                                   // group sx / 2: Y0 U Y1 V (YUYV) or U Y0 V Y1 (UYVY)
+        constexpr uint32_t kY = kFmt == kPixelYUYV ? 0 : 1;
+        const uint32_t at = (sx >> 1) * 4 + (comp == 0 ? kY + (sx & 1) * 2 : (1 - kY) + (comp - 1) * 2);
+        return dsub(static_cast<double>(y[static_cast<size_t>(sy) * s.pitch + at]), 128.0);
+    } else {
+        if (comp == 0) return dsub(static_cast<double>(y[static_cast<size_t>(sy) * s.pitch + sx]), 128.0);
+        const uint32_t cx = sx >> chroma_hsub(kFmt);
+        const size_t row = static_cast<size_t>(sy) * s.pitch2;
+        const uint8_t v = kFmt == kPixelNV16 ? s.plane[1][row + 2 * cx + (comp - 1)] : (comp == 1 ? s.plane[1] : s.plane[2])[row + cx];
+        return dsub(static_cast<double>(v), 128.0);
+    }
+}
+
 template <int kFmt>
 __device__ __forceinline__ double exact_sample(const ExactColumn& b, const PixelSource& s, uint32_t real_w, uint32_t real_h, int r, double scale) {
-    if constexpr (is_yuv(kFmt)) {
+    if constexpr (is_yuv(kFmt) && !chroma_vsub(kFmt)) {
+        if (b.comp == 0) return exact_yuv_byte<kFmt>(b.rgb, s, min(b.x, real_w - 1), min(b.y + r, real_h - 1), 0);
+        const uint32_t x0 = min(b.x, real_w - 1), x1 = min(b.x + 1, real_w - 1);
+        const uint32_t y = b.y + 2 * r, y0 = min(y, real_h - 1), y1 = min(y + 1, real_h - 1);
+        const double top = dadd(dadd(0.0, exact_yuv_byte<kFmt>(b.rgb, s, x0, y0, b.comp)), exact_yuv_byte<kFmt>(b.rgb, s, x1, y0, b.comp));
+        const double bot = dadd(dadd(0.0, exact_yuv_byte<kFmt>(b.rgb, s, x0, y1, b.comp)), exact_yuv_byte<kFmt>(b.rgb, s, x1, y1, b.comp));
+        return dmul(dadd(top, bot), 0.25);
+    } else if constexpr (is_yuv(kFmt)) {
         if (b.comp == 0) {
             const uint32_t sx = min(b.x, real_w - 1), sy = min(b.y + r, real_h - 1);
             return dsub(static_cast<double>(b.rgb[static_cast<size_t>(sy) * s.pitch + sx]), 128.0);
@@ -1271,20 +1416,31 @@ static void fill_forward_params(const jpgenc_ctx* c, ForwardParams* p) {
 }
 
 // calls f(std::integral_constant<int, format>) for an internal format, or -1 for tight RGB: the kernels take the format as a
-// template parameter
+// template parameter; false (and no call) for a code that is no format (check_source refuses those before anything is bound)
 template <class F>
-static void with_format(int format, F&& f) {
+static bool with_format(int format, F&& f) {
     switch (format) {
         case -1: f(std::integral_constant<int, -1>{}); break;
         case JPGENC_PIXEL_RGB: f(std::integral_constant<int, JPGENC_PIXEL_RGB>{}); break;
         case JPGENC_PIXEL_BGR: f(std::integral_constant<int, JPGENC_PIXEL_BGR>{}); break;
         case JPGENC_PIXEL_RGBA: f(std::integral_constant<int, JPGENC_PIXEL_RGBA>{}); break;
+        case JPGENC_PIXEL_BGRA: f(std::integral_constant<int, JPGENC_PIXEL_BGRA>{}); break;
         case JPGENC_PIXEL_GRAY: f(std::integral_constant<int, JPGENC_PIXEL_GRAY>{}); break;
         case kPixelPlanar: f(std::integral_constant<int, kPixelPlanar>{}); break;
         case kPixelI420: f(std::integral_constant<int, kPixelI420>{}); break;
         case kPixelNV12: f(std::integral_constant<int, kPixelNV12>{}); break;
-        default: f(std::integral_constant<int, JPGENC_PIXEL_BGRA>{}); break;
+        case kPixelI422: f(std::integral_constant<int, kPixelI422>{}); break;
+        case kPixelNV16: f(std::integral_constant<int, kPixelNV16>{}); break;
+        case kPixelI444: f(std::integral_constant<int, kPixelI444>{}); break;
+        case kPixelYUYV: f(std::integral_constant<int, kPixelYUYV>{}); break;
+        case kPixelUYVY: f(std::integral_constant<int, kPixelUYVY>{}); break;
+        default: return false;
     }
+    return true;
+}
+static int unknown_format(jpgenc_ctx* c) {
+    c->error = "internal: pixel format without kernels";
+    return JPGENC_ERR_ARG;
 }
 
 // the format the kernels of the single image bound take: its own, or -1 when it is tight RGB
@@ -1309,13 +1465,14 @@ static int launch_refine(jpgenc_ctx* c, bool all) {
     const uint32_t bpf = c->mcu_w * c->mcu_h * kBlocksPerMcu;
     const uint32_t cap = all ? 0u : static_cast<uint32_t>(c->refine_cap);
     const uint8_t* const* frames = c->nframes > 1 ? c->d_frame_ptrs : nullptr;
-    with_format(kernel_format(c), [&](auto fmt) {
-        with_refine_grid(c, static_cast<uint64_t>(bpf) * c->nframes, [&](auto k64, unsigned grid) {
-            refine_kernel<decltype(k64)::value, decltype(fmt)::value><<<grid, kRefineThreads, 0, c->stream>>>(
-                c->src.plane[0], frames, bpf, c->d_coef, c->d_refine_list, c->d_counters, cap, all ? 1 : 0, bpf * c->nframes, c->real_w, c->real_h, c->mcu_w, e,
-                c->src);
-        });
-    });
+    if (!with_format(kernel_format(c), [&](auto fmt) {
+            with_refine_grid(c, static_cast<uint64_t>(bpf) * c->nframes, [&](auto k64, unsigned grid) {
+                refine_kernel<decltype(k64)::value, decltype(fmt)::value><<<grid, kRefineThreads, 0, c->stream>>>(
+                    c->src.plane[0], frames, bpf, c->d_coef, c->d_refine_list, c->d_counters, cap, all ? 1 : 0, bpf * c->nframes, c->real_w, c->real_h, c->mcu_w,
+                    e, c->src);
+            });
+        }))
+        return unknown_format(c);
     JPGENC_CUDA(c, cudaGetLastError());
     c->launches += 1;
     return JPGENC_OK;
@@ -1340,13 +1497,14 @@ int launch_forward_rows(jpgenc_ctx* c, uint32_t y0, uint32_t rows, bool first, b
     if (kernel_format(c) >= 0) {
         // each CTA picks its staging path from the image (stage_layout); the tensor store serves every full strip
         const bool bulk = make_block_map(c->d_coef, static_cast<uint64_t>(c->mcu_w) * c->mcu_h * kBlocksPerMcu, 32 * kBlocksPerMcu, &p.coef_map);
-        with_format(c->src.format, [&](auto fmt) {
-            constexpr int kFmt = decltype(fmt)::value;
-            if constexpr (kFmt >= 0) {
-                if (bulk) forward_layout_kernel<32, kFmt, true><<<grid, 128, 0, c->stream>>>(p);
-                else forward_layout_kernel<32, kFmt, false><<<grid, 128, 0, c->stream>>>(p);
-            }
-        });
+        if (!with_format(c->src.format, [&](auto fmt) {
+                constexpr int kFmt = decltype(fmt)::value;
+                if constexpr (kFmt >= 0) {
+                    if (bulk) forward_layout_kernel<32, kFmt, true><<<grid, 128, 0, c->stream>>>(p);
+                    else forward_layout_kernel<32, kFmt, false><<<grid, 128, 0, c->stream>>>(p);
+                }
+            }))
+            return unknown_format(c);
         JPGENC_CUDA(c, cudaGetLastError());
         c->launches += 1;
         return last ? launch_refine(c, false) : JPGENC_OK;
@@ -1379,13 +1537,14 @@ int launch_forward_mixed(jpgenc_ctx* c) {
     p.extra = source_planes(c->mixed.format) == 3 ? reinterpret_cast<const ExtraPlanes*>(c->d_geom + c->nframes + 1) : nullptr;
     const bool bulk_out = (aligned || layout) && make_block_map(c->d_coef, c->mixed.blocks, 32 * kBlocksPerMcu, &p.coef_map);
     if (layout) {
-        with_format(c->mixed.format, [&](auto fmt) {
-            constexpr int kFmt = decltype(fmt)::value;
-            if constexpr (kFmt >= 0) {
-                if (bulk_out) forward_mixed_layout_kernel<32, kFmt, true><<<c->mixed.strips, 128, 0, c->stream>>>(p);
-                else forward_mixed_layout_kernel<32, kFmt, false><<<c->mixed.strips, 128, 0, c->stream>>>(p);
-            }
-        });
+        if (!with_format(c->mixed.format, [&](auto fmt) {
+                constexpr int kFmt = decltype(fmt)::value;
+                if constexpr (kFmt >= 0) {
+                    if (bulk_out) forward_mixed_layout_kernel<32, kFmt, true><<<c->mixed.strips, 128, 0, c->stream>>>(p);
+                    else forward_mixed_layout_kernel<32, kFmt, false><<<c->mixed.strips, 128, 0, c->stream>>>(p);
+                }
+            }))
+            return unknown_format(c);
     } else if (bulk_out) forward_mixed_kernel<32, true, true><<<c->mixed.strips, 128, 0, c->stream>>>(p);
     else if (aligned) forward_mixed_kernel<32, true, false><<<c->mixed.strips, 128, 0, c->stream>>>(p);
     else forward_mixed_kernel<32, false, false><<<c->mixed.strips, 128, 0, c->stream>>>(p);
@@ -1393,12 +1552,13 @@ int launch_forward_mixed(jpgenc_ctx* c) {
     ExactConsts e;
     fill_exact(c, c->qy, c->qc, 255. / c->maxval, &e);
     const uint32_t cap = static_cast<uint32_t>(c->refine_cap);
-    with_format(c->mixed.format, [&](auto fmt) {
-        with_refine_grid(c, c->mixed.blocks, [&](auto k64, unsigned grid) {
-            refine_mixed_kernel<decltype(k64)::value, decltype(fmt)::value><<<grid, kRefineThreads, 0, c->stream>>>(
-                c->d_geom, c->nframes, c->d_coef, c->d_refine_list, c->d_counters, cap, e, p.extra);
-        });
-    });
+    if (!with_format(c->mixed.format, [&](auto fmt) {
+            with_refine_grid(c, c->mixed.blocks, [&](auto k64, unsigned grid) {
+                refine_mixed_kernel<decltype(k64)::value, decltype(fmt)::value><<<grid, kRefineThreads, 0, c->stream>>>(
+                    c->d_geom, c->nframes, c->d_coef, c->d_refine_list, c->d_counters, cap, e, p.extra);
+            });
+        }))
+        return unknown_format(c);
     JPGENC_CUDA(c, cudaGetLastError());
     c->launches += 2;
     return JPGENC_OK;

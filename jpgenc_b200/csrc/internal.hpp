@@ -23,8 +23,8 @@ int ensure(jpgenc_ctx* c, T** ptr, size_t* cap, size_t need_bytes, bool headroom
 }
 
 int set_geometry(jpgenc_ctx* c, uint32_t w, uint32_t h, uint32_t maxval);
-// A caller's image: a known format, its planes (NV12: v must be NULL), sides 1..65535 and pitches that hold a row (0 -> the row
-// size, filled in; planar RGB: pitch2 = pitch); JPGENC_ERR_ARG otherwise
+// A caller's image: a known format, its planes (NV12 / NV16: v must be NULL; YUYV / UYVY: u and v NULL, pitch2 0), sides 1..65535
+// and pitches that hold a row (0 -> the row size, filled in; planar RGB: pitch2 = pitch); JPGENC_ERR_ARG otherwise
 int check_source(jpgenc_ctx* c, PixelSource* s, uint32_t w, uint32_t h);
 // every colour sample of a host source is <= maxval (maxval 0 or 255: true): a 4th byte and the bytes between rows are not read;
 // planar RGB: all three planes; YUV frames have no maxval
@@ -32,11 +32,13 @@ bool source_within_maxval(const PixelSource& s, uint32_t w, uint32_t h, uint32_t
 // the sources of the C entry points (a format code they do not take becomes -1, which check_source refuses)
 PixelSource image_source(const void* px, uint32_t pitch, int format);
 PixelSource planar_source(const void* r, const void* g, const void* b, uint32_t pitch);
-PixelSource yuv420_source(const void* y, const void* u, const void* v, uint32_t y_pitch, uint32_t c_pitch, int layout);
+PixelSource yuv_source(const void* y, const void* u, const void* v, uint32_t y_pitch, uint32_t c_pitch, int layout);
+// the layouts the jpgenc_*_yuv420 calls take
+inline bool is_yuv420_layout(int layout) { return layout == JPGENC_YUV_I420 || layout == JPGENC_YUV_NV12; }
 
 // One plane of a checked host source as it is uploaded: `rows` host rows of `row` bytes, `pitch` bytes apart (vsub 1: the chroma
-// planes of YUV, half the image's rows rounded up), staged as tight rows at `dev_off` of the device copy; YUV planes start on
-// 256 bytes
+// planes of YUV 4:2:0, half the image's rows rounded up), staged as tight rows at `dev_off` of the device copy; YUV planes start
+// on 256 bytes
 struct StagedPlane {
     const uint8_t* host;
     size_t pitch, row, rows, dev_off;

@@ -663,18 +663,28 @@ int jpgenc_encode_images_packed_planar(jpgenc_ctx* c, uint32_t n, const void* co
     return encode_packed(c, src, images_on_device, widths, heights, maxval, out, cap, offsets, sizes, total_bytes);
 } JPGENC_CATCH(c)
 
+int jpgenc_encode_images_packed_yuv(jpgenc_ctx* c, uint32_t n, const void* const* planes, int images_on_device, const uint32_t* widths,
+                                    const uint32_t* heights, const uint32_t* y_pitches, const uint32_t* c_pitches, int layout, uint8_t* out,
+                                    uint64_t cap, uint64_t* offsets, uint64_t* sizes, uint64_t* total_bytes) try {
+    if (!c) return JPGENC_ERR_ARG;
+    if (total_bytes) *total_bytes = 0;
+    if (yuv_source(nullptr, nullptr, nullptr, 0, 0, layout).format < 0) return fail(c, JPGENC_ERR_ARG, "unknown YUV layout");
+    if (n == 0) return JPGENC_OK;                                // an empty batch is legal and touches nothing
+    if (!planes || !widths || !heights || !offsets || !sizes) return fail(c, JPGENC_ERR_ARG, "null argument");
+    std::vector<PixelSource> src(n);
+    for (uint32_t i = 0; i < n; ++i)
+        src[i] = yuv_source(planes[3 * i], planes[3 * i + 1], planes[3 * i + 2], y_pitches ? y_pitches[i] : 0, c_pitches ? c_pitches[i] : 0, layout);
+    return encode_packed(c, src, images_on_device, widths, heights, 255, out, cap, offsets, sizes, total_bytes);
+} JPGENC_CATCH(c)
+
 int jpgenc_encode_images_packed_yuv420(jpgenc_ctx* c, uint32_t n, const void* const* planes, int images_on_device, const uint32_t* widths,
                                        const uint32_t* heights, const uint32_t* y_pitches, const uint32_t* c_pitches, int layout, uint8_t* out,
                                        uint64_t cap, uint64_t* offsets, uint64_t* sizes, uint64_t* total_bytes) try {
     if (!c) return JPGENC_ERR_ARG;
     if (total_bytes) *total_bytes = 0;
-    if (layout != JPGENC_YUV_I420 && layout != JPGENC_YUV_NV12) return fail(c, JPGENC_ERR_ARG, "unknown YUV layout");
-    if (n == 0) return JPGENC_OK;                                // an empty batch is legal and touches nothing
-    if (!planes || !widths || !heights || !offsets || !sizes) return fail(c, JPGENC_ERR_ARG, "null argument");
-    std::vector<PixelSource> src(n);
-    for (uint32_t i = 0; i < n; ++i)
-        src[i] = yuv420_source(planes[3 * i], planes[3 * i + 1], planes[3 * i + 2], y_pitches ? y_pitches[i] : 0, c_pitches ? c_pitches[i] : 0, layout);
-    return encode_packed(c, src, images_on_device, widths, heights, 255, out, cap, offsets, sizes, total_bytes);
+    if (!is_yuv420_layout(layout)) return fail(c, JPGENC_ERR_ARG, "unknown YUV 4:2:0 layout");
+    return jpgenc_encode_images_packed_yuv(c, n, planes, images_on_device, widths, heights, y_pitches, c_pitches, layout, out, cap, offsets,
+                                          sizes, total_bytes);
 } JPGENC_CATCH(c)
 
 }  // extern "C"
